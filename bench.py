@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — objective+gradient evaluations/sec of the traceobjgrad hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cnot2] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cnot2] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one batched obj+grad evaluation (`jq_traceobjgrad_batch`) of B synthetic pcof candidates per GPU on the
 named BASELINE configuration (default: cnot2, "batched random pcof evaluations").  Ranks shard the candidates
@@ -18,6 +18,9 @@ named BASELINE configuration (default: cnot2, "batched random pcof evaluations")
             weak (16384 samples per GPU) and strong (16384 samples in total; the 1001-point sweep) scaling, and a parity
             self-check of the sharded + all-reduced result against one rank evaluating every sample (<= 1e-12)
   --impl reference   the same oracle with every host thread, as the reference arm
+  --dump-outputs DIR   after the timed steps, the arrays the last timed step returned (infid, leak, trace_infid, grad, and
+            infidgrad / leakgrad when objFuncType != 1) as DIR/<name>.npy in float64, so that two builds can be compared output for
+            output on the same seeded inputs; above DUMP_BYTES a fixed, seeded sample of the candidates is written
 """
 from __future__ import annotations
 
@@ -39,6 +42,27 @@ WORKLOADS = ["rabi", "cnot1", "cnot2", "cnot3", "risk_neutral"]
 DEFAULT_BATCH = {"rabi": 262144, "cnot1": 37888, "cnot2": 16384, "cnot3": 2368, "risk_neutral": 3946}
 KERNEL_NAMES = {1: "jq_generic_kernel", 2: "jq_traj_kernel<SlotLane>", 3: "jq_traj_kernel<FiberLane>", 4: "jq_traj_kernel<TileLane>", 5: "jq_traj_kernel<latency layout, pipelined roles>", 6: "jq_dense_kernel (FP64 MMA)",
                 7: "time-parallel: jq_traj_kernel<segment sweeps> + jq_seg_chain joins"}
+DUMP_BYTES = 64_000_000          # --dump-outputs: bytes written per run, .npy headers included
+
+
+def dump_outputs(out, directory, suffix="", budget=DUMP_BYTES):
+    """Write the CUDA tensors of one evaluate_device() result as <directory>/<name><suffix>.npy (float64).  When they exceed `budget`
+    bytes, only a sample of the candidates (first axis) is written: the same rows, in ascending order, for every run with the same
+    arguments.  Returns what was written, for the JSON line."""
+    arrs = {k: v.cpu().numpy() for k, v in out.items()}
+    nbatch = next(iter(arrs.values())).shape[0]
+    total = sum(a.nbytes for a in arrs.values())
+    room = budget - 256 * len(arrs)                    # an .npy header takes 128 bytes here; leave twice that
+    rows = None
+    if total > room:
+        rows = np.sort(np.random.default_rng(0).choice(nbatch, nbatch * room // total, replace=False))
+        arrs = {k: a[rows] for k, a in arrs.items()}
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(directory, f"{k}{suffix}.npy"), a)
+    return {"dir": directory, "arrays": {k + suffix: list(a.shape) for k, a in arrs.items()},
+            "candidates_written": nbatch if rows is None else len(rows), "candidates": nbatch,
+            "sample": None if rows is None else "rows np.sort(np.random.default_rng(0).choice(candidates, candidates_written, replace=False))"}
 
 
 def alg_flops_per_eval(p, npar, dense=False):
@@ -128,7 +152,7 @@ def ncu_summary(workload):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cnot2", choices=WORKLOADS)
@@ -137,10 +161,16 @@ def main():
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--cpu-budget", type=float, default=12.0, help="seconds of CPU work for the cpu_baseline sample")
     ap.add_argument("--per-config-cpu-budget", type=float, default=2.5, help="seconds of CPU work per extra.per_config baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the last timed step returned as DIR/<name>.npy (float64; a seeded sample of the candidates "
+                         "above 64 MB); with several ranks each rank writes <name>_rank<r>.npy")
     args = ap.parse_args()
     if args.impl != "reference" and args.warmup < 3:
         args.warmup = 3          # timing rules: at least 3 warm-up steps; the JSON line reports the value actually used
-    args.steps = max(1, args.steps)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; the reference arm has no timed GPU step")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -236,6 +266,9 @@ def main():
         e1.record(stream)
         kernel_ms.append(wa.last_kernel_ms)      # library's own events around the trajectory kernel (synchronises)
     barrier()
+    dumped = None
+    if args.dump_outputs:
+        dumped = dump_outputs(out, args.dump_outputs, f"_rank{rank}" if world > 1 else "", DUMP_BYTES // world)
     launches += 2 * args.steps
     total_ms = max_over_ranks(sum(e0.elapsed_time(e1) for e0, e1 in evs))
     evals_per_step = world * B * nsamp
@@ -514,6 +547,8 @@ def main():
                 "roofline": roofline, "clocks": clocks, "extra": extra}
         if cpu is not None:
             line["cpu_baseline"] = cpu
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         print(json.dumps(line))
     wa.close()
     if world > 1:
