@@ -147,6 +147,27 @@ int64_t jq_abi_info(int32_t what);
 int jq_eval_forward(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
                     const double *h0_diag_shift, int32_t save_every, double *hist_r, double *hist_i, double *infid, double *leak);
 
+/* Forward sensitivities (the reference's traceobjgrad(verbose=true, evaladjoint=true) check, src/evalobjgrad.jl:724-745,768-784, for
+ * ndir directions at once).  Trajectory (b, s, k) evaluates candidate b with sample shift s and differentiates along
+ * dirs[(b*ndir + k)*npar ..].  One launch of the forward-sensitivity kernel (jq_query(h, 0) = 8) runs the forward sweep and its tangent
+ * (step_fwdGrad!, src/StormerVerlet.jl:151-251; fgradforce!, src/evalobjgrad.jl:2467-2563) side by side for every trajectory, so
+ * dirs = the unit vectors give the whole forward-mode gradient in one call, and dstate the sensitivity of the final state.
+ * pcof, dirs, h0_diag_shift and weights as in jq_traceobjgrad_batch; with pFidType 3 every pcof and direction vector carries the
+ * global phase as its last entry.
+ * weights == NULL: infid[t], leak[t] with t = b*nsamples + s (the objective-only outputs of the generic kernel, bit for bit);
+ *   dinfid[t*ndir + k], dleak[t*ndir + k], their directional derivatives; dstate_r / dstate_i [(t*ndir + k)][n*m] the tangents of
+ *   Re and Im of the final state (vr' and -vi', the convention of jq_eval_forward), column-major n x m blocks.
+ * weights != NULL ([nsamples]): infid[b], leak[b], dinfid[b*ndir + k], dleak[b*ndir + k], the weighted sums over s that
+ *   eval_f_g_grad! forms (fixed summation order); dstate must then be NULL.
+ * Any output may be NULL.  JQ_ERR_ARG (no launch) for ndir < 1, dirs == NULL, nbatch*nsamples*ndir > 2^31 - 1, the Jacobi solver,
+ * weights with a dstate output, weights while a communicator of more than one rank is attached (this entry never communicates:
+ * shard directions, not samples), or a problem whose trajectory does not fit in 227 KB of shared memory.
+ * Host pointers, blocking. */
+int jq_forward_sensitivity(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                           const double *h0_diag_shift, const double *weights, int32_t ndir, const double *dirs,
+                           double *infid, double *leak, double *dinfid, double *dleak,
+                           double *dstate_r, double *dstate_i);
+
 /* evalctrl(params, pcof, td, func) (src/plotstatectrl.jl:246-276): the control functions p_q(t), q_q(t) (rad/ns) of EVERY
  * coupled control q on the time grid `times`, evaluated by the device function the time loop uses (bcarrier2,
  * src/bsplines.jl:211-304).  p, q: [ncoupled][ntimes] doubles, host pointers, blocking. */
@@ -192,8 +213,9 @@ int jq_set_time_segments(jq_handle *h, int32_t nseg);
  * (src/evalobjgrad.jl:745) has at the segment's first step, t_last[p] the value its backward recurrence t = t - dt from T (:810, :919)
  * has at the segment's last step -- bit-identical to what a single sweep sees, not k dt.  Returns the steps of the longest segment. */
 int64_t jq_time_segments(double T, int64_t nsteps, int32_t nseg, double *t_first, double *t_last);
-/* what: 0 = kernel actually used by the last evaluation (1 ... 7), 1 = CUDA-event time of the last evaluation's
- * trajectory kernel(s) in ms (synchronises), 2 = number of kernels launched by the last evaluation,
+/* what: 0 = kernel actually used by the last evaluation (1 ... 7, or 8 = the forward-sensitivity kernel of jq_forward_sensitivity),
+ * 1 = CUDA-event time of the last evaluation's trajectory kernel(s) in ms (synchronises), 2 = number of kernels launched by the last
+ * evaluation,
  * 3 = trajectories resident per CTA, 4 = CTAs launched, 5 = registers per thread, 6 = dynamic smem bytes per CTA,
  * 7 = time segments of the last evaluation (kernel 7; else 0). */
 int jq_query(jq_handle *h, int32_t what, double *value);

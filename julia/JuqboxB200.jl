@@ -189,6 +189,29 @@ function eval_forward(pcof0::Array{Float64,1}, params::objparams, wa::Working_Ar
     return hr .+ im .* hi
 end
 
+# Forward sensitivities (the forward-sensitivity check of traceobjgrad(pcof, params, wa, true, true), src/evalobjgrad.jl:724-745,768-784,
+# for ndir directions in one launch): dirs is Npar x ndir, one direction per column (dirs = I: the whole forward-mode gradient;
+# dirs = e_kpar: the reference's component kpar).  Without weights: infid, leak [nsamples] and dinfid, dleak ndir x nsamples;
+# with weights: the weighted sums over the nodes, infid, leak [1] and dinfid, dleak [ndir].  The column-major arrays are the ABI's
+# row-major views, nothing is transposed.
+function forward_sensitivity(pcof::Vector{Float64}, params::objparams, wa::Working_Arrays_B200, dirs::Array{Float64,2};
+                             nodes::AbstractArray = [0.0], weights::Union{Nothing,AbstractArray} = nothing)
+    Npar, ndir = size(dirs)
+    Npar == length(pcof) || error("forward_sensitivity: dirs must be Npar x ndir with Npar = length(pcof)")
+    shifts = jq_shifts(params, nodes)
+    nsamples = length(nodes)
+    w = weights === nothing ? nothing : Vector{Float64}(weights)
+    nout = w === nothing ? nsamples : 1
+    infid = zeros(nout); leak = zeros(nout)
+    dinfid = zeros(ndir, nout); dleak = zeros(ndir, nout)
+    jq_check(ccall((:jq_forward_sensitivity, libjq), Cint,
+                   (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Ptr{Float64}, Int32, Ptr{Float64},
+                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                   wa.handle, 1, pcof, Npar, nsamples, shifts, w === nothing ? C_NULL : w, ndir, dirs,
+                   infid, leak, dinfid, dleak, C_NULL, C_NULL))
+    return w === nothing ? (infid, leak, dinfid, dleak) : (infid, leak, vec(dinfid), vec(dleak))
+end
+
 
 # ---- the four Ipopt callbacks as ONE ccall each (src/ipopt_interface.jl:77-179): jq_eval_f_grad keeps the last-pcof cache, runs
 # eval_f_g_grad!'s sample loop as one launch and adds the Tikhonov terms on the device.  params.last_* scalars are kept for

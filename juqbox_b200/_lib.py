@@ -32,7 +32,7 @@ JQ_DENSE, JQ_CSC = 0, 1
 JQ_ERR_PCOF_LENGTH = -2
 
 EXPORTS = ["jq_create", "jq_destroy", "jq_update_target", "jq_traceobjgrad_batch", "jq_traceobjgrad_batch_device", "jq_eval_f_grad",
-           "jq_cache_invalidate", "jq_eval_forward", "jq_eval_controls",
+           "jq_cache_invalidate", "jq_eval_forward", "jq_eval_controls", "jq_forward_sensitivity",
            "jq_set_kernel", "jq_set_time_segments", "jq_time_segments", "jq_query", "jq_fp64_peak", "jq_fp64_peak_3op", "jq_fp64_peak_dmma", "jq_comm_unique_id", "jq_comm_init", "jq_comm_destroy", "jq_comm_set_cooperative",
            "jq_abi_info", "jq_last_error", "jq_version"]
 ABI_VERSION = 2
@@ -71,6 +71,7 @@ def load(build_if_missing: bool = True):
     lib.jq_traceobjgrad_batch_device.argtypes = [vp, i32, dp, i32, i32, dp, dp, i32, dp, dp, dp, dp, dp, dp, vp]
     lib.jq_eval_forward.argtypes = [vp, i32, dp, i32, i32, dp, i32, dp, dp, dp, dp]
     lib.jq_eval_controls.argtypes = [vp, dp, i32, i32, dp, dp, dp]
+    lib.jq_forward_sensitivity.argtypes = [vp, i32, dp, i32, i32, dp, dp, i32, dp, dp, dp, dp, dp, dp, dp]
     lib.jq_set_kernel.argtypes = [vp, i32]
     lib.jq_set_time_segments.argtypes = [vp, i32]
     lib.jq_comm_set_cooperative.argtypes = [vp, i32]

@@ -272,6 +272,54 @@ class Working_Arrays:
                                              infid.ctypes.data_as(C.c_void_p), leak.ctypes.data_as(C.c_void_p)))
         return hr + 1j * hi, infid, leak
 
+    def forward_sensitivity(self, pcof, dirs, shifts=None, weights=None, final_state: bool = False):
+        """Forward sensitivities (jq_forward_sensitivity): the forward sweep and its tangent along every direction in one launch.
+
+        pcof [nbatch, npar], dirs [nbatch, ndir, npar] (direction k of candidate b is dirs[b, k]; with pFidType 3 the last entry is the
+        global phase's component).  Returns a dict: infid, leak [nbatch, nsamples] and dinfid, dleak, dobjf [nbatch, nsamples, ndir]
+        (the directional derivatives; dobjf = dinfid + dleak, the derivative of the total objective); with weights the sample axis is
+        summed away as in evaluate().  final_state=True adds dstate, the tangent of the final state, complex
+        [nbatch, nsamples, ndir, Ntot, N]."""
+        p = self.params
+        self._check_params()
+        pcof = _f64(np.atleast_2d(pcof))
+        if pcof.ndim != 2:
+            raise ValueError("pcof must be [nbatch, npar]")
+        nbatch, npar = pcof.shape
+        dirs = np.asarray(dirs)
+        if dirs.ndim != 3 or dirs.shape[0] != nbatch or dirs.shape[2] != npar or dirs.shape[1] < 1:
+            raise ValueError(f"dirs must be [nbatch, ndir, npar] = [{nbatch}, ndir >= 1, {npar}], not {list(dirs.shape)}")
+        dirs = _f64(dirs)
+        ndir = dirs.shape[1]
+        nsamples, sp, wp = 1, None, None
+        if shifts is not None:
+            shifts = _f64(np.atleast_2d(shifts))
+            if shifts.ndim != 2 or shifts.shape[1] != p.Ntot:
+                raise ValueError("shifts must be [nsamples, Ntot]")
+            nsamples, sp = shifts.shape[0], shifts.ctypes.data_as(C.c_void_p)
+        if weights is not None:
+            weights = _f64(np.atleast_1d(weights))
+            if weights.shape != (nsamples,):
+                raise ValueError("weights must have one entry per sample")
+            if final_state:
+                raise ValueError("final_state=True needs per-sample outputs (weights=None): a weighted sum of states is not defined")
+            wp = weights.ctypes.data_as(C.c_void_p)
+        shape = (nbatch,) if weights is not None else (nbatch, nsamples)
+        out = {"infid": np.zeros(shape), "leak": np.zeros(shape), "dinfid": np.zeros(shape + (ndir,)), "dleak": np.zeros(shape + (ndir,))}
+        sr = si = None
+        if final_state:
+            sr = np.zeros((nbatch, nsamples, ndir, p.N, p.Ntot))      # the C layout: column-major Ntot x N blocks
+            si = np.zeros_like(sr)
+        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        _lib.check(self._lib.jq_forward_sensitivity(
+            self._handle, nbatch, ptr(pcof), npar, nsamples, sp, wp, ndir, ptr(dirs), ptr(out["infid"]), ptr(out["leak"]),
+            ptr(out["dinfid"]), ptr(out["dleak"]), ptr(sr), ptr(si)))
+        out["objf"] = out["infid"] + out["leak"]
+        out["dobjf"] = out["dinfid"] + out["dleak"]
+        if final_state:
+            out["dstate"] = (sr + 1j * si).swapaxes(-1, -2)
+        return out
+
     def eval_f_grad(self, pcof, shifts=None, weights=None, tik0: float = 0.0, prior=None):
         """The fused Ipopt-callback entry (jq_eval_f_grad): objective with Tikhonov, its gradient, infidelity, leak and leak
         gradient of ONE pcof in one call, with the last-pcof cache inside the handle.  Returns a dict; `evaluated` is False
@@ -372,6 +420,25 @@ def traceobjgrad(pcof0, params: objparams, wa: Working_Arrays, verbose: bool = F
     else:
         infidelgrad, leakgrad = totalgrad, np.zeros(0)
     return objfv, totalgrad, primary, secondary, r["trace_infid"][0, 0], infidelgrad, leakgrad
+
+
+def forward_sensitivity(pcof0, params: objparams, wa: Working_Arrays, dirs, nodes=None, weights=None):
+    """Forward sensitivities of one pcof along the rows of `dirs` ([ndir, npar], or one direction [npar]) in one launch: the
+    reference's forward-sensitivity check (traceobjgrad with verbose=true, evaladjoint=true, src/evalobjgrad.jl:724-745,768-784)
+    for many directions at once.  dirs = e_kpar is the reference's component kpar; dirs = I gives the whole forward-mode gradient.
+    nodes: epsilons of the risk-neutral noise model (samples); weights: their quadrature weights (sums over the samples).
+    Returns the dict of Working_Arrays.forward_sensitivity without the candidate axis."""
+    pcof0 = np.asarray(pcof0, dtype=np.float64)
+    if pcof0.ndim != 1:
+        raise ValueError("pcof0 must be one parameter vector")
+    dirs = np.asarray(dirs, dtype=np.float64)
+    if dirs.ndim == 1:
+        dirs = dirs[None, :]
+    if dirs.ndim != 2 or dirs.shape[1] != len(pcof0):
+        raise ValueError(f"dirs must be [ndir, {len(pcof0)}] (one direction per row)")
+    shifts = None if nodes is None else noise_shift(params.Ntot, nodes)
+    r = wa.forward_sensitivity(pcof0[None, :], dirs[None], shifts, weights)
+    return {k: v[0] for k, v in r.items()}
 
 
 def eval_forward(pcof0, params: objparams, wa: Working_Arrays, saveEndOnly: bool = True, saveEvery: int = 1):

@@ -937,3 +937,78 @@ extern "C" int jq_traceobjgrad_batch(jq_handle *h, int32_t nbatch, const double 
     CU(cudaStreamSynchronize(st));
     return 0;
 }
+
+extern "C" int jq_forward_sensitivity(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                                      const double *shift, const double *weights, int32_t ndir, const double *dirs, double *infid,
+                                      double *leak, double *dinfid, double *dleak, double *dstate_r, double *dstate_i) {
+    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
+    if (rc) return rc;
+    if (ndir < 1 || !dirs) return fail(JQ_ERR_ARG, "jq_forward_sensitivity: need ndir >= 1 and a dirs array");
+    if ((long long)nbatch * nsamples * ndir > 0x7fffffffLL)
+        return fail(JQ_ERR_ARG, "jq_forward_sensitivity: nbatch * nsamples * ndir exceeds 2^31 - 1 trajectories per call");
+    if (h->P.solver == 2) return fail(JQ_ERR_ARG, "jq_forward_sensitivity: the Jacobi solver has no tangent sweep (use the Neumann solver)");
+    if (weights && (dstate_r || dstate_i))
+        return fail(JQ_ERR_ARG, "jq_forward_sensitivity: a weighted sum of final-state tangents is not defined (pass weights or dstate, not both)");
+    if (weights && h->comm && h->comm_size > 1)
+        return fail(JQ_ERR_ARG, "jq_forward_sensitivity: never communicates; with a communicator attached shard the directions, not the samples (no weights)");
+    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
+    if (jq_fwdsens_smem_bytes(h->P, nspl) > 227 * 1024)
+        return fail(JQ_ERR_ARG, "jq_forward_sensitivity: problem too large for the tangent kernel's shared memory (n*m = %d)", h->n * h->m);
+    CU(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    if (h->have_last && h->last_stream != st) CU(cudaStreamWaitEvent(st, h->ev_done, 0));      // shared scratch, see jq_traceobjgrad_batch_device
+    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ndir, len = (size_t)h->n * h->m;
+    const size_t nout = weights ? (size_t)nbatch : nt, ndout = nout * ndir;
+    const size_t n_pcof = (size_t)nbatch * npar, n_dirs = (size_t)nbatch * ndir * npar;
+    const size_t n_shift = shift ? (size_t)nsamples * h->n : 0, n_w = weights ? (size_t)nsamples : 0;
+    const bool want_state = dstate_r || dstate_i;
+    const size_t n_state = want_state ? ntraj * len : 0;
+    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_dirs + n_shift + n_w)) != 0) return rc;
+    if ((rc = grow(&h->d_out, &h->cap_out, 2 * nout + 2 * ndout + 2 * n_state)) != 0) return rc;
+    if ((rc = grow(&h->d_scal, &h->cap_traj, nt * 4)) != 0) return rc;
+    if ((rc = grow(&h->d_grad, &h->cap_grad, ntraj)) != 0) return rc;
+    if ((rc = grow(&h->d_igrad, &h->cap_igrad, ntraj)) != 0) return rc;
+    double *d_pcof = h->d_in, *d_dirs = d_pcof + n_pcof, *d_shift = shift ? d_dirs + n_dirs : nullptr;
+    double *d_w = weights ? d_dirs + n_dirs + n_shift : nullptr;
+    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_dirs, dirs, n_dirs * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (n_w) CU(cudaMemcpyAsync(d_w, weights, n_w * sizeof(double), cudaMemcpyHostToDevice, st));
+    double *o_infid = h->d_out, *o_leak = o_infid + nout, *o_dinf = o_leak + nout, *o_dleak = o_dinf + ndout;
+    double *o_sr = want_state ? o_dleak + ndout : nullptr, *o_si = want_state ? o_sr + n_state : nullptr;
+
+    SensArgs S{};
+    S.ntraj = (int)ntraj; S.nsamples = nsamples; S.ndir = ndir; S.Npar = nspl; S.D1 = nspl / (2 * h->Nc * h->Nfreq); S.pstride = npar;
+    S.pcof = d_pcof; S.dirs = d_dirs; S.shift = d_shift;
+    S.scal = h->d_scal; S.dinfid = h->d_grad; S.dleak = h->d_igrad; S.dstate_r = o_sr; S.dstate_i = o_si;
+    int ctas = 0, regs = 0, gpc = 1;
+    size_t smem = 0;
+    CU(cudaEventRecord(h->ev0, st));
+    CU(jq_fwdsens_launch(h->P, S, st, &ctas, &regs, &smem, &gpc));
+    CU(cudaEventRecord(h->ev1, st));
+    h->timed = true;
+    h->last_kernel = 8; h->last_ctas = ctas; h->last_regs = regs; h->last_smem = smem; h->last_tpc = gpc; h->last_traj_launches = 1;
+    // per-trajectory outputs or the weighted sums over the samples, in the fixed order of the evaluation path's reductions: the
+    // directions take the place of the gradient columns (dinfid as `grad`, dleak as `infidgrad`)
+    if (weights && nsamples >= 64)
+        jq_weighted_sum_kernel<<<dim3(nbatch, (ndir + 3 + 31) / 32), 32 * WS_LANES, 0, st>>>(nsamples, ndir, 2, 1, d_w, h->d_scal, h->d_grad,
+                                          h->d_igrad, o_infid, o_leak, nullptr, o_dinf, o_dleak, nullptr);
+    else {
+        const long long total = (long long)nout * (ndir + 1);
+        const int fb = 256, fg = (int)std::min<long long>((total + fb - 1) / fb, 148 * 8);
+        jq_finalize_kernel<<<fg, fb, 0, st>>>(nbatch, nsamples, ndir, 2, 1, d_w, h->d_scal, h->d_grad, h->d_igrad, o_infid, o_leak, nullptr,
+                                              o_dinf, o_dleak, nullptr);
+    }
+    CU(cudaGetLastError());
+    h->last_launches = 2;
+    CU(cudaEventRecord(h->ev_done, st));
+    h->last_stream = st; h->have_last = true;
+    if (infid) CU(cudaMemcpyAsync(infid, o_infid, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (leak) CU(cudaMemcpyAsync(leak, o_leak, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (dinfid) CU(cudaMemcpyAsync(dinfid, o_dinf, ndout * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (dleak) CU(cudaMemcpyAsync(dleak, o_dleak, ndout * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (dstate_r) CU(cudaMemcpyAsync(dstate_r, o_sr, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (dstate_i) CU(cudaMemcpyAsync(dstate_i, o_si, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return 0;
+}

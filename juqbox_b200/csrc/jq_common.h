@@ -87,6 +87,20 @@ cudaError_t jq_generic_launch(const DevProblem &P, const LaunchArgs &A, cudaStre
 cudaError_t jq_controls_launch(const DevProblem &P, int D1, const double *pcof, int ntimes, const double *times, double *p, double *q,
                                cudaStream_t st);
 
+// ---- forward-sensitivity kernel (jq_generic.cu): the forward sweep and its tangent along one direction per trajectory, generic layout ----
+struct SensArgs {
+    int ntraj, nsamples, ndir, Npar, D1;   // ntraj = nbatch * nsamples * ndir; Npar: spline coefficients (without the pFidType 3 phase)
+    int pstride;           // length of every pcof and direction vector: Npar, or Npar + 1 with the global phase (pFidType 3)
+    const double *pcof;    // [nbatch][pstride]
+    const double *dirs;    // [nbatch][ndir][pstride]
+    const double *shift;   // [nsamples][n] or nullptr
+    double *scal;          // [nbatch * nsamples][4]: infid, leak, trace_infid, spare (written by direction 0)
+    double *dinfid, *dleak;            // [ntraj]: traj = (b * nsamples + s) * ndir + k
+    double *dstate_r, *dstate_i;       // [ntraj][n*m] tangents of Re and Im of the final state (vr', -vi'), or nullptr
+};
+size_t jq_fwdsens_smem_bytes(const DevProblem &P, int Npar);     // one group
+cudaError_t jq_fwdsens_launch(const DevProblem &P, const SensArgs &S, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc);
+
 // ---- dense-operator kernel on the FP64 tensor-core path (jq_dense.cu): one CTA per (candidate, tile of samples) ----
 bool jq_dense_supported(const DevProblem &P, char *why, size_t len);
 void jq_dense_padding(int n, int *n8, int *ldk);      // layout of DevProblem::dense_ops: [1 + 2 Nc][n8][ldk], zero padded

@@ -19,6 +19,10 @@
 
 #define GEN_THREADS 256
 
+// Geometry of one launch (host-computed): threads per group, groups per CTA, doubles of shared memory per group, and whether
+// the operator table is staged into shared memory.
+struct GenGeom { int tpt, gpc, per_group, stage; };
+
 namespace {
 
 __device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -61,16 +65,44 @@ __device__ __forceinline__ double op_apply(const Ctx &c, int o, const double *x,
     for (int p = rp[i]; p < rp[i + 1]; ++p) s += c.vl[p] * xc[c.cl[p]];
     return s;
 }
-__device__ __forceinline__ double applyK(const Ctx &c, int level, const double *x, int i, int j) {
+// Tangents of the forward sweep along one direction d (forward-sensitivity kernel): the tangent of every state block the step
+// touches, and the control tables differentiated along d (ctrl_dot = the same table with d in place of pcof: p, q and the
+// uncoupled f are linear in pcof).
+struct Tan {
+    double *vr, *vi, *vi05, *vr0, *rhs, *scr, *k1, *k2, *l1, *l2;
+    double *ctrl;
+};
+// a tangent block when the tangent is carried, nullptr otherwise (td is only dereferenced with TAN)
+#define TD(f) (TAN ? td->f : nullptr)
+
+// K(t) x.  TAN: also *yd = (K x)' = K xd + sum_q p_q' Hsym_q x, one product of Hsym_q x feeding both sums.
+template <bool TAN = false>
+__device__ __forceinline__ double applyK(const Ctx &c, int level, const double *x, int i, int j, const Tan *td = nullptr,
+                                         const double *xd = nullptr, double *yd = nullptr) {
     double s = op_apply(c, 0, x, i, j) + c.shift[i] * x[i + j * c.n];
     const double *ct = c.ctrl + level * 2 * c.Nc;
-    for (int q = 0; q < c.Nc; ++q) s += ct[2 * q] * op_apply(c, 1 + q, x, i, j);
+    double sd = 0.0;
+    if constexpr (TAN) sd = op_apply(c, 0, xd, i, j) + c.shift[i] * xd[i + j * c.n];
+    for (int q = 0; q < c.Nc; ++q) {
+        const double hx = op_apply(c, 1 + q, x, i, j);
+        s += ct[2 * q] * hx;
+        if constexpr (TAN) sd += ct[2 * q] * op_apply(c, 1 + q, xd, i, j) + td->ctrl[level * 2 * c.Nc + 2 * q] * hx;
+    }
+    if constexpr (TAN) *yd = sd;
     return s;
 }
-__device__ __forceinline__ double applyS(const Ctx &c, int level, const double *x, int i, int j) {
+// S(t) x.  TAN: also *yd = (S x)' = S xd + sum_q q_q' Hanti_q x.
+template <bool TAN = false>
+__device__ __forceinline__ double applyS(const Ctx &c, int level, const double *x, int i, int j, const Tan *td = nullptr,
+                                         const double *xd = nullptr, double *yd = nullptr) {
     const double *ct = c.ctrl + level * 2 * c.Nc;
-    double s = 0.0;
-    for (int q = 0; q < c.Nc; ++q) s += ct[2 * q + 1] * op_apply(c, 1 + c.Nc + q, x, i, j);
+    double s = 0.0, sd = 0.0;
+    for (int q = 0; q < c.Nc; ++q) {
+        const double hx = op_apply(c, 1 + c.Nc + q, x, i, j);
+        s += ct[2 * q + 1] * hx;
+        if constexpr (TAN) sd += ct[2 * q + 1] * op_apply(c, 1 + c.Nc + q, xd, i, j) + td->ctrl[level * 2 * c.Nc + 2 * q + 1] * hx;
+    }
+    if constexpr (TAN) *yd = sd;
     return s;
 }
 
@@ -129,14 +161,22 @@ __device__ void eval_controls(const Ctx &c, double t, double dt) {
                    e += c.tpt, i += di_, j += dj_ + (i >= c.n ? 1 : 0), i -= (i >= c.n ? c.n : 0))
 
 // X = sum_{j<=J} (h/2)^j S^j B ; B destroyed, T scratch (src/linear_solvers.jl:94-106)
-__device__ void neumann(const Ctx &c, int level, double h, double *B, double *T, double *X) {
-    FOR_E X[e] = B[e];
+// TAN: the tangent alongside, Td_j = S Td_{j-1} + S' T_{j-1}, Xd += (h/2)^j Td_j; Bd destroyed, Td scratch.
+template <bool TAN = false>
+__device__ void neumann(const Ctx &c, int level, double h, double *B, double *T, double *X, const Tan *td = nullptr,
+                        double *Bd = nullptr, double *Td = nullptr, double *Xd = nullptr) {
+    FOR_E { X[e] = B[e]; if constexpr (TAN) Xd[e] = Bd[e]; }
     double coeff = 1.0;
     for (int it = 0; it < c.J; ++it) {
         coeff *= 0.5 * h;
-        FOR_E { double tv = applyS(c, level, B, i, j); T[e] = tv; X[e] += coeff * tv; }
+        FOR_E {
+            double yd;
+            double tv = applyS<TAN>(c, level, B, i, j, td, Bd, &yd); T[e] = tv; X[e] += coeff * tv;
+            if constexpr (TAN) { Td[e] = yd; Xd[e] += coeff * yd; }
+        }
         gsync(c);
         double *sw = B; B = T; T = sw;
+        if constexpr (TAN) { sw = Bd; Bd = Td; Td = sw; }
     }
 }
 
@@ -157,29 +197,105 @@ __device__ void jacobi(const Ctx &c, int level, double h, const double *B, doubl
     }
 }
 
-__device__ __forceinline__ void solve(const Ctx &c, int level, double h, double *B, double *T, double *X) {
-    if (c.P->solver == 2) jacobi(c, level, h, B, T, X);
+// TAN: Neumann only (the Jacobi solver has no tangent; the host rejects it for the forward-sensitivity kernel)
+template <bool TAN = false>
+__device__ __forceinline__ void solve(const Ctx &c, int level, double h, double *B, double *T, double *X, const Tan *td = nullptr,
+                                      double *Bd = nullptr, double *Td = nullptr, double *Xd = nullptr) {
+    if constexpr (TAN) neumann<true>(c, level, h, B, T, X, td, Bd, Td, Xd);
+    else if (c.P->solver == 2) jacobi(c, level, h, B, T, X);
     else neumann(c, level, h, B, T, X);
 }
 
-// src/StormerVerlet.jl:461-504
-__device__ void state_step(const Ctx &c, double h) {
+// src/StormerVerlet.jl:461-504.  TAN: every statement differentiated along d as well (step_fwdGrad!, src/StormerVerlet.jl:151-251).
+template <bool TAN = false>
+__device__ void state_step(const Ctx &c, double h, const Tan *td = nullptr) {
     double *u = c.vr, *v = c.vi, *v05 = c.vi05;
-    FOR_E c.rhs[e] = applyK(c, 1, u, i, j) + applyS(c, 1, v, i, j);
+    FOR_E {
+        double kd, sd;
+        c.rhs[e] = applyK<TAN>(c, 1, u, i, j, td, TD(vr), &kd) + applyS<TAN>(c, 1, v, i, j, td, TD(vi), &sd);
+        if constexpr (TAN) td->rhs[e] = kd + sd;
+    }
     gsync(c);
-    solve(c, 1, h, c.rhs, c.scr, c.l1);
-    FOR_E v05[e] = v[e] + 0.5 * h * c.l1[e];
+    solve<TAN>(c, 1, h, c.rhs, c.scr, c.l1, td, TD(rhs), TD(scr), TD(l1));
+    FOR_E { v05[e] = v[e] + 0.5 * h * c.l1[e]; if constexpr (TAN) td->vi05[e] = td->vi[e] + 0.5 * h * td->l1[e]; }
     gsync(c);
-    FOR_E c.k1[e] = applyS(c, 0, u, i, j) - applyK(c, 0, v05, i, j);
+    FOR_E {
+        double sd, kd;
+        c.k1[e] = applyS<TAN>(c, 0, u, i, j, td, TD(vr), &sd) - applyK<TAN>(c, 0, v05, i, j, td, TD(vi05), &kd);
+        if constexpr (TAN) td->k1[e] = sd - kd;
+    }
     gsync(c);
-    FOR_E c.rhs[e] = applyS(c, 2, u, i, j) + 0.5 * h * applyS(c, 2, c.k1, i, j) - applyK(c, 2, v05, i, j);
+    FOR_E {
+        double ad, bd, kd;
+        c.rhs[e] = applyS<TAN>(c, 2, u, i, j, td, TD(vr), &ad) + 0.5 * h * applyS<TAN>(c, 2, c.k1, i, j, td, TD(k1), &bd) -
+                   applyK<TAN>(c, 2, v05, i, j, td, TD(vi05), &kd);
+        if constexpr (TAN) td->rhs[e] = ad + 0.5 * h * bd - kd;
+    }
     gsync(c);
-    FOR_E u[e] += 0.5 * h * c.k1[e];
-    solve(c, 2, h, c.rhs, c.scr, c.k2);
-    FOR_E u[e] += 0.5 * h * c.k2[e];
+    FOR_E { u[e] += 0.5 * h * c.k1[e]; if constexpr (TAN) td->vr[e] += 0.5 * h * td->k1[e]; }
+    solve<TAN>(c, 2, h, c.rhs, c.scr, c.k2, td, TD(rhs), TD(scr), TD(k2));
+    FOR_E { u[e] += 0.5 * h * c.k2[e]; if constexpr (TAN) td->vr[e] += 0.5 * h * td->k2[e]; }
     gsync(c);
-    FOR_E { c.l2[e] = applyK(c, 1, u, i, j) + applyS(c, 1, v05, i, j); v[e] += 0.5 * h * (c.l1[e] + c.l2[e]); }
+    FOR_E {
+        double kd, sd;
+        c.l2[e] = applyK<TAN>(c, 1, u, i, j, td, TD(vr), &kd) + applyS<TAN>(c, 1, v05, i, j, td, TD(vi05), &sd);
+        v[e] += 0.5 * h * (c.l1[e] + c.l2[e]);
+        if constexpr (TAN) { td->l2[e] = kd + sd; td->vi[e] += 0.5 * h * (td->l1[e] + td->l2[e]); }
+    }
     gsync(c);
+}
+
+// Forbidden-state penalty of one forward step, accumulated per thread into *pen (summed over the group by the caller).
+// Before the step: penalf2aTrap(vr) (diagonal W), its dense form (src/evalobjgrad.jl:2210-2223) and the vr0 copy for penalf2imag.
+// TAN: the tangent along d into *pd: 2 sum W vr vr' (diagonal), vr'^T W vr + vr^T W vr' (dense).  The tangent runs in its own element
+// loop behind a group barrier: sharing products such as W vr with the primal loop lets the compiler contract the primal sum
+// differently, and the primal penalty must stay the generic kernel's to the bit.
+template <bool TAN = false>
+__device__ __forceinline__ void penalty_pre(const Ctx &c, double *pen, const Tan *td = nullptr, double *pd = nullptr) {
+    const DevProblem &P = *c.P;
+    if (!P.wreal) {
+        FOR_E *pen += P.wdiag[i] * c.vr[e] * c.vr[e];
+    } else {
+        FOR_E { *pen += c.vr[e] * wapply(c, P.wreal, c.vr, i, j); c.vr0[e] = c.vr[e]; }
+    }
+    if constexpr (TAN) {
+        gsync(c);
+        if (!P.wreal) {
+            FOR_E *pd += 2.0 * P.wdiag[i] * c.vr[e] * td->vr[e];
+        } else {
+            FOR_E {
+                *pd += td->vr[e] * wapply(c, P.wreal, c.vr, i, j) + c.vr[e] * wapply(c, P.wreal, td->vr, i, j);
+                td->vr0[e] = td->vr[e];
+            }
+        }
+    }
+}
+// After the step: penalf2a(vr, vi05) (diagonal W); dense penalf2a (:2183-2197) and -2 penalf2imag(vr0, vi05, wmat_imag) =
+// -2 tr(vi05' Wi vr0) (:716-718,:2226-2228).  The caller's next barrier orders the reads of vr0 before its rewrite.
+template <bool TAN = false>
+__device__ __forceinline__ void penalty_post(const Ctx &c, double *pen, const Tan *td = nullptr, double *pd = nullptr) {
+    const DevProblem &P = *c.P;
+    if (!P.wreal) {
+        FOR_E *pen += P.wdiag[i] * (c.vr[e] * c.vr[e] + 2.0 * c.vi05[e] * c.vi05[e]);
+    } else {
+        FOR_E {
+            *pen += c.vr[e] * wapply(c, P.wreal, c.vr, i, j) + 2.0 * c.vi05[e] * wapply(c, P.wreal, c.vi05, i, j);
+            if (P.wimag) *pen -= 2.0 * c.vi05[e] * wapply(c, P.wimag, c.vr0, i, j);
+        }
+    }
+    if constexpr (TAN) {
+        gsync(c);
+        if (!P.wreal) {
+            FOR_E *pd += 2.0 * P.wdiag[i] * (c.vr[e] * td->vr[e] + 2.0 * c.vi05[e] * td->vi05[e]);
+        } else {
+            FOR_E {
+                *pd += td->vr[e] * wapply(c, P.wreal, c.vr, i, j) + c.vr[e] * wapply(c, P.wreal, td->vr, i, j) +
+                       2.0 * (td->vi05[e] * wapply(c, P.wreal, c.vi05, i, j) + c.vi05[e] * wapply(c, P.wreal, td->vi05, i, j));
+                if (P.wimag)
+                    *pd -= 2.0 * (td->vi05[e] * wapply(c, P.wimag, c.vr0, i, j) + c.vi05[e] * wapply(c, P.wimag, td->vr0, i, j));
+            }
+        }
+    }
 }
 
 // src/StormerVerlet.jl:255-303 (forcing) / :365-406 (no forcing).  Forcing with diagonal W:
@@ -303,17 +419,13 @@ __device__ void trace_fid(const Ctx &c, double *re, double *im) {
     *im = v[1] / c.m;
 }
 
-// Geometry of one launch (host-computed): threads per group, groups per CTA, doubles of shared memory per group, and whether
-// the operator table is staged into shared memory.
-struct GenGeom { int tpt, gpc, per_group, stage; };
-
-__global__ void __launch_bounds__(GEN_THREADS) jq_generic_kernel(DevProblem P, LaunchArgs A, GenGeom G) {
-    extern __shared__ __align__(16) double sm[];
-    Ctx c;
+// Context of this thread's group and the operator table (staged into shared memory when G.stage); returns the start of the
+// group's own shared-memory region.  Every thread of the CTA calls it (the staging waits on a CTA-wide barrier).
+__device__ __forceinline__ double *group_setup(Ctx &c, const DevProblem &P, int Npar, int D1, const GenGeom &G, double *sm) {
     c.P = &P;
     c.n = P.n; c.m = P.m; c.len = P.n * P.m; c.Nc = P.Nc; c.Nfreq = P.Nfreq; c.J = P.J;
-    c.Npar = A.Npar; c.D1 = A.D1;
-    c.dtknot = P.T / (A.D1 - 2);
+    c.Npar = Npar; c.D1 = D1;
+    c.dtknot = P.T / (D1 - 2);
     c.tinv = 1.0 / P.T;
     c.tpt = G.tpt; c.gwarps = G.tpt / 32;
     const int grp = threadIdx.x / G.tpt;
@@ -344,7 +456,14 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_generic_kernel(DevProblem P, L
         c.vl = reinterpret_cast<const double *>(blob + P.csr_off_val);
         off = (P.csr_bytes + 16) / sizeof(double);
     }
-    double *p = sm + off + (size_t)grp * G.per_group;
+    return sm + off + (size_t)grp * G.per_group;
+}
+
+__global__ void __launch_bounds__(GEN_THREADS) jq_generic_kernel(DevProblem P, LaunchArgs A, GenGeom G) {
+    extern __shared__ __align__(16) double sm[];
+    Ctx c;
+    double *p = group_setup(c, P, A.Npar, A.D1, G, sm);
+    const int grp = threadIdx.x / G.tpt;
     double **blk[] = {&c.vr, &c.vi, &c.vi05, &c.vr0, &c.lr, &c.li, &c.lr05, &c.li0, &c.lrn, &c.lin, &c.lr05n, &c.li0n,
                       &c.rhs, &c.scr, &c.k1, &c.k2, &c.l1, &c.l2};
     for (int b = 0; b < 18; ++b) {
@@ -375,22 +494,12 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_generic_kernel(DevProblem P, L
         if (hr) FOR_E { hr[e] = c.vr[e]; hi[e] = -c.vi[e]; }
         const bool densew = P.wreal != nullptr;
         for (long long step = 0; step < P.nsteps; ++step) {
-            if (!densew) { FOR_E pen += P.wdiag[i] * c.vr[e] * c.vr[e]; }          // penalf2aTrap(vr)
-            else {
-                FOR_E { pen += c.vr[e] * wapply(c, P.wreal, c.vr, i, j); c.vr0[e] = c.vr[e]; }   // dense penalf2aTrap (:2210-2223); vr0 for penalf2imag
-            }
+            penalty_pre(c, &pen);
             eval_controls(c, t, dt);                                               // (its barrier also orders the vr0 copy)
             state_step(c, dt);
             t = t + dt;
-            if (!densew) { FOR_E pen += P.wdiag[i] * (c.vr[e] * c.vr[e] + 2.0 * c.vi05[e] * c.vi05[e]); }  // penalf2a(vr, vi05)
-            else {
-                // dense penalf2a (:2183-2197) and -2 penalf2imag(vr0, vi05, wmat_imag) = -2 tr(vi05' Wi vr0) (:716-718,:2226-2228)
-                FOR_E {
-                    pen += c.vr[e] * wapply(c, P.wreal, c.vr, i, j) + 2.0 * c.vi05[e] * wapply(c, P.wreal, c.vi05, i, j);
-                    if (P.wimag) pen -= 2.0 * c.vi05[e] * wapply(c, P.wimag, c.vr0, i, j);
-                }
-                gsync(c);                                                   // vr0 is rewritten at the top of the next step
-            }
+            penalty_post(c, &pen);
+            if (densew) gsync(c);                                                  // vr0 is rewritten at the top of the next step
             if (hr && (step + 1) % A.save_every == 0) {                                      // src/evalobjgrad.jl:2847-2849
                 const size_t o = (size_t)((step + 1) / A.save_every) * c.len;
                 FOR_E { hr[o + e] = c.vr[e]; hi[o + e] = -c.vi[e]; }
@@ -460,6 +569,84 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_generic_kernel(DevProblem P, L
 
 }  // namespace
 
+// Forward sensitivities (the reference's traceobjgrad(verbose = true, evaladjoint = true) check, src/evalobjgrad.jl:724-745,768-784,
+// with step_fwdGrad! src/StormerVerlet.jl:151-251 and fgradforce! src/evalobjgrad.jl:2467-2563): the forward sweep and its tangent
+// along a direction d side by side, in the generic kernel's layout.  Trajectory traj = t * ndir + k, t = b * nsamples + s.  The primal
+// statements are the generic kernel's own helpers (TAN = true adds the tangent next to each), so infid / leak are its objective-only
+// outputs bit for bit.
+__global__ void __launch_bounds__(GEN_THREADS) jq_forward_sensitivity_kernel(DevProblem P, SensArgs S, GenGeom G) {
+    extern __shared__ __align__(16) double sm[];
+    Ctx c{};
+    double *p = group_setup(c, P, S.Npar, S.D1, G, sm);
+    const int grp = threadIdx.x / G.tpt;
+    Tan td;
+    double **blk[] = {&c.vr, &c.vi, &c.vi05, &c.vr0, &c.rhs, &c.scr, &c.k1, &c.k2, &c.l1, &c.l2,
+                      &td.vr, &td.vi, &td.vi05, &td.vr0, &td.rhs, &td.scr, &td.k1, &td.k2, &td.l1, &td.l2};
+    for (int b = 0; b < 20; ++b) { *blk[b] = p; p += c.len; }
+    c.pcof = p; p += c.Npar;
+    double *dv = p; p += c.Npar;
+    c.ctrl = p; p += 6 * c.Nc;
+    td.ctrl = p; p += 6 * c.Nc;
+    c.shift = p; p += c.n;
+    c.red = p;
+    // the tangent seen through the primal helpers: the controls of d are the control tables' tangents, trace_fid is linear in the state
+    Ctx cd = c;
+    cd.pcof = dv; cd.ctrl = td.ctrl; cd.vr = td.vr; cd.vi = td.vi;
+    if (grp >= G.gpc) return;
+
+    const double tinv = 1.0 / P.T;
+    for (int traj = blockIdx.x * G.gpc + grp; traj < S.ntraj; traj += gridDim.x * G.gpc) {
+        const int t_ = traj / S.ndir, k_ = traj % S.ndir, b = t_ / S.nsamples, s = t_ % S.nsamples;
+        const double *pc = S.pcof + (size_t)b * S.pstride, *dd = S.dirs + ((size_t)b * S.ndir + k_) * S.pstride;
+        for (int k = c.gtid; k < c.Npar; k += c.tpt) { c.pcof[k] = pc[k]; dv[k] = dd[k]; }
+        const double phase = P.pFidType == 3 ? pc[c.Npar] : P.globalPhase, dphase = P.pFidType == 3 ? dd[c.Npar] : 0.0;
+        for (int k = c.gtid; k < c.n; k += c.tpt) c.shift[k] = S.shift ? S.shift[(size_t)s * c.n + k] : 0.0;
+        FOR_E { c.vr[e] = P.uinit[e]; c.vi[e] = 0.0; c.vi05[e] = 0.0; td.vr[e] = 0.0; td.vi[e] = 0.0; td.vi05[e] = 0.0; }
+        gsync(c);
+
+        double dt = P.T / (double)P.nsteps, t = 0.0, pen = 0.0, pend = 0.0;
+        const bool densew = P.wreal != nullptr;
+        for (long long step = 0; step < P.nsteps; ++step) {
+            penalty_pre<true>(c, &pen, &td, &pend);
+            eval_controls(c, t, dt);
+            eval_controls(cd, t, dt);                                              // ctrl_dot: bcarrier2 of d
+            state_step<true>(c, dt, &td);
+            t = t + dt;
+            penalty_post<true>(c, &pen, &td, &pend);
+            if (densew) gsync(c);
+        }
+        double re, im, red, imd, pv[2] = {pen, pend};
+        block_sum(c, pv, 2);
+        trace_fid(c, &re, &im);
+        trace_fid(cd, &red, &imd);
+        double sph, cph;
+        sincos(phase, &sph, &cph);
+        const int pfid = P.pFidType;
+        const double abs2 = re * re + im * im;
+        const double infid = pfid == 1 ? 1.0 + abs2 - 2.0 * (re * cph + im * sph) : pfid == 2 ? 1.0 - abs2 : 1.0 - (re * cph - im * sph);
+        const double leak = 0.5 * dt * tinv * pv[0];
+        // tangents of the four pFidType formulas (the phase of type 3 is the last entry of pcof, and of d)
+        const double dabs2 = 2.0 * (re * red + im * imd);
+        const double dinfid = pfid == 1 ? dabs2 - 2.0 * (red * cph + imd * sph)
+                            : pfid == 2 ? -dabs2
+                                        : -(red * cph - imd * sph) + dphase * (re * sph + im * cph);
+        const double dleak = 0.5 * dt * tinv * pv[1];
+        if (c.gtid == 0) {
+            if (k_ == 0) {
+                double *o = S.scal + (size_t)t_ * 4;
+                o[0] = infid; o[1] = leak; o[2] = 1.0 - abs2; o[3] = 0.0;
+            }
+            S.dinfid[traj] = dinfid;
+            S.dleak[traj] = dleak;
+        }
+        if (S.dstate_r) {
+            double *dr = S.dstate_r + (size_t)traj * c.len, *di = S.dstate_i + (size_t)traj * c.len;
+            FOR_E { dr[e] = td.vr[e]; di[e] = -td.vi[e]; }
+        }
+        gsync(c);
+    }
+}
+
 // doubles of shared memory per trajectory group
 static size_t per_group_doubles(const DevProblem &P, int Npar) {
     const size_t len = (size_t)P.n * P.m;
@@ -468,12 +655,19 @@ static size_t per_group_doubles(const DevProblem &P, int Npar) {
     return (d + 1) & ~(size_t)1;                       // keep every group's region 16-byte aligned
 }
 
-static GenGeom generic_geometry(const DevProblem &P, int Npar, size_t *bytes) {
+// forward-sensitivity kernel: the 10 forward-sweep blocks and their tangents, pcof, d, the control table and its tangent
+static size_t fwdsens_group_doubles(const DevProblem &P, int Npar) {
+    const size_t len = (size_t)P.n * P.m;
+    size_t d = 20 * len + 2 * (size_t)Npar + 12 * P.Nc + P.n + (GEN_THREADS / 32) * 8;
+    return (d + 1) & ~(size_t)1;
+}
+
+static GenGeom generic_geometry(const DevProblem &P, size_t per_group, size_t *bytes) {
     const size_t len = (size_t)P.n * P.m, limit = 227 * 1024;
     GenGeom G{};
     G.tpt = len <= 32 ? 32 : len <= 64 ? 64 : len <= 128 ? 128 : 256;
     G.gpc = GEN_THREADS / G.tpt;
-    G.per_group = (int)per_group_doubles(P, Npar);
+    G.per_group = (int)per_group;
     const size_t blob = P.csr_blob ? (size_t)P.csr_bytes + 16 : 0;      // + mbarrier
     while (G.gpc > 1 && (size_t)G.gpc * G.per_group * sizeof(double) > limit) G.gpc >>= 1;
     size_t need = (size_t)G.gpc * G.per_group * sizeof(double);
@@ -490,6 +684,10 @@ static GenGeom generic_geometry(const DevProblem &P, int Npar, size_t *bytes) {
 
 size_t jq_generic_smem_bytes(const DevProblem &P, int Npar) {          // minimum: one group, operators through L1
     return per_group_doubles(P, Npar) * sizeof(double);
+}
+
+size_t jq_fwdsens_smem_bytes(const DevProblem &P, int Npar) {
+    return fwdsens_group_doubles(P, Npar) * sizeof(double);
 }
 
 // evalctrl (src/plotstatectrl.jl:246-276): the control functions of every coupled control on an arbitrary time grid,
@@ -516,7 +714,7 @@ cudaError_t jq_controls_launch(const DevProblem &P, int D1, const double *pcof, 
 
 cudaError_t jq_generic_launch(const DevProblem &P, const LaunchArgs &A, cudaStream_t st, int *nctas, int *regs, size_t *smem) {
     size_t bytes = 0;
-    const GenGeom G = generic_geometry(P, A.Npar, &bytes);
+    const GenGeom G = generic_geometry(P, per_group_doubles(P, A.Npar), &bytes);
     cudaError_t e = cudaFuncSetAttribute(jq_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
     cudaFuncAttributes fa;
@@ -533,5 +731,28 @@ cudaError_t jq_generic_launch(const DevProblem &P, const LaunchArgs &A, cudaStre
     if (nctas) *nctas = grid;
     if (regs) *regs = fa.numRegs;
     if (smem) *smem = bytes;
+    return cudaGetLastError();
+}
+
+cudaError_t jq_fwdsens_launch(const DevProblem &P, const SensArgs &S, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc) {
+    size_t bytes = 0;
+    const GenGeom G = generic_geometry(P, fwdsens_group_doubles(P, S.Npar), &bytes);
+    cudaError_t e = cudaFuncSetAttribute(jq_forward_sensitivity_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e != cudaSuccess) return e;
+    cudaFuncAttributes fa;
+    e = cudaFuncGetAttributes(&fa, jq_forward_sensitivity_kernel);
+    if (e != cudaSuccess) return e;
+    int dev = 0, sms = 148, occ = 1;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, jq_forward_sensitivity_kernel, G.tpt * G.gpc, bytes);
+    if (occ < 1) occ = 1;
+    const int want = (S.ntraj + G.gpc - 1) / G.gpc;
+    const int grid = want < sms * occ ? want : sms * occ;   // persistent: groups loop over trajectories
+    jq_forward_sensitivity_kernel<<<grid, G.tpt * G.gpc, bytes, st>>>(P, S, G);
+    if (nctas) *nctas = grid;
+    if (regs) *regs = fa.numRegs;
+    if (smem) *smem = bytes;
+    if (gpc) *gpc = G.gpc;
     return cudaGetLastError();
 }
