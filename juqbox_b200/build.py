@@ -59,7 +59,7 @@ def build_library(force: bool = False, verbose: bool = False, extra_flags=()) ->
                 print(" ".join(cmd))
             cmds.append(cmd)
         objs.append(obj)
-    # the translation units are independent (the trajectory-kernel instantiations are split over three of them): compile in parallel
+    # the translation units are independent (the trajectory-kernel instantiations are split over jq_traj.cu and jq_traj_inst_*.cu): compile in parallel
     from concurrent.futures import ThreadPoolExecutor
     with ThreadPoolExecutor(max_workers=max(1, min(len(cmds), os.cpu_count() or 1))) as pool:
         list(pool.map(subprocess.check_call, cmds))

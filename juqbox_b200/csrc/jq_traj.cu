@@ -1,26 +1,39 @@
 // Planners, launch and instantiation lookup of the register-resident trajectory kernels; the kernels themselves are in
-// jq_traj_kernels.cuh (shared with jq_traj_inst_b.cu / jq_traj_inst_c.cu, which hold the other parts of the table).
+// jq_traj_kernels.cuh (shared with the jq_traj_inst_*.cu files, which hold the other parts of the table).
 #include "jq_traj_kernels.cuh"
 
 namespace {
 
 const Inst kInst[] = {
-    FIBERM(2, 1, 1, 1, 4), FIBERM(4, 1, 1, 1, 3), FIBERM(4, 1, 1, 2, 3), FIBER(6, 1, 1, 2), FIBERM(3, 1, 1, 1, 3), FIBERM(3, 1, 1, 2, 3),
-    FIBER(4, 2, 1, 1), FIBER(3, 2, 1, 1), FIBER(2, 2, 1, 1), FIBER(4, 3, 1, 1), FIBER(3, 3, 1, 1), FIBER(2, 3, 1, 1),
-    FIBER(5, 2, 1, 1), FIBER(5, 3, 1, 1), FIBER(6, 2, 1, 1), FIBER(5, 1, 1, 2), FIBERO(5, 2, 1, 1),      // 5- and 6-level fastest subsystem
+    traj_inst<FiberLane<2, 1, 1>, 1, 4>(), traj_inst<FiberLane<4, 1, 1>, 1, 3>(), traj_inst<FiberLane<4, 1, 1>, 2, 3>(), traj_inst<FiberLane<6, 1, 1>, 2>(),
+    traj_inst<FiberLane<3, 1, 1>, 1, 3>(), traj_inst<FiberLane<3, 1, 1>, 2, 3>(), traj_inst<FiberLane<4, 2, 1>, 1>(), traj_inst<FiberLane<3, 2, 1>, 1>(),
+    traj_inst<FiberLane<2, 2, 1>, 1>(), traj_inst<FiberLane<4, 3, 1>, 1>(), traj_inst<FiberLane<3, 3, 1>, 1>(), traj_inst<FiberLane<2, 3, 1>, 1>(),
+    traj_inst<FiberLane<5, 2, 1>, 1>(), traj_inst<FiberLane<5, 3, 1>, 1>(), traj_inst<FiberLane<6, 2, 1>, 1>(), traj_inst<FiberLane<5, 1, 1>, 2>(),   // 5- and 6-level fastest subsystem
+    traj_inst<FiberLane<5, 2, 1>, 1, 1, 0, 1>(),
 };
+const InstPart kInstA = inst_part(kInst);
 
-// jt = 0: the run-time-J instantiation; jt > 0: the one with exactly jt Neumann terms compiled in (if any).
-const Inst *find_inst(int kind, int R, int C, int NC, int WQ, int LMASK, int UPL, int variant = 0, int GL = 0, int jt = 0, int nw = 0, int pipe = 0, int seg = 0) {
-    const Inst *parts[6] = {kInst, kInstB, kInstC, kInstD, kInstE, kInstF};
-    const int counts[6] = {(int)(sizeof(kInst) / sizeof(kInst[0])), kInstBCount, kInstCCount, kInstDCount, kInstECount, kInstFCount};
-    for (int p = 0; p < 6; ++p)
-        for (int j = 0; j < counts[p]; ++j) {
-            const Inst &i = parts[p][j];
-            if (i.kind == kind && i.R == R && i.C == C && i.NC == NC && i.WQ == WQ && i.LMASK == LMASK && i.UPL == UPL && i.variant == variant &&
-                i.jt == jt && (i.glt == 0 || i.glt == GL) && (nw == 0 || i.nw == nw) && (i.pipe != 0) == (pipe != 0) && i.seg == seg) return &i;
-        }
+// The entry for `want` with J Neumann terms compiled in, else its run-time-J entry.  Every field matches exactly except: an entry
+// with glt == 0 serves any group size, a query with nw == 0 takes the entry's own warp count, pipe is compared as zero / non-zero.
+const Inst *find_inst(const InstKey &want, int J) {
+    for (int jt : {J, 0})
+        for (const InstPart *part : {&kInstA, &kInstB, &kInstC, &kInstD, &kInstE, &kInstF})
+            for (const Inst *i = part->inst; i < part->inst + part->count; ++i) {
+                const InstKey &k = i->key;
+                if (k.kind == want.kind && k.R == want.R && k.C == want.C && k.NC == want.NC && k.WQ == want.WQ && k.LMASK == want.LMASK &&
+                    k.UPL == want.UPL && k.obj2 == want.obj2 && k.jacobi == want.jacobi && k.hx == want.hx &&
+                    k.general_hanti == want.general_hanti && k.jt == jt && (k.glt == 0 || k.glt == want.glt) &&
+                    (want.nw == 0 || k.nw == want.nw) && (k.pipe != 0) == (want.pipe != 0) && k.seg == want.seg) return i;
+            }
     return nullptr;
+}
+
+// The query of a plan on problem P: the layout comes from the plan, what the kernel must compute from the problem.
+InstKey query(const InstKey &layout, const DevProblem &P) {
+    InstKey q = layout;
+    q.obj2 = P.objFuncType != 1;
+    q.jacobi = P.solver != 1;
+    return q;
 }
 
 double value_at(const HostOps &H, int o, int r, int c) {
@@ -90,16 +103,16 @@ TrajPlan *jq_slot_plan_create(const DevProblem &P, const HostOps &H, const doubl
     while (NL < 32 && NL < Nc * H.Nfreq * 2) NL <<= 1;
     if (NL < Nc * H.Nfreq * 2) return no("more (control, frequency) pairs than lanes");
     const int R = (n + NL - 1) / NL;
-    int C = 1;
-    for (int c = 1; c <= 4; ++c) if (m % c == 0 && R * c <= 4) C = c;
-    const int var = P.objFuncType != 1 ? 64 : 0;
-    const Inst *inst = find_inst(2, R, C, Nc, WQ, 0, 1, var);
-    if (!inst && C > 1) { for (int c = C - 1; c >= 1 && !inst; --c) if (m % c == 0) { inst = find_inst(2, R, c, Nc, WQ, 0, 1, var); if (inst) C = c; } }
-    if (!inst) return no("no slot instantiation for this (rows per lane, columns per lane, controls, objFuncType)");
+    InstKey key{2, R, 1, Nc, WQ, 0, 1};
+    key.glt = NL;
+    for (int c = 1; c <= 4; ++c) if (m % c == 0 && R * c <= 4) key.C = c;
+    while (key.C >= 1 && (m % key.C != 0 || !find_inst(query(key, P), 0))) --key.C;     // the widest instantiated C that divides m
+    if (key.C < 1) return no("no slot instantiation for this (rows per lane, columns per lane, controls, objFuncType)");
+    const int C = key.C;
 
     TrajPlan *pl = new TrajPlan();
-    pl->kind = 2; pl->R = R; pl->C = C; pl->NC = Nc; pl->WQ = WQ; pl->LMASK = 0; pl->UPL = 1; pl->AS = 1;
-    pl->NL = NL; pl->NLR = NL * R; pl->GL = NL; pl->GPT = m / C; pl->CPG = C;
+    pl->key = key;
+    pl->NL = NL; pl->NLR = NL * R; pl->GPT = m / C; pl->CPG = C;
     pl->ngroups = TRAJ_WARPS * (32 / NL);
     pl->TPC = pl->ngroups / pl->GPT;
     pl->exch_per_unit = 4 * pl->NLR * C;      // 2 parities x 2 blocks per round
@@ -224,28 +237,25 @@ TrajPlan *jq_fiber_plan_create(const DevProblem &P, const HostOps &H, const doub
     const int CPG = GL / NL, GPT = (m + CPG - 1) / CPG;
     const int NU = Nc * H.Nfreq * 2, UPL = (NU + GL - 1) / GL;
     if (UPL > 2) return no("too many (control, frequency) pairs for the group size");
-    const Inst *inst = find_inst(3, R, 1, Nc, 2, LMASK, UPL, P.objFuncType != 1 ? 64 : (AS ? 0 : 16));
-    if (P.objFuncType != 1 && !AS) inst = nullptr;
-    if (P.solver != 1) {       // Jacobi: residual norm over the whole block = one group reduction -> one group per trajectory only
-        inst = (AS && P.objFuncType == 1 && GPT == 1) ? find_inst(3, R, 1, Nc, 2, LMASK, UPL, 128) : nullptr;
-        if (!inst) return no("Jacobi solver: no fibre instantiation for this shape (or the trajectory spans several groups)");
-    }
-    if (HX) {
-        inst = AS ? find_inst(3, R, 1, Nc, 2, LMASK, UPL, 8) : nullptr;
-        if (!inst) return no("off-diagonal (exchange) Hconst: no fibre instantiation for this shape");
-    }
-    if (!inst) return no("no fibre instantiation for this (fibre length, controls, updaters per lane, Hanti form, objFuncType)");
+    InstKey key{3, R, 1, Nc, 2, LMASK, UPL};
+    key.hx = HX != 0; key.general_hanti = !AS; key.glt = GL;
+    const bool found = find_inst(query(key, P), 0) != nullptr;
+    // Jacobi: residual norm over the whole block = one group reduction -> one group per trajectory only
+    if (P.solver != 1 && (!found || GPT != 1)) return no("Jacobi solver: no fibre instantiation for this shape (or the trajectory spans several groups)");
+    if (HX && !found) return no("off-diagonal (exchange) Hconst: no fibre instantiation for this shape");
+    if (!found) return no("no fibre instantiation for this (fibre length, controls, updaters per lane, Hanti form, objFuncType)");
     // lane offsets of remote neighbours must stay inside the column block of NL lanes
     TrajPlan *pl = new TrajPlan();
-    pl->kind = 3; pl->R = R; pl->C = 1; pl->NC = Nc; pl->WQ = 2; pl->LMASK = LMASK; pl->UPL = UPL; pl->AS = AS ? 1 : 0; pl->HX = HX;
-    pl->NL = NL; pl->NLR = NL * R; pl->GL = GL; pl->GPT = GPT; pl->CPG = CPG;
+    pl->key = key;
+    pl->NL = NL; pl->NLR = NL * R; pl->GPT = GPT; pl->CPG = CPG;
     pl->ngroups = TRAJ_WARPS * (32 / GL);
     pl->TPC = pl->ngroups / GPT;
     pl->exch_per_unit = 4 * R * 32;           // 2 parities x 2 fibres per round
     if (pl->TPC < 1) {
-        // a trajectory wider than 4 warps (e.g. 45 x 12): the 8-warp instantiations, plain problems only
-        const bool plain = AS && !HX && P.objFuncType == 1 && P.solver == 1;
-        if (GPT <= 8 && plain && find_inst(3, R, 1, Nc, 2, LMASK, UPL, 0, GL, 0, 8)) { pl->nw = 8; pl->ngroups = 8 * (32 / GL); pl->TPC = pl->ngroups / GPT; }
+        // a trajectory wider than 4 warps (e.g. 45 x 12): the 8-warp instantiations (plain problems only)
+        InstKey wide = query(key, P);
+        wide.nw = 8;
+        if (GPT <= 8 && find_inst(wide, 0)) { pl->key.nw = 8; pl->ngroups = 8 * (32 / GL); pl->TPC = pl->ngroups / GPT; }
         else { delete pl; return no("a trajectory does not fit in one CTA"); }
     }
     const int perq = 4 * (R - 1) + 4 + (HX ? 2 * (R - 1) : 0), per = Nc * perq;
@@ -278,11 +288,9 @@ TrajPlan *jq_fiber_plan_create(const DevProblem &P, const HostOps &H, const doub
     }
     if (pipe) {      // pipelined roles: single-fibre columns only (no exchange buffer), plain problems; NW = warps that hold one group set
         const int nwp = (GPT * GL + 31) / 32;
-        const bool plain = AS && !HX && P.objFuncType == 1 && P.solver == 1 && LMASK == (1 << Nc) - 1;
-        if (!plain || !(find_inst(3, R, 1, Nc, 2, LMASK, UPL, 0, GL, P.J, nwp, 1) || find_inst(3, R, 1, Nc, 2, LMASK, UPL, 0, GL, 0, nwp, 1))) {
-            delete pl; return no("no pipelined fibre instantiation for this shape");
-        }
-        pl->pipe = 1; pl->nw = nwp; pl->ngroups = nwp * (32 / GL); pl->TPC = pl->ngroups / GPT;
+        pl->key.pipe = 1; pl->key.nw = nwp;
+        if (LMASK != (1 << Nc) - 1 || !find_inst(query(pl->key, P), P.J)) { delete pl; return no("no pipelined fibre instantiation for this shape"); }
+        pl->ngroups = nwp * (32 / GL); pl->TPC = pl->ngroups / GPT;
     }
     if (!upload_plan(pl, pi, pd, d0p, wp)) { jq_traj_plan_destroy(pl); return no("cudaMalloc failed for the fibre plan"); }
     err[0] = 0;
@@ -333,14 +341,16 @@ TrajPlan *jq_tile_plan_create(const DevProblem &P, const HostOps &H, const doubl
     const int NU = Nc * H.Nfreq * 2, UPL = (NU + GL - 1) / GL;
     if (UPL > 1) return no("tile layout: too many (control, frequency) pairs for the group size");
     const int nwp = pipe ? (GPT * GL + 31) / 32 : 0;
-    if (!find_inst(4, NT, 1, Nc, 0, 0, UPL, 0, GL, 0, nwp, pipe) && !find_inst(4, NT, 1, Nc, 0, 0, UPL, 0, GL, P.J, nwp, pipe)) return no("tile layout: no instantiation");
+    InstKey key{4, NT, 1, Nc, 0, 0, UPL};
+    key.glt = GL; key.nw = nwp; key.pipe = pipe ? 1 : 0;      // nw = 0: the 4 x 4 x 4 tiles run 8 warps per CTA
+    if (!find_inst(query(key, P), P.J)) return no("tile layout: no instantiation");
     TrajPlan *pl = new TrajPlan();
-    pl->kind = 4; pl->R = NT; pl->C = 1; pl->NC = Nc; pl->WQ = 0; pl->LMASK = 0; pl->UPL = UPL; pl->AS = 1; pl->HX = 0;
-    pl->NL = NL; pl->NLR = n; pl->GL = GL; pl->GPT = GPT; pl->CPG = CPG;
+    pl->key = key;
+    pl->NL = NL; pl->NLR = n; pl->GPT = GPT; pl->CPG = CPG;
     pl->ngroups = TRAJ_WARPS * (32 / GL);
     pl->TPC = pl->ngroups / GPT;
     pl->exch_per_unit = 0;                         // shuffles only
-    if (pipe) { pl->pipe = 1; pl->nw = nwp; pl->ngroups = nwp * (32 / GL); pl->TPC = pl->ngroups / GPT; }
+    if (pipe) { pl->ngroups = nwp * (32 / GL); pl->TPC = pl->ngroups / GPT; }
     if (pl->TPC < 1) { delete pl; return no("a trajectory does not fit in one CTA"); }
     const int nrem = Nc - NT, per = 3 * NT + 2 * nrem;
     std::vector<int> pi((size_t)NL * (nrem > 0 ? nrem : 1) * 2, 0);
@@ -371,75 +381,55 @@ void jq_traj_plan_destroy(TrajPlan *pl) {
     delete pl;
 }
 
+// Segment-sweep instantiations exist only for Neumann problems on non-pipelined 4-warp (tile: their own) plans without drift
+// couplings and with the ladder form of Hanti.
 bool jq_seg_supported(const TrajPlan *pl, const DevProblem &P, bool second_adjoint) {
-    if (!pl || pl->pipe || pl->nw || !pl->AS || pl->HX || P.solver != 1 || 2 * P.n > 512) return false;
-    if (second_adjoint) return find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, 64, pl->GL, 0, 0, 0, 1) != nullptr;
-    return find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, 0, pl->GL, P.J, 0, 0, 1) ||
-           find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, 0, pl->GL, 0, 0, 0, 1);
+    if (!pl || 2 * P.n > 512) return false;
+    InstKey want = query(pl->key, P);
+    want.seg = 1;
+    want.obj2 = second_adjoint;
+    return find_inst(want, P.J) != nullptr;
 }
 
-int jq_traj_plan_kind(const TrajPlan *pl) { return pl ? pl->kind : 0; }
+int jq_traj_plan_kind(const TrajPlan *pl) { return pl ? pl->key.kind : 0; }
 int jq_traj_plan_tpc(const TrajPlan *pl) { return pl ? pl->TPC : 0; }
-int jq_traj_plan_lanes(const TrajPlan *pl) { return pl ? pl->GPT * pl->GL : 0; }
+int jq_traj_plan_lanes(const TrajPlan *pl) { return pl ? pl->GPT * pl->key.glt : 0; }
 
 cudaError_t jq_traj_launch(TrajPlan *pl, const DevProblem &P, const LaunchArgs &A, cudaStream_t st, int *nctas, int *regs,
                            size_t *smem, int *traj_per_cta) {
-    // What the kernel must compute fixes the variant; exchange-mode twins (1, 512) are a development override for plain problems only.
-    int want = 0;
-    if (P.objFuncType != 1) want = 64;
-    else if (P.solver != 1) want = 128;
-    else if (pl->HX) want = 8;
-    else if (!pl->AS) want = 16;
-    if ((want == 64 || want == 128 || want == 8) && !pl->AS) return cudaErrorNotSupported;
-    const Inst *inst = nullptr;
+    // never substitute: Neumann for Jacobi, one adjoint set for two, no drift couplings
+    InstKey want = query(pl->key, P);
     const bool seg = A.seg.nseg > 0;
-    if (seg) {                  // segment sweeps of the time-parallel evaluation: Neumann problems on a non-pipelined plan
+    if (seg) {                  // segment sweeps of the time-parallel evaluation
+        if (A.hist_r) return cudaErrorNotSupported;
+        want.seg = 1;
         // objFuncType 2/3: only the gradient sweep (mode 5) carries the second adjoint set; every other mode is the plain one
-        const int segwant = A.seg.mode[0] == 5 ? want : (want == 64 ? 0 : want);
-        if ((segwant != 0 && segwant != 64) || pl->pipe || pl->nw || A.hist_r) return cudaErrorNotSupported;
-        if (segwant == 0) inst = find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, 0, pl->GL, P.J, 0, 0, 1);
-        if (!inst) inst = find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, segwant, pl->GL, 0, 0, 0, 1);
-        if (!inst) return cudaErrorNotSupported;
-    } else if (pl->pipe) {
-        if (want != 0 || P.nsteps > 0x7ffffff0LL) return cudaErrorNotSupported;      // the hand-over counters are ints
-        inst = find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, 0, pl->GL, P.J, pl->nw, 1);
-        if (!inst) inst = find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, 0, pl->GL, 0, pl->nw, 1);
-        if (!inst) return cudaErrorNotSupported;
-    } else if (want == 0 && !pl->nw) {
-        const char *xm = getenv("JQ_TRAJ_XMODE");
-        const int xv = xm ? atoi(xm) : 0;
-        if (xv > 0) {
-            inst = find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, xv, pl->GL, P.J);
-            if (!inst) inst = find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, xv, pl->GL, 0);
-        }
-        if (!inst && P.J > 0)     // instantiation with the number of Neumann terms known at compile time
-            inst = find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, 0, pl->GL, P.J);
+        want.obj2 = want.obj2 && A.seg.mode[0] == 5;
     }
-    if (pl->nw && !inst) inst = find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, want, pl->GL, 0, pl->nw);
-    if (!inst) inst = find_inst(pl->kind, pl->R, pl->C, pl->NC, pl->WQ, pl->LMASK, pl->UPL, want, pl->GL, 0);
-    if (!inst) return cudaErrorNotSupported;       // never substitute: Neumann for Jacobi, one adjoint set for two, no drift couplings
-    if (inst->jt != 0 && inst->jt != P.J) return cudaErrorNotSupported;
+    if (want.pipe && P.nsteps > 0x7ffffff0LL) return cudaErrorNotSupported;      // the hand-over counters are ints
+    const Inst *inst = find_inst(want, P.J);
+    if (!inst || (inst->key.jt != 0 && inst->key.jt != P.J)) return cudaErrorNotSupported;
     TrajParams S{};
     S.P = P; S.A = A;
-    S.NL = pl->NL; S.NLR = pl->NLR; S.GL = pl->GL; S.GPT = pl->GPT; S.CPG = pl->CPG;
+    S.NL = pl->NL; S.NLR = pl->NLR; S.GL = pl->key.glt; S.GPT = pl->GPT; S.CPG = pl->CPG;
     S.plan_i = pl->d_i; S.plan_d = pl->d_d; S.plan_d0 = pl->d_d0; S.plan_w = pl->d_w;
     S.exch_per_unit = pl->exch_per_unit;
     S.NparS = A.Npar | 1;
-    S.GPW = 32 / pl->GL;
-    const int npts = 2 * TRAJ_CH + 1, NC = pl->NC;
+    S.GPW = 32 / pl->key.glt;
+    const int npts = 2 * TRAJ_CH + 1, NC = pl->key.NC;
     // warps per CTA: 4 normally; fewer when the per-CTA gradient windows / pcof staging of very long coefficient
     // vectors would not fit in shared memory (the kernel only uses blockDim.x and the counts below)
-    int nw = inst->nw, TPC = 0, ngroups = 0;
+    int nw = inst->key.nw, TPC = 0, ngroups = 0;
     size_t bytes = 0;
-    const int pipe = inst->pipe;
-    const int Eper = pl->kind == 4 ? (1 << pl->R) : pl->kind == 3 ? pl->R : pl->R * pl->C;      // elements per lane
+    const int pipe = inst->key.pipe;
+    const int kind = pl->key.kind, Eper = kind == 4 ? (1 << pl->key.R) : kind == 3 ? pl->key.R : pl->key.R * pl->key.C;      // elements per lane
     for (; nw >= 1; nw >>= 1) {
         ngroups = nw * S.GPW;
         TPC = ngroups / pl->GPT;
         if (TPC < 1) return cudaErrorInvalidConfiguration;
         int o = 0;
         auto take = [&](int cnt) { int at = o; o += (cnt + 1) & ~1; return at; };   // keep 16-byte alignment
-        S.o_exch = take(pl->exch_per_unit * (pl->kind == 2 ? ngroups : nw));
+        S.o_exch = take(pl->exch_per_unit * (kind == 2 ? ngroups : nw));
         S.o_pcof = take(TPC * S.NparS);
         S.o_gsm = take(ngroups * A.Npar);
         S.o_times = take(npts);                              // control table: one contiguous block per role

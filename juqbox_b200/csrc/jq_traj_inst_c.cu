@@ -1,11 +1,15 @@
 // Part of the instantiation table of the register-resident trajectory kernels (see jq_traj_kernels.cuh).
 #include "jq_traj_kernels.cuh"
 
-const Inst kInstC[] = {
-    FIBERO(3, 2, 1, 1), FIBERO(4, 2, 1, 1), FIBERO(4, 1, 1, 1), FIBERO(4, 1, 1, 2), FIBERO(6, 1, 1, 2), FIBERO(4, 3, 1, 1), FIBERO(2, 1, 1, 1),
-    FIBERHX(4, 2, 1, 1), FIBERHX(3, 2, 1, 1), FIBERHX(2, 2, 1, 1), FIBERHX(4, 3, 1, 1),      // drift with exchange couplings to the fibre subsystem
-    FIBERJAC(3, 2, 1, 1), FIBERJAC(4, 2, 1, 1), FIBERJAC(4, 1, 1, 2), FIBERJAC(6, 1, 1, 2),
-    FIBERG(4, 2, 1, 1), FIBERG(4, 1, 1, 1), FIBERG(4, 1, 1, 2), FIBERG(2, 1, 1, 1),
-    FIBERW(5, 3, 1, 1, 8), FIBERW(4, 3, 1, 1, 8), FIBERW(3, 3, 1, 1, 8),      // trajectories of 5 ... 8 warps (e.g. 45 x 12)
+const Inst kInst[] = {
+    traj_inst<FiberLane<3, 2, 1>, 1, 1, 0, 1>(), traj_inst<FiberLane<4, 2, 1>, 1, 1, 0, 1>(), traj_inst<FiberLane<4, 1, 1>, 1, 1, 0, 1>(),   // objFuncType 2/3
+    traj_inst<FiberLane<4, 1, 1>, 2, 1, 0, 1>(), traj_inst<FiberLane<6, 1, 1>, 2, 1, 0, 1>(), traj_inst<FiberLane<4, 3, 1>, 1, 1, 0, 1>(),
+    traj_inst<FiberLane<2, 1, 1>, 1, 1, 0, 1>(),
+    // drift with exchange couplings to the fibre subsystem (HX: every control outside LMASK)
+    traj_inst<FiberLane<4, 2, 1, 1, 0, 2>, 1>(), traj_inst<FiberLane<3, 2, 1, 1, 0, 2>, 1>(), traj_inst<FiberLane<2, 2, 1, 1, 0, 2>, 1>(), traj_inst<FiberLane<4, 3, 1, 1, 0, 6>, 1>(),
+    traj_inst<FiberLane<3, 2, 1>, 1, 1, -1>(), traj_inst<FiberLane<4, 2, 1>, 1, 1, -1>(), traj_inst<FiberLane<4, 1, 1>, 2, 1, -1>(),      // Jacobi solver
+    traj_inst<FiberLane<6, 1, 1>, 2, 1, -1>(),
+    traj_inst<FiberLane<4, 2, 1, 0>, 1>(), traj_inst<FiberLane<4, 1, 1, 0>, 1>(), traj_inst<FiberLane<4, 1, 1, 0>, 2>(), traj_inst<FiberLane<2, 1, 1, 0>, 1>(),   // general Hanti (AS = 0)
+    traj_inst<FiberLane<5, 3, 1>, 1, 1, 0, 0, 0, 8>(), traj_inst<FiberLane<4, 3, 1>, 1, 1, 0, 0, 0, 8>(), traj_inst<FiberLane<3, 3, 1>, 1, 1, 0, 0, 0, 8>(),   // trajectories of 5 ... 8 warps (e.g. 45 x 12)
 };
-const int kInstCCount = (int)(sizeof(kInstC) / sizeof(kInstC[0]));
+const InstPart kInstC = inst_part(kInst);

@@ -61,28 +61,34 @@ struct TrajParams {
     int o_ring, o_cnt, tab_role_stride;      // rings of (vr0, vi05, vr) and of lane-partial traces, the int step / chunk counters, size of one control-table buffer
 };
 
+typedef void (*traj_kernel_t)(const TrajParams);
+
+// What an instantiation of jq_traj_kernel computes and for which layout.  In a table entry every field follows from the template
+// arguments (traj_inst); a plan holds the key of its layout, and a query adds what the problem asks for (find_inst in jq_traj.cu).
+//   kind 2 slot, 3 fibre, 4 tile; R rows per lane (tile: tiled directions NT), C columns per lane, NC controls, WQ entries per row
+//   and control, LMASK controls coupling inside a fibre, UPL gradient-scatter roles per lane;
+//   obj2 second adjoint set (objFuncType 2/3), jacobi Jacobi solver, hx exchange-coupled drift, general_hanti Hanti not of the
+//   ladder form (AS = 0);
+//   glt group size (entry: compile-time, 0 = any); jt Neumann terms compiled in (0 = run-time J; a query passes J instead);
+//   nw warps per CTA and role (query: 0 = the entry's own); pipe pipelined roles (matched as zero / non-zero); seg segment sweep
+//   of the time-parallel evaluation.
+struct InstKey {
+    int kind, R, C, NC, WQ, LMASK, UPL;
+    bool obj2 = false, jacobi = false, hx = false, general_hanti = false;
+    int glt = 0, jt = 0, nw = TRAJ_WARPS, pipe = 0, seg = 0;
+};
+struct Inst { InstKey key; traj_kernel_t fn; };
+// The instantiation table is split over jq_traj.cu and the jq_traj_inst_*.cu files so that they compile in parallel.
+struct InstPart { const Inst *inst; int count; };
+template <int N> constexpr InstPart inst_part(const Inst (&t)[N]) { return {t, N}; }
+extern const InstPart kInstB, kInstC, kInstD, kInstE, kInstF;
+
 struct TrajPlan {
-    int kind;                                // 2 slot, 3 fibre
-    int R, C, NC, WQ, LMASK, UPL, AS, HX = 0;
-    int NL, GL, GPT, TPC, ngroups, CPG, NLR, exch_per_unit;
-    int nw = 0;                              // warps per CTA (per role) the plan needs (0: the instantiation's own)
-    int pipe = 0;                            // pipelined state / adjoint roles (latency plans)
+    InstKey key;                             // glt: the group size GL; nw: warps per CTA (per role), 0 for the instantiation's own
+    int NL, GPT, TPC, ngroups, CPG, NLR, exch_per_unit;
     int *d_i = nullptr;
     double *d_d = nullptr, *d_d0 = nullptr, *d_w = nullptr;
 };
-
-typedef void (*traj_kernel_t)(const TrajParams);
-// variant (what the kernel computes / how it exchanges): 0 default, 8 exchange-coupled drift, 16 general Hanti, 64 objFuncType 2/3,
-// 128 Jacobi solver; 1 (warp-shuffle exchange) and 512 (shared-memory twin of the cnot2 instantiation) are exchange-mode
-// twins selectable for comparisons with the env variable JQ_TRAJ_XMODE.  jt: number of Neumann terms fixed at compile time
-// (0 = run-time J) -- its own field, never folded into `variant`.  glt: compile-time group size (0 = run-time).
-struct Inst { int kind, R, C, NC, WQ, LMASK, UPL, variant; traj_kernel_t fn; int glt = 0; int jt = 0; int nw = TRAJ_WARPS; int pipe = 0; int seg = 0; };
-// The instantiation table is split over jq_traj.cu / jq_traj_inst_b.cu / jq_traj_inst_c.cu so that they compile in parallel.
-extern const Inst kInstB[]; extern const int kInstBCount;
-extern const Inst kInstC[]; extern const int kInstCCount;
-extern const Inst kInstD[]; extern const int kInstDCount;
-extern const Inst kInstE[]; extern const int kInstECount;
-extern const Inst kInstF[]; extern const int kInstFCount;
 
 namespace {
 
@@ -139,7 +145,7 @@ struct Geo {
 
 template <int R_, int C_, int NC_, int WQ_>
 struct SlotLane {
-    static constexpr int R = R_, C = C_, NC = NC_, WQ = WQ_, E = R_ * C_, HX = 0;
+    static constexpr int KIND = 2, R = R_, C = C_, NC = NC_, WQ = WQ_, LMASK = 0, AS = 1, E = R_ * C_, HX = 0;
     int pos[R][NC][WQ], own[R];
     double hs[R][NC][WQ], ha[R][NC][WQ];
     double d0[E], w[E];
@@ -247,7 +253,7 @@ struct SlotLane {
 // control q -- fibres every K-product fetches anyway.
 template <int R_, int NC_, int LMASK_, int AS_ = 1, int XM_ = 0, int HX_ = 0>
 struct FiberLane {
-    static constexpr int R = R_, NC = NC_, LMASK = LMASK_, E = R_, AS = AS_, XM = XM_, HX = HX_;   // XM: 0 = shared-memory exchange, 1 = warp shuffles (16 instead of 24 data-pipe wavefronts per round for R = 4, NC = 2, but 16 instead of 7 instructions)
+    static constexpr int KIND = 3, R = R_, C = 1, NC = NC_, WQ = 2, LMASK = LMASK_, E = R_, AS = AS_, XM = XM_, HX = HX_;   // XM: 0 = shared-memory exchange, 1 = warp shuffles (16 instead of 24 data-pipe wavefronts per round for R = 4, NC = 2, but 16 instead of 7 instructions)
     static constexpr bool REMOTE = (LMASK_ != (1 << NC_) - 1);
     static constexpr int RM1 = R_ > 1 ? R_ - 1 : 1;
     // local (inside the fibre) tridiagonal coefficients: x_{k+1} -> row k ("u"), x_k -> row k+1 ("l")
@@ -428,7 +434,7 @@ struct FiberLane {
 // Requires Hanti = upper(Hsym) - lower(Hsym) and a diagonal Hconst (the planner checks).
 template <int NC_, int NT_>
 struct TileLane {
-    static constexpr int NC = NC_, NT = NT_, E = 1 << NT_, HX = 0, R = NT_;
+    static constexpr int KIND = 4, NC = NC_, NT = NT_, E = 1 << NT_, HX = 0, R = NT_, C = 1, WQ = 0, LMASK = 0, AS = 1;
     static constexpr bool SIGNED = true;
     static constexpr int NT1 = NT_ > 0 ? NT_ : 1, EH = NT_ > 0 ? (1 << NT_) / 2 : 1;      // array extents (NT = 0: one element per lane, all directions remote)
     double cin[NT1], cx[NT1], sg[NT1];       // in-lane pair coupling, cross-lane (interface) coupling, mirror sign
@@ -1365,28 +1371,11 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
     }
 }
 
-#define SLOT(R, C, NC, WQ) {2, R, C, NC, WQ, 0, 1, 0, jq_traj_kernel<SlotLane<R, C, NC, WQ>, 1>}
-#define SLOTO(R, C, NC, WQ) {2, R, C, NC, WQ, 0, 1, 64, jq_traj_kernel<SlotLane<R, C, NC, WQ>, 1, 1, 0, 1>}   /* objFuncType 2/3 */
-#define FIBER(R, NC, LMASK, UPL) {3, R, 1, NC, 2, LMASK, UPL, 0, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL>}
-#define FIBERM(R, NC, LMASK, UPL, MINB) {3, R, 1, NC, 2, LMASK, UPL, 0, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, MINB>}
-#define FIBERJ(R, NC, LMASK, UPL, JT) {3, R, 1, NC, 2, LMASK, UPL, 0, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, 1, JT>, 0, JT}   /* compile-time J */
-#define FIBERJG(R, NC, LMASK, UPL, JT, GLT) {3, R, 1, NC, 2, LMASK, UPL, 0, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, 1, JT, 0, GLT>, GLT, JT}   /* compile-time J and group size */
-#define FIBERO(R, NC, LMASK, UPL) {3, R, 1, NC, 2, LMASK, UPL, 64, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, 1, 0, 1>}   /* objFuncType 2/3 */
-#define FIBERJGM(R, NC, LMASK, UPL, JT, GLT, MINB, VAR) {3, R, 1, NC, 2, LMASK, UPL, VAR, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, MINB, JT, 0, GLT>, GLT, JT}
-#define FIBERX(R, NC, LMASK, UPL, JT, GLT, XM, VAR) {3, R, 1, NC, 2, LMASK, UPL, VAR, jq_traj_kernel<FiberLane<R, NC, LMASK, 1, XM>, UPL, 1, JT, 0, GLT>, GLT, JT}   /* compile-time J and group size, exchange mode XM */
-#define FIBERHX(R, NC, LMASK, UPL) {3, R, 1, NC, 2, LMASK, UPL, 8, jq_traj_kernel<FiberLane<R, NC, LMASK, 1, 0, ((1 << NC) - 1) & ~LMASK>, UPL>}   /* exchange-coupled drift */
-#define FIBERJAC(R, NC, LMASK, UPL) {3, R, 1, NC, 2, LMASK, UPL, 128, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, 1, -1>}   /* Jacobi solver */
-#define FIBERG(R, NC, LMASK, UPL) {3, R, 1, NC, 2, LMASK, UPL, 16, jq_traj_kernel<FiberLane<R, NC, LMASK, 0>, UPL>}   /* general Hanti (AS = 0) */
-#define TILEJ(NC, NT, UPL, JT, GLT) {4, NT, 1, NC, 0, 0, UPL, 0, jq_traj_kernel<TileLane<NC, NT>, UPL, 1, JT, 0, GLT>, GLT, JT}   /* tile layout */
-#define TILEP(NC, NT, UPL, JT, GLT, NW) {4, NT, 1, NC, 0, 0, UPL, 0, jq_traj_kernel<TileLane<NC, NT>, UPL, 1, JT, 0, GLT, NW, 1>, GLT, JT, NW, 1}   /* tile layout, pipelined roles (2 NW warps) */
-#define TILEP2(NC, NT, UPL, JT, GLT, NW) {4, NT, 1, NC, 0, 0, UPL, 0, jq_traj_kernel<TileLane<NC, NT>, UPL, 1, JT, 0, GLT, NW, 2>, GLT, JT, NW, 2}   /* roles (state + adjoint) | (gradient + tables) */
-#define FIBERP(R, NC, LMASK, UPL, JT, GLT, NW) {3, R, 1, NC, 2, LMASK, UPL, 0, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, 1, JT, 0, GLT, NW, 1>, GLT, JT, NW, 1}   /* single-fibre layout, pipelined roles */
-#define TILEJW(NC, NT, UPL, JT, GLT, NW, MINB, VAR) {4, NT, 1, NC, 0, 0, UPL, VAR, jq_traj_kernel<TileLane<NC, NT>, UPL, MINB, JT, 0, GLT, NW>, GLT, JT, NW}   /* tile layout, NW warps per CTA */
-#define FIBERW(R, NC, LMASK, UPL, NW) {3, R, 1, NC, 2, LMASK, UPL, 0, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, 1, 0, 0, 0, NW>, 0, 0, NW}   /* NW warps per CTA: trajectories wider than 4 warps */
-#define FIBERV(R, NC, LMASK, UPL, XM) {3, R, 1, NC, 2, LMASK, UPL, XM, jq_traj_kernel<FiberLane<R, NC, LMASK, 1, XM>, UPL>}   /* exchange mode XM (1 = warp shuffle) */
+// Table entry of one instantiation: the key is derived from the template arguments, so it cannot disagree with the kernel.
+template <class LaneT, int UPL, int MINB = 1, int JT = 0, int OBJ = 0, int GLT = 0, int NW = TRAJ_WARPS, int PIPE = 0, bool SEG = false>
+constexpr Inst traj_inst() {
+    return {{LaneT::KIND, LaneT::R, LaneT::C, LaneT::NC, LaneT::WQ, LaneT::LMASK, UPL, OBJ != 0, JT < 0, LaneT::HX != 0, !LaneT::AS,
+             GLT, JT > 0 ? JT : 0, NW, PIPE, SEG},
+            jq_traj_kernel<LaneT, UPL, MINB, JT, OBJ, GLT, NW, PIPE, SEG>};
+}
 }  // namespace
-/* time-parallel evaluation: segment sweeps (SEG) on the tile / fibre layouts */
-#define TILES(NC, NT, UPL, JT, GLT) {4, NT, 1, NC, 0, 0, UPL, 0, jq_traj_kernel<TileLane<NC, NT>, UPL, 1, JT, 0, GLT, TRAJ_WARPS, 0, true>, GLT, JT, TRAJ_WARPS, 0, 1}
-#define FIBERS(R, NC, LMASK, UPL, JT, GLT) {3, R, 1, NC, 2, LMASK, UPL, 0, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, 1, JT, 0, GLT, TRAJ_WARPS, 0, true>, GLT, JT, TRAJ_WARPS, 0, 1}
-#define TILESW(NC, NT, UPL, JT, GLT, NW) {4, NT, 1, NC, 0, 0, UPL, 0, jq_traj_kernel<TileLane<NC, NT>, UPL, 1, JT, 0, GLT, NW, 0, true>, GLT, JT, NW, 0, 1}
-#define FIBERSO(R, NC, LMASK, UPL) {3, R, 1, NC, 2, LMASK, UPL, 64, jq_traj_kernel<FiberLane<R, NC, LMASK, 1>, UPL, 1, 0, 1, 0, TRAJ_WARPS, 0, true>, 0, 0, TRAJ_WARPS, 0, 1}   /* objFuncType 2/3 */
