@@ -64,6 +64,8 @@ struct jq_handle {
     std::vector<int> rowptr, col;
     std::vector<double> val;
     TrajPlan *slot = nullptr, *fiber = nullptr, *tile = nullptr, *tile_lat = nullptr;     // tile_lat: fewest elements per lane (small batches)
+    TrajPlan *tile_in = nullptr;        // tile layout with the first subsystem whole in the lane (large batches; nullptr: none)
+    int tile_in_ntraj = 0;              // automatic mode: launches with at least this many trajectories use tile_in
     bool dense_ok = false;              // the dense (FP64 MMA) kernel can serve this problem
     bool dense_auto = false;            // ... and the operators are dense enough for it to beat the row-wise generic kernel
     char dense_reason[128] = "";
@@ -347,16 +349,20 @@ extern "C" int jq_create(const jq_problem *pb, int device, jq_handle **out) {
     h->fiber = jq_fiber_plan_create(P, H, pb->wdiag, h->fiber_reason, sizeof(h->fiber_reason));
     {
         const char *nt = getenv("JQ_TILE_NT");      // development: number of tiled directions of the tile layout (default: all)
-        h->tile = jq_tile_plan_create(P, H, pb->wdiag, nt ? atoi(nt) : Nc, h->tile_reason, sizeof(h->tile_reason));
+        h->tile = jq_tile_plan_create(P, H, pb->wdiag, nt ? atoi(nt) : Nc, 0, h->tile_reason, sizeof(h->tile_reason));
+        char why[256];
+        // Two subsystems, first one whole in the lane (TileLane<2,1,1>): half the exchange shuffles per element of the 2 x 2 tiles
+        // and twice the independent element chains per lane, but 4 instead of 2 trajectories per warp
+        const char *ti = getenv("JQ_TILE_INLANE");      // development: 0 = never, 1 = for every launch, unset = automatic
+        if (h->tile && !nt && !(ti && atoi(ti) == 0)) h->tile_in = jq_tile_plan_create(P, H, pb->wdiag, 1, 1, why, sizeof(why));
         // Latency layout: a trajectory spread over as many lanes as the warp-local exchange allows (one element per lane for two
         // subsystems, two for three).  A lone evaluation (the reference's own call pattern, one pcof per Ipopt callback) is bound
         // by the instruction stream of ONE lane, so fewer elements per lane is what shortens it; throughput layouts win once the
         // SMs are full.
-        char why[256];
         const char *lnt = getenv("JQ_TILE_LAT_NT");
         const char *lp = getenv("JQ_LAT_PIPE");        // development: 0 = latency layout without the pipelined roles
         const int pipe = lp ? atoi(lp) : 1;
-        h->tile_lat = jq_tile_plan_create(P, H, pb->wdiag, lnt ? atoi(lnt) : (Nc == 2 ? 0 : 1), why, sizeof(why), pipe);
+        h->tile_lat = jq_tile_plan_create(P, H, pb->wdiag, lnt ? atoi(lnt) : (Nc == 2 ? 0 : 1), 0, why, sizeof(why), pipe);
         if (!h->tile_lat && pipe) h->tile_lat = jq_fiber_plan_create(P, H, pb->wdiag, why, sizeof(why), 1);     // single-fibre shapes: same layout, pipelined roles
         int sms = 148;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
@@ -369,10 +375,15 @@ extern "C" int jq_create(const jq_problem *pb, int device, jq_handle **out) {
         for (double v : h->val) nnz += v != 0.0;
         h->dense_auto = h->dense_ok && n >= 8 && (double)nnz >= 0.2 * (double)(1 + 2 * Nc) * n * n;
         h->lat_ntraj = lt ? atoi(lt) : sms * (h->tile_lat ? jq_traj_plan_tpc(h->tile_lat) : 1);
+        // in-lane tiles from one full resident wave of them (2 CTAs of 16 trajectories per SM, 4736 on 148 SMs): below it their
+        // CTAs leave SMs half empty where the 2 x 2 tiles (wave 2368) fill them.  Measured cnot2 speed-up over the 2 x 2 tiles (B200,
+        // 1000 W; profiles/r03_tile_inlane.md): 0.88x at 2368 and 0.85x at 3552 candidates; 1.09x at 4736, 1.06x at 7104, 1.10x at
+        // 9472 and 16384, 1.12x at 32768.
+        if (h->tile_in) h->tile_in_ntraj = ti && atoi(ti) == 1 ? 0 : 2 * sms * jq_traj_plan_tpc(h->tile_in);
         // Time-parallel evaluation for launches of very few trajectories (one pcof per Ipopt callback): segments of the time axis
         // swept concurrently and joined through their propagators
         h->sms = sms;
-        h->seg_plan = jq_tile_plan_create(P, H, pb->wdiag, Nc == 2 ? 0 : 1, why, sizeof(why), 0);
+        h->seg_plan = jq_tile_plan_create(P, H, pb->wdiag, Nc == 2 ? 0 : 1, 0, why, sizeof(why), 0);
         if (!h->seg_plan) h->seg_plan = h->fiber;
         if (h->seg_plan && !jq_seg_supported(h->seg_plan, P)) { if (h->seg_plan != h->fiber) jq_traj_plan_destroy(h->seg_plan); h->seg_plan = nullptr; }
         // objFuncType 2/3: the gradient sweep needs the second adjoint set, which the fibre layout has
@@ -407,6 +418,7 @@ extern "C" int jq_destroy(jq_handle *h) {
     if (h->slot) jq_traj_plan_destroy(h->slot);
     if (h->tile) jq_traj_plan_destroy(h->tile);
     if (h->tile_lat) jq_traj_plan_destroy(h->tile_lat);
+    if (h->tile_in) jq_traj_plan_destroy(h->tile_in);
     if (h->seg_plan && h->seg_plan != h->fiber) jq_traj_plan_destroy(h->seg_plan);
     if (h->fiber) jq_traj_plan_destroy(h->fiber);
     if (h->d_seg) cudaFree(h->d_seg);
@@ -590,13 +602,16 @@ __global__ void __launch_bounds__(32 * WS_LANES) jq_weighted_sum_kernel(int nsam
 // generic kernel.  In automatic mode a layout that cannot serve this launch (no instantiation for the variant, shared-memory
 // layout does not fit, out of launch resources) hands over to the next one; an explicitly requested kernel fails instead.
 static int launch_trajectories(jq_handle *h, const LaunchArgs &A, cudaStream_t st) {
-    TrajPlan *cands[4] = {nullptr, nullptr, nullptr, nullptr};
+    TrajPlan *cands[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
     int ncand = 0;
     const int pref = h->kernel_pref;
     const bool small = A.ntraj <= h->lat_ntraj;
     if (pref == 5 || (pref == 0 && h->tile_lat && small)) cands[ncand++] = h->tile_lat;
     if (pref == 0 && small && h->fiber && h->tile && h->Nc >= 3) cands[ncand++] = h->fiber;     // three subsystems: the fibre layout (4 elements per lane) before the 8-element tiles
-    if (pref == 4 || (pref == 0 && h->tile && h->prefer_tile)) cands[ncand++] = h->tile;
+    if (pref == 4 || (pref == 0 && h->tile && h->prefer_tile)) {
+        if (h->tile_in && A.ntraj >= h->tile_in_ntraj) cands[ncand++] = h->tile_in;
+        cands[ncand++] = h->tile;
+    }
     if (pref == 3 || (pref == 0 && h->fiber && !(ncand && cands[ncand - 1] == h->fiber) && !(ncand > 1 && cands[ncand - 2] == h->fiber))) cands[ncand++] = h->fiber;
     if (pref == 2 || (pref == 0 && h->slot)) cands[ncand++] = h->slot;
     TrajPlan *plan = nullptr;

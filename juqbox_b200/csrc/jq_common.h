@@ -118,7 +118,7 @@ struct HostOps {
 struct TrajPlan;   // opaque, built at jq_create; nullptr + reason when the problem shape has no instantiation
 TrajPlan *jq_slot_plan_create(const DevProblem &Pdev, const HostOps &H, const double *wdiag_host, char *err, size_t errlen);
 TrajPlan *jq_fiber_plan_create(const DevProblem &Pdev, const HostOps &H, const double *wdiag_host, char *err, size_t errlen, int pipe = 0);
-TrajPlan *jq_tile_plan_create(const DevProblem &Pdev, const HostOps &H, const double *wdiag_host, int NT, char *err, size_t errlen, int pipe = 0);
+TrajPlan *jq_tile_plan_create(const DevProblem &Pdev, const HostOps &H, const double *wdiag_host, int NT, int NF, char *err, size_t errlen, int pipe = 0);
 void jq_traj_plan_destroy(TrajPlan *);
 int jq_traj_plan_kind(const TrajPlan *);
 int jq_traj_plan_tpc(const TrajPlan *);      // trajectories per CTA

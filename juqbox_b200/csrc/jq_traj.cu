@@ -22,7 +22,7 @@ const Inst *find_inst(const InstKey &want, int J) {
                 const InstKey &k = i->key;
                 if (k.kind == want.kind && k.R == want.R && k.C == want.C && k.NC == want.NC && k.WQ == want.WQ && k.LMASK == want.LMASK &&
                     k.UPL == want.UPL && k.obj2 == want.obj2 && k.jacobi == want.jacobi && k.hx == want.hx &&
-                    k.general_hanti == want.general_hanti && k.jt == jt && (k.glt == 0 || k.glt == want.glt) &&
+                    k.general_hanti == want.general_hanti && k.NF == want.NF && k.jt == jt && (k.glt == 0 || k.glt == want.glt) &&
                     (want.nw == 0 || k.nw == want.nw) && (k.pipe != 0) == (want.pipe != 0) && k.seg == want.seg) return i;
             }
     return nullptr;
@@ -299,14 +299,14 @@ TrajPlan *jq_fiber_plan_create(const DevProblem &P, const HostOps &H, const doub
 
 
 // Tile layout: every subsystem has 4 levels, control q is the ladder pair (a_q + a_q', a_q - a_q') of subsystem q (row stride
-// 4^q), Hconst diagonal.  NT tiled directions cut in mirrored halves, the others remote (see TileLane).
-TrajPlan *jq_tile_plan_create(const DevProblem &P, const HostOps &H, const double *wdiag, int NT, char *err, size_t errlen, int pipe) {
+// 4^q), Hconst diagonal.  NF in-lane directions, then NT tiled directions cut in mirrored halves, the others remote (see TileLane).
+TrajPlan *jq_tile_plan_create(const DevProblem &P, const HostOps &H, const double *wdiag, int NT, int NF, char *err, size_t errlen, int pipe) {
     const int n = H.n, m = H.m, Nc = H.Nc;
     auto no = [&](const char *why) { snprintf(err, errlen, "%s", why); return (TrajPlan *)nullptr; };
     if (P.wreal || P.any_unc) return no("dense forbidden-state weights / uncoupled controls run on the generic kernel");
     if (P.solver != 1 || P.objFuncType != 1) return no("tile layout: only objFuncType 1 with the Neumann solver is instantiated");
     if (Nc < 2 || Nc > 3) return no("tile layout: 2 or 3 controls");
-    if (NT < 0 || NT > Nc) return no("tile layout: bad number of tiled directions");
+    if (NT < 0 || NF < 0 || NF + NT > Nc) return no("tile layout: bad number of in-lane / tiled directions");
     int n4 = 1;
     for (int q = 0; q < Nc; ++q) n4 *= 4;
     if (n != n4) return no("tile layout: every subsystem must have 4 levels");
@@ -334,7 +334,7 @@ TrajPlan *jq_tile_plan_create(const DevProblem &P, const HostOps &H, const doubl
         }
     }
     int NL = 1 << NT;
-    for (int q = NT; q < Nc; ++q) NL *= 4;
+    for (int q = NF + NT; q < Nc; ++q) NL *= 4;
     const int GL = pow2ceil(NL * m) > 32 ? 32 : pow2ceil(NL * m);
     if (NL > 32) return no("tile layout: more than 32 lanes per column");
     const int CPG = GL / NL, GPT = (m + CPG - 1) / CPG;
@@ -343,6 +343,7 @@ TrajPlan *jq_tile_plan_create(const DevProblem &P, const HostOps &H, const doubl
     const int nwp = pipe ? (GPT * GL + 31) / 32 : 0;
     InstKey key{4, NT, 1, Nc, 0, 0, UPL};
     key.glt = GL; key.nw = nwp; key.pipe = pipe ? 1 : 0;      // nw = 0: the 4 x 4 x 4 tiles run 8 warps per CTA
+    key.NF = NF;
     if (!find_inst(query(key, P), P.J)) return no("tile layout: no instantiation");
     TrajPlan *pl = new TrajPlan();
     pl->key = key;
@@ -352,20 +353,23 @@ TrajPlan *jq_tile_plan_create(const DevProblem &P, const HostOps &H, const doubl
     pl->exch_per_unit = 0;                         // shuffles only
     if (pipe) { pl->ngroups = nwp * (32 / GL); pl->TPC = pl->ngroups / GPT; }
     if (pl->TPC < 1) { delete pl; return no("a trajectory does not fit in one CTA"); }
-    const int nrem = Nc - NT, per = 3 * NT + 2 * nrem;
+    const int nrem = Nc - NF - NT, per = 3 * NF + 3 * NT + 2 * nrem;
     std::vector<int> pi((size_t)NL * (nrem > 0 ? nrem : 1) * 2, 0);
     std::vector<double> pd((size_t)NL * per, 0.0), d0p(n), wp(n);
     for (int r = 0; r < n; ++r) { d0p[r] = d0[r]; wp[r] = wdiag[r]; }
     for (int rho = 0; rho < NL; ++rho) {
         double *c = pd.data() + (size_t)rho * per;
+        for (int d = 0; d < NF; ++d)
+            for (int l = 0; l < 3; ++l) c[3 * d + l] = sq[d * 3 + l];
+        c += 3 * NF;
         for (int d = 0; d < NT; ++d) {
-            const int hb = (rho >> d) & 1;
-            c[3 * d] = sq[d * 3 + (hb ? 2 : 0)];
-            c[3 * d + 1] = sq[d * 3 + 1];
+            const int hb = (rho >> d) & 1, q = NF + d;
+            c[3 * d] = sq[q * 3 + (hb ? 2 : 0)];
+            c[3 * d + 1] = sq[q * 3 + 1];
             c[3 * d + 2] = hb ? -1.0 : 1.0;
         }
         for (int r = 0, gs = 1; r < nrem; ++r, gs *= 4) {
-            const int g = ((rho >> NT) / gs) % 4, q = NT + r;
+            const int g = ((rho >> NT) / gs) % 4, q = NF + NT + r;
             if (g > 0) { pi[((size_t)rho * nrem + r) * 2] = -(gs << NT); c[3 * NT + 2 * r] = sq[q * 3 + g - 1]; }
             if (g < 3) { pi[((size_t)rho * nrem + r) * 2 + 1] = gs << NT; c[3 * NT + 2 * r + 1] = sq[q * 3 + g]; }
         }
@@ -422,7 +426,7 @@ cudaError_t jq_traj_launch(TrajPlan *pl, const DevProblem &P, const LaunchArgs &
     int nw = inst->key.nw, TPC = 0, ngroups = 0;
     size_t bytes = 0;
     const int pipe = inst->key.pipe;
-    const int kind = pl->key.kind, Eper = kind == 4 ? (1 << pl->key.R) : kind == 3 ? pl->key.R : pl->key.R * pl->key.C;      // elements per lane
+    const int kind = pl->key.kind, Eper = kind == 4 ? (1 << (2 * pl->key.NF + pl->key.R)) : kind == 3 ? pl->key.R : pl->key.R * pl->key.C;      // elements per lane
     for (; nw >= 1; nw >>= 1) {
         ngroups = nw * S.GPW;
         TPC = ngroups / pl->GPT;

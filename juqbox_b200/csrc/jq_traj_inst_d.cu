@@ -3,6 +3,7 @@
 
 const Inst kInst[] = {
     traj_inst<TileLane<2, 2>, 1, 1, 4, 0, 16>(),            // cnot2 example shape: 4 x 4 levels, 2 x 2 tiles, J = 4, 16-lane groups (two trajectories per warp)
+    traj_inst<TileLane<2, 1, 1>, 1, 2, 4, 0, 8>(),          // the same, first subsystem whole in the lane: 8 elements per lane, 8-lane groups (four trajectories per warp)
     traj_inst<TileLane<2, 2>, 1>(),                          // 4 x 4 levels, run-time J and group size
     traj_inst<TileLane<3, 3>, 1, 1, 3, 0, 32, 8>(),         // cnot3 example shape: 4 x 4 x 4 levels, 2 x 2 x 2 tiles (one warp per trajectory), J = 3, 8 warps per CTA
     traj_inst<TileLane<3, 3>, 1, 1, 0, 0, 0, 8>(),          // 4 x 4 x 4 levels, run-time J and group size

@@ -66,7 +66,7 @@ typedef void (*traj_kernel_t)(const TrajParams);
 // What an instantiation of jq_traj_kernel computes and for which layout.  In a table entry every field follows from the template
 // arguments (traj_inst); a plan holds the key of its layout, and a query adds what the problem asks for (find_inst in jq_traj.cu).
 //   kind 2 slot, 3 fibre, 4 tile; R rows per lane (tile: tiled directions NT), C columns per lane, NC controls, WQ entries per row
-//   and control, LMASK controls coupling inside a fibre, UPL gradient-scatter roles per lane;
+//   and control, LMASK controls coupling inside a fibre, UPL gradient-scatter roles per lane, NF tile: in-lane directions;
 //   obj2 second adjoint set (objFuncType 2/3), jacobi Jacobi solver, hx exchange-coupled drift, general_hanti Hanti not of the
 //   ladder form (AS = 0);
 //   glt group size (entry: compile-time, 0 = any); jt Neumann terms compiled in (0 = run-time J; a query passes J instead);
@@ -76,6 +76,7 @@ struct InstKey {
     int kind, R, C, NC, WQ, LMASK, UPL;
     bool obj2 = false, jacobi = false, hx = false, general_hanti = false;
     int glt = 0, jt = 0, nw = TRAJ_WARPS, pipe = 0, seg = 0;
+    int NF = 0;
 };
 struct Inst { InstKey key; traj_kernel_t fn; };
 // The instantiation table is split over jq_traj.cu and the jq_traj_inst_*.cu files so that they compile in parallel.
@@ -145,7 +146,7 @@ struct Geo {
 
 template <int R_, int C_, int NC_, int WQ_>
 struct SlotLane {
-    static constexpr int KIND = 2, R = R_, C = C_, NC = NC_, WQ = WQ_, LMASK = 0, AS = 1, E = R_ * C_, HX = 0;
+    static constexpr int KIND = 2, R = R_, C = C_, NC = NC_, WQ = WQ_, LMASK = 0, AS = 1, E = R_ * C_, HX = 0, NF = 0;
     int pos[R][NC][WQ], own[R];
     double hs[R][NC][WQ], ha[R][NC][WQ];
     double d0[E], w[E];
@@ -253,7 +254,7 @@ struct SlotLane {
 // control q -- fibres every K-product fetches anyway.
 template <int R_, int NC_, int LMASK_, int AS_ = 1, int XM_ = 0, int HX_ = 0>
 struct FiberLane {
-    static constexpr int KIND = 3, R = R_, C = 1, NC = NC_, WQ = 2, LMASK = LMASK_, E = R_, AS = AS_, XM = XM_, HX = HX_;   // XM: 0 = shared-memory exchange, 1 = warp shuffles (16 instead of 24 data-pipe wavefronts per round for R = 4, NC = 2, but 16 instead of 7 instructions)
+    static constexpr int KIND = 3, R = R_, C = 1, NC = NC_, WQ = 2, LMASK = LMASK_, E = R_, AS = AS_, XM = XM_, HX = HX_, NF = 0;   // XM: 0 = shared-memory exchange, 1 = warp shuffles (16 instead of 24 data-pipe wavefronts per round for R = 4, NC = 2, but 16 instead of 7 instructions)
     static constexpr bool REMOTE = (LMASK_ != (1 << NC_) - 1);
     static constexpr int RM1 = R_ > 1 ? R_ - 1 : 1;
     // local (inside the fibre) tridiagonal coefficients: x_{k+1} -> row k ("u"), x_k -> row k+1 ("l")
@@ -421,24 +422,30 @@ struct FiberLane {
 
 
 // Tile layout (kernel id 4): Kronecker ladder Hamiltonians whose subsystems all have 4 levels (the cnot2 and cnot3 examples).
-// The first NT subsystems ("tiled directions", control q <-> direction q, row stride 4^q) are cut in HALVES: a lane owns
-// 2 of the 4 levels of every tiled direction, E = 2^NT elements, element e = sum_d i_d 2^d with i_d the position inside the
-// half.  The upper half keeps its levels in MIRRORED order (i = 0 -> level 3, i = 1 -> level 2; lower half i = 0 -> level 0,
-// i = 1 -> level 1), so in every lane i = 1 is the level at the interface and i = 0 the outer level: the code is uniform,
-// each lane has exactly ONE neighbour lane per tiled direction (lane ^ 2^d) and needs only the interface face of its tile
-// (2^(NT-1) values) from it -- 4 doubles per product for the cnot2 shape where the fibre layout moves 8, and the in-lane
-// pair coupling needs no traffic at all.  Mirroring swaps "upper" and "lower" neighbour, i.e. flips the sign of the
-// antisymmetric product D = Hanti x of that direction; the sign sg[d] is folded into the lane's copy of q_d(t) (LOAD_LEVELS)
-// and applied to the lane's partial traces that contain D (dsign).  Controls NT..NC-1 are remote as in the fibre layout
-// (a lane per level, lower and upper neighbour lane, lane-uniform coefficients).  Exchange is by warp shuffle only.
-// Requires Hanti = upper(Hsym) - lower(Hsym) and a diagonal Hconst (the planner checks).
-template <int NC_, int NT_>
+// Control q <-> direction q (row stride 4^q).  The first NF directions lie WHOLE in the lane ("in-lane directions": all 4
+// levels, a tridiagonal product with no traffic, coefficients the same in every lane).  The next NT ("tiled directions") are
+// cut in HALVES: a lane owns 2 of the 4 levels.  E = 4^NF 2^NT elements, element e = sum_{d<NF} l_d 4^d + 4^NF sum_d i_d 2^d
+// with l_d the level of in-lane direction d and i_d the position inside the half of tiled direction NF + d.  The upper half
+// keeps its levels in MIRRORED order (i = 0 -> level 3, i = 1 -> level 2; lower half i = 0 -> level 0, i = 1 -> level 1), so in
+// every lane i = 1 is the level at the interface and i = 0 the outer level: the code is uniform, each lane has exactly ONE
+// neighbour lane per tiled direction (lane ^ 2^d) and needs only the interface face of its tile (E/2 values) from it -- for
+// cnot2, 4 doubles per product for 4 elements (NF = 0, NT = 2) where the fibre layout moves 8, or 4 doubles for 8 elements
+// (NF = 1, NT = 1) -- and the in-lane pair coupling needs no traffic at all.  Mirroring swaps "upper" and "lower" neighbour,
+// i.e. flips the sign of the antisymmetric product D = Hanti x of that direction; the sign sg[d] is folded into the lane's copy
+// of q_d(t) (LOAD_LEVELS) and applied to the lane's partial traces that contain D (dsign); in-lane directions have none.
+// Controls NF+NT..NC-1 are remote as in the fibre layout (a lane per level, lower and upper neighbour lane, lane-uniform
+// coefficients).  Exchange is by warp shuffle only.  Requires Hanti = upper(Hsym) - lower(Hsym) and a diagonal Hconst (the
+// planner checks).
+template <int NC_, int NT_, int NF_ = 0>
 struct TileLane {
-    static constexpr int KIND = 4, NC = NC_, NT = NT_, E = 1 << NT_, HX = 0, R = NT_, C = 1, WQ = 0, LMASK = 0, AS = 1;
+    static constexpr int KIND = 4, NC = NC_, NT = NT_, NF = NF_, E = (1 << (2 * NF_)) << NT_, HX = 0, R = NT_, C = 1, WQ = 0, LMASK = 0, AS = 1;
     static constexpr bool SIGNED = true;
-    static constexpr int NT1 = NT_ > 0 ? NT_ : 1, EH = NT_ > 0 ? (1 << NT_) / 2 : 1;      // array extents (NT = 0: one element per lane, all directions remote)
+    static constexpr int HB = 2 * NF_;                  // bit of the element index where the tiled directions start
+    static constexpr int NT1 = NT_ > 0 ? NT_ : 1, EH = NT_ > 0 ? E / 2 : 1;      // array extents (NT = 0: no faces)
+    static constexpr int NF1 = NF_ > 0 ? NF_ : 1;
+    double cf[NF1][3];                       // in-lane ladder coefficients between levels l and l+1
     double cin[NT1], cx[NT1], sg[NT1];       // in-lane pair coupling, cross-lane (interface) coupling, mirror sign
-    static constexpr int NREM = NC_ > NT_ ? NC_ - NT_ : 1;
+    static constexpr int NRC = NC_ - NT_ - NF_, NREM = NRC > 0 ? NRC : 1;
     int rpos[NREM][2];
     double rhs[NREM][2];
     double d0[E], w[E];
@@ -450,64 +457,79 @@ struct TileLane {
         lane = g.lane;
         rho = g.lg % S.NL;
         colj = g.gi * S.CPG + g.lg / S.NL;
-        gdim = rho >> NT;                                  // level index of the remote directions (row offset 4^NT * gdim)
-        const double *pd = S.plan_d + rho * (3 * NT + 2 * (NC - NT));
+        gdim = rho >> NT;                                  // level index of the remote directions (row offset 4^(NF+NT) * gdim)
+        const double *pd = S.plan_d + rho * (3 * NF + 3 * NT + 2 * NRC);
+        UNROLL for (int d = 0; d < NF; ++d) UNROLL for (int l = 0; l < 3; ++l) cf[d][l] = pd[3 * d + l];
+        pd += 3 * NF;
         UNROLL for (int d = 0; d < NT; ++d) { cin[d] = pd[3 * d]; cx[d] = pd[3 * d + 1]; sg[d] = pd[3 * d + 2]; }
-        UNROLL for (int r = 0; r < NC - NT; ++r) {
+        UNROLL for (int r = 0; r < NRC; ++r) {
             UNROLL for (int e = 0; e < 2; ++e) {
-                rpos[r][e] = g.lane + S.plan_i[(rho * (NC - NT) + r) * 2 + e];
+                rpos[r][e] = g.lane + S.plan_i[(rho * NRC + r) * 2 + e];
                 rhs[r][e] = pd[3 * NT + 2 * r + e];
             }
         }
     }
     __device__ __forceinline__ int row(int e) const {
         int r = 0, st = 1;
+        UNROLL for (int d = 0; d < NF; ++d) { r += st * ((e >> (2 * d)) & 3); st *= 4; }
         UNROLL for (int d = 0; d < NT; ++d) {
-            const int i = (e >> d) & 1, hb = (rho >> d) & 1;
+            const int i = (e >> (HB + d)) & 1, hb = (rho >> d) & 1;
             r += st * (hb ? 3 - i : i);
             st *= 4;
         }
         return r + st * gdim;
     }
     __device__ __forceinline__ int col(int) const { return colj; }
-    __device__ __forceinline__ double dsign(int qq) const { return qq < NT ? sg[qq] : 1.0; }
+    __device__ __forceinline__ double dsign(int qq) const { return qq >= NF && qq < NF + NT ? sg[qq - NF] : 1.0; }
     __device__ __forceinline__ void sync_reset() {}
 
-    // index of element e inside the interface face of direction d (bit d removed)
-    static __device__ __forceinline__ constexpr int face(int e, int d) { return (e & ((1 << d) - 1)) | ((e >> (d + 1)) << d); }
+    // index of element e inside the interface face of tiled direction d (its bit removed)
+    static __device__ __forceinline__ constexpr int face(int e, int d) { return (e & ((1 << (HB + d)) - 1)) | ((e >> (HB + d + 1)) << (HB + d)); }
     struct Nbr { double t[NT1][EH]; double r[NREM][2][E]; };
     __device__ __forceinline__ void exchange(const double (&x)[E], Nbr &nb) const {
         UNROLL for (int d = 0; d < NT; ++d)
             UNROLL for (int e = 0; e < E; ++e)
-                if ((e >> d) & 1) nb.t[d][face(e, d)] = __shfl_xor_sync(0xffffffffu, x[e], 1 << d);
-        UNROLL for (int r = 0; r < NC - NT; ++r)
+                if ((e >> (HB + d)) & 1) nb.t[d][face(e, d)] = __shfl_xor_sync(0xffffffffu, x[e], 1 << d);
+        UNROLL for (int r = 0; r < NRC; ++r)
             UNROLL for (int e = 0; e < E; ++e) {
                 nb.r[r][0][e] = __shfl_sync(0xffffffffu, x[e], rpos[r][0]);
                 nb.r[r][1][e] = __shfl_sync(0xffffffffu, x[e], rpos[r][1]);
             }
     }
 
-    struct SC { double a[NT1], b[NT1], r[NREM][2]; };
+    struct SC { double f[NF1][3], a[NT1], b[NT1], r[NREM][2]; };
     __device__ __forceinline__ void s_prescale(int level, SC &sc) const {          // q[level] already carries sg
-        UNROLL for (int d = 0; d < NT; ++d) { sc.a[d] = q[level][d] * cin[d]; sc.b[d] = q[level][d] * cx[d]; }
-        UNROLL for (int r = 0; r < NC - NT; ++r) { sc.r[r][0] = -q[level][NT + r] * rhs[r][0]; sc.r[r][1] = q[level][NT + r] * rhs[r][1]; }
+        UNROLL for (int d = 0; d < NF; ++d) UNROLL for (int l = 0; l < 3; ++l) sc.f[d][l] = q[level][d] * cf[d][l];
+        UNROLL for (int d = 0; d < NT; ++d) { sc.a[d] = q[level][NF + d] * cin[d]; sc.b[d] = q[level][NF + d] * cx[d]; }
+        UNROLL for (int r = 0; r < NRC; ++r) { sc.r[r][0] = -q[level][NF + NT + r] * rhs[r][0]; sc.r[r][1] = q[level][NF + NT + r] * rhs[r][1]; }
     }
     __device__ __forceinline__ void s_scale(SC &sc, double f) const {
+        UNROLL for (int d = 0; d < NF; ++d) UNROLL for (int l = 0; l < 3; ++l) sc.f[d][l] *= f;
         UNROLL for (int d = 0; d < NT; ++d) { sc.a[d] *= f; sc.b[d] *= f; }
-        UNROLL for (int r = 0; r < NC - NT; ++r) { sc.r[r][0] *= f; sc.r[r][1] *= f; }
+        UNROLL for (int r = 0; r < NRC; ++r) { sc.r[r][0] *= f; sc.r[r][1] *= f; }
     }
     template <bool ADD>
     __device__ __forceinline__ void s_from(const SC &sc, const double (&x)[E], const Nbr &nb, const double (&add)[E], double (&t)[E]) const {
-        if constexpr (NT == 0) { UNROLL for (int e = 0; e < E; ++e) t[e] = ADD ? add[e] : 0.0; }
-        UNROLL for (int d = 0; d < NT; ++d)                // in-lane pair couplings first: independent of the exchange;
-            UNROLL for (int e = 0; e < E; ++e) {           // direction outer / element inner: neighbouring FMAs share the coefficient register
-                const double c = ((e >> d) & 1) ? -sc.a[d] : sc.a[d];
-                t[e] = d == 0 ? (ADD ? fma(c, x[e ^ 1], add[e]) : c * x[e ^ 1]) : fma(c, x[e ^ (1 << d)], t[e]);
+        if constexpr (NT == 0 && NF == 0) { UNROLL for (int e = 0; e < E; ++e) t[e] = ADD ? add[e] : 0.0; }
+        // in-lane products first (independent of the exchange), direction outer / element inner: neighbouring FMAs share the
+        // coefficient register.  In-lane directions: (S x)_l = c_l x_{l+1} - c_{l-1} x_{l-1}; the first term met starts the sum.
+        UNROLL for (int d = 0; d < NF; ++d)
+            UNROLL for (int e = 0; e < E; ++e) {
+                const int l = (e >> (2 * d)) & 3, st = 1 << (2 * d);
+                if (l < 3) t[e] = d == 0 ? (ADD ? fma(sc.f[d][l], x[e + st], add[e]) : sc.f[d][l] * x[e + st]) : fma(sc.f[d][l], x[e + st], t[e]);
+                if (l > 0) t[e] = d == 0 && l == 3 ? (ADD ? fma(-sc.f[d][2], x[e - st], add[e]) : -sc.f[d][2] * x[e - st])
+                                                   : fma(-sc.f[d][l - 1], x[e - st], t[e]);
+            }
+        UNROLL for (int d = 0; d < NT; ++d)
+            UNROLL for (int e = 0; e < E; ++e) {
+                const double c = ((e >> (HB + d)) & 1) ? -sc.a[d] : sc.a[d];
+                const int en = e ^ (1 << (HB + d));
+                t[e] = NF == 0 && d == 0 ? (ADD ? fma(c, x[en], add[e]) : c * x[en]) : fma(c, x[en], t[e]);
             }
         UNROLL for (int d = 0; d < NT; ++d)
             UNROLL for (int e = 0; e < E; ++e)
-                if ((e >> d) & 1) t[e] = fma(sc.b[d], nb.t[d][face(e, d)], t[e]);
-        UNROLL for (int r = 0; r < NC - NT; ++r)
+                if ((e >> (HB + d)) & 1) t[e] = fma(sc.b[d], nb.t[d][face(e, d)], t[e]);
+        UNROLL for (int r = 0; r < NRC; ++r)
             UNROLL for (int e = 0; e < E; ++e) t[e] = fma(sc.r[r][1], nb.r[r][1][e], fma(sc.r[r][0], nb.r[r][0][e], t[e]));
     }
     __device__ __forceinline__ void s_pass(const SC &sc, const double (&x)[E], double (&t)[E]) {
@@ -526,18 +548,24 @@ struct TileLane {
         UNROLL for (int e = 0; e < E; ++e) {
             double Ae[NC + 1], De[NC];
             Ae[NC] = 0.0;
+            UNROLL for (int d = 0; d < NF; ++d) {          // up = c_l x_{l+1}, lo = c_{l-1} x_{l-1}: A = up + lo, D = up - lo
+                const int l = (e >> (2 * d)) & 3, st = 1 << (2 * d);
+                if (l == 0) { const double up = cf[d][0] * x[e + st]; Ae[d] = up; De[d] = up; }
+                else if (l == 3) { const double lo = cf[d][2] * x[e - st]; Ae[d] = lo; De[d] = -lo; }
+                else { const double up = cf[d][l] * x[e + st], lo = cf[d][l - 1] * x[e - st]; Ae[d] = up + lo; De[d] = up - lo; }
+            }
             UNROLL for (int d = 0; d < NT; ++d) {
-                const double pin = cin[d] * x[e ^ (1 << d)];
-                if ((e >> d) & 1) {
+                const double pin = cin[d] * x[e ^ (1 << (HB + d))];
+                if ((e >> (HB + d)) & 1) {
                     const double xc = cx[d] * nb.t[d][face(e, d)];
-                    Ae[d] = xc + pin; De[d] = xc - pin;
+                    Ae[NF + d] = xc + pin; De[NF + d] = xc - pin;
                 } else {
-                    Ae[d] = pin; De[d] = pin;
+                    Ae[NF + d] = pin; De[NF + d] = pin;
                 }
             }
-            UNROLL for (int r = 0; r < NC - NT; ++r) {
+            UNROLL for (int r = 0; r < NRC; ++r) {
                 const double lo = rhs[r][0] * nb.r[r][0][e], up = rhs[r][1] * nb.r[r][1][e];
-                Ae[NT + r] = up + lo; De[NT + r] = up - lo;
+                Ae[NF + NT + r] = up + lo; De[NF + NT + r] = up - lo;
             }
             f(e, Ae, De);
         }
@@ -1375,7 +1403,7 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
 template <class LaneT, int UPL, int MINB = 1, int JT = 0, int OBJ = 0, int GLT = 0, int NW = TRAJ_WARPS, int PIPE = 0, bool SEG = false>
 constexpr Inst traj_inst() {
     return {{LaneT::KIND, LaneT::R, LaneT::C, LaneT::NC, LaneT::WQ, LaneT::LMASK, UPL, OBJ != 0, JT < 0, LaneT::HX != 0, !LaneT::AS,
-             GLT, JT > 0 ? JT : 0, NW, PIPE, SEG},
+             GLT, JT > 0 ? JT : 0, NW, PIPE, SEG, LaneT::NF},
             jq_traj_kernel<LaneT, UPL, MINB, JT, OBJ, GLT, NW, PIPE, SEG>};
 }
 }  // namespace
