@@ -12,6 +12,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <vector>
 
 static thread_local char g_err[512] = "";
@@ -46,6 +47,28 @@ struct NcclApi {
 static NcclApi g_nccl;
 static int load_nccl();
 
+struct PlanFree { void operator()(TrajPlan *p) const { jq_traj_plan_destroy(p); } };
+using PlanPtr = std::unique_ptr<TrajPlan, PlanFree>;
+
+// A way to serve a launch: a kernel (jq_set_kernel / jq_query(0) id) and, for the register-resident layouts, its plan (for the
+// time-parallel evaluation the plan of its segment sweeps).  Indices 0-6 are the routes of kernel ids 1-7; the in-lane tiles are a
+// second route of id 4.
+enum RouteId { GENERIC, SLOT, FIBER, TILE, LATENCY, DENSE, TIME_PARALLEL, TILE_INLANE, NROUTES };
+struct Route {
+    int kernel = 0;
+    TrajPlan *plan = nullptr;
+    bool ok = false;
+    char why[300] = "";     // !ok: why jq_set_kernel refuses the kernel id
+};
+
+// What the last evaluation ran (jq_query items 0 and 3-7)
+struct Ran {
+    int kernel = 0, ctas = 0, regs = 0, tpc = 1;
+    size_t smem = 0;
+    int nseg = 0;           // time segments (kernel 7)
+    int launches = 1;       // kernel launches of the trajectory work (the time-parallel evaluation makes several)
+};
+
 struct jq_handle {
     nccl_comm_t comm = nullptr;
     int comm_rank = 0, comm_size = 1;
@@ -63,22 +86,20 @@ struct jq_handle {
     // host copies of the row-wise operators (for the planners)
     std::vector<int> rowptr, col;
     std::vector<double> val;
-    TrajPlan *slot = nullptr, *fiber = nullptr, *tile = nullptr, *tile_lat = nullptr;     // tile_lat: fewest elements per lane (small batches)
-    TrajPlan *tile_in = nullptr;        // tile layout with the first subsystem whole in the lane (large batches; nullptr: none)
-    int tile_in_ntraj = 0;              // automatic mode: launches with at least this many trajectories use tile_in
-    bool dense_ok = false;              // the dense (FP64 MMA) kernel can serve this problem
-    bool dense_auto = false;            // ... and the operators are dense enough for it to beat the row-wise generic kernel
-    char dense_reason[128] = "";
+    std::vector<PlanPtr> plans;         // every trajectory plan; the routes and the roles below point into it
+    Route route[NROUTES];
+    int tile_in_ntraj = 0;              // automatic mode: launches with at least this many trajectories use the in-lane tiles
+    bool dense_auto = false;            // the dense kernel can serve this problem and the operators are dense enough for it to beat the
+                                        // row-wise generic kernel
     int lat_ntraj = 0;                  // automatic mode: launches with at most this many trajectories use the latency layout
-    // time-parallel evaluation (jq_seg.cu, kernel id 7): plan whose instantiations have segment sweeps (the non-pipelined latency
-    // tile layout, else the fibre plan -- then shared with `fiber`), workspace, segments (0 = automatic)
-    TrajPlan *seg_plan = nullptr, *seg_prop = nullptr, *seg_obj = nullptr;      // seg_prop: plan of the propagator launch (nullptr: seg_plan); seg_obj: of the gradient sweep for objFuncType 2/3
+    // time-parallel evaluation (jq_seg.cu, kernel id 7): its route's plan runs the segment sweeps (the tile layout with the fewest
+    // elements per lane, else the fibre plan); seg_prop: plan of the propagator launch; seg_obj: of the gradient sweep for
+    // objFuncType 2/3.  Workspace, segments (0 = automatic)
+    TrajPlan *seg_prop = nullptr, *seg_obj = nullptr;
     double *d_seg = nullptr; size_t cap_seg = 0;
     double *d_segt = nullptr; size_t cap_segt = 0; int segt_nseg = 0; std::vector<double> segt;
-    int seg_nseg = 0, seg_ntraj = 0, sms = 148, last_nseg = 0;
-    char slot_reason[256] = "", fiber_reason[256] = "", tile_reason[256] = "";
+    int seg_nseg = 0, seg_ntraj = 0, sms = 148;
     int kernel_pref = 0;
-    bool prefer_tile = true;            // automatic mode: tile layout before the fibre layout
     // growable scratch
     double *d_scal = nullptr, *d_grad = nullptr, *d_igrad = nullptr;
     size_t cap_traj = 0, cap_grad = 0, cap_igrad = 0;
@@ -89,8 +110,8 @@ struct jq_handle {
     std::vector<double> c_pcof, c_shift, c_w, c_igrad, c_lgrad;
     double c_infid = 0.0, c_leak = 0.0;
     // last-evaluation facts
-    int last_kernel = 0, last_launches = 0, last_ctas = 0, last_regs = 0, last_tpc = 1, last_traj_launches = 1;
-    size_t last_smem = 0;
+    Ran ran;
+    int last_launches = 0;              // every launch of the last entry (jq_query(2)): the trajectory work, reductions, all-reduce
     bool timed = false;
 };
 
@@ -345,65 +366,68 @@ extern "C" int jq_create(const jq_problem *pb, int device, jq_handle **out) {
         return fail(JQ_ERR_CUDA, "jq_create: stream/event creation failed");
     }
     HostOps H{n, m, Nc, pb->nfreq, h->rowptr.data(), h->col.data(), h->val.data()};
-    h->slot = jq_slot_plan_create(P, H, pb->wdiag, h->slot_reason, sizeof(h->slot_reason));
-    h->fiber = jq_fiber_plan_create(P, H, pb->wdiag, h->fiber_reason, sizeof(h->fiber_reason));
-    {
-        const char *nt = getenv("JQ_TILE_NT");      // development: number of tiled directions of the tile layout (default: all)
-        h->tile = jq_tile_plan_create(P, H, pb->wdiag, nt ? atoi(nt) : Nc, 0, h->tile_reason, sizeof(h->tile_reason));
-        char why[256];
-        // Two subsystems, first one whole in the lane (TileLane<2,1,1>): half the exchange shuffles per element of the 2 x 2 tiles
-        // and twice the independent element chains per lane, but 4 instead of 2 trajectories per warp
-        const char *ti = getenv("JQ_TILE_INLANE");      // development: 0 = never, 1 = for every launch, unset = automatic
-        if (h->tile && !nt && !(ti && atoi(ti) == 0)) h->tile_in = jq_tile_plan_create(P, H, pb->wdiag, 1, 1, why, sizeof(why));
-        // Latency layout: a trajectory spread over as many lanes as the warp-local exchange allows (one element per lane for two
-        // subsystems, two for three).  A lone evaluation (the reference's own call pattern, one pcof per Ipopt callback) is bound
-        // by the instruction stream of ONE lane, so fewer elements per lane is what shortens it; throughput layouts win once the
-        // SMs are full.
-        const char *lnt = getenv("JQ_TILE_LAT_NT");
-        const char *lp = getenv("JQ_LAT_PIPE");        // development: 0 = latency layout without the pipelined roles
-        const int pipe = lp ? atoi(lp) : 1;
-        h->tile_lat = jq_tile_plan_create(P, H, pb->wdiag, lnt ? atoi(lnt) : (Nc == 2 ? 0 : 1), 0, why, sizeof(why), pipe);
-        if (!h->tile_lat && pipe) h->tile_lat = jq_fiber_plan_create(P, H, pb->wdiag, why, sizeof(why), 1);     // single-fibre shapes: same layout, pipelined roles
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-        const char *lt = getenv("JQ_LAT_NTRAJ");
-        // one latency CTA per SM: beyond that the throughput layouts win (measured)
-        h->dense_ok = jq_dense_supported(P, h->dense_reason, sizeof(h->dense_reason));
-        // a dense contraction executes n^2 multiply-adds per product and column whatever the sparsity: worth it from ~20% fill
-        // (measured: 5%-filled ladder operators with remote exchange run 1.6x faster on the row-wise generic kernel)
-        size_t nnz = 0;
-        for (double v : h->val) nnz += v != 0.0;
-        h->dense_auto = h->dense_ok && n >= 8 && (double)nnz >= 0.2 * (double)(1 + 2 * Nc) * n * n;
-        h->lat_ntraj = lt ? atoi(lt) : sms * (h->tile_lat ? jq_traj_plan_tpc(h->tile_lat) : 1);
-        // in-lane tiles from one full resident wave of them (2 CTAs of 16 trajectories per SM, 4736 on 148 SMs): below it their
-        // CTAs leave SMs half empty where the 2 x 2 tiles (wave 2368) fill them.  Measured cnot2 speed-up over the 2 x 2 tiles (B200,
-        // 1000 W; profiles/r03_tile_inlane.md): 0.88x at 2368 and 0.85x at 3552 candidates; 1.09x at 4736, 1.06x at 7104, 1.10x at
-        // 9472 and 16384, 1.12x at 32768.
-        if (h->tile_in) h->tile_in_ntraj = ti && atoi(ti) == 1 ? 0 : 2 * sms * jq_traj_plan_tpc(h->tile_in);
-        // Time-parallel evaluation for launches of very few trajectories (one pcof per Ipopt callback): segments of the time axis
-        // swept concurrently and joined through their propagators
-        h->sms = sms;
-        h->seg_plan = jq_tile_plan_create(P, H, pb->wdiag, Nc == 2 ? 0 : 1, 0, why, sizeof(why), 0);
-        if (!h->seg_plan) h->seg_plan = h->fiber;
-        if (h->seg_plan && !jq_seg_supported(h->seg_plan, P)) { if (h->seg_plan != h->fiber) jq_traj_plan_destroy(h->seg_plan); h->seg_plan = nullptr; }
-        // objFuncType 2/3: the gradient sweep needs the second adjoint set, which the fibre layout has
-        if (h->seg_plan && P.objFuncType != 1) {
-            if (h->fiber && jq_seg_supported(h->fiber, P, true)) h->seg_obj = h->fiber;
-            else { if (h->seg_plan != h->fiber) jq_traj_plan_destroy(h->seg_plan); h->seg_plan = nullptr; }
-        }
+    auto own = [h](TrajPlan *p) { if (p) h->plans.emplace_back(p); return p; };
+    auto set_route = [h](RouteId id, int kernel, TrajPlan *plan, bool ok, const char *missing, const char *reason) {
+        Route &r = h->route[id];
+        r.kernel = kernel; r.plan = plan; r.ok = ok;
+        if (!ok) snprintf(r.why, sizeof(r.why), reason ? "%s (%s)" : "%s", missing, reason);
+    };
+    char why[256];
+    set_route(GENERIC, 1, nullptr, true, "", nullptr);
+    TrajPlan *slot = own(jq_slot_plan_create(P, H, pb->wdiag, why, sizeof(why)));
+    set_route(SLOT, 2, slot, slot, "no slot-layout instantiation for this problem", why);
+    TrajPlan *fiber = own(jq_fiber_plan_create(P, H, pb->wdiag, why, sizeof(why)));
+    set_route(FIBER, 3, fiber, fiber, "no fibre-layout instantiation for this problem", why);
+    TrajPlan *tile = own(jq_tile_plan_create(P, H, pb->wdiag, Nc, 0, why, sizeof(why)));
+    set_route(TILE, 4, tile, tile, "no tile-layout instantiation for this problem", why);
+    // Two subsystems, first one whole in the lane (TileLane<2,1,1>): half the exchange shuffles per element of the 2 x 2 tiles
+    // and twice the independent element chains per lane, but 4 instead of 2 trajectories per warp
+    const char *ti = getenv("JQ_TILE_INLANE");      // development: 0 = never, 1 = for every launch, unset = automatic
+    TrajPlan *tile_in = tile && !(ti && atoi(ti) == 0) ? own(jq_tile_plan_create(P, H, pb->wdiag, 1, 1, why, sizeof(why))) : nullptr;
+    set_route(TILE_INLANE, 4, tile_in, tile_in, "no in-lane tile instantiation for this problem", nullptr);
+    // Latency layout: a trajectory spread over as many lanes as the warp-local exchange allows (one element per lane for two
+    // subsystems, two for three), with pipelined roles.  A lone evaluation (the reference's own call pattern, one pcof per Ipopt
+    // callback) is bound by the instruction stream of ONE lane, so fewer elements per lane is what shortens it; throughput layouts
+    // win once the SMs are full.
+    TrajPlan *lat = own(jq_tile_plan_create(P, H, pb->wdiag, Nc == 2 ? 0 : 1, 0, why, sizeof(why), 1));
+    if (!lat) lat = own(jq_fiber_plan_create(P, H, pb->wdiag, why, sizeof(why), 1));     // single-fibre shapes: same layout, pipelined roles
+    set_route(LATENCY, 5, lat, lat, "no latency layout for this problem", nullptr);
+    const bool dense_ok = jq_dense_supported(P, why, sizeof(why));
+    set_route(DENSE, 6, nullptr, dense_ok, "the dense (tensor-core) kernel cannot serve this problem", why);
+    // a dense contraction executes n^2 multiply-adds per product and column whatever the sparsity: worth it from ~20% fill
+    // (measured: 5%-filled ladder operators with remote exchange run 1.6x faster on the row-wise generic kernel)
+    size_t nnz = 0;
+    for (double v : h->val) nnz += v != 0.0;
+    h->dense_auto = dense_ok && n >= 8 && (double)nnz >= 0.2 * (double)(1 + 2 * Nc) * n * n;
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    h->sms = sms;
+    // one latency CTA per SM: beyond that the throughput layouts win (measured)
+    h->lat_ntraj = sms * (lat ? jq_traj_plan_tpc(lat) : 1);
+    // in-lane tiles from one full resident wave of them (2 CTAs of 16 trajectories per SM, 4736 on 148 SMs): below it their
+    // CTAs leave SMs half empty where the 2 x 2 tiles (wave 2368) fill them.  Measured cnot2 speed-up over the 2 x 2 tiles (B200,
+    // 1000 W; profiles/r03_tile_inlane.md): 0.88x at 2368 and 0.85x at 3552 candidates; 1.09x at 4736, 1.06x at 7104, 1.10x at
+    // 9472 and 16384, 1.12x at 32768.
+    if (tile_in) h->tile_in_ntraj = ti && atoi(ti) == 1 ? 0 : 2 * sms * jq_traj_plan_tpc(tile_in);
+    // Time-parallel evaluation for launches of very few trajectories (one pcof per Ipopt callback): segments of the time axis
+    // swept concurrently and joined through their propagators.  The segment sweeps run on the tile layout with the fewest elements
+    // per lane, else on the fibre plan; objFuncType 2/3: the gradient sweep needs the second adjoint set, which the fibre layout has
+    TrajPlan *seg = own(jq_tile_plan_create(P, H, pb->wdiag, Nc == 2 ? 0 : 1, 0, why, sizeof(why), 0, true));
+    if (!seg) seg = fiber;
+    if (!jq_seg_supported(seg, P) || (P.objFuncType != 1 && !jq_seg_supported(fiber, P, true))) seg = nullptr;
+    set_route(TIME_PARALLEL, 7, seg, seg,
+              "no time-parallel evaluation for this problem (needs a tile / fibre layout, the Neumann solver, diagonal weights)", nullptr);
+    if (seg) {
+        h->seg_obj = P.objFuncType != 1 ? fiber : nullptr;
         // propagator launch (many independent unit-vector sweeps): the throughput tile layout when the problem has one
-        const char *pe = getenv("JQ_SEG_PROP_TILE");
-        if (h->seg_plan && h->tile && jq_seg_supported(h->tile, P) && (pe ? atoi(pe) != 0 : true)) h->seg_prop = h->tile;
-        // automatic mode: time-parallel while the propagator launch (2 x 2n/m unit-vector sweeps per trajectory and segment) stays within
-        // about four warps per SM -- measured cross-overs against the other kernels: cnot2 ~60 candidates, cnot3 ~30, risk-neutral ~1100
-        // samples (profiles/r02_timeparallel.md)
-        const char *sn = getenv("JQ_SEG_NTRAJ");
-        if (h->seg_plan) {
-            const int lanes = std::max(1, jq_traj_plan_lanes(h->seg_prop ? h->seg_prop : h->seg_plan)), nblk = (2 * n + m - 1) / m;
-            h->seg_ntraj = std::max(1, (4 * sms * 32) / (2 * nblk * lanes));
-        }
-        if (sn) h->seg_ntraj = atoi(sn);
+        h->seg_prop = jq_seg_supported(tile, P) ? tile : seg;
+        // automatic mode: time-parallel while the propagator launch (2 x 2n/m unit-vector sweeps per trajectory and segment) stays
+        // within about four warps per SM -- measured cross-overs against the other kernels: cnot2 ~60 candidates, cnot3 ~30,
+        // risk-neutral ~1100 samples (profiles/r02_timeparallel.md)
+        const int lanes = std::max(1, jq_traj_plan_lanes(h->seg_prop)), nblk = (2 * n + m - 1) / m;
+        h->seg_ntraj = std::max(1, (4 * sms * 32) / (2 * nblk * lanes));
     }
+    if (const char *sn = getenv("JQ_SEG_NTRAJ")) h->seg_ntraj = atoi(sn);
     *out = h;
     return 0;
 }
@@ -415,12 +439,7 @@ extern "C" int jq_destroy(jq_handle *h) {
     if (h->comm && g_nccl.ok) { g_nccl.CommDestroy(h->comm); h->comm = nullptr; }
     for (void *p : h->owned) cudaFree(p);
     for (double *p : {h->d_scal, h->d_grad, h->d_igrad, h->d_in, h->d_out}) if (p) cudaFree(p);
-    if (h->slot) jq_traj_plan_destroy(h->slot);
-    if (h->tile) jq_traj_plan_destroy(h->tile);
-    if (h->tile_lat) jq_traj_plan_destroy(h->tile_lat);
-    if (h->tile_in) jq_traj_plan_destroy(h->tile_in);
-    if (h->seg_plan && h->seg_plan != h->fiber) jq_traj_plan_destroy(h->seg_plan);
-    if (h->fiber) jq_traj_plan_destroy(h->fiber);
+    h->plans.clear();
     if (h->d_seg) cudaFree(h->d_seg);
     if (h->d_segt) cudaFree(h->d_segt);
     if (h->ev0) cudaEventDestroy(h->ev0);
@@ -466,12 +485,7 @@ extern "C" int64_t jq_abi_info(int32_t what) {
 
 extern "C" int jq_set_kernel(jq_handle *h, int32_t kernel) {
     if (!h || kernel < 0 || kernel > 7) return fail(JQ_ERR_ARG, "jq_set_kernel: kernel must be 0 ... 7");
-    if (kernel == 7 && !h->seg_plan) return fail(JQ_ERR_ARG, "jq_set_kernel: no time-parallel evaluation for this problem (needs a tile / fibre layout, the Neumann solver, diagonal weights)");
-    if (kernel == 6 && !h->dense_ok) return fail(JQ_ERR_ARG, "jq_set_kernel: the dense (tensor-core) kernel cannot serve this problem (%s)", h->dense_reason);
-    if (kernel == 5 && !h->tile_lat) return fail(JQ_ERR_ARG, "jq_set_kernel: no latency layout for this problem");
-    if (kernel == 4 && !h->tile) return fail(JQ_ERR_ARG, "jq_set_kernel: no tile-layout instantiation for this problem (%s)", h->tile_reason);
-    if (kernel == 2 && !h->slot) return fail(JQ_ERR_ARG, "jq_set_kernel: no slot-layout instantiation for this problem (%s)", h->slot_reason);
-    if (kernel == 3 && !h->fiber) return fail(JQ_ERR_ARG, "jq_set_kernel: no fibre-layout instantiation for this problem (%s)", h->fiber_reason);
+    if (kernel > 0 && !h->route[kernel - 1].ok) return fail(JQ_ERR_ARG, "jq_set_kernel: %s", h->route[kernel - 1].why);
     h->kernel_pref = kernel;
     return 0;
 }
@@ -499,7 +513,7 @@ extern "C" int64_t jq_time_segments(double T, int64_t nsteps, int32_t nseg, doub
 extern "C" int jq_query(jq_handle *h, int32_t what, double *value) {
     if (!h || !value) return fail(JQ_ERR_ARG, "jq_query: null argument");
     switch (what) {
-    case 0: *value = h->last_kernel; break;
+    case 0: *value = h->ran.kernel; break;
     case 1: {
         if (!h->timed) return fail(JQ_ERR_ARG, "jq_query: no evaluation has run yet");
         CU(cudaEventSynchronize(h->ev1));
@@ -509,11 +523,11 @@ extern "C" int jq_query(jq_handle *h, int32_t what, double *value) {
         break;
     }
     case 2: *value = h->last_launches; break;
-    case 3: *value = h->last_tpc; break;
-    case 4: *value = h->last_ctas; break;
-    case 5: *value = h->last_regs; break;
-    case 6: *value = (double)h->last_smem; break;
-    case 7: *value = h->last_kernel == 7 ? h->last_nseg : 0; break;
+    case 3: *value = h->ran.tpc; break;
+    case 4: *value = h->ran.ctas; break;
+    case 5: *value = h->ran.regs; break;
+    case 6: *value = (double)h->ran.smem; break;
+    case 7: *value = h->ran.nseg; break;
     default: return fail(JQ_ERR_ARG, "jq_query: unknown item %d", what);
     }
     return 0;
@@ -598,95 +612,148 @@ __global__ void __launch_bounds__(32 * WS_LANES) jq_weighted_sum_kernel(int nsam
 }
 
 
-// Launch the trajectory kernel for `A`: the register-resident layouts in order of preference (tile, fibre, slot), then the
-// generic kernel.  In automatic mode a layout that cannot serve this launch (no instantiation for the variant, shared-memory
-// layout does not fit, out of launch resources) hands over to the next one; an explicitly requested kernel fails instead.
-static int launch_trajectories(jq_handle *h, const LaunchArgs &A, cudaStream_t st) {
-    TrajPlan *cands[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    int ncand = 0;
-    const int pref = h->kernel_pref;
-    const bool small = A.ntraj <= h->lat_ntraj;
-    if (pref == 5 || (pref == 0 && h->tile_lat && small)) cands[ncand++] = h->tile_lat;
-    if (pref == 0 && small && h->fiber && h->tile && h->Nc >= 3) cands[ncand++] = h->fiber;     // three subsystems: the fibre layout (4 elements per lane) before the 8-element tiles
-    if (pref == 4 || (pref == 0 && h->tile && h->prefer_tile)) {
-        if (h->tile_in && A.ntraj >= h->tile_in_ntraj) cands[ncand++] = h->tile_in;
-        cands[ncand++] = h->tile;
+// Per-candidate outputs of `ncol` columns (gradient entries or directions) and the three scalars of every trajectory: copies
+// (w == nullptr) or weighted sums over the samples, with jq_weighted_sum_kernel from 64 samples on.  The two kernels add in
+// different orders, so the rule that picks one fixes the bits of the sums.
+static void launch_finalize(int nbatch, int nsamples, int ncol, int objFuncType, int evaladjoint, const double *w, const double *scal,
+                            const double *gt, const double *igt, double *infid, double *leak, double *tinfid, double *grad,
+                            double *infidgrad, double *leakgrad, cudaStream_t st) {
+    if (w && nsamples >= 64) {
+        jq_weighted_sum_kernel<<<dim3(nbatch, (ncol + 3 + 31) / 32), 32 * WS_LANES, 0, st>>>(nsamples, ncol, objFuncType, evaladjoint, w, scal,
+                                          gt, igt, infid, leak, tinfid, grad, infidgrad, leakgrad);
+        return;
     }
-    if (pref == 3 || (pref == 0 && h->fiber && !(ncand && cands[ncand - 1] == h->fiber) && !(ncand > 1 && cands[ncand - 2] == h->fiber))) cands[ncand++] = h->fiber;
-    if (pref == 2 || (pref == 0 && h->slot)) cands[ncand++] = h->slot;
-    TrajPlan *plan = nullptr;
-    int ctas = 0, regs = 0, tpc = 1;
-    size_t smem = 0;
-    CU(cudaEventRecord(h->ev0, st));
+    const long long total = (long long)(w ? nbatch : nbatch * nsamples) * (ncol + 1);
+    const int fb = 256, fg = (int)std::min<long long>((total + fb - 1) / fb, 148 * 8);
+    jq_finalize_kernel<<<fg, fb, 0, st>>>(nbatch, nsamples, ncol, objFuncType, evaladjoint, w, scal, gt, igt, infid, leak, tinfid, grad,
+                                          infidgrad, leakgrad);
+}
+
+// The handle's scratch (d_scal, d_grad, d_igrad) is shared by every call: a call on a different stream than the previous one
+// (host-pointer entries = the handle's own stream, device entry = the caller's) first waits for that one to finish
+static int scratch_acquire(jq_handle *h, cudaStream_t st) {
+    if (h->have_last && h->last_stream != st) CU(cudaStreamWaitEvent(st, h->ev_done, 0));
+    return 0;
+}
+
+static int scratch_release(jq_handle *h, cudaStream_t st) {
+    CU(cudaEventRecord(h->ev_done, st));
+    h->last_stream = st; h->have_last = true;
+    return 0;
+}
+
+// Arguments of a launch over nbatch x nsamples trajectories.  npar is the caller's vector length: the spline coefficients, plus the
+// global phase as last entry for pFidType 3; gradients have the same length.
+static LaunchArgs launch_args(const jq_handle *h, int nbatch, int npar, int nsamples, const double *pcof, const double *shift) {
+    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
+    LaunchArgs A{};
+    A.ntraj = nbatch * nsamples; A.nsamples = nsamples; A.Npar = nspl; A.D1 = nspl / (2 * h->Nc * h->Nfreq);
+    A.pstride = npar; A.gstride = npar;
+    A.pcof = pcof; A.shift = shift; A.scal = h->d_scal;
+    return A;
+}
+
+// The routes a launch tries, in order.  An explicit preference has only its own routes; automatic mode lists every route that may
+// serve the launch, the fastest for its size first.
+static int launch_routes(const jq_handle *h, const LaunchArgs &A, int pref, const Route *out[NROUTES]) {
+    int n = 0;
+    auto add = [&](RouteId id) {
+        if (!h->route[id].ok) return;
+        for (int i = 0; i < n; ++i) if (out[i] == &h->route[id]) return;
+        out[n++] = &h->route[id];
+    };
+    auto tiles = [&]() { if (A.ntraj >= h->tile_in_ntraj) add(TILE_INLANE); add(TILE); };
+    if (pref == 4) tiles();
+    else if (pref > 0) add(RouteId(pref - 1));
+    if (pref != 0) return n;
     // very few trajectories: time-parallel evaluation (segments of the time axis swept concurrently)
-    const bool seg_able = h->seg_plan && h->P.solver == 1 && !A.hist_r;
-    if (pref == 7 || (pref == 0 && seg_able && A.ntraj <= h->seg_ntraj && h->P.nsteps >= 256)) {
-        if (!seg_able) return fail(JQ_ERR_ARG, "time-parallel evaluation: Neumann solver, no state history");
-        TrajPlan *prop = h->seg_prop ? h->seg_prop : h->seg_plan;
-        int nseg = h->seg_nseg > 0 ? h->seg_nseg : jq_seg_auto_segments(h->P, A.ntraj, A.evaladjoint, jq_traj_plan_tpc(prop), h->sms);
-        if (nseg > h->P.nsteps) nseg = (int)h->P.nsteps;
-        // cooperative evaluation: the segments are shared out evenly over the ranks (every rank computes the same nseg)
-        // ... when the propagator launch is at least two waves of CTAs: below that its collective costs more than it saves
-        const long long l1_ctas = 2LL * nseg * (((long long)((2 * h->n + h->m - 1) / h->m) * A.ntraj + jq_traj_plan_tpc(prop) - 1) / jq_traj_plan_tpc(prop));
-        const char *cf = getenv("JQ_SEG_COOP_FORCE");     // tests: share out small problems too
-        const bool coop_on = h->cooperative && h->comm && h->comm_size > 1 && h->P.nsteps >= h->comm_size &&
-                             (l1_ctas >= 2LL * h->sms || (cf && atoi(cf)));
-        if (coop_on) {
-            nseg = std::max(h->comm_size, (nseg + h->comm_size - 1) / h->comm_size * h->comm_size);
-            if (nseg > h->P.nsteps) nseg = (int)(h->P.nsteps / h->comm_size) * h->comm_size;       // >= comm_size by the test above
-        }
-        SegCoop coop{h->comm_rank, h->comm_size, seg_allgather, h};
-        int rc = grow(&h->d_seg, &h->cap_seg, jq_seg_workspace_doubles(h->P, A.ntraj, A.Npar, nseg, A.evaladjoint));
-        if (rc) return rc;
-        if (h->segt_nseg != nseg) {           // segment start / end times: host recurrence, once per segment count
-            h->segt.resize(2 * (size_t)nseg);
-            jq_seg_times(h->P, nseg, h->segt.data());
-            if ((rc = grow(&h->d_segt, &h->cap_segt, 2 * (size_t)nseg + 2)) != 0) return rc;      // times, then the four refinement flags
-            CU(cudaMemcpyAsync(h->d_segt, h->segt.data(), 2 * (size_t)nseg * sizeof(double), cudaMemcpyHostToDevice, st));
-            h->segt_nseg = nseg;
-        }
-        int nl = 0;
-        cudaError_t e = jq_seg_launch(h->seg_prop, h->seg_plan, h->seg_obj, h->P, A, nseg, h->d_segt, reinterpret_cast<int *>(h->d_segt + 2 * (size_t)nseg), h->d_seg, st, coop_on && nseg >= h->comm_size ? &coop : nullptr, &ctas, &regs, &smem, &tpc, &nl);
-        if (e == cudaSuccess) {
-            CU(cudaEventRecord(h->ev1, st));
-            h->timed = true;
-            h->last_kernel = 7; h->last_nseg = nseg; h->last_traj_launches = nl;
-            h->last_ctas = ctas; h->last_regs = regs; h->last_smem = smem; h->last_tpc = tpc;
-            return 0;
-        }
-        cudaGetLastError();
-        const bool soft = e == cudaErrorInvalidConfiguration || e == cudaErrorNotSupported || e == cudaErrorLaunchOutOfResources;
-        if (!soft || pref != 0) return fail(JQ_ERR_CUDA, "time-parallel evaluation failed: %s", cudaGetErrorString(e));
+    if (h->P.solver == 1 && !A.hist_r && A.ntraj <= h->seg_ntraj && h->P.nsteps >= 256) add(TIME_PARALLEL);
+    const bool small = A.ntraj <= h->lat_ntraj;
+    if (small) add(LATENCY);
+    if (small && h->route[TILE].ok && h->Nc >= 3) add(FIBER);     // three subsystems: the fibre layout (4 elements per lane) before the 8-element tiles
+    tiles();
+    add(FIBER);
+    add(SLOT);
+    // unstructured operators: the products are real contractions -> FP64 tensor-core kernel, samples of a candidate batched
+    if (h->dense_auto && !A.hist_r) add(DENSE);
+    add(GENERIC);
+    return n;
+}
+
+// Outcome of a route's launch: 0, HANDED_OVER for an error after which automatic mode tries the next route (the route cannot serve
+// this launch: no instantiation for the variant, shared-memory layout does not fit, out of launch resources), else the error
+static const int HANDED_OVER = 1;
+static int launched(cudaError_t e, bool hand_over, const char *what) {
+    if (e == cudaSuccess) return 0;
+    cudaGetLastError();                                   // clear the (non-sticky) launch error before trying the next route
+    const bool soft = e == cudaErrorInvalidConfiguration || e == cudaErrorNotSupported || e == cudaErrorLaunchOutOfResources;
+    return soft && hand_over ? HANDED_OVER : fail(JQ_ERR_CUDA, "%s failed: %s", what, cudaGetErrorString(e));
+}
+
+// The time-parallel evaluation of `A`
+static int launch_time_parallel(jq_handle *h, const LaunchArgs &A, cudaStream_t st, Ran &ran, bool hand_over) {
+    if (h->P.solver != 1 || A.hist_r) return fail(JQ_ERR_ARG, "time-parallel evaluation: Neumann solver, no state history");
+    const int tpc = jq_traj_plan_tpc(h->seg_prop);
+    int nseg = h->seg_nseg > 0 ? h->seg_nseg : jq_seg_auto_segments(h->P, A.ntraj, A.evaladjoint, tpc, h->sms);
+    if (nseg > h->P.nsteps) nseg = (int)h->P.nsteps;
+    // cooperative evaluation: the segments are shared out evenly over the ranks (every rank computes the same nseg)
+    // ... when the propagator launch is at least two waves of CTAs: below that its collective costs more than it saves
+    const long long l1_ctas = 2LL * nseg * (((long long)((2 * h->n + h->m - 1) / h->m) * A.ntraj + tpc - 1) / tpc);
+    const char *cf = getenv("JQ_SEG_COOP_FORCE");     // tests: share out small problems too
+    const bool coop_on = h->cooperative && h->comm && h->comm_size > 1 && h->P.nsteps >= h->comm_size &&
+                         (l1_ctas >= 2LL * h->sms || (cf && atoi(cf)));
+    if (coop_on) {
+        nseg = std::max(h->comm_size, (nseg + h->comm_size - 1) / h->comm_size * h->comm_size);
+        if (nseg > h->P.nsteps) nseg = (int)(h->P.nsteps / h->comm_size) * h->comm_size;       // >= comm_size by the test above
     }
-    h->last_traj_launches = 1;
-    for (int i = 0; i < ncand && !plan; ++i) {
-        cudaError_t e = jq_traj_launch(cands[i], h->P, A, st, &ctas, &regs, &smem, &tpc);
-        if (e == cudaSuccess) { plan = cands[i]; break; }
-        cudaGetLastError();                                   // clear the (non-sticky) launch error before trying the next kernel
-        const bool soft = e == cudaErrorInvalidConfiguration || e == cudaErrorNotSupported || e == cudaErrorLaunchOutOfResources;
-        if (!soft || pref != 0) return fail(JQ_ERR_CUDA, "trajectory kernel launch failed: %s", cudaGetErrorString(e));
+    SegCoop coop{h->comm_rank, h->comm_size, seg_allgather, h};
+    int rc = grow(&h->d_seg, &h->cap_seg, jq_seg_workspace_doubles(h->P, A.ntraj, A.Npar, nseg, A.evaladjoint));
+    if (rc) return rc;
+    if (h->segt_nseg != nseg) {           // segment start / end times: host recurrence, once per segment count
+        h->segt.resize(2 * (size_t)nseg);
+        jq_seg_times(h->P, nseg, h->segt.data());
+        if ((rc = grow(&h->d_segt, &h->cap_segt, 2 * (size_t)nseg + 2)) != 0) return rc;      // times, then the four refinement flags
+        CU(cudaMemcpyAsync(h->d_segt, h->segt.data(), 2 * (size_t)nseg * sizeof(double), cudaMemcpyHostToDevice, st));
+        h->segt_nseg = nseg;
     }
-    bool dense = false;
-    if (!plan && (pref == 6 || (pref == 0 && h->dense_auto && !A.hist_r))) {
-        // unstructured operators: the products are real contractions -> FP64 tensor-core kernel, samples of a candidate batched
-        cudaError_t e = jq_dense_launch(h->P, A, st, &ctas, &regs, &smem, &tpc);
-        if (e == cudaSuccess) dense = true;
-        else {
-            cudaGetLastError();
-            if (pref == 6) return fail(JQ_ERR_CUDA, "dense kernel launch failed: %s", cudaGetErrorString(e));
-        }
-    }
-    if (!plan && !dense) {
-        if (pref > 1) return fail(JQ_ERR_ARG, "requested kernel is not available for this problem");
+    ran.nseg = nseg;
+    return launched(jq_seg_launch(h->seg_prop, h->route[TIME_PARALLEL].plan, h->seg_obj, h->P, A, nseg, h->d_segt,
+                                  reinterpret_cast<int *>(h->d_segt + 2 * (size_t)nseg), h->d_seg, st, coop_on && nseg >= h->comm_size ? &coop : nullptr,
+                                  &ran.ctas, &ran.regs, &ran.smem, &ran.tpc, &ran.launches),
+                    hand_over, "time-parallel evaluation");
+}
+
+// Launch route `r` for `A`, recording what ran in `ran`
+static int launch_route(jq_handle *h, const Route &r, const LaunchArgs &A, cudaStream_t st, Ran &ran, bool hand_over) {
+    switch (r.kernel) {
+    case 7: return launch_time_parallel(h, A, st, ran, hand_over);
+    case 6: return launched(jq_dense_launch(h->P, A, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc), hand_over, "dense kernel launch");
+    case 1:
         if (jq_generic_smem_bytes(h->P, A.Npar) > 227 * 1024)
             return fail(JQ_ERR_ARG, "problem too large for the generic kernel's shared memory (n*m = %d)", h->n * h->m);
-        tpc = 1;
-        CU(jq_generic_launch(h->P, A, st, &ctas, &regs, &smem));
+        return launched(jq_generic_launch(h->P, A, st, &ran.ctas, &ran.regs, &ran.smem), hand_over, "generic kernel launch");
+    default: return launched(jq_traj_launch(r.plan, h->P, A, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc), hand_over, "trajectory kernel launch");
     }
+}
+
+// Launch the trajectory work for `A` on the first of its routes that serves it: automatic mode hands over to the next route, an
+// explicitly requested kernel fails instead.
+static int launch_trajectories(jq_handle *h, const LaunchArgs &A, cudaStream_t st) {
+    const int pref = h->kernel_pref;
+    const Route *routes[NROUTES];
+    const int n = launch_routes(h, A, pref, routes);
+    CU(cudaEventRecord(h->ev0, st));
+    Ran ran;
+    int rc = HANDED_OVER;
+    for (int i = 0; i < n && rc == HANDED_OVER; ++i) {
+        ran = Ran();
+        ran.kernel = routes[i]->kernel;
+        rc = launch_route(h, *routes[i], A, st, ran, pref == 0 && i + 1 < n);
+    }
+    if (rc) return rc;
     CU(cudaEventRecord(h->ev1, st));
     h->timed = true;
-    h->last_kernel = plan ? (plan == h->tile_lat ? 5 : jq_traj_plan_kind(plan)) : dense ? 6 : 1;
-    h->last_ctas = ctas; h->last_regs = regs; h->last_smem = smem; h->last_tpc = tpc;
+    h->ran = ran;
     return 0;
 }
 
@@ -716,33 +783,19 @@ extern "C" int jq_traceobjgrad_batch_device(jq_handle *h, int32_t nbatch, const 
     CU(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)cuda_stream;
     const size_t ntraj = (size_t)nbatch * nsamples;
-    // the handle's scratch (d_scal, d_grad, d_igrad) is shared by every call: a call on a different stream than the previous one
-    // (host-pointer entry = the handle's own stream, device entry = the caller's) first waits for that one to finish
-    if (h->have_last && h->last_stream != st) CU(cudaStreamWaitEvent(st, h->ev_done, 0));
+    if ((rc = scratch_acquire(h, st)) != 0) return rc;
     if ((rc = grow(&h->d_scal, &h->cap_traj, ntraj * 4)) != 0) return rc;
     if (evaladjoint && (rc = grow(&h->d_grad, &h->cap_grad, ntraj * npar)) != 0) return rc;
     if (evaladjoint && h->P.objFuncType != 1 && (rc = grow(&h->d_igrad, &h->cap_igrad, ntraj * npar)) != 0) return rc;
 
-    // npar is the caller's vector length: the spline coefficients, plus the global phase as last entry for pFidType 3; gradients
-    // have the same length, so the finalize kernels just see npar columns
-    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
-    LaunchArgs A{};
-    A.ntraj = (int)ntraj; A.nsamples = nsamples; A.Npar = nspl; A.D1 = nspl / (2 * h->Nc * h->Nfreq); A.evaladjoint = evaladjoint ? 1 : 0;
-    A.pstride = npar; A.gstride = npar;
-    A.pcof = pcof; A.shift = shift; A.scal = h->d_scal; A.grad = h->d_grad; A.infidgrad = h->P.objFuncType != 1 ? h->d_igrad : nullptr;
-
+    LaunchArgs A = launch_args(h, nbatch, npar, nsamples, pcof, shift);
+    A.evaladjoint = evaladjoint ? 1 : 0;
+    A.grad = h->d_grad; A.infidgrad = h->P.objFuncType != 1 ? h->d_igrad : nullptr;
     if (ntraj > 0 && (rc = launch_trajectories(h, A, st)) != 0) return rc;
-    const int nout = weights ? nbatch : (int)ntraj;
-    const long long total = (long long)nout * (npar + 1);
-    const int fb = 256, fg = (int)std::min<long long>((total + fb - 1) / fb, 148 * 8);
-    if (weights && nsamples >= 64)
-        jq_weighted_sum_kernel<<<dim3(nbatch, (npar + 3 + 31) / 32), 32 * WS_LANES, 0, st>>>(nsamples, npar, h->P.objFuncType, A.evaladjoint,
-                                          weights, h->d_scal, h->d_grad, h->d_igrad, infid, leak, trace_infid, grad, infidgrad, leakgrad);
-    else
-        jq_finalize_kernel<<<fg, fb, 0, st>>>(nbatch, nsamples, npar, h->P.objFuncType, A.evaladjoint, weights, h->d_scal, h->d_grad,
-                                              h->d_igrad, infid, leak, trace_infid, grad, infidgrad, leakgrad);
+    launch_finalize(nbatch, nsamples, npar, h->P.objFuncType, A.evaladjoint, weights, h->d_scal, h->d_grad, h->d_igrad, infid, leak,
+                    trace_infid, grad, infidgrad, leakgrad, st);
     CU(cudaGetLastError());
-    h->last_launches = 1 + h->last_traj_launches;
+    h->last_launches = 1 + h->ran.launches;
     if (h->comm && weights && h->comm_size > 1) {
         // the path's one exchange step: weighted sums over the sample shards of all ranks (sum, FP64), one grouped call
         const size_t nb = (size_t)nbatch, ng = (size_t)nbatch * npar;
@@ -760,9 +813,7 @@ extern "C" int jq_traceobjgrad_batch_device(jq_handle *h, int32_t nbatch, const 
         if (nrc != 0) return fail(JQ_ERR_CUDA, "ncclAllReduce of the weighted sample sums: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(nrc) : "nccl error");
         h->last_launches += 1;
     }
-    CU(cudaEventRecord(h->ev_done, st));
-    h->last_stream = st; h->have_last = true;
-    return 0;
+    return scratch_release(h, st);
 }
 
 
@@ -880,11 +931,7 @@ extern "C" int jq_eval_forward(jq_handle *h, int32_t nbatch, const double *pcof,
     double *d_pcof = h->d_in, *d_shift = shift ? h->d_in + n_pcof : nullptr;
     CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
     if (shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
-    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
-    LaunchArgs A{};
-    A.ntraj = (int)ntraj; A.nsamples = nsamples; A.Npar = nspl; A.D1 = nspl / (2 * h->Nc * h->Nfreq); A.evaladjoint = 0;
-    A.pstride = npar; A.gstride = npar;
-    A.pcof = d_pcof; A.shift = d_shift; A.scal = h->d_scal; A.grad = nullptr; A.infidgrad = nullptr;
+    LaunchArgs A = launch_args(h, nbatch, npar, nsamples, d_pcof, d_shift);
     A.hist_r = h->d_out; A.hist_i = h->d_out + n_hist; A.save_every = save_every; A.nsave = nsave;
     if ((rc = launch_trajectories(h, A, st)) != 0) return rc;      // same kernel choice as jq_traceobjgrad_batch
     h->last_launches = 1;
@@ -971,7 +1018,7 @@ extern "C" int jq_forward_sensitivity(jq_handle *h, int32_t nbatch, const double
         return fail(JQ_ERR_ARG, "jq_forward_sensitivity: problem too large for the tangent kernel's shared memory (n*m = %d)", h->n * h->m);
     CU(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
-    if (h->have_last && h->last_stream != st) CU(cudaStreamWaitEvent(st, h->ev_done, 0));      // shared scratch, see jq_traceobjgrad_batch_device
+    if ((rc = scratch_acquire(h, st)) != 0) return rc;
     const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ndir, len = (size_t)h->n * h->m;
     const size_t nout = weights ? (size_t)nbatch : nt, ndout = nout * ndir;
     const size_t n_pcof = (size_t)nbatch * npar, n_dirs = (size_t)nbatch * ndir * npar;
@@ -996,28 +1043,19 @@ extern "C" int jq_forward_sensitivity(jq_handle *h, int32_t nbatch, const double
     S.ntraj = (int)ntraj; S.nsamples = nsamples; S.ndir = ndir; S.Npar = nspl; S.D1 = nspl / (2 * h->Nc * h->Nfreq); S.pstride = npar;
     S.pcof = d_pcof; S.dirs = d_dirs; S.shift = d_shift;
     S.scal = h->d_scal; S.dinfid = h->d_grad; S.dleak = h->d_igrad; S.dstate_r = o_sr; S.dstate_i = o_si;
-    int ctas = 0, regs = 0, gpc = 1;
-    size_t smem = 0;
+    Ran ran;
+    ran.kernel = 8;
     CU(cudaEventRecord(h->ev0, st));
-    CU(jq_fwdsens_launch(h->P, S, st, &ctas, &regs, &smem, &gpc));
+    CU(jq_fwdsens_launch(h->P, S, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc));
     CU(cudaEventRecord(h->ev1, st));
     h->timed = true;
-    h->last_kernel = 8; h->last_ctas = ctas; h->last_regs = regs; h->last_smem = smem; h->last_tpc = gpc; h->last_traj_launches = 1;
+    h->ran = ran;
     // per-trajectory outputs or the weighted sums over the samples, in the fixed order of the evaluation path's reductions: the
     // directions take the place of the gradient columns (dinfid as `grad`, dleak as `infidgrad`)
-    if (weights && nsamples >= 64)
-        jq_weighted_sum_kernel<<<dim3(nbatch, (ndir + 3 + 31) / 32), 32 * WS_LANES, 0, st>>>(nsamples, ndir, 2, 1, d_w, h->d_scal, h->d_grad,
-                                          h->d_igrad, o_infid, o_leak, nullptr, o_dinf, o_dleak, nullptr);
-    else {
-        const long long total = (long long)nout * (ndir + 1);
-        const int fb = 256, fg = (int)std::min<long long>((total + fb - 1) / fb, 148 * 8);
-        jq_finalize_kernel<<<fg, fb, 0, st>>>(nbatch, nsamples, ndir, 2, 1, d_w, h->d_scal, h->d_grad, h->d_igrad, o_infid, o_leak, nullptr,
-                                              o_dinf, o_dleak, nullptr);
-    }
+    launch_finalize(nbatch, nsamples, ndir, 2, 1, d_w, h->d_scal, h->d_grad, h->d_igrad, o_infid, o_leak, nullptr, o_dinf, o_dleak, nullptr, st);
     CU(cudaGetLastError());
     h->last_launches = 2;
-    CU(cudaEventRecord(h->ev_done, st));
-    h->last_stream = st; h->have_last = true;
+    if ((rc = scratch_release(h, st)) != 0) return rc;
     if (infid) CU(cudaMemcpyAsync(infid, o_infid, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (leak) CU(cudaMemcpyAsync(leak, o_leak, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (dinfid) CU(cudaMemcpyAsync(dinfid, o_dinf, ndout * sizeof(double), cudaMemcpyDeviceToHost, st));

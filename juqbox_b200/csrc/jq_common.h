@@ -118,9 +118,10 @@ struct HostOps {
 struct TrajPlan;   // opaque, built at jq_create; nullptr + reason when the problem shape has no instantiation
 TrajPlan *jq_slot_plan_create(const DevProblem &Pdev, const HostOps &H, const double *wdiag_host, char *err, size_t errlen);
 TrajPlan *jq_fiber_plan_create(const DevProblem &Pdev, const HostOps &H, const double *wdiag_host, char *err, size_t errlen, int pipe = 0);
-TrajPlan *jq_tile_plan_create(const DevProblem &Pdev, const HostOps &H, const double *wdiag_host, int NT, int NF, char *err, size_t errlen, int pipe = 0);
+// seg: a plan for the segment sweeps of the time-parallel evaluation only (it must have segment-sweep instantiations)
+TrajPlan *jq_tile_plan_create(const DevProblem &Pdev, const HostOps &H, const double *wdiag_host, int NT, int NF, char *err, size_t errlen, int pipe = 0,
+                              bool seg = false);
 void jq_traj_plan_destroy(TrajPlan *);
-int jq_traj_plan_kind(const TrajPlan *);
 int jq_traj_plan_tpc(const TrajPlan *);      // trajectories per CTA
 int jq_traj_plan_lanes(const TrajPlan *);    // lanes per trajectory
 cudaError_t jq_traj_launch(TrajPlan *plan, const DevProblem &P, const LaunchArgs &A, cudaStream_t st, int *nctas, int *regs,

@@ -300,7 +300,8 @@ TrajPlan *jq_fiber_plan_create(const DevProblem &P, const HostOps &H, const doub
 
 // Tile layout: every subsystem has 4 levels, control q is the ladder pair (a_q + a_q', a_q - a_q') of subsystem q (row stride
 // 4^q), Hconst diagonal.  NF in-lane directions, then NT tiled directions cut in mirrored halves, the others remote (see TileLane).
-TrajPlan *jq_tile_plan_create(const DevProblem &P, const HostOps &H, const double *wdiag, int NT, int NF, char *err, size_t errlen, int pipe) {
+TrajPlan *jq_tile_plan_create(const DevProblem &P, const HostOps &H, const double *wdiag, int NT, int NF, char *err, size_t errlen, int pipe,
+                              bool seg) {
     const int n = H.n, m = H.m, Nc = H.Nc;
     auto no = [&](const char *why) { snprintf(err, errlen, "%s", why); return (TrajPlan *)nullptr; };
     if (P.wreal || P.any_unc) return no("dense forbidden-state weights / uncoupled controls run on the generic kernel");
@@ -344,7 +345,9 @@ TrajPlan *jq_tile_plan_create(const DevProblem &P, const HostOps &H, const doubl
     InstKey key{4, NT, 1, Nc, 0, 0, UPL};
     key.glt = GL; key.nw = nwp; key.pipe = pipe ? 1 : 0;      // nw = 0: the 4 x 4 x 4 tiles run 8 warps per CTA
     key.NF = NF;
-    if (!find_inst(query(key, P), P.J)) return no("tile layout: no instantiation");
+    InstKey want = query(key, P);
+    want.seg = seg;
+    if (!find_inst(want, P.J)) return no("tile layout: no instantiation");
     TrajPlan *pl = new TrajPlan();
     pl->key = key;
     pl->NL = NL; pl->NLR = n; pl->GPT = GPT; pl->CPG = CPG;
@@ -395,7 +398,6 @@ bool jq_seg_supported(const TrajPlan *pl, const DevProblem &P, bool second_adjoi
     return find_inst(want, P.J) != nullptr;
 }
 
-int jq_traj_plan_kind(const TrajPlan *pl) { return pl ? pl->key.kind : 0; }
 int jq_traj_plan_tpc(const TrajPlan *pl) { return pl ? pl->TPC : 0; }
 int jq_traj_plan_lanes(const TrajPlan *pl) { return pl ? pl->GPT * pl->key.glt : 0; }
 

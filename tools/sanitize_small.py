@@ -74,7 +74,7 @@ pcs = np.concatenate([configs.synthetic_pcof(cfg, 4) * 20, np.linspace(-1, 1, 4)
 for k in (1, 3, 5):
     try:
         wa.set_kernel(k)
-    except Exception:      # JQ_LAT_PIPE=0: single-qudit shapes have no latency layout without the pipelined roles
+    except Exception:      # no instantiation of this layout for the shape
         continue
     wa.evaluate(pcs)
 wa.close()
