@@ -422,7 +422,7 @@ cudaError_t jq_traj_launch(TrajPlan *pl, const DevProblem &P, const LaunchArgs &
     S.exch_per_unit = pl->exch_per_unit;
     S.NparS = A.Npar | 1;
     S.GPW = 32 / pl->key.glt;
-    const int npts = 2 * TRAJ_CH + 1, NC = pl->key.NC;
+    const int npts = 2 * TRAJ_CH + 2, NC = pl->key.NC;     // control-table points per chunk, with fill_table's extra point
     // warps per CTA: 4 normally; fewer when the per-CTA gradient windows / pcof staging of very long coefficient
     // vectors would not fit in shared memory (the kernel only uses blockDim.x and the counts below)
     int nw = inst->key.nw, TPC = 0, ngroups = 0;

@@ -497,40 +497,60 @@ struct TileLane {
             }
     }
 
+    // Control-weighted neighbour coefficients of W x = sum_q wt_q (Hsym_q x) (symmetric form) or sum_q wt_q (Hanti_q x) (antisymmetric
+    // form, wt = q[level], which already carries sg).  The remote lower coefficients carry the sign of their form; the in-lane and pair
+    // terms get it in w_from.
     struct SC { double f[NF1][3], a[NT1], b[NT1], r[NREM][2]; };
-    __device__ __forceinline__ void s_prescale(int level, SC &sc) const {          // q[level] already carries sg
-        UNROLL for (int d = 0; d < NF; ++d) UNROLL for (int l = 0; l < 3; ++l) sc.f[d][l] = q[level][d] * cf[d][l];
-        UNROLL for (int d = 0; d < NT; ++d) { sc.a[d] = q[level][NF + d] * cin[d]; sc.b[d] = q[level][NF + d] * cx[d]; }
-        UNROLL for (int r = 0; r < NRC; ++r) { sc.r[r][0] = -q[level][NF + NT + r] * rhs[r][0]; sc.r[r][1] = q[level][NF + NT + r] * rhs[r][1]; }
+    template <bool ANTI>
+    __device__ __forceinline__ void w_prescale(const double (&wt)[NC], SC &sc) const {
+        UNROLL for (int d = 0; d < NF; ++d) UNROLL for (int l = 0; l < 3; ++l) sc.f[d][l] = wt[d] * cf[d][l];
+        UNROLL for (int d = 0; d < NT; ++d) { sc.a[d] = wt[NF + d] * cin[d]; sc.b[d] = wt[NF + d] * cx[d]; }
+        UNROLL for (int r = 0; r < NRC; ++r) { sc.r[r][0] = (ANTI ? -wt[NF + NT + r] : wt[NF + NT + r]) * rhs[r][0]; sc.r[r][1] = wt[NF + NT + r] * rhs[r][1]; }
     }
+    __device__ __forceinline__ void s_prescale(int level, SC &sc) const { w_prescale<true>(q[level], sc); }
     __device__ __forceinline__ void s_scale(SC &sc, double f) const {
         UNROLL for (int d = 0; d < NF; ++d) UNROLL for (int l = 0; l < 3; ++l) sc.f[d][l] *= f;
         UNROLL for (int d = 0; d < NT; ++d) { sc.a[d] *= f; sc.b[d] *= f; }
         UNROLL for (int r = 0; r < NRC; ++r) { sc.r[r][0] *= f; sc.r[r][1] *= f; }
     }
+    // t[o] = (bit o of ADDM: add) +- ((bit o of DIAG: d0.*x) + W_o x) for the N coefficient sets sc[o], all from one exchange; bit o
+    // of ANTI: W_o has the antisymmetric form, of NEG: the minus sign (it rides on the FMAs).  In-lane products first (independent of
+    // the exchange), direction outer / element inner: neighbouring FMAs share the coefficient register.  In-lane directions:
+    // (W x)_l = c_l x_{l+1} +- c_{l-1} x_{l-1}; without a diagonal or an addend the first term met starts the sum.
+    template <int N, unsigned ANTI, unsigned DIAG, unsigned ADDM, unsigned NEG = 0u>
+    __device__ __forceinline__ void w_from(const SC *sc, const double (&x)[E], const Nbr &nb, const double (&add)[E], double (*t)[E]) const {
+        UNROLL for (int o = 0; o < N; ++o) {
+            const bool an = (ANTI >> o) & 1, dg = (DIAG >> o) & 1, ad = (ADDM >> o) & 1, ng = (NEG >> o) & 1;
+            const bool open = !dg && !ad && (NF > 0 || NT > 0);      // the first neighbour term starts the sum
+            auto sgn = [ng](double c) { return ng ? -c : c; };
+            if (!open) { UNROLL for (int e = 0; e < E; ++e) t[o][e] = dg ? (ad ? fma(sgn(d0[e]), x[e], add[e]) : sgn(d0[e]) * x[e]) : (ad ? add[e] : 0.0); }
+            UNROLL for (int d = 0; d < NF; ++d)
+                UNROLL for (int e = 0; e < E; ++e) {
+                    const int l = (e >> (2 * d)) & 3, st = 1 << (2 * d);
+                    if (l < 3) { const double c = sgn(sc[o].f[d][l]); t[o][e] = open && d == 0 ? c * x[e + st] : fma(c, x[e + st], t[o][e]); }
+                    if (l > 0) {
+                        const double c = sgn(an ? -sc[o].f[d][l - 1] : sc[o].f[d][l - 1]);
+                        t[o][e] = open && d == 0 && l == 3 ? c * x[e - st] : fma(c, x[e - st], t[o][e]);
+                    }
+                }
+            UNROLL for (int d = 0; d < NT; ++d)
+                UNROLL for (int e = 0; e < E; ++e) {
+                    const double c = sgn(an && ((e >> (HB + d)) & 1) ? -sc[o].a[d] : sc[o].a[d]);
+                    const int en = e ^ (1 << (HB + d));
+                    t[o][e] = open && NF == 0 && d == 0 ? c * x[en] : fma(c, x[en], t[o][e]);
+                }
+            UNROLL for (int d = 0; d < NT; ++d)
+                UNROLL for (int e = 0; e < E; ++e)
+                    if ((e >> (HB + d)) & 1) t[o][e] = fma(sgn(sc[o].b[d]), nb.t[d][face(e, d)], t[o][e]);
+            UNROLL for (int r = 0; r < NRC; ++r)
+                UNROLL for (int e = 0; e < E; ++e)
+                    t[o][e] = fma(sgn(sc[o].r[r][1]), nb.r[r][1][e], fma(sgn(sc[o].r[r][0]), nb.r[r][0][e], t[o][e]));
+        }
+    }
+    // t = S x  (ADD: t = add + S x)
     template <bool ADD>
     __device__ __forceinline__ void s_from(const SC &sc, const double (&x)[E], const Nbr &nb, const double (&add)[E], double (&t)[E]) const {
-        if constexpr (NT == 0 && NF == 0) { UNROLL for (int e = 0; e < E; ++e) t[e] = ADD ? add[e] : 0.0; }
-        // in-lane products first (independent of the exchange), direction outer / element inner: neighbouring FMAs share the
-        // coefficient register.  In-lane directions: (S x)_l = c_l x_{l+1} - c_{l-1} x_{l-1}; the first term met starts the sum.
-        UNROLL for (int d = 0; d < NF; ++d)
-            UNROLL for (int e = 0; e < E; ++e) {
-                const int l = (e >> (2 * d)) & 3, st = 1 << (2 * d);
-                if (l < 3) t[e] = d == 0 ? (ADD ? fma(sc.f[d][l], x[e + st], add[e]) : sc.f[d][l] * x[e + st]) : fma(sc.f[d][l], x[e + st], t[e]);
-                if (l > 0) t[e] = d == 0 && l == 3 ? (ADD ? fma(-sc.f[d][2], x[e - st], add[e]) : -sc.f[d][2] * x[e - st])
-                                                   : fma(-sc.f[d][l - 1], x[e - st], t[e]);
-            }
-        UNROLL for (int d = 0; d < NT; ++d)
-            UNROLL for (int e = 0; e < E; ++e) {
-                const double c = ((e >> (HB + d)) & 1) ? -sc.a[d] : sc.a[d];
-                const int en = e ^ (1 << (HB + d));
-                t[e] = NF == 0 && d == 0 ? (ADD ? fma(c, x[en], add[e]) : c * x[en]) : fma(c, x[en], t[e]);
-            }
-        UNROLL for (int d = 0; d < NT; ++d)
-            UNROLL for (int e = 0; e < E; ++e)
-                if ((e >> (HB + d)) & 1) t[e] = fma(sc.b[d], nb.t[d][face(e, d)], t[e]);
-        UNROLL for (int r = 0; r < NRC; ++r)
-            UNROLL for (int e = 0; e < E; ++e) t[e] = fma(sc.r[r][1], nb.r[r][1][e], fma(sc.r[r][0], nb.r[r][0][e], t[e]));
+        w_from<1, 1u, 0u, ADD ? 1u : 0u>(&sc, x, nb, add, &t);
     }
     __device__ __forceinline__ void s_pass(const SC &sc, const double (&x)[E], double (&t)[E]) {
         Nbr nb;
@@ -581,6 +601,11 @@ struct TileLane {
 // Sign of the lane's antisymmetric products of control qq relative to Hanti_qq x (tile layout: mirrored halves); 1 elsewhere.
 template <class LaneT, class = void> struct LaneSigned : std::false_type {};
 template <class LaneT> struct LaneSigned<LaneT, std::enable_if_t<LaneT::SIGNED>> : std::true_type {};
+// Layouts with control-weighted neighbour products (w_prescale / w_from): the state steps weight the coefficients instead of forming
+// the per-control products A_q x, D_q x, which no trace of a state step reads.
+template <class LaneT, class = void> struct LaneWeighted : std::false_type {};
+// With fewer than 4 elements per lane (the latency layouts) the coefficient prescales would cost more than the weighting saves.
+template <class LaneT> struct LaneWeighted<LaneT, std::void_t<decltype(&LaneT::template w_from<1, 0u, 0u, 0u>)>> : std::bool_constant<(LaneT::E >= 4)> {};
 
 // ------------------------------------------------------------------------------------------------ steppers
 // Sum over the GL lanes of a group, result on every lane.  Power-of-two groups use the xor butterfly; other sizes
@@ -670,10 +695,74 @@ __device__ __forceinline__ void solve(LaneT &L, typename LaneT::SC &sc, int J, d
     else neumann<JT, SCALED>(L, sc, J, h, B, X);
 }
 
+// Weighted layouts: the boundary products of a state step, bp[0] = K05 u and bp[1] = S0 u of the state u it starts from.
+template <class LaneT>
+__device__ __forceinline__ void step_open(LaneT &L, const double (&u)[LaneT::E], const double (&p05)[LaneT::NC], const double (&q0)[LaneT::NC],
+                                          double (&bp)[2][LaneT::E]) {
+    typename LaneT::SC w[2];
+    L.template w_prescale<false>(p05, w[0]);
+    L.template w_prescale<true>(q0, w[1]);
+    typename LaneT::Nbr nb;
+    L.exchange(u, nb);
+    L.template w_from<2, 2u, 1u, 0u>(w, u, nb, u, bp);
+}
+
+// src/StormerVerlet.jl:461-504 for the weighted layouts, entered with the boundary products bp of u (step_open).  SHARE: the last
+// product pass also forms those of the outgoing u for the next step (p05 of the next step = pn; its S0 is this step's S1) and leaves
+// them in bp, so consecutive steps share one exchange of u.
+template <int JT, bool SHARE, class LaneT>
+__device__ __forceinline__ void state_step_w(LaneT &L, int J, double h, double (&u)[LaneT::E], double (&v)[LaneT::E], double (&v05)[LaneT::E],
+                                             double (&bp)[2][LaneT::E], const double (&pn)[LaneT::NC]) {
+    constexpr int E = LaneT::E;
+    double rhs[E], l1[E];
+    typename LaneT::SC sc;
+    typename LaneT::Nbr nb;
+    L.s_prescale(1, sc);
+    L.s_pass_add(sc, v, bp[0], rhs);                                                           // K05 u + S05 v
+    solve<JT>(L, sc, J, h, rhs, l1);
+    UNROLL for (int e = 0; e < E; ++e) v05[e] = fma(0.5 * h, l1[e], v[e]);
+    double k1v[E], s05v[E];
+    {
+        typename LaneT::SC w[3];
+        L.template w_prescale<false>(L.p[0], w[0]);
+        L.template w_prescale<false>(L.p[2], w[1]);
+        L.template w_prescale<true>(L.q[1], w[2]);
+        double t[3][E];                                                                        // kappa1 = S0 u - K0 v05, -K1 v05, S05 v05
+        L.exchange(v05, nb);
+        L.template w_from<3, 4u, 3u, 1u, 3u>(w, v05, nb, bp[1], t);
+        UNROLL for (int e = 0; e < E; ++e) {
+            k1v[e] = t[1][e];
+            s05v[e] = t[2][e];
+            u[e] = fma(0.5 * h, t[0][e], u[e]);            // u + (h/2) kappa1
+        }
+    }
+    constexpr int NO = SHARE ? 3 : 1;
+    typename LaneT::SC w[NO];
+    L.s_prescale(2, sc);
+    if constexpr (SHARE) w[2] = sc;                                                            // the next step's S0
+    L.s_pass_add(sc, u, k1v, rhs);                                                             // S1 (u + (h/2) kappa1) - K1 v05
+    double k2[E];
+    solve<JT>(L, sc, J, h, rhs, k2);
+    UNROLL for (int e = 0; e < E; ++e) u[e] = fma(0.5 * h, k2[e], u[e]);
+    L.template w_prescale<false>(L.p[1], w[0]);
+    if constexpr (SHARE) L.template w_prescale<false>(pn, w[1]);
+    double t[NO][E];                                                                           // l2 = K05 u + S05 v05 (, next K05 u, S0 u)
+    L.exchange(u, nb);
+    L.template w_from<NO, 4u, 3u, 1u>(w, u, nb, s05v, t);
+    UNROLL for (int e = 0; e < E; ++e) v[e] = fma(0.5 * h, t[0][e], v05[e]);                   // v + (h/2)(l1 + l2) = v05 + (h/2) l2
+    if constexpr (SHARE) { UNROLL for (int e = 0; e < E; ++e) { bp[0][e] = t[1][e]; bp[1][e] = t[2][e]; } }
+}
+
 // src/StormerVerlet.jl:461-504.  u, v updated in place; v05 returned.
 template <int JT, class LaneT>
 __device__ __forceinline__ void state_step(LaneT &L, int J, double h, double (&u)[LaneT::E], double (&v)[LaneT::E], double (&v05)[LaneT::E]) {
     constexpr int E = LaneT::E, NC = LaneT::NC;
+    if constexpr (LaneWeighted<LaneT>::value) {
+        double bp[2][E];
+        step_open(L, u, L.p[1], L.q[0], bp);
+        state_step_w<JT, false>(L, J, h, u, v, v05, bp, L.p[1]);
+        return;
+    }
     double rhs[E], l1[E], s0u[E];
     L.sync_reset();        // buffer parity restarts at 0: with compile-time J every exchange address is a constant offset
     L.template pass_each<true, true>(u, [&](int e, const double (&Ae)[NC + 1], const double (&De)[NC]) {
@@ -718,11 +807,13 @@ __device__ __forceinline__ void state_step(LaneT &L, int J, double h, double (&u
 // The group-reduced traces are left in shared memory at tred[q*5 + a] (written by lane 0 of the group).
 // DEFER: the lane's partial traces are returned in tpart[q*5 + a] instead of being reduced over the group (pipelined
 // instantiations hand them to the gradient role).
+// tcar: the lane-partial tr(vr0,Hs,li0) of this step on entry -- the tr(vr,Hs,li) of the step before (trace_hs before the first) --
+// and tr(vr,Hs,li) on return, so that every boundary trace is summed once.
 template <int JT, bool FORCING, class LaneT, bool DEFER = false>
 __device__ __forceinline__ void adjoint_step(LaneT &L, int J, double h, double (&mu)[LaneT::E], double (&nu)[LaneT::E],
                                              const double (&vr0)[LaneT::E], const double (&vi05)[LaneT::E],
                                              const double (&vr)[LaneT::E], double *tred, int GL, int gbase_lane, bool writer,
-                                             double *tpart = nullptr) {
+                                             double *tpart = nullptr, double *tcar = nullptr) {
     constexpr int E = LaneT::E, NC = LaneT::NC;
     double rhs[E], s05n[E], Tb[NC][2];
     typename LaneT::SC sc;
@@ -735,7 +826,7 @@ __device__ __forceinline__ void adjoint_step(LaneT &L, int J, double h, double (
         UNROLL for (int qq = 0; qq < NC; ++qq) {
             kk = fma(L.p[1][qq], Ae[qq], kk);
             s = fma(L.q[1][qq], De[qq], s);
-            Tb[qq][0] = fma(vr0[e], Ae[qq], Tb[qq][0]);      // tr(vr0, Hs, li0)
+            if (!tcar) Tb[qq][0] = fma(vr0[e], Ae[qq], Tb[qq][0]);      // tr(vr0, Hs, li0)
             Tb[qq][1] = fma(vi05[e], De[qq], Tb[qq][1]);     // tr(vi05, Ha, li0)
         }
         rhs[e] = (FORCING ? fma(L.w[e], vr0[e], rhs[e]) : rhs[e]) - kk;   // S0 mu + hr0 - K05 nu
@@ -798,6 +889,7 @@ __device__ __forceinline__ void adjoint_step(LaneT &L, int J, double h, double (
     {
         double tv2[NC * 2];
         UNROLL for (int qq = 0; qq < NC; ++qq) UNROLL for (int a = 0; a < 2; ++a) tv2[qq * 2 + a] = Tb[qq][a];
+        if (tcar) { UNROLL for (int qq = 0; qq < NC; ++qq) { tv2[qq * 2] += tcar[qq]; tcar[qq] = Tb[qq][0]; } }
         if constexpr (LaneSigned<LaneT>::value) { UNROLL for (int qq = 0; qq < NC; ++qq) tv2[qq * 2 + 1] *= L.dsign(qq); }
         if constexpr (DEFER) { UNROLL for (int qq = 0; qq < NC; ++qq) UNROLL for (int a = 0; a < 2; ++a) tpart[qq * 5 + 3 + a] = tv2[qq * 2 + a]; }
         else {
@@ -806,6 +898,17 @@ __device__ __forceinline__ void adjoint_step(LaneT &L, int J, double h, double (
         }
     }
     if constexpr (!DEFER) __syncwarp();
+}
+
+// Lane-partial tr(v, Hs_q, x) for every control q: the boundary trace adjoint_step carries from step to step (tcar).
+template <class LaneT>
+__device__ __forceinline__ void trace_hs(LaneT &L, const double (&v)[LaneT::E], const double (&x)[LaneT::E], double (&tc)[LaneT::NC]) {
+    constexpr int NC = LaneT::NC;
+    UNROLL for (int qq = 0; qq < NC; ++qq) tc[qq] = 0.0;
+    L.sync_reset();
+    L.template pass_each<true, false>(x, [&](int e, const double (&Ae)[NC + 1], const double (&)[NC]) {
+        UNROLL for (int qq = 0; qq < NC; ++qq) tc[qq] = fma(v[e], Ae[qq], tc[qq]);
+    });
 }
 
 // ---- pipelined instantiations: hand-over between the state role and the adjoint role of one CTA through two step counters per
@@ -830,12 +933,14 @@ __device__ __forceinline__ void role_sync(int nthr) {
 
 // Fill the control table for `nst` steps starting at time t: all threads of the CTA into the table at offset 0 (SYNC = 0), or the
 // 32 lanes of the table warp (SYNC = 1) / the rnthr threads of the gradient role (SYNC = 2) into the table buffer at offset `toff`.
-template <int NC, int SYNC = 0>
+// XPT: one extra point, the midpoint of the step after the chunk (the shared boundary pass of the chunk's last forward step needs
+// its p05): the same recurrence, so the same value as the next chunk's row 1.
+template <int NC, int SYNC = 0, bool XPT = false>
 __device__ void fill_table(const TrajParams &S, double *sm, double t, double dt, int nst, double dtknot, int toff = 0, int rtid = 0, int rnthr = 0) {
     if (SYNC == 0) { rtid = threadIdx.x; rnthr = blockDim.x; toff = 0; }
     double *times = sm + S.o_times + toff, *tabb = sm + S.o_tabb + toff, *tabph = sm + S.o_tabph + toff, *tabpq = sm + S.o_tabpq + toff;
     int *tabk = reinterpret_cast<int *>(sm + S.o_tabk + toff);
-    const int npts = 2 * nst + 1, Nfreq = S.P.Nfreq, D1 = S.A.D1;
+    const int npts = 2 * nst + 1 + XPT, Nfreq = S.P.Nfreq, D1 = S.A.D1;
     role_sync<SYNC>(rnthr);          // the previous chunk's table is no longer in use
     if (rtid == 0) {
         double tt = t;
@@ -845,6 +950,7 @@ __device__ void fill_table(const TrajParams &S, double *sm, double t, double dt,
             tt = tt + dt;
             times[2 * i + 2] = tt;
         }
+        if (XPT) times[2 * nst + 1] = tt + 0.5 * dt;
     }
     role_sync<SYNC>(rnthr);
     const double width = 3.0 * dtknot;
@@ -1107,24 +1213,50 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
     };
     if (hist) save_state();
     // two copies of the loop (generic lambda, both inlined): the evaluation path carries no per-step history test
+    // SHARE (weighted layouts, not pipelined): a step's last product pass also gives the next step's boundary products (bp, with
+    // the next p05 from the table row past the step: the table carries one extra point for the last step of a chunk).  The penalty
+    // (penalf2aTrap + penalf2a), the sum over the steps of w.*(vr_k^2 + vr_k+1^2 + 2 vi05^2), is then evaluated as twice
+    // (w.*vr_0^2 / 2 + sum of w.*(vr_k+1^2 + vi05^2) - w.*vr_N^2 / 2), so that every state is squared once.  The other layouts keep
+    // the step-by-step form: several of them spill, and the end terms would add spill loads to their forward loops.
+    constexpr bool SHARE = LaneWeighted<LaneT>::value && !PIPE;
     auto forward_sweep = [&](auto with_hist) {
+        if constexpr (SHARE) { UNROLL for (int e = 0; e < E; ++e) pen = fma(0.5 * L.w[e], vr[e] * vr[e], pen); }
+        double bp[SHARE ? 2 : 1][SHARE ? E : 1];
         for (long long s0 = 0; s0 < (SEG ? nstl : P.nsteps); s0 += TRAJ_CH) {
             const int nst = (int)(((SEG ? nstl : P.nsteps) - s0) < TRAJ_CH ? ((SEG ? nstl : P.nsteps) - s0) : TRAJ_CH);
             if constexpr (PIPE) {
                 const int gk = (int)(s0 / TRAJ_CH);
                 pipe_wait(tabs_ready, gk + 1);
                 tabpq = sm + S.o_tabpq + (gk % TRAJ_TABS) * S.tab_role_stride;
-            } else fill_table<NC>(S, sm, t, dt, nst, dtknot);
+            } else fill_table<NC, 0, SHARE>(S, sm, t, dt, nst, dtknot);
             LOAD_LEVEL0();
+            if constexpr (SHARE) {
+                if (s0 == 0) {
+                    double p05[NC];
+                    UNROLL for (int qq = 0; qq < NC; ++qq) p05[qq] = tabpq[(S.TPC + tl) * 2 * NC + 2 * qq];
+                    step_open(L, vr, p05, L.q[2], bp);
+                }
+            }
             for (int ls = 0; ls < nst; ++ls) {
                 LOAD_LEVELS(ls);
-                UNROLL for (int e = 0; e < E; ++e) pen = fma(L.w[e], vr[e] * vr[e], pen);                              // penalf2aTrap
-                state_step<JT>(L, J, dt, vr, vi, vi05);
-                UNROLL for (int e = 0; e < E; ++e) pen = fma(L.w[e], vr[e] * vr[e] + 2.0 * vi05[e] * vi05[e], pen);   // penalf2a
+                if constexpr (SHARE) {
+                    double pn[NC];
+                    UNROLL for (int qq = 0; qq < NC; ++qq) pn[qq] = tabpq[((2 * ls + 3) * S.TPC + tl) * 2 * NC + 2 * qq];
+                    state_step_w<JT, true>(L, J, dt, vr, vi, vi05, bp, pn);
+                    UNROLL for (int e = 0; e < E; ++e) pen = fma(L.w[e], fma(vr[e], vr[e], vi05[e] * vi05[e]), pen);
+                } else {
+                    UNROLL for (int e = 0; e < E; ++e) pen = fma(L.w[e], vr[e] * vr[e], pen);                              // penalf2aTrap
+                    state_step<JT>(L, J, dt, vr, vi, vi05);
+                    UNROLL for (int e = 0; e < E; ++e) pen = fma(L.w[e], vr[e] * vr[e] + 2.0 * vi05[e] * vi05[e], pen);   // penalf2a
+                }
                 t = t + dt;
                 if constexpr (decltype(with_hist)::value) { if (--hcount == 0) { hcount = A.save_every; save_state(); } }
             }
             if constexpr (PIPE) pipe_post(cdone + pwarp, (int)(s0 / TRAJ_CH) + 1, g.lane);
+        }
+        if constexpr (SHARE) {
+            UNROLL for (int e = 0; e < E; ++e) pen = fma(-0.5 * L.w[e], vr[e] * vr[e], pen);
+            pen *= 2.0;
         }
     };
     double *red = sm + S.o_red;
@@ -1257,6 +1389,14 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
     if constexpr (SEG) t = A.seg.times[A.seg.nseg + seg];
     dt = -dt;
     if constexpr (!PIPE) {
+        // weighted layouts carry the boundary trace from step to step; in the other layouts' backward loops, several of which
+        // spill, the carried sums would be more live registers
+        constexpr bool CARRY = LaneWeighted<LaneT>::value;
+        double tcar[NC], tcar2[OBJ ? NC : 1];
+        if constexpr (CARRY) {
+            trace_hs(L, vr, li, tcar);
+            if constexpr (OBJ != 0) trace_hs(L, vr, lin, tcar2);
+        }
         for (long long s0 = 0; s0 < (SEG ? nstl : P.nsteps); s0 += TRAJ_CH) {
             const int nst = (int)(((SEG ? nstl : P.nsteps) - s0) < TRAJ_CH ? ((SEG ? nstl : P.nsteps) - s0) : TRAJ_CH);
             fill_table<NC>(S, sm, t, dt, nst, dtknot);
@@ -1279,10 +1419,10 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
                 }
                 UNROLL for (int e = 0; e < E; ++e) vr0[e] = vr[e];
                 state_step<JT>(L, J, dt, vr, vi, vi05);
-                adjoint_step<JT, true>(L, J, dt, lr, li, vr0, vi05, vr, tred, GL, gbase_lane, lane_on && g.lg == 0);   // traces -> tred
+                adjoint_step<JT, true>(L, J, dt, lr, li, vr0, vi05, vr, tred, GL, gbase_lane, lane_on && g.lg == 0, nullptr, CARRY ? tcar : nullptr);   // traces -> tred
                 grad_scatter<NC, UPL>(U, gsm, tred, tabb, tabph, tabk, ls, Nfreq);
                 if constexpr (OBJ != 0) {
-                    adjoint_step<JT, false>(L, J, dt, lrn, lin, vr0, vi05, vr, tred, GL, gbase_lane, lane_on && g.lg == 0);
+                    adjoint_step<JT, false>(L, J, dt, lrn, lin, vr0, vi05, vr, tred, GL, gbase_lane, lane_on && g.lg == 0, nullptr, CARRY ? tcar2 : nullptr);
                     grad_scatter<NC, UPL>(U2, gsm2, tred, tabb, tabph, tabk, ls, Nfreq);
                 }
                 t = t + dt;
