@@ -168,6 +168,26 @@ int jq_forward_sensitivity(jq_handle *h, int32_t nbatch, const double *pcof, int
                            double *infid, double *leak, double *dinfid, double *dleak,
                            double *dstate_r, double *dstate_i);
 
+/* Final-state vector-Jacobian products: the gradient of any real objective of the final state U(T), one backward sweep per cotangent
+ * whatever npar is (the dual of dstate in jq_forward_sensitivity).  Trajectory (b, s, k) evaluates candidate b with sample shift s and
+ * pulls back cotangent k.  One launch of the final-state VJP kernel (jq_query(h, 0) = 9) runs, per trajectory, the forward sweep and
+ * then the backward sweep of the reference's unforced adjoint (the objFuncType 2/3 set, src/StormerVerlet.jl:365-406, gradient
+ * src/evalobjgrad.jl:2567-2619) from the terminal condition lambda_r(T) = -cot_r / 2, lambda_i(T) = cot_i / 2.
+ * Conventions: U(T) = vr - i vi as in jq_eval_forward, so Re U = vr and Im U = -vi.  With c = cot_r + i cot_i,
+ *   vjp[p] = sum_e cot_r[e] dRe U[e]/dpcof[p] + cot_i[e] dIm U[e]/dpcof[p]  (= Re vdot(c, dU . e_p), vdot conjugating c),
+ * which for a real loss L and c = dL/dRe U + i dL/dIm U is dL/dpcof.  With c = dinfid/d(Re U, Im U) the result is the infidelity
+ * gradient of jq_traceobjgrad_batch for every pFidType.  The guard penalty, its weights and obj_func_type play no part; the solver and
+ * uncoupled controls do.  pcof, h0_diag_shift as in jq_traceobjgrad_batch; with pFidType 3 every pcof and vjp vector carries the global
+ * phase as its last entry, and U(T) does not depend on it: that entry of vjp is 0.
+ * cot_r, cot_i: [(t*ncot + k)][n*m] with t = b*nsamples + s, column-major n x m blocks (the layout of dstate); NULL means zero, not both.
+ * vjp: [(t*ncot + k)][npar].  state_r, state_i: [t][n*m], Re and Im of U(T), or NULL.
+ * JQ_ERR_ARG (no launch) for ncot < 1, both cotangent parts NULL, vjp == NULL, nbatch*nsamples*ncot > 2^31 - 1, or a problem whose
+ * trajectory does not fit in 227 KB of shared memory.  Never communicates; jq_set_kernel and jq_comm_set_cooperative do not affect it.
+ * Host pointers, blocking. */
+int jq_final_state_vjp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                       const double *h0_diag_shift, int32_t ncot, const double *cot_r, const double *cot_i,
+                       double *vjp, double *state_r, double *state_i);
+
 /* evalctrl(params, pcof, td, func) (src/plotstatectrl.jl:246-276): the control functions p_q(t), q_q(t) (rad/ns) of EVERY
  * coupled control q on the time grid `times`, evaluated by the device function the time loop uses (bcarrier2,
  * src/bsplines.jl:211-304).  p, q: [ncoupled][ntimes] doubles, host pointers, blocking. */
@@ -213,7 +233,8 @@ int jq_set_time_segments(jq_handle *h, int32_t nseg);
  * (src/evalobjgrad.jl:745) has at the segment's first step, t_last[p] the value its backward recurrence t = t - dt from T (:810, :919)
  * has at the segment's last step -- bit-identical to what a single sweep sees, not k dt.  Returns the steps of the longest segment. */
 int64_t jq_time_segments(double T, int64_t nsteps, int32_t nseg, double *t_first, double *t_last);
-/* what: 0 = kernel actually used by the last evaluation (1 ... 7, or 8 = the forward-sensitivity kernel of jq_forward_sensitivity),
+/* what: 0 = kernel actually used by the last evaluation (1 ... 7, 8 = the forward-sensitivity kernel of jq_forward_sensitivity, or
+ * 9 = the final-state VJP kernel of jq_final_state_vjp),
  * 1 = CUDA-event time of the last evaluation's trajectory kernel(s) in ms (synchronises), 2 = number of kernels launched by the last
  * evaluation,
  * 3 = trajectories resident per CTA, 4 = CTAs launched, 5 = registers per thread, 6 = dynamic smem bytes per CTA,

@@ -212,6 +212,27 @@ function forward_sensitivity(pcof::Vector{Float64}, params::objparams, wa::Worki
     return w === nothing ? (infid, leak, dinfid, dleak) : (infid, leak, vec(dinfid), vec(dleak))
 end
 
+# Final-state vector-Jacobian products (jq_final_state_vjp): for each node and each cotangent c = cot_r + im cot_i of the final
+# state U(T) (Ntot x N), vjp = sum of cot_r .* dRe U / dpcof + cot_i .* dIm U / dpcof, one backward sweep per cotangent whatever
+# Npar is.  With cot = dL/dRe U + im dL/dIm U this is dL/dpcof for any real loss L of U(T); with pFidType 3 the phase entry is 0.
+# cot_r, cot_i are Ntot x N x ncot x nsamples; returns vjp, Npar x ncot x nsamples, and U(T), Ntot x N x nsamples.
+function final_state_vjp(pcof::Vector{Float64}, params::objparams, wa::Working_Arrays_B200, cot_r::Array{Float64,4},
+                         cot_i::Array{Float64,4}; nodes::AbstractArray = [0.0])
+    Ntot = params.N + params.Nguard
+    nsamples = length(nodes)
+    size(cot_r) == size(cot_i) && size(cot_r, 1) == Ntot && size(cot_r, 2) == params.N && size(cot_r, 4) == nsamples ||
+        error("final_state_vjp: cot_r and cot_i must be Ntot x N x ncot x nsamples")
+    ncot = size(cot_r, 3)
+    Npar = length(pcof)
+    vjp = zeros(Npar, ncot, nsamples)
+    ur = zeros(Ntot, params.N, nsamples); ui = zeros(Ntot, params.N, nsamples)
+    jq_check(ccall((:jq_final_state_vjp, libjq), Cint,
+                   (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Int32, Ptr{Float64}, Ptr{Float64},
+                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                   wa.handle, 1, pcof, Npar, nsamples, jq_shifts(params, nodes), ncot, cot_r, cot_i, vjp, ur, ui))
+    return vjp, ur .+ im .* ui
+end
+
 
 # ---- the four Ipopt callbacks as ONE ccall each (src/ipopt_interface.jl:77-179): jq_eval_f_grad keeps the last-pcof cache, runs
 # eval_f_g_grad!'s sample loop as one launch and adds the Tikhonov terms on the device.  params.last_* scalars are kept for

@@ -320,6 +320,46 @@ class Working_Arrays:
             out["dstate"] = (sr + 1j * si).swapaxes(-1, -2)
         return out
 
+    def final_state_vjp(self, pcof, cot, shifts=None, final_state: bool = False):
+        """Final-state vector-Jacobian products (jq_final_state_vjp): one backward sweep per cotangent of U(T).
+
+        pcof [nbatch, npar]; cot complex [nbatch, nsamples, ncot, Ntot, N] (the shape of forward_sensitivity's dstate).  Returns a
+        dict with vjp [nbatch, nsamples, ncot, npar], vjp[b, s, k] = sum over the entries of Re(cot) dRe U + Im(cot) dIm U by pcof,
+        i.e. dL/dpcof for a real loss L when cot = dL/dRe U + i dL/dIm U (PyTorch's convention for complex outputs).  With pFidType 3
+        the last entry (the global phase) is 0.  final_state=True adds state, U(T) complex [nbatch, nsamples, Ntot, N]."""
+        p = self.params
+        self._check_params()
+        pcof = np.asarray(pcof)
+        if pcof.ndim != 2:
+            raise ValueError("pcof must be [nbatch, npar]")
+        pcof = _f64(pcof)
+        nbatch, npar = pcof.shape
+        nsamples, sp = 1, None
+        if shifts is not None:
+            shifts = _f64(np.atleast_2d(shifts))
+            if shifts.ndim != 2 or shifts.shape[1] != p.Ntot:
+                raise ValueError("shifts must be [nsamples, Ntot]")
+            nsamples, sp = shifts.shape[0], shifts.ctypes.data_as(C.c_void_p)
+        cot = np.asarray(cot)
+        if cot.ndim != 5 or cot.shape[:2] != (nbatch, nsamples) or cot.shape[2] < 1 or cot.shape[3:] != (p.Ntot, p.N):
+            raise ValueError(f"cot must be [nbatch, nsamples, ncot, Ntot, N] = [{nbatch}, {nsamples}, ncot >= 1, {p.Ntot}, {p.N}], "
+                             f"not {list(cot.shape)}")
+        ncot = cot.shape[2]
+        cr = _f64(cot.real.swapaxes(-1, -2))                     # the C layout: column-major Ntot x N blocks
+        ci = _f64(cot.imag.swapaxes(-1, -2)) if np.iscomplexobj(cot) else None
+        vjp = np.zeros((nbatch, nsamples, ncot, npar))
+        sr = si = None
+        if final_state:
+            sr = np.zeros((nbatch, nsamples, p.N, p.Ntot))
+            si = np.zeros_like(sr)
+        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        _lib.check(self._lib.jq_final_state_vjp(self._handle, nbatch, ptr(pcof), npar, nsamples, sp, ncot, ptr(cr), ptr(ci), ptr(vjp),
+                                                ptr(sr), ptr(si)))
+        out = {"vjp": vjp}
+        if final_state:
+            out["state"] = (sr + 1j * si).swapaxes(-1, -2)
+        return out
+
     def eval_f_grad(self, pcof, shifts=None, weights=None, tik0: float = 0.0, prior=None):
         """The fused Ipopt-callback entry (jq_eval_f_grad): objective with Tikhonov, its gradient, infidelity, leak and leak
         gradient of ONE pcof in one call, with the last-pcof cache inside the handle.  Returns a dict; `evaluated` is False
@@ -439,6 +479,38 @@ def forward_sensitivity(pcof0, params: objparams, wa: Working_Arrays, dirs, node
     shifts = None if nodes is None else noise_shift(params.Ntot, nodes)
     r = wa.forward_sensitivity(pcof0[None, :], dirs[None], shifts, weights)
     return {k: v[0] for k, v in r.items()}
+
+
+_FinalState = None
+
+
+def final_state(wa: Working_Arrays, pcof, shifts=None):
+    """U(T) as a differentiable torch function of pcof: a complex tensor [nbatch, nsamples, Ntot, N] on pcof's device.
+
+    pcof: float64 tensor [nbatch, npar] on any device; shifts: host array [nsamples, Ntot] or None.  The forward pass is
+    wa.forward_history(save_every=nsteps); the backward pass is one wa.final_state_vjp call with the incoming gradient as the
+    cotangent (summed over the samples, which all share pcof).  First derivatives in reverse mode only."""
+    global _FinalState
+    import torch
+    if pcof.dim() != 2 or pcof.dtype != torch.float64:
+        raise ValueError("pcof must be a float64 tensor [nbatch, npar]")
+    if _FinalState is None:
+        class _Fn(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, wa_, pc, sh):
+                ctx.wa, ctx.pcof, ctx.shifts = wa_, pc.detach().cpu().numpy(), sh
+                hist, _, _ = wa_.forward_history(ctx.pcof, sh, save_every=wa_.params.nsteps)
+                return torch.from_numpy(np.ascontiguousarray(hist[:, :, -1].swapaxes(-1, -2))).to(pc.device)
+
+            @staticmethod
+            @torch.autograd.function.once_differentiable
+            def backward(ctx, grad_out):
+                cot = grad_out.detach().resolve_conj().cpu().numpy()[:, :, None]
+                g = ctx.wa.final_state_vjp(ctx.pcof, cot, ctx.shifts)["vjp"][:, :, 0].sum(axis=1)
+                return None, torch.from_numpy(g).to(grad_out.device), None
+
+        _FinalState = _Fn
+    return _FinalState.apply(wa, pcof, shifts)
 
 
 def eval_forward(pcof0, params: objparams, wa: Working_Arrays, saveEndOnly: bool = True, saveEvery: int = 1):

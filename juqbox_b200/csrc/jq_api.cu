@@ -1065,3 +1065,50 @@ extern "C" int jq_forward_sensitivity(jq_handle *h, int32_t nbatch, const double
     CU(cudaStreamSynchronize(st));
     return 0;
 }
+
+extern "C" int jq_final_state_vjp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples, const double *shift,
+                                  int32_t ncot, const double *cot_r, const double *cot_i, double *vjp, double *state_r, double *state_i) {
+    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
+    if (rc) return rc;
+    if (ncot < 1 || (!cot_r && !cot_i)) return fail(JQ_ERR_ARG, "jq_final_state_vjp: need ncot >= 1 and at least one of cot_r, cot_i");
+    if (!vjp) return fail(JQ_ERR_ARG, "jq_final_state_vjp: null vjp output");
+    if ((long long)nbatch * nsamples * ncot > 0x7fffffffLL)
+        return fail(JQ_ERR_ARG, "jq_final_state_vjp: nbatch * nsamples * ncot exceeds 2^31 - 1 trajectories per call");
+    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
+    if (jq_vjp_smem_bytes(h->P, nspl) > 227 * 1024)
+        return fail(JQ_ERR_ARG, "jq_final_state_vjp: problem too large for the VJP kernel's shared memory (n*m = %d)", h->n * h->m);
+    CU(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ncot, len = (size_t)h->n * h->m;
+    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)nsamples * h->n : 0, n_cot = ntraj * len;
+    const size_t n_vjp = ntraj * npar, n_state = (state_r || state_i) ? nt * len : 0;
+    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_shift + (cot_r ? n_cot : 0) + (cot_i ? n_cot : 0))) != 0) return rc;
+    if ((rc = grow(&h->d_out, &h->cap_out, n_vjp + 2 * n_state)) != 0) return rc;
+    double *d_pcof = h->d_in, *cur = d_pcof + n_pcof;
+    double *d_shift = shift ? cur : nullptr; cur += n_shift;
+    double *d_cr = cot_r ? cur : nullptr; cur += cot_r ? n_cot : 0;
+    double *d_ci = cot_i ? cur : nullptr;
+    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (cot_r) CU(cudaMemcpyAsync(d_cr, cot_r, n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (cot_i) CU(cudaMemcpyAsync(d_ci, cot_i, n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
+
+    VjpArgs V{};
+    V.ntraj = (int)ntraj; V.nsamples = nsamples; V.ncot = ncot; V.Npar = nspl; V.D1 = nspl / (2 * h->Nc * h->Nfreq); V.pstride = npar;
+    V.pcof = d_pcof; V.shift = d_shift; V.cot_r = d_cr; V.cot_i = d_ci;
+    V.vjp = h->d_out;
+    V.state_r = n_state ? h->d_out + n_vjp : nullptr; V.state_i = n_state ? h->d_out + n_vjp + n_state : nullptr;
+    Ran ran;
+    ran.kernel = 9;
+    CU(cudaEventRecord(h->ev0, st));
+    CU(jq_vjp_launch(h->P, V, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc));
+    CU(cudaEventRecord(h->ev1, st));
+    h->timed = true;
+    h->ran = ran;
+    h->last_launches = 1;
+    CU(cudaMemcpyAsync(vjp, V.vjp, n_vjp * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (state_r) CU(cudaMemcpyAsync(state_r, V.state_r, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (state_i) CU(cudaMemcpyAsync(state_i, V.state_i, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return 0;
+}

@@ -101,6 +101,19 @@ struct SensArgs {
 size_t jq_fwdsens_smem_bytes(const DevProblem &P, int Npar);     // one group
 cudaError_t jq_fwdsens_launch(const DevProblem &P, const SensArgs &S, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc);
 
+// ---- final-state VJP kernel (jq_generic.cu): forward sweep, then one unforced adjoint sweep from a caller-supplied cotangent of U(T) ----
+struct VjpArgs {
+    int ntraj, nsamples, ncot, Npar, D1;   // ntraj = nbatch * nsamples * ncot; Npar: spline coefficients (without the pFidType 3 phase)
+    int pstride;           // length of every pcof and vjp vector: Npar, or Npar + 1 with the global phase (pFidType 3)
+    const double *pcof;    // [nbatch][pstride]
+    const double *shift;   // [nsamples][n] or nullptr
+    const double *cot_r, *cot_i;       // [ntraj][n*m] cotangents of Re and Im of U(T), or nullptr (zero); traj = (b * nsamples + s) * ncot + k
+    double *vjp;           // [ntraj][pstride]; the phase entry is 0
+    double *state_r, *state_i;         // [nbatch * nsamples][n*m] Re and Im of U(T) (vr, -vi; written by cotangent 0), or nullptr
+};
+size_t jq_vjp_smem_bytes(const DevProblem &P, int Npar);         // one group
+cudaError_t jq_vjp_launch(const DevProblem &P, const VjpArgs &V, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc);
+
 // ---- dense-operator kernel on the FP64 tensor-core path (jq_dense.cu): one CTA per (candidate, tile of samples) ----
 bool jq_dense_supported(const DevProblem &P, char *why, size_t len);
 void jq_dense_padding(int n, int *n8, int *ldk);      // layout of DevProblem::dense_ops: [1 + 2 Nc][n8][ldk], zero padded

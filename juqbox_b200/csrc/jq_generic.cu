@@ -647,6 +647,69 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_forward_sensitivity_kernel(Dev
     }
 }
 
+// Final-state vector-Jacobian products: g = sum_e c_r[e] dRe U(T)[e]/dpcof + c_i[e] dIm U(T)[e]/dpcof for a caller-supplied cotangent
+// c = c_r + i c_i.  The generic kernel's forward sweep without the penalty, then its backward sweep with one unforced adjoint set
+// (the objFuncType 2/3 set) from the terminal condition lambda_r(T) = -c_r / 2, lambda_i(T) = c_i / 2: with c = dinfid/d(Re U, Im U)
+// that is the generic kernel's own terminal condition for every pFidType, so the result is its infidgrad.  Trajectory
+// traj = t * ncot + k, t = b * nsamples + s.
+__global__ void __launch_bounds__(GEN_THREADS) jq_final_state_vjp_kernel(DevProblem P, VjpArgs V, GenGeom G) {
+    extern __shared__ __align__(16) double sm[];
+    Ctx c{};
+    double *p = group_setup(c, P, V.Npar, V.D1, G, sm);
+    const int grp = threadIdx.x / G.tpt;
+    double **blk[] = {&c.vr, &c.vi, &c.vi05, &c.vr0, &c.lr, &c.li, &c.lr05, &c.li0, &c.rhs, &c.scr, &c.k1, &c.k2, &c.l1, &c.l2};
+    for (int b = 0; b < 14; ++b) { *blk[b] = p; p += c.len; }
+    c.pcof = p; p += c.Npar;
+    c.grad = p; p += c.Npar;
+    c.ctrl = p; p += 6 * c.Nc;
+    c.shift = p; p += c.n;
+    c.red = p;
+    if (grp >= G.gpc) return;
+
+    for (int traj = blockIdx.x * G.gpc + grp; traj < V.ntraj; traj += gridDim.x * G.gpc) {
+        const int t_ = traj / V.ncot, k_ = traj % V.ncot, b = t_ / V.nsamples, s = t_ % V.nsamples;
+        const double *pc = V.pcof + (size_t)b * V.pstride;
+        for (int k = c.gtid; k < c.Npar; k += c.tpt) { c.pcof[k] = pc[k]; c.grad[k] = 0.0; }
+        for (int k = c.gtid; k < c.n; k += c.tpt) c.shift[k] = V.shift ? V.shift[(size_t)s * c.n + k] : 0.0;
+        FOR_E { c.vr[e] = P.uinit[e]; c.vi[e] = 0.0; c.vi05[e] = 0.0; }
+        gsync(c);
+
+        double dt = P.T / (double)P.nsteps, t = 0.0;
+        for (long long step = 0; step < P.nsteps; ++step) {
+            eval_controls(c, t, dt);
+            state_step(c, dt);
+            t = t + dt;
+        }
+        if (V.state_r && k_ == 0) {
+            double *sr = V.state_r + (size_t)t_ * c.len, *si = V.state_i + (size_t)t_ * c.len;
+            FOR_E { sr[e] = c.vr[e]; si[e] = -c.vi[e]; }
+        }
+        const double *cr = V.cot_r ? V.cot_r + (size_t)traj * c.len : nullptr, *ci = V.cot_i ? V.cot_i + (size_t)traj * c.len : nullptr;
+        FOR_E {
+            const double lr = cr ? -0.5 * cr[e] : 0.0, li = ci ? 0.5 * ci[e] : 0.0;
+            c.lr[e] = lr; c.lr05[e] = lr; c.li[e] = li; c.li0[e] = li;
+        }
+        t = P.T;
+        dt = -dt;
+        gsync(c);
+        for (long long step = P.nsteps - 1; step >= 0; --step) {
+            const double t0 = t;
+            FOR_E c.vr0[e] = c.vr[e];
+            eval_controls(c, t, dt);
+            state_step(c, dt);
+            t = t + dt;
+            adjoint_step(c, c.lr, c.li, c.lr05, dt, false, c.tinv);
+            grad_step(c, c.lr05, c.li, c.li0, t0, dt, c.grad);
+            FOR_E c.li0[e] = c.li[e];
+            gsync(c);
+        }
+        double *g = V.vjp + (size_t)traj * V.pstride;
+        for (int k = c.gtid; k < c.Npar; k += c.tpt) g[k] = dt * c.grad[k];
+        if (V.pstride > c.Npar && c.gtid == 0) g[c.Npar] = 0.0;      // pFidType 3: U(T) does not depend on the global phase
+        gsync(c);
+    }
+}
+
 // doubles of shared memory per trajectory group
 static size_t per_group_doubles(const DevProblem &P, int Npar) {
     const size_t len = (size_t)P.n * P.m;
@@ -659,6 +722,13 @@ static size_t per_group_doubles(const DevProblem &P, int Npar) {
 static size_t fwdsens_group_doubles(const DevProblem &P, int Npar) {
     const size_t len = (size_t)P.n * P.m;
     size_t d = 20 * len + 2 * (size_t)Npar + 12 * P.Nc + P.n + (GEN_THREADS / 32) * 8;
+    return (d + 1) & ~(size_t)1;
+}
+
+// final-state VJP kernel: the generic kernel's objFuncType-1 footprint (14 blocks, pcof, grad, the control table)
+static size_t vjp_group_doubles(const DevProblem &P, int Npar) {
+    const size_t len = (size_t)P.n * P.m;
+    size_t d = 14 * len + 2 * (size_t)Npar + 6 * P.Nc + P.n + (GEN_THREADS / 32) * 8;
     return (d + 1) & ~(size_t)1;
 }
 
@@ -688,6 +758,10 @@ size_t jq_generic_smem_bytes(const DevProblem &P, int Npar) {          // minimu
 
 size_t jq_fwdsens_smem_bytes(const DevProblem &P, int Npar) {
     return fwdsens_group_doubles(P, Npar) * sizeof(double);
+}
+
+size_t jq_vjp_smem_bytes(const DevProblem &P, int Npar) {
+    return vjp_group_doubles(P, Npar) * sizeof(double);
 }
 
 // evalctrl (src/plotstatectrl.jl:246-276): the control functions of every coupled control on an arbitrary time grid,
@@ -734,25 +808,37 @@ cudaError_t jq_generic_launch(const DevProblem &P, const LaunchArgs &A, cudaStre
     return cudaGetLastError();
 }
 
-cudaError_t jq_fwdsens_launch(const DevProblem &P, const SensArgs &S, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc) {
+// One launch of a persistent generic-layout kernel (forward sensitivities, final-state VJPs): at most one resident wave of CTAs, whose
+// groups loop over the ntraj trajectories.
+template <class Args>
+static cudaError_t persistent_launch(void (*kernel)(DevProblem, Args, GenGeom), const DevProblem &P, const Args &A, int ntraj,
+                                     size_t per_group, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc) {
     size_t bytes = 0;
-    const GenGeom G = generic_geometry(P, fwdsens_group_doubles(P, S.Npar), &bytes);
-    cudaError_t e = cudaFuncSetAttribute(jq_forward_sensitivity_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    const GenGeom G = generic_geometry(P, per_group, &bytes);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
     cudaFuncAttributes fa;
-    e = cudaFuncGetAttributes(&fa, jq_forward_sensitivity_kernel);
+    e = cudaFuncGetAttributes(&fa, kernel);
     if (e != cudaSuccess) return e;
     int dev = 0, sms = 148, occ = 1;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, jq_forward_sensitivity_kernel, G.tpt * G.gpc, bytes);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, G.tpt * G.gpc, bytes);
     if (occ < 1) occ = 1;
-    const int want = (S.ntraj + G.gpc - 1) / G.gpc;
-    const int grid = want < sms * occ ? want : sms * occ;   // persistent: groups loop over trajectories
-    jq_forward_sensitivity_kernel<<<grid, G.tpt * G.gpc, bytes, st>>>(P, S, G);
+    const int want = (ntraj + G.gpc - 1) / G.gpc;
+    const int grid = want < sms * occ ? want : sms * occ;
+    kernel<<<grid, G.tpt * G.gpc, bytes, st>>>(P, A, G);
     if (nctas) *nctas = grid;
     if (regs) *regs = fa.numRegs;
     if (smem) *smem = bytes;
     if (gpc) *gpc = G.gpc;
     return cudaGetLastError();
+}
+
+cudaError_t jq_fwdsens_launch(const DevProblem &P, const SensArgs &S, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc) {
+    return persistent_launch(jq_forward_sensitivity_kernel, P, S, S.ntraj, fwdsens_group_doubles(P, S.Npar), st, nctas, regs, smem, gpc);
+}
+
+cudaError_t jq_vjp_launch(const DevProblem &P, const VjpArgs &V, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc) {
+    return persistent_launch(jq_final_state_vjp_kernel, P, V, V.ntraj, vjp_group_doubles(P, V.Npar), st, nctas, regs, smem, gpc);
 }
