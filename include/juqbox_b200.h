@@ -188,6 +188,35 @@ int jq_final_state_vjp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t
                        const double *h0_diag_shift, int32_t ncot, const double *cot_r, const double *cot_i,
                        double *vjp, double *state_r, double *state_i);
 
+/* Derivatives of the state history of jq_eval_forward, U_j = U(t_j) with t_j after step j*save_every, j = 0 ... nsave - 1,
+ * nsave = nsteps/save_every + 1 (U_0 = Uinit does not depend on pcof).  A block is a column-major n x m matrix; Re U_j = vr,
+ * Im U_j = -vi as in jq_eval_forward.  Both entries use host pointers, block until done, never communicate, and are not affected by
+ * jq_set_kernel or jq_comm_set_cooperative.  pcof, h0_diag_shift as in jq_traceobjgrad_batch, with t = b*nsamples + s.
+ * JQ_ERR_ARG (no launch) for save_every < 1 or nsteps % save_every != 0 (the message of jq_eval_forward), ncot / ndir < 1, a NULL
+ * required array, more than 2^31 - 1 trajectories, or a problem whose trajectory does not fit in 227 KB of shared memory.
+ * Histories are large: one history of nsave blocks is 16 * nsave * n * m bytes (the cnot3 example, 64 x 4 with 31325 steps, at
+ * save_every = 1: 128 MB per trajectory and cotangent or direction), and every cotangent and tangent history of a call sits on the
+ * device at once; a request the device cannot hold returns JQ_ERR_ALLOC.
+ *
+ * jq_history_vjp: reverse mode, vjp[p] = sum_j sum_e cot_r[j,e] dRe U_j[e]/dpcof[p] + cot_i[j,e] dIm U_j[e]/dpcof[p], i.e. dL/dpcof of
+ * L = sum_j Re vdot(c_j, U_j), one forward and one backward sweep per cotangent whatever npar and nsave are.  One launch of the VJP
+ * kernel of jq_final_state_vjp (jq_query(h, 0) = 9): its adjoint sweep starts from the last block as in jq_final_state_vjp, and the
+ * cotangent of every earlier saved state jumps into the adjoint when the backward sweep reaches that state (block 0 has no effect).
+ * cot_r, cot_i: [(t*ncot + k)][nsave][n*m]; NULL means zero, not both.  vjp: [(t*ncot + k)][npar] (pFidType 3: the phase entry is 0).
+ * hist_r, hist_i: [t][nsave][n*m], the states the forward sweep saved (bit-identical to jq_eval_forward on kernel 1), or NULL.
+ * With nsave blocks of which only the last is nonzero the result is jq_final_state_vjp's, bit for bit. */
+int jq_history_vjp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                   const double *h0_diag_shift, int32_t save_every, int32_t ncot, const double *cot_r, const double *cot_i,
+                   double *vjp, double *hist_r, double *hist_i);
+
+/* jq_history_jvp: forward mode, the tangent dU_j . d of every saved state along ndir directions per candidate.  One launch of the
+ * forward-sensitivity kernel (jq_query(h, 0) = 8); dirs as in jq_forward_sensitivity.  dhist_r, dhist_i: [(t*ndir + k)][nsave][n*m],
+ * the tangents of Re and Im of U_j (block 0 is zero; block nsave - 1 is jq_forward_sensitivity's dstate, bit for bit).  The Jacobi
+ * solver has no tangent sweep: JQ_ERR_ARG. */
+int jq_history_jvp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                   const double *h0_diag_shift, int32_t save_every, int32_t ndir, const double *dirs,
+                   double *dhist_r, double *dhist_i);
+
 /* evalctrl(params, pcof, td, func) (src/plotstatectrl.jl:246-276): the control functions p_q(t), q_q(t) (rad/ns) of EVERY
  * coupled control q on the time grid `times`, evaluated by the device function the time loop uses (bcarrier2,
  * src/bsplines.jl:211-304).  p, q: [ncoupled][ntimes] doubles, host pointers, blocking. */
@@ -233,8 +262,8 @@ int jq_set_time_segments(jq_handle *h, int32_t nseg);
  * (src/evalobjgrad.jl:745) has at the segment's first step, t_last[p] the value its backward recurrence t = t - dt from T (:810, :919)
  * has at the segment's last step -- bit-identical to what a single sweep sees, not k dt.  Returns the steps of the longest segment. */
 int64_t jq_time_segments(double T, int64_t nsteps, int32_t nseg, double *t_first, double *t_last);
-/* what: 0 = kernel actually used by the last evaluation (1 ... 7, 8 = the forward-sensitivity kernel of jq_forward_sensitivity, or
- * 9 = the final-state VJP kernel of jq_final_state_vjp),
+/* what: 0 = kernel actually used by the last evaluation (1 ... 7, 8 = the forward-sensitivity kernel of jq_forward_sensitivity and
+ * jq_history_jvp, or 9 = the VJP kernel of jq_final_state_vjp and jq_history_vjp),
  * 1 = CUDA-event time of the last evaluation's trajectory kernel(s) in ms (synchronises), 2 = number of kernels launched by the last
  * evaluation,
  * 3 = trajectories resident per CTA, 4 = CTAs launched, 5 = registers per thread, 6 = dynamic smem bytes per CTA,

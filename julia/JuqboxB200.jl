@@ -233,6 +233,29 @@ function final_state_vjp(pcof::Vector{Float64}, params::objparams, wa::Working_A
     return vjp, ur .+ im .* ui
 end
 
+# State-history vector-Jacobian products (jq_history_vjp): for each node and each cotangent c_j = cot_r[:, :, j] + im cot_i[:, :, j] of
+# the saved states U_j (Ntot x N, j = 1 ... nsave, saved every saveEvery steps as in eval_forward; U_1 = Uinit), vjp = the sum over j of
+# cot_r .* dRe U_j / dpcof + cot_i .* dIm U_j / dpcof, one forward and one backward sweep per cotangent whatever Npar and nsave are.
+# cot_r, cot_i are Ntot x N x nsave x ncot x nsamples; returns vjp, Npar x ncot x nsamples, and the history, Ntot x N x nsave x nsamples.
+function history_vjp(pcof::Vector{Float64}, params::objparams, wa::Working_Arrays_B200, cot_r::Array{Float64,5},
+                     cot_i::Array{Float64,5}; nodes::AbstractArray = [0.0], saveEvery::Int = 1)
+    Ntot = params.N + params.Nguard
+    nsamples = length(nodes)
+    params.nsteps % saveEvery == 0 || error("nsteps must be divisible by saveEvery. nsteps=$(params.nsteps), saveEvery=$saveEvery")
+    nsave = params.nsteps ÷ saveEvery + 1
+    size(cot_r) == size(cot_i) && size(cot_r)[1:3] == (Ntot, params.N, nsave) && size(cot_r, 5) == nsamples ||
+        error("history_vjp: cot_r and cot_i must be Ntot x N x nsave x ncot x nsamples")
+    ncot = size(cot_r, 4)
+    Npar = length(pcof)
+    vjp = zeros(Npar, ncot, nsamples)
+    hr = zeros(Ntot, params.N, nsave, nsamples); hi = zeros(Ntot, params.N, nsave, nsamples)
+    jq_check(ccall((:jq_history_vjp, libjq), Cint,
+                   (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Ptr{Float64},
+                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                   wa.handle, 1, pcof, Npar, nsamples, jq_shifts(params, nodes), saveEvery, ncot, cot_r, cot_i, vjp, hr, hi))
+    return vjp, hr .+ im .* hi
+end
+
 
 # ---- the four Ipopt callbacks as ONE ccall each (src/ipopt_interface.jl:77-179): jq_eval_f_grad keeps the last-pcof cache, runs
 # eval_f_g_grad!'s sample loop as one launch and adds the Tikhonov terms on the device.  params.last_* scalars are kept for

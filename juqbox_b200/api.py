@@ -360,6 +360,74 @@ class Working_Arrays:
             out["state"] = (sr + 1j * si).swapaxes(-1, -2)
         return out
 
+    def _history_inputs(self, pcof, shifts, save_every):
+        """pcof, shifts and save_every of the history entries, checked: (pcof, nbatch, npar, nsamples, shifts pointer, nsave)."""
+        p = self.params
+        self._check_params()
+        pcof = np.asarray(pcof)
+        if pcof.ndim != 2:
+            raise ValueError("pcof must be [nbatch, npar]")
+        pcof = _f64(pcof)
+        nbatch, npar = pcof.shape
+        nsamples, sp = 1, None
+        if shifts is not None:
+            shifts = _f64(np.atleast_2d(shifts))
+            if shifts.ndim != 2 or shifts.shape[1] != p.Ntot:
+                raise ValueError("shifts must be [nsamples, Ntot]")
+            nsamples, sp = shifts.shape[0], shifts
+        if int(save_every) != save_every or save_every < 1 or p.nsteps % save_every != 0:
+            raise ValueError(f"nsteps must be divisible by saveEvery. nsteps={p.nsteps}, saveEvery={save_every}")
+        return pcof, nbatch, npar, nsamples, sp, p.nsteps // int(save_every) + 1
+
+    def history_vjp(self, pcof, cot, shifts=None, save_every: int = 1, history: bool = False):
+        """Vector-Jacobian products of the state history (jq_history_vjp): one forward and one backward sweep per cotangent.
+
+        pcof [nbatch, npar]; cot complex [nbatch, nsamples, ncot, nsave, Ntot, N], nsave = nsteps / save_every + 1, where save j is
+        the state after step j * save_every (save 0 is Uinit).  Returns a dict with vjp [nbatch, nsamples, ncot, npar],
+        vjp[b, s, k] = sum over the saves and entries of Re(cot) dRe U_j + Im(cot) dIm U_j by pcof, i.e. dL/dpcof for a real loss L
+        when cot[..., j, :, :] = dL/dRe U_j + i dL/dIm U_j.  With pFidType 3 the last entry (the global phase) is 0.
+        history=True adds history, the saved states, complex [nbatch, nsamples, nsave, Ntot, N]."""
+        p = self.params
+        pcof, nbatch, npar, nsamples, sh, nsave = self._history_inputs(pcof, shifts, save_every)
+        cot = np.asarray(cot)
+        if cot.ndim != 6 or cot.shape[:2] != (nbatch, nsamples) or cot.shape[2] < 1 or cot.shape[3:] != (nsave, p.Ntot, p.N):
+            raise ValueError(f"cot must be [nbatch, nsamples, ncot, nsave, Ntot, N] = [{nbatch}, {nsamples}, ncot >= 1, {nsave}, "
+                             f"{p.Ntot}, {p.N}], not {list(cot.shape)}")
+        ncot = cot.shape[2]
+        cr = _f64(cot.real.swapaxes(-1, -2))                     # the C layout: column-major Ntot x N blocks
+        ci = _f64(cot.imag.swapaxes(-1, -2)) if np.iscomplexobj(cot) else None
+        vjp = np.zeros((nbatch, nsamples, ncot, npar))
+        hr = hi = None
+        if history:
+            hr = np.zeros((nbatch, nsamples, nsave, p.N, p.Ntot))
+            hi = np.zeros_like(hr)
+        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        _lib.check(self._lib.jq_history_vjp(self._handle, nbatch, ptr(pcof), npar, nsamples, ptr(sh), int(save_every), ncot, ptr(cr),
+                                            ptr(ci), ptr(vjp), ptr(hr), ptr(hi)))
+        out = {"vjp": vjp}
+        if history:
+            out["history"] = (hr + 1j * hi).swapaxes(-1, -2)
+        return out
+
+    def history_jvp(self, pcof, dirs, shifts=None, save_every: int = 1):
+        """Tangents of the state history (jq_history_jvp): the forward sweep and its tangent along every direction in one launch.
+
+        pcof [nbatch, npar], dirs [nbatch, ndir, npar] as in forward_sensitivity.  Returns dhistory, complex
+        [nbatch, nsamples, ndir, nsave, Ntot, N]: dhistory[b, s, k, j] = dU_j . dirs[b, k] for the state after step j * save_every."""
+        p = self.params
+        pcof, nbatch, npar, nsamples, sh, nsave = self._history_inputs(pcof, shifts, save_every)
+        dirs = np.asarray(dirs)
+        if dirs.ndim != 3 or dirs.shape[0] != nbatch or dirs.shape[2] != npar or dirs.shape[1] < 1:
+            raise ValueError(f"dirs must be [nbatch, ndir, npar] = [{nbatch}, ndir >= 1, {npar}], not {list(dirs.shape)}")
+        dirs = _f64(dirs)
+        ndir = dirs.shape[1]
+        dr = np.zeros((nbatch, nsamples, ndir, nsave, p.N, p.Ntot))
+        di = np.zeros_like(dr)
+        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        _lib.check(self._lib.jq_history_jvp(self._handle, nbatch, ptr(pcof), npar, nsamples, ptr(sh), int(save_every), ndir, ptr(dirs),
+                                            ptr(dr), ptr(di)))
+        return (dr + 1j * di).swapaxes(-1, -2)
+
     def eval_f_grad(self, pcof, shifts=None, weights=None, tik0: float = 0.0, prior=None):
         """The fused Ipopt-callback entry (jq_eval_f_grad): objective with Tikhonov, its gradient, infidelity, leak and leak
         gradient of ONE pcof in one call, with the last-pcof cache inside the handle.  Returns a dict; `evaluated` is False
@@ -511,6 +579,39 @@ def final_state(wa: Working_Arrays, pcof, shifts=None):
 
         _FinalState = _Fn
     return _FinalState.apply(wa, pcof, shifts)
+
+
+_StateHistory = None
+
+
+def state_history(wa: Working_Arrays, pcof, shifts=None, save_every: int = 1):
+    """The saved states U_j (j = 0 ... nsteps / save_every, save j after step j * save_every) as a differentiable torch function of
+    pcof: a complex tensor [nbatch, nsamples, nsave, Ntot, N] on pcof's device, the axis order of final_state.
+
+    pcof: float64 tensor [nbatch, npar] on any device; shifts: host array [nsamples, Ntot] or None.  The forward pass is
+    wa.forward_history; the backward pass is one wa.history_vjp call with the incoming gradient as the cotangent (summed over the
+    samples, which all share pcof).  First derivatives in reverse mode only."""
+    global _StateHistory
+    import torch
+    if pcof.dim() != 2 or pcof.dtype != torch.float64:
+        raise ValueError("pcof must be a float64 tensor [nbatch, npar]")
+    if _StateHistory is None:
+        class _Fn(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, wa_, pc, sh, se):
+                ctx.wa, ctx.pcof, ctx.shifts, ctx.save_every = wa_, pc.detach().cpu().numpy(), sh, se
+                hist, _, _ = wa_.forward_history(ctx.pcof, sh, save_every=se)
+                return torch.from_numpy(np.ascontiguousarray(hist.swapaxes(-1, -2))).to(pc.device)
+
+            @staticmethod
+            @torch.autograd.function.once_differentiable
+            def backward(ctx, grad_out):
+                cot = grad_out.detach().resolve_conj().cpu().numpy()[:, :, None]
+                g = ctx.wa.history_vjp(ctx.pcof, cot, ctx.shifts, ctx.save_every)["vjp"][:, :, 0].sum(axis=1)
+                return None, torch.from_numpy(g).to(grad_out.device), None, None
+
+        _StateHistory = _Fn
+    return _StateHistory.apply(wa, pcof, shifts, save_every)
 
 
 def eval_forward(pcof0, params: objparams, wa: Working_Arrays, saveEndOnly: bool = True, saveEvery: int = 1):

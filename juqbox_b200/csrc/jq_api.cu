@@ -913,13 +913,19 @@ extern "C" int jq_eval_f_grad(jq_handle *h, const double *pcof, int32_t npar, in
     return 0;
 }
 
+// the saving stride of the history entries (jq_eval_forward, jq_history_vjp, jq_history_jvp)
+static int check_save_every(const jq_handle *h, int save_every) {
+    if (save_every < 1 || h->P.nsteps % save_every != 0)     // src/evalobjgrad.jl:2797-2799
+        return fail(JQ_ERR_ARG, "nsteps must be divisible by saveEvery. nsteps=%lld, saveEvery=%d", (long long)h->P.nsteps, save_every);
+    return 0;
+}
+
 extern "C" int jq_eval_forward(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples, const double *shift,
                                int32_t save_every, double *hist_r, double *hist_i, double *infid, double *leak) {
     int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
     if (rc) return rc;
     if (!hist_r || !hist_i) return fail(JQ_ERR_ARG, "jq_eval_forward: null history buffer");
-    if (save_every < 1 || h->P.nsteps % save_every != 0)     // src/evalobjgrad.jl:2797-2799
-        return fail(JQ_ERR_ARG, "nsteps must be divisible by saveEvery. nsteps=%lld, saveEvery=%d", (long long)h->P.nsteps, save_every);
+    if ((rc = check_save_every(h, save_every)) != 0) return rc;
     CU(cudaSetDevice(h->device));
     const size_t ntraj = (size_t)nbatch * nsamples, len = (size_t)h->n * h->m;
     const long long nsave = h->P.nsteps / save_every + 1;
@@ -1095,7 +1101,7 @@ extern "C" int jq_final_state_vjp(jq_handle *h, int32_t nbatch, const double *pc
 
     VjpArgs V{};
     V.ntraj = (int)ntraj; V.nsamples = nsamples; V.ncot = ncot; V.Npar = nspl; V.D1 = nspl / (2 * h->Nc * h->Nfreq); V.pstride = npar;
-    V.pcof = d_pcof; V.shift = d_shift; V.cot_r = d_cr; V.cot_i = d_ci;
+    V.pcof = d_pcof; V.shift = d_shift; V.cot_r = d_cr; V.cot_i = d_ci; V.save_every = h->P.nsteps; V.nsave = 1;
     V.vjp = h->d_out;
     V.state_r = n_state ? h->d_out + n_vjp : nullptr; V.state_i = n_state ? h->d_out + n_vjp + n_state : nullptr;
     Ran ran;
@@ -1109,6 +1115,131 @@ extern "C" int jq_final_state_vjp(jq_handle *h, int32_t nbatch, const double *pc
     CU(cudaMemcpyAsync(vjp, V.vjp, n_vjp * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (state_r) CU(cudaMemcpyAsync(state_r, V.state_r, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (state_i) CU(cudaMemcpyAsync(state_i, V.state_i, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// grow() for the buffers of the history derivatives, which reach hundreds of MB (cnot3 at save_every = 1: ~128 MB per trajectory and
+// cotangent or direction): a request larger than the device, or one cudaMalloc cannot satisfy, is JQ_ERR_ALLOC with the size
+static int grow_history(double **buf, size_t *cap, double need, const char *who) {
+    size_t free_b = 0, total_b = 0;
+    CU(cudaMemGetInfo(&free_b, &total_b));
+    if (need * sizeof(double) > (double)total_b)
+        return fail(JQ_ERR_ALLOC, "%s: needs %.1f GB in one device buffer, the device has %.1f GB", who, need * sizeof(double) / 1e9,
+                    total_b / 1e9);
+    if ((size_t)need <= *cap) return 0;
+    if (*buf) cudaFree(*buf);
+    *buf = nullptr;
+    *cap = 0;
+    const cudaError_t e = cudaMalloc((void **)buf, (size_t)need * sizeof(double));
+    if (e != cudaSuccess) {
+        *buf = nullptr;
+        cudaGetLastError();
+        return fail(e == cudaErrorMemoryAllocation ? JQ_ERR_ALLOC : JQ_ERR_CUDA, "%s: cudaMalloc of %.1f GB: %s", who,
+                    need * sizeof(double) / 1e9, cudaGetErrorString(e));
+    }
+    *cap = (size_t)need;
+    return 0;
+}
+
+extern "C" int jq_history_vjp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples, const double *shift,
+                              int32_t save_every, int32_t ncot, const double *cot_r, const double *cot_i, double *vjp, double *hist_r,
+                              double *hist_i) {
+    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
+    if (rc) return rc;
+    if ((rc = check_save_every(h, save_every)) != 0) return rc;
+    if (ncot < 1 || (!cot_r && !cot_i)) return fail(JQ_ERR_ARG, "jq_history_vjp: need ncot >= 1 and at least one of cot_r, cot_i");
+    if (!vjp) return fail(JQ_ERR_ARG, "jq_history_vjp: null vjp output");
+    if ((long long)nbatch * nsamples * ncot > 0x7fffffffLL)
+        return fail(JQ_ERR_ARG, "jq_history_vjp: nbatch * nsamples * ncot exceeds 2^31 - 1 trajectories per call");
+    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
+    if (jq_vjp_smem_bytes(h->P, nspl) > 227 * 1024)
+        return fail(JQ_ERR_ARG, "jq_history_vjp: problem too large for the VJP kernel's shared memory (n*m = %d)", h->n * h->m);
+    CU(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    const long long nsave = h->P.nsteps / save_every + 1;
+    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ncot, len = (size_t)h->n * h->m;
+    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)nsamples * h->n : 0;
+    const double n_cot = (double)ntraj * nsave * len, n_hist = (hist_r || hist_i) ? (double)nt * nsave * len : 0.0;
+    const size_t n_vjp = ntraj * npar;
+    if ((rc = grow_history(&h->d_in, &h->cap_in, n_pcof + n_shift + (cot_r ? n_cot : 0) + (cot_i ? n_cot : 0), "jq_history_vjp")) != 0)
+        return rc;
+    if ((rc = grow_history(&h->d_out, &h->cap_out, n_vjp + 2 * n_hist, "jq_history_vjp")) != 0) return rc;
+    double *d_pcof = h->d_in, *cur = d_pcof + n_pcof;
+    double *d_shift = shift ? cur : nullptr; cur += n_shift;
+    double *d_cr = cot_r ? cur : nullptr; cur += cot_r ? (size_t)n_cot : 0;
+    double *d_ci = cot_i ? cur : nullptr;
+    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (cot_r) CU(cudaMemcpyAsync(d_cr, cot_r, (size_t)n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (cot_i) CU(cudaMemcpyAsync(d_ci, cot_i, (size_t)n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
+
+    VjpArgs V{};
+    V.ntraj = (int)ntraj; V.nsamples = nsamples; V.ncot = ncot; V.Npar = nspl; V.D1 = nspl / (2 * h->Nc * h->Nfreq); V.pstride = npar;
+    V.pcof = d_pcof; V.shift = d_shift; V.cot_r = d_cr; V.cot_i = d_ci; V.save_every = save_every; V.nsave = nsave;
+    V.vjp = h->d_out;
+    V.hist_r = n_hist > 0 ? h->d_out + n_vjp : nullptr; V.hist_i = n_hist > 0 ? h->d_out + n_vjp + (size_t)n_hist : nullptr;
+    Ran ran;
+    ran.kernel = 9;
+    CU(cudaEventRecord(h->ev0, st));
+    CU(jq_vjp_launch(h->P, V, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc));
+    CU(cudaEventRecord(h->ev1, st));
+    h->timed = true;
+    h->ran = ran;
+    h->last_launches = 1;
+    CU(cudaMemcpyAsync(vjp, V.vjp, n_vjp * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (hist_r) CU(cudaMemcpyAsync(hist_r, V.hist_r, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (hist_i) CU(cudaMemcpyAsync(hist_i, V.hist_i, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int jq_history_jvp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples, const double *shift,
+                              int32_t save_every, int32_t ndir, const double *dirs, double *dhist_r, double *dhist_i) {
+    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
+    if (rc) return rc;
+    if ((rc = check_save_every(h, save_every)) != 0) return rc;
+    if (ndir < 1 || !dirs) return fail(JQ_ERR_ARG, "jq_history_jvp: need ndir >= 1 and a dirs array");
+    if (!dhist_r || !dhist_i) return fail(JQ_ERR_ARG, "jq_history_jvp: null tangent-history output");
+    if ((long long)nbatch * nsamples * ndir > 0x7fffffffLL)
+        return fail(JQ_ERR_ARG, "jq_history_jvp: nbatch * nsamples * ndir exceeds 2^31 - 1 trajectories per call");
+    if (h->P.solver == 2) return fail(JQ_ERR_ARG, "jq_history_jvp: the Jacobi solver has no tangent sweep (use the Neumann solver)");
+    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
+    if (jq_fwdsens_smem_bytes(h->P, nspl) > 227 * 1024)
+        return fail(JQ_ERR_ARG, "jq_history_jvp: problem too large for the tangent kernel's shared memory (n*m = %d)", h->n * h->m);
+    CU(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    if ((rc = scratch_acquire(h, st)) != 0) return rc;
+    const long long nsave = h->P.nsteps / save_every + 1;
+    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ndir, len = (size_t)h->n * h->m;
+    const size_t n_pcof = (size_t)nbatch * npar, n_dirs = (size_t)nbatch * ndir * npar, n_shift = shift ? (size_t)nsamples * h->n : 0;
+    const double n_hist = (double)ntraj * nsave * len;
+    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_dirs + n_shift)) != 0) return rc;
+    if ((rc = grow_history(&h->d_out, &h->cap_out, 2 * n_hist, "jq_history_jvp")) != 0) return rc;
+    if ((rc = grow(&h->d_scal, &h->cap_traj, nt * 4)) != 0) return rc;
+    if ((rc = grow(&h->d_grad, &h->cap_grad, ntraj)) != 0) return rc;
+    if ((rc = grow(&h->d_igrad, &h->cap_igrad, ntraj)) != 0) return rc;
+    double *d_pcof = h->d_in, *d_dirs = d_pcof + n_pcof, *d_shift = shift ? d_dirs + n_dirs : nullptr;
+    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_dirs, dirs, n_dirs * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
+
+    SensArgs S{};
+    S.ntraj = (int)ntraj; S.nsamples = nsamples; S.ndir = ndir; S.Npar = nspl; S.D1 = nspl / (2 * h->Nc * h->Nfreq); S.pstride = npar;
+    S.pcof = d_pcof; S.dirs = d_dirs; S.shift = d_shift;
+    S.scal = h->d_scal; S.dinfid = h->d_grad; S.dleak = h->d_igrad;         // written by the kernel, not returned
+    S.dhist_r = h->d_out; S.dhist_i = h->d_out + (size_t)n_hist; S.save_every = save_every; S.nsave = nsave;
+    Ran ran;
+    ran.kernel = 8;
+    CU(cudaEventRecord(h->ev0, st));
+    CU(jq_fwdsens_launch(h->P, S, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc));
+    CU(cudaEventRecord(h->ev1, st));
+    h->timed = true;
+    h->ran = ran;
+    h->last_launches = 1;
+    if ((rc = scratch_release(h, st)) != 0) return rc;
+    CU(cudaMemcpyAsync(dhist_r, S.dhist_r, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(dhist_i, S.dhist_i, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return 0;
 }

@@ -97,19 +97,27 @@ struct SensArgs {
     double *scal;          // [nbatch * nsamples][4]: infid, leak, trace_infid, spare (written by direction 0)
     double *dinfid, *dleak;            // [ntraj]: traj = (b * nsamples + s) * ndir + k
     double *dstate_r, *dstate_i;       // [ntraj][n*m] tangents of Re and Im of the final state (vr', -vi'), or nullptr
+    // tangent history: (vr', -vi') at t = 0 (zero) and after every save_every-th step, [ntraj][nsave][n*m], or nullptr
+    double *dhist_r, *dhist_i;
+    int save_every;
+    long long nsave;
 };
 size_t jq_fwdsens_smem_bytes(const DevProblem &P, int Npar);     // one group
 cudaError_t jq_fwdsens_launch(const DevProblem &P, const SensArgs &S, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc);
 
-// ---- final-state VJP kernel (jq_generic.cu): forward sweep, then one unforced adjoint sweep from a caller-supplied cotangent of U(T) ----
+// ---- VJP kernel (jq_generic.cu): forward sweep, then one unforced adjoint sweep from caller-supplied cotangents of the saved states ----
 struct VjpArgs {
     int ntraj, nsamples, ncot, Npar, D1;   // ntraj = nbatch * nsamples * ncot; Npar: spline coefficients (without the pFidType 3 phase)
     int pstride;           // length of every pcof and vjp vector: Npar, or Npar + 1 with the global phase (pFidType 3)
     const double *pcof;    // [nbatch][pstride]
     const double *shift;   // [nsamples][n] or nullptr
-    const double *cot_r, *cot_i;       // [ntraj][n*m] cotangents of Re and Im of U(T), or nullptr (zero); traj = (b * nsamples + s) * ncot + k
+    // [ntraj][nsave][n*m] cotangents of Re and Im of the saved states, or nullptr (zero); traj = (b * nsamples + s) * ncot + k.  Block
+    // nsave - 1 is U(T); block j < nsave - 1 is the state after step j * save_every.  The final-state entry: nsave = 1, save_every = nsteps.
+    const double *cot_r, *cot_i;
+    long long save_every, nsave;
     double *vjp;           // [ntraj][pstride]; the phase entry is 0
     double *state_r, *state_i;         // [nbatch * nsamples][n*m] Re and Im of U(T) (vr, -vi; written by cotangent 0), or nullptr
+    double *hist_r, *hist_i;           // [nbatch * nsamples][nsave][n*m] the saved states as jq_eval_forward writes them (cotangent 0), or nullptr
 };
 size_t jq_vjp_smem_bytes(const DevProblem &P, int Npar);         // one group
 cudaError_t jq_vjp_launch(const DevProblem &P, const VjpArgs &V, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc);

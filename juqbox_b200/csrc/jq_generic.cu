@@ -573,7 +573,7 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_generic_kernel(DevProblem P, L
 // with step_fwdGrad! src/StormerVerlet.jl:151-251 and fgradforce! src/evalobjgrad.jl:2467-2563): the forward sweep and its tangent
 // along a direction d side by side, in the generic kernel's layout.  Trajectory traj = t * ndir + k, t = b * nsamples + s.  The primal
 // statements are the generic kernel's own helpers (TAN = true adds the tangent next to each), so infid / leak are its objective-only
-// outputs bit for bit.
+// outputs bit for bit.  With dhist_r the tangent of every saved state is written as well (jq_history_jvp).
 __global__ void __launch_bounds__(GEN_THREADS) jq_forward_sensitivity_kernel(DevProblem P, SensArgs S, GenGeom G) {
     extern __shared__ __align__(16) double sm[];
     Ctx c{};
@@ -606,6 +606,10 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_forward_sensitivity_kernel(Dev
 
         double dt = P.T / (double)P.nsteps, t = 0.0, pen = 0.0, pend = 0.0;
         const bool densew = P.wreal != nullptr;
+        // tangent history in the generic kernel's hist_r pattern: t = 0 (a zero tangent), then after every save_every-th step
+        double *hdr = S.dhist_r ? S.dhist_r + (size_t)traj * S.nsave * c.len : nullptr;
+        double *hdi = S.dhist_i ? S.dhist_i + (size_t)traj * S.nsave * c.len : nullptr;
+        if (hdr) FOR_E { hdr[e] = td.vr[e]; hdi[e] = -td.vi[e]; }
         for (long long step = 0; step < P.nsteps; ++step) {
             penalty_pre<true>(c, &pen, &td, &pend);
             eval_controls(c, t, dt);
@@ -614,6 +618,10 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_forward_sensitivity_kernel(Dev
             t = t + dt;
             penalty_post<true>(c, &pen, &td, &pend);
             if (densew) gsync(c);
+            if (hdr && (step + 1) % S.save_every == 0) {
+                const size_t o = (size_t)((step + 1) / S.save_every) * c.len;
+                FOR_E { hdr[o + e] = td.vr[e]; hdi[o + e] = -td.vi[e]; }
+            }
         }
         double re, im, red, imd, pv[2] = {pen, pend};
         block_sum(c, pv, 2);
@@ -652,6 +660,9 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_forward_sensitivity_kernel(Dev
 // (the objFuncType 2/3 set) from the terminal condition lambda_r(T) = -c_r / 2, lambda_i(T) = c_i / 2: with c = dinfid/d(Re U, Im U)
 // that is the generic kernel's own terminal condition for every pFidType, so the result is its infidgrad.  Trajectory
 // traj = t * ncot + k, t = b * nsamples + s.
+// State histories (jq_history_vjp): for L = sum_j Re vdot(c_j, U(t_j)) the same sweep is the exact discrete adjoint once the cotangent
+// of every saved state jumps into the node adjoint right after the backward step that recomputes that state (DESIGN.md section 4.8).
+// With nsave = 1 (the final-state entry) no jump fires and the sweep is the one above.
 __global__ void __launch_bounds__(GEN_THREADS) jq_final_state_vjp_kernel(DevProblem P, VjpArgs V, GenGeom G) {
     extern __shared__ __align__(16) double sm[];
     Ctx c{};
@@ -675,18 +686,27 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_final_state_vjp_kernel(DevProb
         gsync(c);
 
         double dt = P.T / (double)P.nsteps, t = 0.0;
+        double *hr = V.hist_r && k_ == 0 ? V.hist_r + (size_t)t_ * V.nsave * c.len : nullptr;
+        double *hi = V.hist_i && k_ == 0 ? V.hist_i + (size_t)t_ * V.nsave * c.len : nullptr;
+        if (hr) FOR_E { hr[e] = c.vr[e]; hi[e] = -c.vi[e]; }
         for (long long step = 0; step < P.nsteps; ++step) {
             eval_controls(c, t, dt);
             state_step(c, dt);
             t = t + dt;
+            if (hr && (step + 1) % V.save_every == 0) {                            // the generic kernel's hist_r pattern
+                const size_t o = (size_t)((step + 1) / V.save_every) * c.len;
+                FOR_E { hr[o + e] = c.vr[e]; hi[o + e] = -c.vi[e]; }
+            }
         }
         if (V.state_r && k_ == 0) {
             double *sr = V.state_r + (size_t)t_ * c.len, *si = V.state_i + (size_t)t_ * c.len;
             FOR_E { sr[e] = c.vr[e]; si[e] = -c.vi[e]; }
         }
-        const double *cr = V.cot_r ? V.cot_r + (size_t)traj * c.len : nullptr, *ci = V.cot_i ? V.cot_i + (size_t)traj * c.len : nullptr;
+        // the cotangent blocks of this trajectory; the last one (U(T)) is the terminal condition
+        const size_t cb = (size_t)traj * V.nsave * c.len, last = (size_t)(V.nsave - 1) * c.len;
+        const double *cr = V.cot_r ? V.cot_r + cb : nullptr, *ci = V.cot_i ? V.cot_i + cb : nullptr;
         FOR_E {
-            const double lr = cr ? -0.5 * cr[e] : 0.0, li = ci ? 0.5 * ci[e] : 0.0;
+            const double lr = cr ? -0.5 * cr[last + e] : 0.0, li = ci ? 0.5 * ci[last + e] : 0.0;
             c.lr[e] = lr; c.lr05[e] = lr; c.li[e] = li; c.li0[e] = li;
         }
         t = P.T;
@@ -701,6 +721,16 @@ __global__ void __launch_bounds__(GEN_THREADS) jq_final_state_vjp_kernel(DevProb
             adjoint_step(c, c.lr, c.li, c.lr05, dt, false, c.tinv);
             grad_step(c, c.lr05, c.li, c.li0, t0, dt, c.grad);
             FOR_E c.li0[e] = c.li[e];
+            // The state is now the one after step `step`.  If it is saved (j = step / save_every >= 1), its cotangent jumps into the
+            // node adjoint (lr, li) with the terminal condition's scaling; li0 is li at the start of the next step, whose traces read it.
+            // lr05 is written before it is read.  Block 0 (Uinit) does not depend on pcof and is never read.
+            if (step > 0 && step % V.save_every == 0) {
+                const size_t o = (size_t)(step / V.save_every) * c.len;
+                FOR_E {
+                    if (cr) c.lr[e] -= 0.5 * cr[o + e];
+                    if (ci) { c.li[e] += 0.5 * ci[o + e]; c.li0[e] = c.li[e]; }
+                }
+            }
             gsync(c);
         }
         double *g = V.vjp + (size_t)traj * V.pstride;
