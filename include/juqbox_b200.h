@@ -188,6 +188,24 @@ int jq_final_state_vjp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t
                        const double *h0_diag_shift, int32_t ncot, const double *cot_r, const double *cot_i,
                        double *vjp, double *state_r, double *state_i);
 
+/* The same vector-Jacobian products on the time-parallel path (kernel 7, DESIGN.md 4.9): the time axis is cut into segments swept
+ * concurrently and joined through their propagators, so one cotangent at batch 1 takes about one time-parallel evaluation instead of two
+ * serial sweeps.  Kernel 7's stages for its unforced adjoint set, started from lambda_r(T) = -cot_r / 2, lambda_i(T) = cot_i / 2 instead
+ * of the objective's terminal adjoint; trajectory (b, s, k) is one kernel-7 trajectory, its propagators computed per cotangent (few
+ * trajectories: the call pattern of one optimizer step).  Arguments, layouts and conventions as jq_final_state_vjp; the results agree
+ * with it to rounding.
+ * ncot = 0: U(T) only (cotangents and vjp ignored; state_r or state_i required), from the state propagators and their join alone.
+ * Host pointers, blocking; never communicates (jq_comm_set_cooperative does not apply) and ignores jq_set_kernel; honours
+ * jq_set_time_segments (0 = automatic, as for kernel 7).  Afterwards jq_query reports kernel 7, the segments (item 7), the launches
+ * (item 2) and the CUDA-event time (item 1).
+ * JQ_ERR_ARG (no launch) for ncot < 0, a NULL required array, nbatch*nsamples*max(ncot, 1) > 2^31 - 1, a problem without kernel 7
+ * (Jacobi solver, dense weights, uncoupled controls, no tile or fibre layout; the message of jq_set_kernel(h, 7)), or, for ncot >= 1,
+ * one whose fibre layout has no segment gradient sweep with the second adjoint set.  JQ_ERR_ALLOC with the size when the segment
+ * workspace does not fit on the device. */
+int jq_final_state_vjp_time_parallel(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                                     const double *h0_diag_shift, int32_t ncot, const double *cot_r, const double *cot_i,
+                                     double *vjp, double *state_r, double *state_i);
+
 /* Derivatives of the state history of jq_eval_forward, U_j = U(t_j) with t_j after step j*save_every, j = 0 ... nsave - 1,
  * nsave = nsteps/save_every + 1 (U_0 = Uinit does not depend on pcof).  A block is a column-major n x m matrix; Re U_j = vr,
  * Im U_j = -vi as in jq_eval_forward.  Both entries use host pointers, block until done, never communicate, and are not affected by
@@ -263,7 +281,7 @@ int jq_set_time_segments(jq_handle *h, int32_t nseg);
  * has at the segment's last step -- bit-identical to what a single sweep sees, not k dt.  Returns the steps of the longest segment. */
 int64_t jq_time_segments(double T, int64_t nsteps, int32_t nseg, double *t_first, double *t_last);
 /* what: 0 = kernel actually used by the last evaluation (1 ... 7, 8 = the forward-sensitivity kernel of jq_forward_sensitivity and
- * jq_history_jvp, or 9 = the VJP kernel of jq_final_state_vjp and jq_history_vjp),
+ * jq_history_jvp, or 9 = the VJP kernel of jq_final_state_vjp and jq_history_vjp; 7 after jq_final_state_vjp_time_parallel),
  * 1 = CUDA-event time of the last evaluation's trajectory kernel(s) in ms (synchronises), 2 = number of kernels launched by the last
  * evaluation,
  * 3 = trajectories resident per CTA, 4 = CTAs launched, 5 = registers per thread, 6 = dynamic smem bytes per CTA,

@@ -216,8 +216,10 @@ end
 # state U(T) (Ntot x N), vjp = sum of cot_r .* dRe U / dpcof + cot_i .* dIm U / dpcof, one backward sweep per cotangent whatever
 # Npar is.  With cot = dL/dRe U + im dL/dIm U this is dL/dpcof for any real loss L of U(T); with pFidType 3 the phase entry is 0.
 # cot_r, cot_i are Ntot x N x ncot x nsamples; returns vjp, Npar x ncot x nsamples, and U(T), Ntot x N x nsamples.
+# time_parallel = true: the same products on the time-parallel path (jq_final_state_vjp_time_parallel, kernel 7), the latency route
+# for one pcof per optimizer step.  Written against the C header but not executed: no Julia was available to build it.
 function final_state_vjp(pcof::Vector{Float64}, params::objparams, wa::Working_Arrays_B200, cot_r::Array{Float64,4},
-                         cot_i::Array{Float64,4}; nodes::AbstractArray = [0.0])
+                         cot_i::Array{Float64,4}; nodes::AbstractArray = [0.0], time_parallel::Bool = false)
     Ntot = params.N + params.Nguard
     nsamples = length(nodes)
     size(cot_r) == size(cot_i) && size(cot_r, 1) == Ntot && size(cot_r, 2) == params.N && size(cot_r, 4) == nsamples ||
@@ -226,10 +228,18 @@ function final_state_vjp(pcof::Vector{Float64}, params::objparams, wa::Working_A
     Npar = length(pcof)
     vjp = zeros(Npar, ncot, nsamples)
     ur = zeros(Ntot, params.N, nsamples); ui = zeros(Ntot, params.N, nsamples)
-    jq_check(ccall((:jq_final_state_vjp, libjq), Cint,
-                   (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Int32, Ptr{Float64}, Ptr{Float64},
-                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
-                   wa.handle, 1, pcof, Npar, nsamples, jq_shifts(params, nodes), ncot, cot_r, cot_i, vjp, ur, ui))
+    shifts = jq_shifts(params, nodes)
+    if time_parallel
+        jq_check(ccall((:jq_final_state_vjp_time_parallel, libjq), Cint,
+                       (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Int32, Ptr{Float64}, Ptr{Float64},
+                        Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                       wa.handle, 1, pcof, Npar, nsamples, shifts, ncot, cot_r, cot_i, vjp, ur, ui))
+    else
+        jq_check(ccall((:jq_final_state_vjp, libjq), Cint,
+                       (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Int32, Ptr{Float64}, Ptr{Float64},
+                        Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                       wa.handle, 1, pcof, Npar, nsamples, shifts, ncot, cot_r, cot_i, vjp, ur, ui))
+    end
     return vjp, ur .+ im .* ui
 end
 

@@ -320,13 +320,17 @@ class Working_Arrays:
             out["dstate"] = (sr + 1j * si).swapaxes(-1, -2)
         return out
 
-    def final_state_vjp(self, pcof, cot, shifts=None, final_state: bool = False):
+    def final_state_vjp(self, pcof, cot, shifts=None, final_state: bool = False, time_parallel: bool = False):
         """Final-state vector-Jacobian products (jq_final_state_vjp): one backward sweep per cotangent of U(T).
 
         pcof [nbatch, npar]; cot complex [nbatch, nsamples, ncot, Ntot, N] (the shape of forward_sensitivity's dstate).  Returns a
         dict with vjp [nbatch, nsamples, ncot, npar], vjp[b, s, k] = sum over the entries of Re(cot) dRe U + Im(cot) dIm U by pcof,
         i.e. dL/dpcof for a real loss L when cot = dL/dRe U + i dL/dIm U (PyTorch's convention for complex outputs).  With pFidType 3
-        the last entry (the global phase) is 0.  final_state=True adds state, U(T) complex [nbatch, nsamples, Ntot, N]."""
+        the last entry (the global phase) is 0.  final_state=True adds state, U(T) complex [nbatch, nsamples, Ntot, N].
+
+        time_parallel=True: the same products on the time-parallel path (jq_final_state_vjp_time_parallel, kernel 7), the latency
+        route for a few trajectories (one optimizer step); it honours set_time_segments.  There cot=None with final_state=True
+        returns U(T) alone."""
         p = self.params
         self._check_params()
         pcof = np.asarray(pcof)
@@ -340,22 +344,27 @@ class Working_Arrays:
             if shifts.ndim != 2 or shifts.shape[1] != p.Ntot:
                 raise ValueError("shifts must be [nsamples, Ntot]")
             nsamples, sp = shifts.shape[0], shifts.ctypes.data_as(C.c_void_p)
-        cot = np.asarray(cot)
-        if cot.ndim != 5 or cot.shape[:2] != (nbatch, nsamples) or cot.shape[2] < 1 or cot.shape[3:] != (p.Ntot, p.N):
-            raise ValueError(f"cot must be [nbatch, nsamples, ncot, Ntot, N] = [{nbatch}, {nsamples}, ncot >= 1, {p.Ntot}, {p.N}], "
-                             f"not {list(cot.shape)}")
-        ncot = cot.shape[2]
-        cr = _f64(cot.real.swapaxes(-1, -2))                     # the C layout: column-major Ntot x N blocks
-        ci = _f64(cot.imag.swapaxes(-1, -2)) if np.iscomplexobj(cot) else None
-        vjp = np.zeros((nbatch, nsamples, ncot, npar))
+        if cot is None:
+            if not (time_parallel and final_state):
+                raise ValueError("cot=None (U(T) only) needs time_parallel=True and final_state=True")
+            ncot, cr, ci = 0, None, None
+        else:
+            cot = np.asarray(cot)
+            if cot.ndim != 5 or cot.shape[:2] != (nbatch, nsamples) or cot.shape[2] < 1 or cot.shape[3:] != (p.Ntot, p.N):
+                raise ValueError(f"cot must be [nbatch, nsamples, ncot, Ntot, N] = [{nbatch}, {nsamples}, ncot >= 1, {p.Ntot}, {p.N}], "
+                                 f"not {list(cot.shape)}")
+            ncot = cot.shape[2]
+            cr = _f64(cot.real.swapaxes(-1, -2))                 # the C layout: column-major Ntot x N blocks
+            ci = _f64(cot.imag.swapaxes(-1, -2)) if np.iscomplexobj(cot) else None
+        vjp = np.zeros((nbatch, nsamples, ncot, npar)) if ncot else None
         sr = si = None
         if final_state:
             sr = np.zeros((nbatch, nsamples, p.N, p.Ntot))
             si = np.zeros_like(sr)
         ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
-        _lib.check(self._lib.jq_final_state_vjp(self._handle, nbatch, ptr(pcof), npar, nsamples, sp, ncot, ptr(cr), ptr(ci), ptr(vjp),
-                                                ptr(sr), ptr(si)))
-        out = {"vjp": vjp}
+        fn = self._lib.jq_final_state_vjp_time_parallel if time_parallel else self._lib.jq_final_state_vjp
+        _lib.check(fn(self._handle, nbatch, ptr(pcof), npar, nsamples, sp, ncot, ptr(cr), ptr(ci), ptr(vjp), ptr(sr), ptr(si)))
+        out = {} if vjp is None else {"vjp": vjp}
         if final_state:
             out["state"] = (sr + 1j * si).swapaxes(-1, -2)
         return out
@@ -552,12 +561,14 @@ def forward_sensitivity(pcof0, params: objparams, wa: Working_Arrays, dirs, node
 _FinalState = None
 
 
-def final_state(wa: Working_Arrays, pcof, shifts=None):
+def final_state(wa: Working_Arrays, pcof, shifts=None, time_parallel: bool = False):
     """U(T) as a differentiable torch function of pcof: a complex tensor [nbatch, nsamples, Ntot, N] on pcof's device.
 
     pcof: float64 tensor [nbatch, npar] on any device; shifts: host array [nsamples, Ntot] or None.  The forward pass is
     wa.forward_history(save_every=nsteps); the backward pass is one wa.final_state_vjp call with the incoming gradient as the
-    cotangent (summed over the samples, which all share pcof).  First derivatives in reverse mode only."""
+    cotangent (summed over the samples, which all share pcof).  time_parallel=True runs both on the time-parallel path (kernel 7,
+    for a few trajectories): the forward pass is the U(T)-only call (cot=None), the backward pass one time-parallel VJP.  First
+    derivatives in reverse mode only."""
     global _FinalState
     import torch
     if pcof.dim() != 2 or pcof.dtype != torch.float64:
@@ -565,20 +576,25 @@ def final_state(wa: Working_Arrays, pcof, shifts=None):
     if _FinalState is None:
         class _Fn(torch.autograd.Function):
             @staticmethod
-            def forward(ctx, wa_, pc, sh):
-                ctx.wa, ctx.pcof, ctx.shifts = wa_, pc.detach().cpu().numpy(), sh
-                hist, _, _ = wa_.forward_history(ctx.pcof, sh, save_every=wa_.params.nsteps)
-                return torch.from_numpy(np.ascontiguousarray(hist[:, :, -1].swapaxes(-1, -2))).to(pc.device)
+            def forward(ctx, wa_, pc, sh, tp):
+                ctx.wa, ctx.pcof, ctx.shifts, ctx.tp = wa_, pc.detach().cpu().numpy(), sh, tp
+                if tp:
+                    U = wa_.final_state_vjp(ctx.pcof, None, sh, final_state=True, time_parallel=True)["state"]
+                else:
+                    hist, _, _ = wa_.forward_history(ctx.pcof, sh, save_every=wa_.params.nsteps)
+                    U = hist[:, :, -1].swapaxes(-1, -2)
+                return torch.from_numpy(np.ascontiguousarray(U)).to(pc.device)
 
             @staticmethod
             @torch.autograd.function.once_differentiable
             def backward(ctx, grad_out):
                 cot = grad_out.detach().resolve_conj().cpu().numpy()[:, :, None]
-                g = ctx.wa.final_state_vjp(ctx.pcof, cot, ctx.shifts)["vjp"][:, :, 0].sum(axis=1)
-                return None, torch.from_numpy(g).to(grad_out.device), None
+                kw = {"time_parallel": True} if ctx.tp else {}
+                g = ctx.wa.final_state_vjp(ctx.pcof, cot, ctx.shifts, **kw)["vjp"][:, :, 0].sum(axis=1)
+                return None, torch.from_numpy(g).to(grad_out.device), None, None
 
         _FinalState = _Fn
-    return _FinalState.apply(wa, pcof, shifts)
+    return _FinalState.apply(wa, pcof, shifts, bool(time_parallel))
 
 
 _StateHistory = None

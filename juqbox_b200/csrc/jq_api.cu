@@ -690,12 +690,30 @@ static int launched(cudaError_t e, bool hand_over, const char *what) {
     return soft && hand_over ? HANDED_OVER : fail(JQ_ERR_CUDA, "%s failed: %s", what, cudaGetErrorString(e));
 }
 
+// Segments of a time-parallel launch of ntraj trajectories: jq_set_time_segments, or automatic (jq_seg_auto_segments)
+static int seg_count(const jq_handle *h, int ntraj, int evaladjoint) {
+    const int nseg = h->seg_nseg > 0 ? h->seg_nseg : jq_seg_auto_segments(h->P, ntraj, evaladjoint, jq_traj_plan_tpc(h->seg_prop), h->sms);
+    return nseg > h->P.nsteps ? (int)h->P.nsteps : nseg;
+}
+
+// Segment start / end times of nseg segments on the device, then the four refinement flags (int): host recurrence, uploaded once per
+// segment count
+static int seg_times_upload(jq_handle *h, int nseg, cudaStream_t st) {
+    if (h->segt_nseg == nseg) return 0;
+    h->segt.resize(2 * (size_t)nseg);
+    jq_seg_times(h->P, nseg, h->segt.data());
+    int rc = grow(&h->d_segt, &h->cap_segt, 2 * (size_t)nseg + 2);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(h->d_segt, h->segt.data(), 2 * (size_t)nseg * sizeof(double), cudaMemcpyHostToDevice, st));
+    h->segt_nseg = nseg;
+    return 0;
+}
+
 // The time-parallel evaluation of `A`
 static int launch_time_parallel(jq_handle *h, const LaunchArgs &A, cudaStream_t st, Ran &ran, bool hand_over) {
     if (h->P.solver != 1 || A.hist_r) return fail(JQ_ERR_ARG, "time-parallel evaluation: Neumann solver, no state history");
     const int tpc = jq_traj_plan_tpc(h->seg_prop);
-    int nseg = h->seg_nseg > 0 ? h->seg_nseg : jq_seg_auto_segments(h->P, A.ntraj, A.evaladjoint, tpc, h->sms);
-    if (nseg > h->P.nsteps) nseg = (int)h->P.nsteps;
+    int nseg = seg_count(h, A.ntraj, A.evaladjoint);
     // cooperative evaluation: the segments are shared out evenly over the ranks (every rank computes the same nseg)
     // ... when the propagator launch is at least two waves of CTAs: below that its collective costs more than it saves
     const long long l1_ctas = 2LL * nseg * (((long long)((2 * h->n + h->m - 1) / h->m) * A.ntraj + tpc - 1) / tpc);
@@ -709,13 +727,7 @@ static int launch_time_parallel(jq_handle *h, const LaunchArgs &A, cudaStream_t 
     SegCoop coop{h->comm_rank, h->comm_size, seg_allgather, h};
     int rc = grow(&h->d_seg, &h->cap_seg, jq_seg_workspace_doubles(h->P, A.ntraj, A.Npar, nseg, A.evaladjoint));
     if (rc) return rc;
-    if (h->segt_nseg != nseg) {           // segment start / end times: host recurrence, once per segment count
-        h->segt.resize(2 * (size_t)nseg);
-        jq_seg_times(h->P, nseg, h->segt.data());
-        if ((rc = grow(&h->d_segt, &h->cap_segt, 2 * (size_t)nseg + 2)) != 0) return rc;      // times, then the four refinement flags
-        CU(cudaMemcpyAsync(h->d_segt, h->segt.data(), 2 * (size_t)nseg * sizeof(double), cudaMemcpyHostToDevice, st));
-        h->segt_nseg = nseg;
-    }
+    if ((rc = seg_times_upload(h, nseg, st)) != 0) return rc;
     ran.nseg = nseg;
     return launched(jq_seg_launch(h->seg_prop, h->route[TIME_PARALLEL].plan, h->seg_obj, h->P, A, nseg, h->d_segt,
                                   reinterpret_cast<int *>(h->d_segt + 2 * (size_t)nseg), h->d_seg, st, coop_on && nseg >= h->comm_size ? &coop : nullptr,
@@ -1240,6 +1252,75 @@ extern "C" int jq_history_jvp(jq_handle *h, int32_t nbatch, const double *pcof, 
     if ((rc = scratch_release(h, st)) != 0) return rc;
     CU(cudaMemcpyAsync(dhist_r, S.dhist_r, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(dhist_i, S.dhist_i, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int jq_final_state_vjp_time_parallel(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                                                const double *shift, int32_t ncot, const double *cot_r, const double *cot_i, double *vjp,
+                                                double *state_r, double *state_i) {
+    static const char *who = "jq_final_state_vjp_time_parallel";
+    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
+    if (rc) return rc;
+    if (ncot < 0) return fail(JQ_ERR_ARG, "%s: need ncot >= 0 (0: U(T) only)", who);
+    if (ncot == 0 && !state_r && !state_i) return fail(JQ_ERR_ARG, "%s: ncot = 0 returns U(T) only and needs state_r or state_i", who);
+    if (ncot > 0 && !cot_r && !cot_i) return fail(JQ_ERR_ARG, "%s: need at least one of cot_r, cot_i", who);
+    if (ncot > 0 && !vjp) return fail(JQ_ERR_ARG, "%s: null vjp output", who);
+    const int nc = std::max<int>(ncot, 1);
+    if ((long long)nbatch * nsamples * nc > 0x7fffffffLL)
+        return fail(JQ_ERR_ARG, "%s: nbatch * nsamples * ncot exceeds 2^31 - 1 trajectories per call", who);
+    if (!h->route[TIME_PARALLEL].ok) return fail(JQ_ERR_ARG, "%s: %s", who, h->route[TIME_PARALLEL].why);
+    // the pulled-back adjoint is the unforced second set of objFuncType 2/3: every launch sees objFuncType 2, whatever the problem's
+    DevProblem P = h->P;
+    P.objFuncType = 2;
+    TrajPlan *fiber = h->route[FIBER].plan;
+    if (ncot > 0 && !jq_seg_supported(fiber, P, true))
+        return fail(JQ_ERR_ARG, "%s: no segment gradient sweep with the second adjoint set (fibre layout) for this problem", who);
+    CU(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    if ((rc = scratch_acquire(h, st)) != 0) return rc;       // the segment workspace is shared with the evaluation entries
+    // trajectory (b, s, k) is kernel-7 trajectory b * nsamples * nc + s * nc + k: sample s * nc + k of candidate b, whose shift row is s
+    const int ns2 = nsamples * nc;
+    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * nc, len = (size_t)h->n * h->m;
+    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)ns2 * h->n : 0, n_cot = ncot > 0 ? ntraj * len : 0;
+    const size_t n_vjp = ncot > 0 ? ntraj * npar : 0, n_state = (state_r || state_i) ? nt * len : 0;
+    const double *cr = ncot > 0 ? cot_r : nullptr, *ci = ncot > 0 ? cot_i : nullptr;
+    const int nseg = seg_count(h, (int)ntraj, 1);
+    const size_t need = jq_seg_vjp_workspace_doubles(P, (int)ntraj, npar - (h->pfid == 3 ? 1 : 0), nseg, ncot > 0);
+    if (need > h->cap_seg && (rc = grow_history(&h->d_seg, &h->cap_seg, (double)need, who)) != 0) return rc;
+    if ((rc = seg_times_upload(h, nseg, st)) != 0) return rc;
+    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_shift + (cr ? n_cot : 0) + (ci ? n_cot : 0))) != 0) return rc;
+    if ((rc = grow(&h->d_out, &h->cap_out, n_vjp + 2 * n_state)) != 0) return rc;
+    double *d_pcof = h->d_in, *cur = d_pcof + n_pcof;
+    double *d_shift = shift ? cur : nullptr; cur += n_shift;
+    double *d_cr = cr ? cur : nullptr; cur += cr ? n_cot : 0;
+    double *d_ci = ci ? cur : nullptr;
+    std::vector<double> shifts(n_shift);
+    for (size_t r = 0; r < (shift ? (size_t)ns2 : 0); ++r) memcpy(&shifts[r * h->n], shift + (r / nc) * h->n, h->n * sizeof(double));
+    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (n_shift) CU(cudaMemcpyAsync(d_shift, shifts.data(), n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (cr) CU(cudaMemcpyAsync(d_cr, cr, n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (ci) CU(cudaMemcpyAsync(d_ci, ci, n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
+    double *o_vjp = n_vjp ? h->d_out : nullptr, *o_sr = n_state ? h->d_out + n_vjp : nullptr, *o_si = n_state ? o_sr + n_state : nullptr;
+
+    const LaunchArgs A = launch_args(h, nbatch, npar, ns2, d_pcof, d_shift);
+    Ran ran;
+    ran.kernel = 7;
+    ran.nseg = nseg;
+    CU(cudaEventRecord(h->ev0, st));
+    rc = launched(jq_seg_vjp_launch(h->seg_prop, h->route[TIME_PARALLEL].plan, fiber, P, A, nseg, h->d_segt,
+                                    reinterpret_cast<int *>(h->d_segt + 2 * (size_t)nseg), h->d_seg, st, ncot, d_cr, d_ci, o_vjp,
+                                    state_r ? o_sr : nullptr, state_i ? o_si : nullptr, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc, &ran.launches),
+                  false, who);
+    if (rc) return rc;
+    CU(cudaEventRecord(h->ev1, st));
+    h->timed = true;
+    h->ran = ran;
+    h->last_launches = ran.launches;
+    if ((rc = scratch_release(h, st)) != 0) return rc;
+    if (n_vjp) CU(cudaMemcpyAsync(vjp, o_vjp, n_vjp * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (state_r) CU(cudaMemcpyAsync(state_r, o_sr, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (state_i) CU(cudaMemcpyAsync(state_i, o_si, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return 0;
 }

@@ -166,3 +166,10 @@ struct SegCoop {
 };
 cudaError_t jq_seg_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_obj, const DevProblem &P, const LaunchArgs &A, int nseg, const double *times, int *flags /* 4 ints, device */, double *work, cudaStream_t st, const SegCoop *coop,
                           int *nctas, int *regs, size_t *smem, int *traj_per_cta, int *nlaunch);
+// Final-state vector-Jacobian products on the segment sweeps (the unforced adjoint set of jq_seg_launch from caller-supplied
+// cotangents; ncot = 0: U(T) only).  P: objFuncType 2 or 3 whatever the problem's own; plan_obj: the two-set gradient sweep.
+size_t jq_seg_vjp_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, bool cotangents);
+cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_obj, const DevProblem &P, const LaunchArgs &A, int nseg,
+                              const double *times, int *flags /* 4 ints, device */, double *work, cudaStream_t st, int ncot,
+                              const double *cot_r, const double *cot_i, double *vjp, double *state_r, double *state_i, int *nctas, int *regs,
+                              size_t *smem, int *traj_per_cta, int *nlaunch);

@@ -366,6 +366,105 @@ __global__ void __launch_bounds__(256) jq_seg_sum_kernel(const LaunchArgs A) {
     }
 }
 
+// Final-state VJP (jq_seg_vjp_launch): the terminal value of the unforced adjoint set from the cotangent c of trajectory tr, kernel 9's
+// terminal condition lambda_r(T) = -c_r / 2, lambda_i(T) = c_i / 2 (NULL part: zero) in the boundary layout, Lam2_nseg = [column][u
+// rows, then v rows]; and U(T) of X_nseg in the ABI layout (Re U = vr, Im U = -vi, column-major n x m), written by cotangent 0 of
+// every (candidate, sample): trajectory tr = t * nc + k.
+__global__ void __launch_bounds__(256) jq_seg_vjp_terminal_kernel(const DevProblem P, const LaunchArgs A, int nc, const double *cot_r,
+                                                                  const double *cot_i, double *state_r, double *state_i) {
+    const int n = P.n, nseg = A.seg.nseg;
+    const size_t nm = (size_t)n * P.m, nv = 2 * nm, total = (size_t)A.ntraj * nm;
+    for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+        const size_t tr = idx / nm, e = idx % nm;
+        const size_t bx = ((size_t)nseg * A.ntraj + tr) * nv + (e / n) * 2 * n + e % n;
+        if (A.seg.Lam2) {
+            A.seg.Lam2[bx] = cot_r ? -0.5 * cot_r[idx] : 0.0;
+            A.seg.Lam2[bx + n] = cot_i ? 0.5 * cot_i[idx] : 0.0;
+        }
+        if (tr % nc == 0) {
+            const size_t o = (tr / nc) * nm + e;
+            if (state_r) state_r[o] = A.seg.X[bx];
+            if (state_i) state_i[o] = -A.seg.X[bx + n];
+        }
+    }
+}
+
+// vjp[tr][k] = sum_p gpart2[p][tr][k] in jq_seg_sum_kernel's fixed order (one warp per entry, lane l sums the segments l, l + 32, ...,
+// then a butterfly); with pFidType 3 the phase entry k = Npar of the pstride-long rows is 0: U(T) does not depend on it
+__global__ void __launch_bounds__(256) jq_seg_vjp_sum_kernel(const LaunchArgs A, double *vjp) {
+    const int nseg = A.seg.nseg, nt = A.ntraj, Npar = A.Npar, lane = threadIdx.x & 31;
+    const long long total = (long long)nt * A.pstride, nwarps = (long long)gridDim.x * (blockDim.x >> 5);
+    for (long long idx = blockIdx.x * (long long)(blockDim.x >> 5) + (threadIdx.x >> 5); idx < total; idx += nwarps) {
+        const int tr = (int)(idx / A.pstride), k = (int)(idx % A.pstride);
+        double s = 0.0;
+        if (k < Npar) { for (int p = lane; p < nseg; p += 32) s += A.seg.gpart2[((size_t)p * nt + tr) * Npar + k]; }
+        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        if (lane == 0) vjp[idx] = s;
+    }
+}
+
+// Join `kind` of the segment boundaries of A (see the kinds above): one warp per (trajectory, column); small matrices: the columns of a
+// trajectory share a CTA, large ones: a CTA (an SM) each
+void run_join(const DevProblem &P, const LaunchArgs &A, int kind, cudaStream_t st) {
+    const size_t n2 = 2 * (size_t)P.n;
+    const long long nwarps = (long long)A.ntraj * P.m;
+    if (n2 <= 32) {
+        // ring of 8 segments per warp: 8 (NV^2 + 32) + 32 doubles -- one warp per CTA for 2n > 16 (68 KB), up to four otherwise
+        constexpr int D = 8;
+        const int NV = n2 <= 8 ? 8 : n2 <= 16 ? 16 : 32;
+        const int wpb = (int)std::min<long long>(NV == 32 ? 1 : 4, nwarps);
+        const unsigned grid = (unsigned)((nwarps + wpb - 1) / wpb);
+        const size_t sm = (size_t)wpb * (D * (NV * NV + 32) + 32) * sizeof(double);
+        void (*k)(const DevProblem, const LaunchArgs, int) =
+            NV == 8 ? jq_seg_chain_small_kernel<8, D> : NV == 16 ? jq_seg_chain_small_kernel<16, D> : jq_seg_chain_small_kernel<32, D>;
+        if (sm > 48 * 1024) cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        k<<<grid, wpb * 32, sm, st>>>(P, A, kind);
+    } else {
+        // cluster version: CS = 8 CTAs per chain, EPC entries each, NG = 256 / EPC row groups, at most 8 matrix entries per thread
+        {
+            const int CS = 8, EPC = (int)((n2 + CS - 1) / CS), NG = EPC <= 256 ? 256 / EPC : 0, kpt = NG ? (int)((n2 + NG - 1) / NG) : 99;
+            const char *cenv = getenv("JQ_SEG_CLUSTER");
+            if ((cenv ? atoi(cenv) != 0 : true) && kpt <= 8) {
+                cudaLaunchConfig_t cfg = {};
+                cfg.gridDim = dim3((unsigned)(nwarps * CS)); cfg.blockDim = dim3(256);
+                cfg.dynamicSmemBytes = (size_t)(2 * n2 + NG * EPC) * sizeof(double); cfg.stream = st;
+                cudaLaunchAttribute at[1];
+                at[0].id = cudaLaunchAttributeClusterDimension;
+                at[0].val.clusterDim.x = CS; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+                cfg.attrs = at; cfg.numAttrs = 1;
+                cudaError_t ce = kpt <= 4 ? cudaLaunchKernelEx(&cfg, jq_seg_chain_cluster_kernel<4, 4>, P, A, kind, EPC, NG)
+                                          : cudaLaunchKernelEx(&cfg, jq_seg_chain_cluster_kernel<8, 4>, P, A, kind, EPC, NG);
+                if (ce == cudaSuccess) return;
+                cudaGetLastError();                     // fall through to the one-CTA kernel
+            }
+        }
+        const int W = (int)((n2 + 31) / 32 * 32), NJ = std::max(1, 1024 / W), cnt = (int)((n2 + NJ - 1) / NJ);
+        const unsigned grid = (unsigned)nwarps, thr = (unsigned)(W * NJ);
+        const size_t sm = (size_t)(W + NJ * W) * sizeof(double);
+        if (cnt <= 8) jq_seg_chain_block_kernel<8><<<grid, thr, sm, st>>>(P, A, kind, W, NJ);
+        else if (cnt <= 16) jq_seg_chain_block_kernel<16><<<grid, thr, sm, st>>>(P, A, kind, W, NJ);
+        else jq_seg_chain_block_kernel<0><<<grid, thr, sm, st>>>(P, A, kind, W, NJ);
+    }
+}
+
+// development: JQ_SEG_TIMING=1 prints the CUDA-event time of every stage of a time-parallel launch
+struct StageTimer {
+    cudaEvent_t ev[12];
+    int nev = 0;
+    const bool on = getenv("JQ_SEG_TIMING") != nullptr;
+    cudaStream_t st;
+    explicit StageTimer(cudaStream_t s) : st(s) {}
+    void mark() { if (on && nev < 12) { cudaEventCreate(&ev[nev]); cudaEventRecord(ev[nev], st); ++nev; } }
+    void print(const char *what) {
+        if (!on) return;
+        cudaStreamSynchronize(st);
+        printf("%s (us):", what);
+        for (int k = 1; k < nev; ++k) { float ms = 0.f; cudaEventElapsedTime(&ms, ev[k - 1], ev[k]); printf(" %.1f", ms * 1e3); }
+        printf("\n");
+    }
+    ~StageTimer() { for (int k = 0; k < nev; ++k) cudaEventDestroy(ev[k]); }
+};
+
 }   // namespace
 
 // Number of segments for a launch of ntraj trajectories.  Per evaluation the sweeps between boundaries cost ~ nsteps / nseg steps of one
@@ -450,59 +549,14 @@ cudaError_t jq_seg_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_ob
             A.seg.gpart2 = take(ns * nt * (size_t)A.Npar);
         }
     }
-    // joins: one warp per (trajectory, column); small matrices: the columns of a trajectory share a CTA, large ones: a CTA (an SM) each
-    const long long nwarps = (long long)nt * P.m;
-    auto run_join = [&](int kind) {
-        if (n2 <= 32) {
-            // ring of 8 segments per warp: 8 (NV^2 + 32) + 32 doubles -- one warp per CTA for 2n > 16 (68 KB), up to four otherwise
-            constexpr int D = 8;
-            const int NV = n2 <= 8 ? 8 : n2 <= 16 ? 16 : 32;
-            const int wpb = (int)std::min<long long>(NV == 32 ? 1 : 4, nwarps);
-            const unsigned grid = (unsigned)((nwarps + wpb - 1) / wpb);
-            const size_t sm = (size_t)wpb * (D * (NV * NV + 32) + 32) * sizeof(double);
-            void (*k)(const DevProblem, const LaunchArgs, int) =
-                NV == 8 ? jq_seg_chain_small_kernel<8, D> : NV == 16 ? jq_seg_chain_small_kernel<16, D> : jq_seg_chain_small_kernel<32, D>;
-            if (sm > 48 * 1024) cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-            k<<<grid, wpb * 32, sm, st>>>(P, A, kind);
-        } else {
-            // cluster version: CS = 8 CTAs per chain, EPC entries each, NG = 256 / EPC row groups, at most 8 matrix entries per thread
-            {
-                const int CS = 8, EPC = (int)((n2 + CS - 1) / CS), NG = EPC <= 256 ? 256 / EPC : 0, kpt = NG ? (int)((n2 + NG - 1) / NG) : 99;
-                const char *cenv = getenv("JQ_SEG_CLUSTER");
-                if ((cenv ? atoi(cenv) != 0 : true) && kpt <= 8) {
-                    cudaLaunchConfig_t cfg = {};
-                    cfg.gridDim = dim3((unsigned)(nwarps * CS)); cfg.blockDim = dim3(256);
-                    cfg.dynamicSmemBytes = (size_t)(2 * n2 + NG * EPC) * sizeof(double); cfg.stream = st;
-                    cudaLaunchAttribute at[1];
-                    at[0].id = cudaLaunchAttributeClusterDimension;
-                    at[0].val.clusterDim.x = CS; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-                    cfg.attrs = at; cfg.numAttrs = 1;
-                    cudaError_t ce = kpt <= 4 ? cudaLaunchKernelEx(&cfg, jq_seg_chain_cluster_kernel<4, 4>, P, A, kind, EPC, NG)
-                                              : cudaLaunchKernelEx(&cfg, jq_seg_chain_cluster_kernel<8, 4>, P, A, kind, EPC, NG);
-                    if (ce == cudaSuccess) return;
-                    cudaGetLastError();                     // fall through to the one-CTA kernel
-                }
-            }
-            const int W = (int)((n2 + 31) / 32 * 32), NJ = std::max(1, 1024 / W), cnt = (int)((n2 + NJ - 1) / NJ);
-            const unsigned grid = (unsigned)nwarps, thr = (unsigned)(W * NJ);
-            const size_t sm = (size_t)(W + NJ * W) * sizeof(double);
-            if (cnt <= 8) jq_seg_chain_block_kernel<8><<<grid, thr, sm, st>>>(P, A, kind, W, NJ);
-            else if (cnt <= 16) jq_seg_chain_block_kernel<16><<<grid, thr, sm, st>>>(P, A, kind, W, NJ);
-            else jq_seg_chain_block_kernel<0><<<grid, thr, sm, st>>>(P, A, kind, W, NJ);
-        }
-    };
     int launches = 0;
     cudaMemsetAsync(flags, 0, 4 * sizeof(int), st);
     if (ld != n2) {            // the padding of the propagators must read as zero
         cudaMemsetAsync(A.seg.Phi, 0, ns * nt * ld * ld * sizeof(double), st);
         if (A.evaladjoint) cudaMemsetAsync(A.seg.Adj, 0, ns * nt * ld * ld * sizeof(double), st);
     }
-    // development: JQ_SEG_TIMING=1 prints the CUDA-event time of every stage
-    cudaEvent_t ev[12];
-    int nev = 0;
-    const bool timing = getenv("JQ_SEG_TIMING") != nullptr;
-    auto mark = [&]() { if (timing && nev < 12) { cudaEventCreate(&ev[nev]); cudaEventRecord(ev[nev], st); ++nev; } };
-    mark();
+    StageTimer timer(st);
+    timer.mark();
     // launch 1: propagators
     A.seg.mode[0] = 1; A.seg.mode[1] = A.evaladjoint ? 3 : 0;
     const bool shared = coop && coop->nranks > 1 && nseg % coop->nranks == 0;
@@ -516,55 +570,153 @@ cudaError_t jq_seg_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_ob
         A.seg.seg_lo = 0; A.seg.seg_cnt = 0;
         launches += A.evaladjoint ? 2 : 1;
     }
-    mark();
-    run_join(0);
-    mark();
+    timer.mark();
+    run_join(P, A, 0, st);
+    timer.mark();
     jq_seg_objective_kernel<<<(unsigned)nt, 256, 0, st>>>(P, A);
-    mark();
+    timer.mark();
     // launch 2: penalty shares; defects of the backward state recomputation
     A.seg.mode[0] = 2; A.seg.mode[1] = A.evaladjoint ? 6 : 0;
     e = jq_traj_launch(plan, P, A, st, nullptr, nullptr, nullptr, nullptr);
     if (e != cudaSuccess) return e;
     launches += 4;
-    mark();
+    timer.mark();
     if (A.evaladjoint) {
-        run_join(2);
+        run_join(P, A, 2, st);
         // refinement passes of the boundary states of the backward sweep: no-ops unless the defects are large (coarse time steps)
         for (int r = 1; r <= 2; ++r) {
             A.seg.pass = r; A.seg.mode[0] = 6; A.seg.mode[1] = 0;
             e = jq_traj_launch(plan, P, A, st, nullptr, nullptr, nullptr, nullptr);
             if (e != cudaSuccess) return e;
-            run_join(3);
+            run_join(P, A, 3, st);
             launches += 2;
         }
         A.seg.pass = 0;
-        mark();
+        timer.mark();
         // launch 3: particular adjoint solutions
         A.seg.mode[0] = 4; A.seg.mode[1] = 0;
         e = jq_traj_launch(plan, P, A, st, nullptr, nullptr, nullptr, nullptr);
         if (e != cudaSuccess) return e;
-        mark();
-        run_join(1);
-        if (P.objFuncType != 1) { run_join(4); ++launches; }
-        mark();
+        timer.mark();
+        run_join(P, A, 1, st);
+        if (P.objFuncType != 1) { run_join(P, A, 4, st); ++launches; }
+        timer.mark();
         // launch 4: gradient shares (objFuncType 2/3: with the second adjoint set, on the plan that has it)
         A.seg.mode[0] = 5; A.seg.mode[1] = 0;
         e = jq_traj_launch(P.objFuncType != 1 ? plan_obj : plan, P, A, st, nullptr, nullptr, nullptr, nullptr);
         if (e != cudaSuccess) return e;
         launches += 4;
-        mark();
+        timer.mark();
     }
     const long long total = (long long)nt * (A.Npar + 1);
     jq_seg_sum_kernel<<<(unsigned)std::min<long long>((total + 7) / 8, 148 * 8), 256, 0, st>>>(A);
     ++launches;
-    mark();
-    if (timing) {
-        cudaStreamSynchronize(st);
-        printf("seg stages (us):");
-        for (int k = 1; k < nev; ++k) { float ms = 0.f; cudaEventElapsedTime(&ms, ev[k - 1], ev[k]); printf(" %.1f", ms * 1e3); }
-        printf("\n");
-        for (int k = 0; k < nev; ++k) cudaEventDestroy(ev[k]);
+    timer.mark();
+    timer.print("seg stages");
+    if (nlaunch) *nlaunch = launches;
+    return cudaGetLastError();
+}
+
+size_t jq_seg_vjp_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, bool cotangents) {
+    const size_t ld = (size_t)jq_seg_ld(P), nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)ntraj, ns = (size_t)nseg;
+    size_t tot = ns * nt * ld * ld + (ns + 1) * nt * nm2;                                               // Phi, X
+    if (cotangents) tot += ns * nt * ld * ld + 2 * (ns + 1) * nt * nm2 + ns * nt * nm2 + 2 * ns * nt * (size_t)Npar;    // Adj, Lam2, Eta, dpart, gpart, gpart2
+    return tot + 16;                                                                                    // even-count padding of every array
+}
+
+// Final-state vector-Jacobian products on the segment sweeps (DESIGN.md §4.9): the stages of jq_seg_launch that the unforced adjoint
+// set (kind 4, Lam2) needs, started from the callers' cotangents instead of the objective's terminal adjoint --
+//   launch 1  Phi_p (mode 1) and, with cotangents, Adj_p (mode 3)
+//   join X    X_{p+1} = Phi_p X_p, then jq_seg_vjp_terminal_kernel: Lam2_nseg from the cotangents, U(T) from X_nseg
+//   launch 2  defect sweeps only (mode 6, pass 0): the penalty plays no part
+//   join Eta  and the two refinement passes
+//   join Lam2 Lam2_p = Adj_p Lam2_{p+1}
+//   launch 4  gradient sweeps (mode 5) on plan_obj, the two-set instantiation: gpart2 is the VJP's share of segment p
+//   sum       vjp = sum_p gpart2 (jq_seg_vjp_sum_kernel)
+// Launch 3 and join Lam (the forced set's particular solutions) are not run: mode 5 still sweeps the forced set next to the unforced
+// one, from Lam = Lam2 (a finite input), and its gpart is discarded.  ncot = 0: launch 1 (Phi only), join X and U(T).
+// P.objFuncType must be 2 or 3, so that mode 5 selects the two-set instantiation (the other modes select the plain ones whatever it is).
+// Trajectory tr = t * nc + k of A, nc = max(ncot, 1), pulls back cotangent k (cot_r, cot_i [tr][n*m], NULL: zero) of candidate x sample
+// t; vjp [tr][A.pstride]; state_r, state_i [t][n*m] or NULL.
+cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_obj, const DevProblem &P, const LaunchArgs &A0, int nseg,
+                              const double *times, int *flags, double *work, cudaStream_t st, int ncot, const double *cot_r,
+                              const double *cot_i, double *vjp, double *state_r, double *state_i, int *nctas, int *regs, size_t *smem,
+                              int *traj_per_cta, int *nlaunch) {
+    if (nseg < 1 || nseg > P.nsteps) return cudaErrorInvalidValue;
+    const bool cot = ncot > 0;
+    if (P.solver != 1 || P.objFuncType == 1 || A0.hist_r || 2 * P.n > 512 || (cot && !plan_obj)) return cudaErrorNotSupported;
+    const size_t n2 = 2 * (size_t)P.n, nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)A0.ntraj, ns = (size_t)nseg;
+    LaunchArgs A = A0;
+    A.evaladjoint = cot ? 1 : 0;
+    A.seg.nseg = nseg;
+    A.seg.times = times;
+    const size_t ld = (size_t)jq_seg_ld(P);
+    A.seg.ld = (int)ld;
+    A.seg.pass = 0;
+    A.seg.flags = flags;
+    A.seg.refine_tol = 1.0e-9 / (double)nseg;              // as in jq_seg_launch
+    double *w = work;
+    auto take = [&](size_t cnt) { double *p = w; w += (cnt + 1) & ~(size_t)1; return p; };
+    A.seg.Phi = take(ns * nt * ld * ld);
+    A.seg.X = take((ns + 1) * nt * nm2);
+    if (cot) {
+        A.seg.Adj = take(ns * nt * ld * ld);
+        A.seg.Lam2 = take((ns + 1) * nt * nm2);
+        A.seg.Eta = take((ns + 1) * nt * nm2);
+        A.seg.dpart = take(ns * nt * nm2);
+        A.seg.gpart = take(ns * nt * (size_t)A.Npar);
+        A.seg.gpart2 = take(ns * nt * (size_t)A.Npar);
+        A.seg.Lam = A.seg.Lam2;
     }
+    int launches = 0;
+    cudaMemsetAsync(flags, 0, 4 * sizeof(int), st);
+    if (ld != n2) {            // the padding of the propagators must read as zero
+        cudaMemsetAsync(A.seg.Phi, 0, ns * nt * ld * ld * sizeof(double), st);
+        if (cot) cudaMemsetAsync(A.seg.Adj, 0, ns * nt * ld * ld * sizeof(double), st);
+    }
+    // Eta_0, which no join writes, enters the refinement passes' defect of segment 0 (dpart_0 feeds nothing, but the flag does): zero,
+    // so that a stale workspace cannot start a pass
+    if (cot) cudaMemsetAsync(A.seg.Eta, 0, nt * nm2 * sizeof(double), st);
+    StageTimer timer(st);
+    timer.mark();
+    A.seg.mode[0] = 1; A.seg.mode[1] = cot ? 3 : 0;
+    cudaError_t e = jq_traj_launch(plan_prop ? plan_prop : plan, P, A, st, nctas, regs, smem, traj_per_cta);
+    if (e != cudaSuccess) return e;
+    timer.mark();
+    run_join(P, A, 0, st);
+    timer.mark();
+    const size_t nel = nt * nm2 / 2;
+    jq_seg_vjp_terminal_kernel<<<(unsigned)std::min<size_t>((nel + 255) / 256, 148 * 8), 256, 0, st>>>(P, A, std::max(ncot, 1), cot_r, cot_i,
+                                                                                                      state_r, state_i);
+    launches += 3;
+    timer.mark();
+    if (cot) {
+        A.seg.mode[0] = 6; A.seg.mode[1] = 0;
+        e = jq_traj_launch(plan, P, A, st, nullptr, nullptr, nullptr, nullptr);
+        if (e != cudaSuccess) return e;
+        run_join(P, A, 2, st);
+        launches += 2;
+        for (int r = 1; r <= 2; ++r) {         // refinement passes: no-ops unless the defects are large (coarse time steps)
+            A.seg.pass = r;
+            e = jq_traj_launch(plan, P, A, st, nullptr, nullptr, nullptr, nullptr);
+            if (e != cudaSuccess) return e;
+            run_join(P, A, 3, st);
+            launches += 2;
+        }
+        A.seg.pass = 0;
+        timer.mark();
+        run_join(P, A, 4, st);
+        timer.mark();
+        A.seg.mode[0] = 5;
+        e = jq_traj_launch(plan_obj, P, A, st, nullptr, nullptr, nullptr, nullptr);
+        if (e != cudaSuccess) return e;
+        timer.mark();
+        const long long total = (long long)nt * A.pstride;
+        jq_seg_vjp_sum_kernel<<<(unsigned)std::min<long long>((total + 7) / 8, 148 * 8), 256, 0, st>>>(A, vjp);
+        launches += 3;
+        timer.mark();
+    }
+    timer.print("seg vjp stages");
     if (nlaunch) *nlaunch = launches;
     return cudaGetLastError();
 }
