@@ -227,6 +227,20 @@ int jq_history_vjp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npa
                    const double *h0_diag_shift, int32_t save_every, int32_t ncot, const double *cot_r, const double *cot_i,
                    double *vjp, double *hist_r, double *hist_i);
 
+/* jq_history_vjp_time_parallel: jq_history_vjp on the time-parallel path (kernel 7), the latency route for one or a few trajectories
+ * (a path-dependent loss inside an optimizer loop).  Arguments, layouts and conventions as jq_history_vjp; the results agree with it to
+ * rounding, and a cotangent history that is nonzero only in its last block gives jq_final_state_vjp_time_parallel's vjp bit for bit at
+ * the same segments.  The cotangent of a save jumps into the segment that recomputes it (DESIGN.md §4.10), so the call costs about one
+ * final-state VJP on kernel 7 whatever nsave is.  ncot = 0: the history only (cotangents and vjp ignored; hist_r or hist_i required).
+ * Semantics and restrictions as jq_final_state_vjp_time_parallel: host pointers, blocking, never communicates, ignores jq_set_kernel,
+ * honours jq_set_time_segments; afterwards jq_query reports kernel 7, the segments, the launches and the event time.  JQ_ERR_ARG (no
+ * launch) for the rejections of both entries (save_every, ncot < 0, NULL required arrays, trajectories, no kernel 7, for ncot >= 1 no
+ * segment gradient sweep with the second adjoint set) and for a layout without segment sweeps carrying the history paths; JQ_ERR_ALLOC
+ * with the size when the workspace and histories do not fit. */
+int jq_history_vjp_time_parallel(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                                 const double *h0_diag_shift, int32_t save_every, int32_t ncot, const double *cot_r,
+                                 const double *cot_i, double *vjp, double *hist_r, double *hist_i);
+
 /* jq_history_jvp: forward mode, the tangent dU_j . d of every saved state along ndir directions per candidate.  One launch of the
  * forward-sensitivity kernel (jq_query(h, 0) = 8); dirs as in jq_forward_sensitivity.  dhist_r, dhist_i: [(t*ndir + k)][nsave][n*m],
  * the tangents of Re and Im of U_j (block 0 is zero; block nsave - 1 is jq_forward_sensitivity's dstate, bit for bit).  The Jacobi
@@ -281,7 +295,8 @@ int jq_set_time_segments(jq_handle *h, int32_t nseg);
  * has at the segment's last step -- bit-identical to what a single sweep sees, not k dt.  Returns the steps of the longest segment. */
 int64_t jq_time_segments(double T, int64_t nsteps, int32_t nseg, double *t_first, double *t_last);
 /* what: 0 = kernel actually used by the last evaluation (1 ... 7, 8 = the forward-sensitivity kernel of jq_forward_sensitivity and
- * jq_history_jvp, or 9 = the VJP kernel of jq_final_state_vjp and jq_history_vjp; 7 after jq_final_state_vjp_time_parallel),
+ * jq_history_jvp, or 9 = the VJP kernel of jq_final_state_vjp and jq_history_vjp; 7 after jq_final_state_vjp_time_parallel and
+ * jq_history_vjp_time_parallel),
  * 1 = CUDA-event time of the last evaluation's trajectory kernel(s) in ms (synchronises), 2 = number of kernels launched by the last
  * evaluation,
  * 3 = trajectories resident per CTA, 4 = CTAs launched, 5 = registers per thread, 6 = dynamic smem bytes per CTA,

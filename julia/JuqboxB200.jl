@@ -247,8 +247,10 @@ end
 # the saved states U_j (Ntot x N, j = 1 ... nsave, saved every saveEvery steps as in eval_forward; U_1 = Uinit), vjp = the sum over j of
 # cot_r .* dRe U_j / dpcof + cot_i .* dIm U_j / dpcof, one forward and one backward sweep per cotangent whatever Npar and nsave are.
 # cot_r, cot_i are Ntot x N x nsave x ncot x nsamples; returns vjp, Npar x ncot x nsamples, and the history, Ntot x N x nsave x nsamples.
+# time_parallel = true: the same products on the time-parallel path (jq_history_vjp_time_parallel, kernel 7), the latency route for
+# one pcof per optimizer step.  Written against the C header but not executed: no Julia was available to build it.
 function history_vjp(pcof::Vector{Float64}, params::objparams, wa::Working_Arrays_B200, cot_r::Array{Float64,5},
-                     cot_i::Array{Float64,5}; nodes::AbstractArray = [0.0], saveEvery::Int = 1)
+                     cot_i::Array{Float64,5}; nodes::AbstractArray = [0.0], saveEvery::Int = 1, time_parallel::Bool = false)
     Ntot = params.N + params.Nguard
     nsamples = length(nodes)
     params.nsteps % saveEvery == 0 || error("nsteps must be divisible by saveEvery. nsteps=$(params.nsteps), saveEvery=$saveEvery")
@@ -259,10 +261,17 @@ function history_vjp(pcof::Vector{Float64}, params::objparams, wa::Working_Array
     Npar = length(pcof)
     vjp = zeros(Npar, ncot, nsamples)
     hr = zeros(Ntot, params.N, nsave, nsamples); hi = zeros(Ntot, params.N, nsave, nsamples)
-    jq_check(ccall((:jq_history_vjp, libjq), Cint,
-                   (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Ptr{Float64},
-                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
-                   wa.handle, 1, pcof, Npar, nsamples, jq_shifts(params, nodes), saveEvery, ncot, cot_r, cot_i, vjp, hr, hi))
+    if time_parallel
+        jq_check(ccall((:jq_history_vjp_time_parallel, libjq), Cint,
+                       (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Ptr{Float64},
+                        Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                       wa.handle, 1, pcof, Npar, nsamples, jq_shifts(params, nodes), saveEvery, ncot, cot_r, cot_i, vjp, hr, hi))
+    else
+        jq_check(ccall((:jq_history_vjp, libjq), Cint,
+                       (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Int32, Int32, Ptr{Float64}, Ptr{Float64},
+                        Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                       wa.handle, 1, pcof, Npar, nsamples, jq_shifts(params, nodes), saveEvery, ncot, cot_r, cot_i, vjp, hr, hi))
+    end
     return vjp, hr .+ im .* hi
 end
 

@@ -388,32 +388,42 @@ class Working_Arrays:
             raise ValueError(f"nsteps must be divisible by saveEvery. nsteps={p.nsteps}, saveEvery={save_every}")
         return pcof, nbatch, npar, nsamples, sp, p.nsteps // int(save_every) + 1
 
-    def history_vjp(self, pcof, cot, shifts=None, save_every: int = 1, history: bool = False):
+    def history_vjp(self, pcof, cot, shifts=None, save_every: int = 1, history: bool = False, time_parallel: bool = False):
         """Vector-Jacobian products of the state history (jq_history_vjp): one forward and one backward sweep per cotangent.
 
         pcof [nbatch, npar]; cot complex [nbatch, nsamples, ncot, nsave, Ntot, N], nsave = nsteps / save_every + 1, where save j is
         the state after step j * save_every (save 0 is Uinit).  Returns a dict with vjp [nbatch, nsamples, ncot, npar],
         vjp[b, s, k] = sum over the saves and entries of Re(cot) dRe U_j + Im(cot) dIm U_j by pcof, i.e. dL/dpcof for a real loss L
         when cot[..., j, :, :] = dL/dRe U_j + i dL/dIm U_j.  With pFidType 3 the last entry (the global phase) is 0.
-        history=True adds history, the saved states, complex [nbatch, nsamples, nsave, Ntot, N]."""
+        history=True adds history, the saved states, complex [nbatch, nsamples, nsave, Ntot, N].
+
+        time_parallel=True: the same products on the time-parallel path (jq_history_vjp_time_parallel, kernel 7), the latency route
+        for a few trajectories (one optimizer step); it honours set_time_segments.  There cot=None with history=True returns the
+        saved states alone."""
         p = self.params
         pcof, nbatch, npar, nsamples, sh, nsave = self._history_inputs(pcof, shifts, save_every)
-        cot = np.asarray(cot)
-        if cot.ndim != 6 or cot.shape[:2] != (nbatch, nsamples) or cot.shape[2] < 1 or cot.shape[3:] != (nsave, p.Ntot, p.N):
-            raise ValueError(f"cot must be [nbatch, nsamples, ncot, nsave, Ntot, N] = [{nbatch}, {nsamples}, ncot >= 1, {nsave}, "
-                             f"{p.Ntot}, {p.N}], not {list(cot.shape)}")
-        ncot = cot.shape[2]
-        cr = _f64(cot.real.swapaxes(-1, -2))                     # the C layout: column-major Ntot x N blocks
-        ci = _f64(cot.imag.swapaxes(-1, -2)) if np.iscomplexobj(cot) else None
-        vjp = np.zeros((nbatch, nsamples, ncot, npar))
+        if cot is None:
+            if not (time_parallel and history):
+                raise ValueError("cot=None (the history only) needs time_parallel=True and history=True")
+            ncot, cr, ci = 0, None, None
+        else:
+            cot = np.asarray(cot)
+            if cot.ndim != 6 or cot.shape[:2] != (nbatch, nsamples) or cot.shape[2] < 1 or cot.shape[3:] != (nsave, p.Ntot, p.N):
+                raise ValueError(f"cot must be [nbatch, nsamples, ncot, nsave, Ntot, N] = [{nbatch}, {nsamples}, ncot >= 1, {nsave}, "
+                                 f"{p.Ntot}, {p.N}], not {list(cot.shape)}")
+            ncot = cot.shape[2]
+            cr = _f64(cot.real.swapaxes(-1, -2))                 # the C layout: column-major Ntot x N blocks
+            ci = _f64(cot.imag.swapaxes(-1, -2)) if np.iscomplexobj(cot) else None
+        vjp = np.zeros((nbatch, nsamples, ncot, npar)) if ncot else None
         hr = hi = None
         if history:
             hr = np.zeros((nbatch, nsamples, nsave, p.N, p.Ntot))
             hi = np.zeros_like(hr)
         ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
-        _lib.check(self._lib.jq_history_vjp(self._handle, nbatch, ptr(pcof), npar, nsamples, ptr(sh), int(save_every), ncot, ptr(cr),
-                                            ptr(ci), ptr(vjp), ptr(hr), ptr(hi)))
-        out = {"vjp": vjp}
+        fn = self._lib.jq_history_vjp_time_parallel if time_parallel else self._lib.jq_history_vjp
+        _lib.check(fn(self._handle, nbatch, ptr(pcof), npar, nsamples, ptr(sh), int(save_every), ncot, ptr(cr), ptr(ci), ptr(vjp),
+                      ptr(hr), ptr(hi)))
+        out = {} if vjp is None else {"vjp": vjp}
         if history:
             out["history"] = (hr + 1j * hi).swapaxes(-1, -2)
         return out
@@ -600,13 +610,15 @@ def final_state(wa: Working_Arrays, pcof, shifts=None, time_parallel: bool = Fal
 _StateHistory = None
 
 
-def state_history(wa: Working_Arrays, pcof, shifts=None, save_every: int = 1):
+def state_history(wa: Working_Arrays, pcof, shifts=None, save_every: int = 1, time_parallel: bool = False):
     """The saved states U_j (j = 0 ... nsteps / save_every, save j after step j * save_every) as a differentiable torch function of
     pcof: a complex tensor [nbatch, nsamples, nsave, Ntot, N] on pcof's device, the axis order of final_state.
 
     pcof: float64 tensor [nbatch, npar] on any device; shifts: host array [nsamples, Ntot] or None.  The forward pass is
     wa.forward_history; the backward pass is one wa.history_vjp call with the incoming gradient as the cotangent (summed over the
-    samples, which all share pcof).  First derivatives in reverse mode only."""
+    samples, which all share pcof).  time_parallel=True runs both on the time-parallel path (kernel 7, for a few trajectories): the
+    forward pass is the history-only call (cot=None), the backward pass one time-parallel history VJP.  First derivatives in reverse
+    mode only."""
     global _StateHistory
     import torch
     if pcof.dim() != 2 or pcof.dtype != torch.float64:
@@ -614,20 +626,24 @@ def state_history(wa: Working_Arrays, pcof, shifts=None, save_every: int = 1):
     if _StateHistory is None:
         class _Fn(torch.autograd.Function):
             @staticmethod
-            def forward(ctx, wa_, pc, sh, se):
-                ctx.wa, ctx.pcof, ctx.shifts, ctx.save_every = wa_, pc.detach().cpu().numpy(), sh, se
-                hist, _, _ = wa_.forward_history(ctx.pcof, sh, save_every=se)
-                return torch.from_numpy(np.ascontiguousarray(hist.swapaxes(-1, -2))).to(pc.device)
+            def forward(ctx, wa_, pc, sh, se, tp):
+                ctx.wa, ctx.pcof, ctx.shifts, ctx.save_every, ctx.tp = wa_, pc.detach().cpu().numpy(), sh, se, tp
+                if tp:
+                    H = wa_.history_vjp(ctx.pcof, None, sh, se, history=True, time_parallel=True)["history"]
+                else:
+                    H = wa_.forward_history(ctx.pcof, sh, save_every=se)[0].swapaxes(-1, -2)
+                return torch.from_numpy(np.ascontiguousarray(H)).to(pc.device)
 
             @staticmethod
             @torch.autograd.function.once_differentiable
             def backward(ctx, grad_out):
                 cot = grad_out.detach().resolve_conj().cpu().numpy()[:, :, None]
-                g = ctx.wa.history_vjp(ctx.pcof, cot, ctx.shifts, ctx.save_every)["vjp"][:, :, 0].sum(axis=1)
-                return None, torch.from_numpy(g).to(grad_out.device), None, None
+                kw = {"time_parallel": True} if ctx.tp else {}
+                g = ctx.wa.history_vjp(ctx.pcof, cot, ctx.shifts, ctx.save_every, **kw)["vjp"][:, :, 0].sum(axis=1)
+                return None, torch.from_numpy(g).to(grad_out.device), None, None, None
 
         _StateHistory = _Fn
-    return _StateHistory.apply(wa, pcof, shifts, save_every)
+    return _StateHistory.apply(wa, pcof, shifts, save_every, bool(time_parallel))
 
 
 def eval_forward(pcof0, params: objparams, wa: Working_Arrays, saveEndOnly: bool = True, saveEvery: int = 1):

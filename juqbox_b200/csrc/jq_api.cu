@@ -1256,14 +1256,18 @@ extern "C" int jq_history_jvp(jq_handle *h, int32_t nbatch, const double *pcof, 
     return 0;
 }
 
-extern "C" int jq_final_state_vjp_time_parallel(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
-                                                const double *shift, int32_t ncot, const double *cot_r, const double *cot_i, double *vjp,
-                                                double *state_r, double *state_i) {
-    static const char *who = "jq_final_state_vjp_time_parallel";
+// The VJP entries on the time-parallel path: cotangents [traj][nsave][n*m] of the saved states (nsave = 1, save_every = nsteps: of U(T),
+// whose stages jq_seg_vjp_launch runs unchanged); ncot = 0 returns U(T) (state) and / or the history alone.  `history`: the history
+// entry's rejections and buffers, sized by nsave.
+static int vjp_time_parallel(jq_handle *h, const char *who, bool history, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                             const double *shift, int32_t save_every, int32_t ncot, const double *cot_r, const double *cot_i, double *vjp,
+                             double *state_r, double *state_i, double *hist_r, double *hist_i) {
     int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
     if (rc) return rc;
-    if (ncot < 0) return fail(JQ_ERR_ARG, "%s: need ncot >= 0 (0: U(T) only)", who);
-    if (ncot == 0 && !state_r && !state_i) return fail(JQ_ERR_ARG, "%s: ncot = 0 returns U(T) only and needs state_r or state_i", who);
+    if (history && (rc = check_save_every(h, save_every)) != 0) return rc;
+    if (ncot < 0) return fail(JQ_ERR_ARG, "%s: need ncot >= 0 (0: %s only)", who, history ? "the history" : "U(T)");
+    if (ncot == 0 && !history && !state_r && !state_i) return fail(JQ_ERR_ARG, "%s: ncot = 0 returns U(T) only and needs state_r or state_i", who);
+    if (ncot == 0 && history && !hist_r && !hist_i) return fail(JQ_ERR_ARG, "%s: ncot = 0 returns the history only and needs hist_r or hist_i", who);
     if (ncot > 0 && !cot_r && !cot_i) return fail(JQ_ERR_ARG, "%s: need at least one of cot_r, cot_i", who);
     if (ncot > 0 && !vjp) return fail(JQ_ERR_ARG, "%s: null vjp output", who);
     const int nc = std::max<int>(ncot, 1);
@@ -1274,34 +1278,42 @@ extern "C" int jq_final_state_vjp_time_parallel(jq_handle *h, int32_t nbatch, co
     DevProblem P = h->P;
     P.objFuncType = 2;
     TrajPlan *fiber = h->route[FIBER].plan;
-    if (ncot > 0 && !jq_seg_supported(fiber, P, true))
+    if (ncot > 0 && !jq_seg_supported(fiber, P, true, history))
         return fail(JQ_ERR_ARG, "%s: no segment gradient sweep with the second adjoint set (fibre layout) for this problem", who);
+    if (history && !jq_seg_supported(h->route[TIME_PARALLEL].plan, P, false, true))
+        return fail(JQ_ERR_ARG, "%s: no segment sweep with the history paths for this problem's layout", who);
     CU(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
     if ((rc = scratch_acquire(h, st)) != 0) return rc;       // the segment workspace is shared with the evaluation entries
     // trajectory (b, s, k) is kernel-7 trajectory b * nsamples * nc + s * nc + k: sample s * nc + k of candidate b, whose shift row is s
     const int ns2 = nsamples * nc;
+    const long long nsave = history ? h->P.nsteps / save_every + 1 : 1;
     const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * nc, len = (size_t)h->n * h->m;
-    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)ns2 * h->n : 0, n_cot = ncot > 0 ? ntraj * len : 0;
+    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)ns2 * h->n : 0;
+    const double n_cot = ncot > 0 ? (double)ntraj * nsave * len : 0.0;
     const size_t n_vjp = ncot > 0 ? ntraj * npar : 0, n_state = (state_r || state_i) ? nt * len : 0;
+    const double n_hist = (hist_r || hist_i) ? (double)nt * nsave * len : 0.0;
     const double *cr = ncot > 0 ? cot_r : nullptr, *ci = ncot > 0 ? cot_i : nullptr;
     const int nseg = seg_count(h, (int)ntraj, 1);
-    const size_t need = jq_seg_vjp_workspace_doubles(P, (int)ntraj, npar - (h->pfid == 3 ? 1 : 0), nseg, ncot > 0);
+    const size_t need = jq_seg_vjp_workspace_doubles(P, (int)ntraj, npar - (h->pfid == 3 ? 1 : 0), nseg, ncot > 0, nsave > 1);
     if (need > h->cap_seg && (rc = grow_history(&h->d_seg, &h->cap_seg, (double)need, who)) != 0) return rc;
     if ((rc = seg_times_upload(h, nseg, st)) != 0) return rc;
-    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_shift + (cr ? n_cot : 0) + (ci ? n_cot : 0))) != 0) return rc;
-    if ((rc = grow(&h->d_out, &h->cap_out, n_vjp + 2 * n_state)) != 0) return rc;
+    // histories reach hundreds of MB: JQ_ERR_ALLOC with the size when they do not fit
+    auto grow_io = [&](double **buf, size_t *cap, double cnt) { return history ? grow_history(buf, cap, cnt, who) : grow(buf, cap, (size_t)cnt); };
+    if ((rc = grow_io(&h->d_in, &h->cap_in, n_pcof + n_shift + (cr ? n_cot : 0) + (ci ? n_cot : 0))) != 0) return rc;
+    if ((rc = grow_io(&h->d_out, &h->cap_out, n_vjp + 2 * n_state + 2 * n_hist)) != 0) return rc;
     double *d_pcof = h->d_in, *cur = d_pcof + n_pcof;
     double *d_shift = shift ? cur : nullptr; cur += n_shift;
-    double *d_cr = cr ? cur : nullptr; cur += cr ? n_cot : 0;
+    double *d_cr = cr ? cur : nullptr; cur += cr ? (size_t)n_cot : 0;
     double *d_ci = ci ? cur : nullptr;
     std::vector<double> shifts(n_shift);
     for (size_t r = 0; r < (shift ? (size_t)ns2 : 0); ++r) memcpy(&shifts[r * h->n], shift + (r / nc) * h->n, h->n * sizeof(double));
     CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
     if (n_shift) CU(cudaMemcpyAsync(d_shift, shifts.data(), n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (cr) CU(cudaMemcpyAsync(d_cr, cr, n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (ci) CU(cudaMemcpyAsync(d_ci, ci, n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (cr) CU(cudaMemcpyAsync(d_cr, cr, (size_t)n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (ci) CU(cudaMemcpyAsync(d_ci, ci, (size_t)n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
     double *o_vjp = n_vjp ? h->d_out : nullptr, *o_sr = n_state ? h->d_out + n_vjp : nullptr, *o_si = n_state ? o_sr + n_state : nullptr;
+    double *o_hr = n_hist > 0 ? h->d_out + n_vjp + 2 * n_state : nullptr, *o_hi = n_hist > 0 ? o_hr + (size_t)n_hist : nullptr;
 
     const LaunchArgs A = launch_args(h, nbatch, npar, ns2, d_pcof, d_shift);
     Ran ran;
@@ -1309,8 +1321,9 @@ extern "C" int jq_final_state_vjp_time_parallel(jq_handle *h, int32_t nbatch, co
     ran.nseg = nseg;
     CU(cudaEventRecord(h->ev0, st));
     rc = launched(jq_seg_vjp_launch(h->seg_prop, h->route[TIME_PARALLEL].plan, fiber, P, A, nseg, h->d_segt,
-                                    reinterpret_cast<int *>(h->d_segt + 2 * (size_t)nseg), h->d_seg, st, ncot, d_cr, d_ci, o_vjp,
-                                    state_r ? o_sr : nullptr, state_i ? o_si : nullptr, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc, &ran.launches),
+                                    reinterpret_cast<int *>(h->d_segt + 2 * (size_t)nseg), h->d_seg, st, ncot,
+                                    history ? save_every : (int)h->P.nsteps, nsave, d_cr, d_ci, o_vjp, state_r ? o_sr : nullptr,
+                                    state_i ? o_si : nullptr, o_hr, o_hi, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc, &ran.launches),
                   false, who);
     if (rc) return rc;
     CU(cudaEventRecord(h->ev1, st));
@@ -1321,6 +1334,22 @@ extern "C" int jq_final_state_vjp_time_parallel(jq_handle *h, int32_t nbatch, co
     if (n_vjp) CU(cudaMemcpyAsync(vjp, o_vjp, n_vjp * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (state_r) CU(cudaMemcpyAsync(state_r, o_sr, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (state_i) CU(cudaMemcpyAsync(state_i, o_si, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (hist_r) CU(cudaMemcpyAsync(hist_r, o_hr, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (hist_i) CU(cudaMemcpyAsync(hist_i, o_hi, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return 0;
+}
+
+extern "C" int jq_final_state_vjp_time_parallel(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                                                const double *shift, int32_t ncot, const double *cot_r, const double *cot_i, double *vjp,
+                                                double *state_r, double *state_i) {
+    return vjp_time_parallel(h, "jq_final_state_vjp_time_parallel", false, nbatch, pcof, npar, nsamples, shift, 0, ncot, cot_r, cot_i, vjp,
+                             state_r, state_i, nullptr, nullptr);
+}
+
+extern "C" int jq_history_vjp_time_parallel(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                                            const double *shift, int32_t save_every, int32_t ncot, const double *cot_r, const double *cot_i,
+                                            double *vjp, double *hist_r, double *hist_i) {
+    return vjp_time_parallel(h, "jq_history_vjp_time_parallel", true, nbatch, pcof, npar, nsamples, shift, save_every, ncot, cot_r, cot_i,
+                             vjp, nullptr, nullptr, hist_r, hist_i);
 }

@@ -40,15 +40,18 @@ struct DevProblem {
 
 // Time-parallel evaluation (jq_seg.cu): the time axis is cut into nseg segments, every segment is swept by its own sub-trajectories
 // and the segments are joined through the discrete propagators (the one-step maps are linear in the state / the adjoint).
-// What the CTAs of one trajectory-kernel launch do: CTAs [0, ctas0) run mode[0], the others mode[1] (0 = none)
+// What the CTAs of one trajectory-kernel launch do: CTAs [0, ctas0) run mode[0], the others mode[1] (0 = none; SegHist adds a third)
 //   1 forward sweep of a block of m unit vectors of R^2n           -> Phi   (state propagator of the segment, column by column)
-//   2 forward sweep of the true state from X[seg]                  -> penpart (the segment's share of the guard-level penalty)
+//   2 forward sweep of the true state from X[seg]                  -> penpart (the segment's share of the guard-level penalty); with
+//     LaunchArgs::hist_r (SegHist) also the saved states in (k0, k1], segment 0 also block 0, and penpart may be nullptr
 //   3 adjoint sweep without forcing from a block of unit vectors   -> Adj   (homogeneous adjoint propagator)
 //   4 backward sweep (state from Xb[seg+1], zero terminal adjoint) -> cpart (particular adjoint solution at the segment start)
 //   5 backward sweep (state from Xb[seg+1], adjoint from Lam[seg+1]) -> gpart (the segment's share of the gradient)
 //   6 backward state sweep of the true state from X[seg+1]         -> dpart = J (state reached - X[seg]), J (u; v) = (v; -u): the
 //     defect of the backward recomputation, from which the join builds Xb = X + J' Eta, the states the reference's backward sweep
 //     sees (its time recurrence from T is shifted against the forward one by the rounding of nsteps additions, ~1e-10)
+//   7 adjoint sweep without forcing from zero with the cotangent jumps of SegHist -> cpart (history VJP: the particular solution of
+//     the unforced set; it needs no state)
 // Layouts: Phi, Adj [seg][traj][ld (unit vector j)][ld (u rows, then v rows)]; X, Lam, Eta, cpart, dpart [seg][traj][m (column)][2n
 // (u rows, then v rows)] (X, Lam, Eta have nseg + 1 boundary entries); gpart [seg][traj][Npar]; penpart [seg][traj].
 struct SegArgs {
@@ -63,6 +66,19 @@ struct SegArgs {
     double refine_tol;
     const double *times;   // [2][nseg]: time at the first step of segment p in the reference's forward recurrence t = t + dt from 0, and at
                            // its last step in the backward recurrence t = t - dt from T (jq_seg_times): the sweeps see bit-identical times
+};
+
+// History VJP on the segment sweeps (jq_seg_vjp_launch).  A separate argument of jq_traj_launch, stored at the end of TrajParams, so
+// that the parameter layout of every other kernel stays as it was; a launch with it runs the HIST instantiations, which alone carry
+// the history paths (the saves of mode 2, mode 7, the jumps of mode 5).
+//   mode2, ctas1: a third mode for the CTAs [ctas1, grid) of the launch (0 = none)
+//   hist_nc:      mode 2 with LaunchArgs::hist_r writes the saves of trajectories tr % hist_nc == 0 into history row tr / hist_nc
+//   cot_r, cot_i: cotangents [traj][nsave][n*m] of the saved states (LaunchArgs::save_every, nsave), or nullptr.  When one is set,
+//                 modes 5 (second adjoint set) and 7 add the cotangent of save j >= 1 after the iteration that recomputes state
+//                 j * save_every: lambda_r -= c_r[j] / 2, lambda_i += c_i[j] / 2 (DESIGN.md §4.10)
+struct SegHist {
+    int mode2, ctas1, hist_nc;
+    const double *cot_r, *cot_i;
 };
 
 // Per-launch arguments common to both kernels.
@@ -146,10 +162,11 @@ void jq_traj_plan_destroy(TrajPlan *);
 int jq_traj_plan_tpc(const TrajPlan *);      // trajectories per CTA
 int jq_traj_plan_lanes(const TrajPlan *);    // lanes per trajectory
 cudaError_t jq_traj_launch(TrajPlan *plan, const DevProblem &P, const LaunchArgs &A, cudaStream_t st, int *nctas, int *regs,
-                           size_t *smem, int *traj_per_cta);
+                           size_t *smem, int *traj_per_cta, const SegHist *hist = nullptr);
 
 // ---- time-parallel evaluation (jq_seg.cu): segment sweeps on a trajectory plan, joined through the segment propagators ----
-bool jq_seg_supported(const TrajPlan *plan, const DevProblem &P, bool second_adjoint = false);      // the plan has segment-sweep instantiations
+// the plan has segment-sweep instantiations (hist: with the history VJP's paths)
+bool jq_seg_supported(const TrajPlan *plan, const DevProblem &P, bool second_adjoint = false, bool hist = false);
 int jq_seg_ld(const DevProblem &P);
 int jq_seg_auto_segments(const DevProblem &P, int ntraj, int evaladjoint, int tpc, int sms);
 size_t jq_seg_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, int evaladjoint);
@@ -166,10 +183,12 @@ struct SegCoop {
 };
 cudaError_t jq_seg_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_obj, const DevProblem &P, const LaunchArgs &A, int nseg, const double *times, int *flags /* 4 ints, device */, double *work, cudaStream_t st, const SegCoop *coop,
                           int *nctas, int *regs, size_t *smem, int *traj_per_cta, int *nlaunch);
-// Final-state vector-Jacobian products on the segment sweeps (the unforced adjoint set of jq_seg_launch from caller-supplied
-// cotangents; ncot = 0: U(T) only).  P: objFuncType 2 or 3 whatever the problem's own; plan_obj: the two-set gradient sweep.
-size_t jq_seg_vjp_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, bool cotangents);
+// Vector-Jacobian products of the saved states on the segment sweeps (the unforced adjoint set of jq_seg_launch from caller-supplied
+// cotangents [traj][nsave][n*m]; nsave = 1, save_every = nsteps: of U(T) alone; ncot = 0: U(T) and / or the history only).  P:
+// objFuncType 2 or 3 whatever the problem's own; plan_obj: the two-set gradient sweep.
+size_t jq_seg_vjp_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, bool cotangents, bool jumps);
 cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_obj, const DevProblem &P, const LaunchArgs &A, int nseg,
                               const double *times, int *flags /* 4 ints, device */, double *work, cudaStream_t st, int ncot,
-                              const double *cot_r, const double *cot_i, double *vjp, double *state_r, double *state_i, int *nctas, int *regs,
-                              size_t *smem, int *traj_per_cta, int *nlaunch);
+                              int save_every, long long nsave, const double *cot_r, const double *cot_i, double *vjp, double *state_r,
+                              double *state_i, double *hist_r, double *hist_i, int *nctas, int *regs, size_t *smem, int *traj_per_cta,
+                              int *nlaunch);

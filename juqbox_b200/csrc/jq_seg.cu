@@ -366,20 +366,21 @@ __global__ void __launch_bounds__(256) jq_seg_sum_kernel(const LaunchArgs A) {
     }
 }
 
-// Final-state VJP (jq_seg_vjp_launch): the terminal value of the unforced adjoint set from the cotangent c of trajectory tr, kernel 9's
-// terminal condition lambda_r(T) = -c_r / 2, lambda_i(T) = c_i / 2 (NULL part: zero) in the boundary layout, Lam2_nseg = [column][u
-// rows, then v rows]; and U(T) of X_nseg in the ABI layout (Re U = vr, Im U = -vi, column-major n x m), written by cotangent 0 of
-// every (candidate, sample): trajectory tr = t * nc + k.
+// VJP (jq_seg_vjp_launch): the terminal value of the unforced adjoint set from the cotangent c of trajectory tr (cot_r + tr * cstride,
+// the last block of a cotangent history), kernel 9's terminal condition lambda_r(T) = -c_r / 2, lambda_i(T) = c_i / 2 (NULL part: zero)
+// in the boundary layout, Lam2_nseg = [column][u rows, then v rows]; and U(T) of X_nseg in the ABI layout (Re U = vr, Im U = -vi,
+// column-major n x m), written by cotangent 0 of every (candidate, sample): trajectory tr = t * nc + k.
 __global__ void __launch_bounds__(256) jq_seg_vjp_terminal_kernel(const DevProblem P, const LaunchArgs A, int nc, const double *cot_r,
-                                                                  const double *cot_i, double *state_r, double *state_i) {
+                                                                  const double *cot_i, size_t cstride, double *state_r, double *state_i) {
     const int n = P.n, nseg = A.seg.nseg;
     const size_t nm = (size_t)n * P.m, nv = 2 * nm, total = (size_t)A.ntraj * nm;
     for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
         const size_t tr = idx / nm, e = idx % nm;
         const size_t bx = ((size_t)nseg * A.ntraj + tr) * nv + (e / n) * 2 * n + e % n;
         if (A.seg.Lam2) {
-            A.seg.Lam2[bx] = cot_r ? -0.5 * cot_r[idx] : 0.0;
-            A.seg.Lam2[bx + n] = cot_i ? 0.5 * cot_i[idx] : 0.0;
+            const size_t c = tr * cstride + e;
+            A.seg.Lam2[bx] = cot_r ? -0.5 * cot_r[c] : 0.0;
+            A.seg.Lam2[bx + n] = cot_i ? 0.5 * cot_i[c] : 0.0;
         }
         if (tr % nc == 0) {
             const size_t o = (tr / nc) * nm + e;
@@ -617,34 +618,42 @@ cudaError_t jq_seg_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_ob
     return cudaGetLastError();
 }
 
-size_t jq_seg_vjp_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, bool cotangents) {
+size_t jq_seg_vjp_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, bool cotangents, bool jumps) {
     const size_t ld = (size_t)jq_seg_ld(P), nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)ntraj, ns = (size_t)nseg;
     size_t tot = ns * nt * ld * ld + (ns + 1) * nt * nm2;                                               // Phi, X
     if (cotangents) tot += ns * nt * ld * ld + 2 * (ns + 1) * nt * nm2 + ns * nt * nm2 + 2 * ns * nt * (size_t)Npar;    // Adj, Lam2, Eta, dpart, gpart, gpart2
-    return tot + 16;                                                                                    // even-count padding of every array
+    if (cotangents && jumps) tot += ns * nt * nm2;                                                      // cpart
+    return tot + 18;                                                                                    // even-count padding of every array
 }
 
-// Final-state vector-Jacobian products on the segment sweeps (DESIGN.md §4.9): the stages of jq_seg_launch that the unforced adjoint
-// set (kind 4, Lam2) needs, started from the callers' cotangents instead of the objective's terminal adjoint --
+// Vector-Jacobian products of the saved states on the segment sweeps (DESIGN.md §4.9, §4.10): the stages of jq_seg_launch that the
+// unforced adjoint set (kind 4, Lam2) needs, started from the callers' cotangents instead of the objective's terminal adjoint --
 //   launch 1  Phi_p (mode 1) and, with cotangents, Adj_p (mode 3)
-//   join X    X_{p+1} = Phi_p X_p, then jq_seg_vjp_terminal_kernel: Lam2_nseg from the cotangents, U(T) from X_nseg
-//   launch 2  defect sweeps only (mode 6, pass 0): the penalty plays no part
-//   join Eta  and the two refinement passes
-//   join Lam2 Lam2_p = Adj_p Lam2_{p+1}
-//   launch 4  gradient sweeps (mode 5) on plan_obj, the two-set instantiation: gpart2 is the VJP's share of segment p
+//   join X    X_{p+1} = Phi_p X_p, then jq_seg_vjp_terminal_kernel: Lam2_nseg from the last cotangent block, U(T) from X_nseg
+//   launch 2  the saved states (mode 2, with a history; no penalty shares: penpart is nullptr), defect sweeps (mode 6, pass 0; the penalty plays no part) and, with jumps,
+//             the particular solutions of the unforced set (mode 7): adjoint sweeps from zero with the segment's cotangent jumps
+//   join Eta  and the two refinement passes (mode 6 only)
+//   join Lam2 Lam2_p = Adj_p Lam2_{p+1} (kind 4), with jumps Lam2_p = Adj_p Lam2_{p+1} + c_p (kind 1 with Lam = Lam2, cpart = c)
+//   launch 4  gradient sweeps (mode 5) on plan_obj, the two-set instantiation, jumps applied to the second set: gpart2 is the VJP's
+//             share of segment p
 //   sum       vjp = sum_p gpart2 (jq_seg_vjp_sum_kernel)
 // Launch 3 and join Lam (the forced set's particular solutions) are not run: mode 5 still sweeps the forced set next to the unforced
-// one, from Lam = Lam2 (a finite input), and its gpart is discarded.  ncot = 0: launch 1 (Phi only), join X and U(T).
+// one, from Lam = Lam2 (a finite input), and its gpart is discarded.  A save at global step k belongs to the segment p with
+// k0 <= k < k1: its jump is in c_p, so Lam2_p contains it; save nsave - 1 is the terminal value, save 0 has no effect.
+// ncot = 0: launch 1 (Phi only), join X, then U(T) and / or the history.
 // P.objFuncType must be 2 or 3, so that mode 5 selects the two-set instantiation (the other modes select the plain ones whatever it is).
-// Trajectory tr = t * nc + k of A, nc = max(ncot, 1), pulls back cotangent k (cot_r, cot_i [tr][n*m], NULL: zero) of candidate x sample
-// t; vjp [tr][A.pstride]; state_r, state_i [t][n*m] or NULL.
+// Trajectory tr = t * nc + k of A, nc = max(ncot, 1), pulls back cotangent k (cot_r, cot_i [tr][nsave][n*m], NULL: zero) of
+// candidate x sample t; nsave = 1 (save_every = nsteps): the final-state VJP, whose stages and arithmetic do not depend on this
+// function's history arguments.  vjp [tr][A.pstride]; state_r, state_i [t][n*m] or NULL; hist_r, hist_i [t][nsave][n*m] or NULL.
 cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_obj, const DevProblem &P, const LaunchArgs &A0, int nseg,
-                              const double *times, int *flags, double *work, cudaStream_t st, int ncot, const double *cot_r,
-                              const double *cot_i, double *vjp, double *state_r, double *state_i, int *nctas, int *regs, size_t *smem,
-                              int *traj_per_cta, int *nlaunch) {
+                              const double *times, int *flags, double *work, cudaStream_t st, int ncot, int save_every, long long nsave,
+                              const double *cot_r, const double *cot_i, double *vjp, double *state_r, double *state_i, double *hist_r,
+                              double *hist_i, int *nctas, int *regs, size_t *smem, int *traj_per_cta, int *nlaunch) {
     if (nseg < 1 || nseg > P.nsteps) return cudaErrorInvalidValue;
-    const bool cot = ncot > 0;
+    if (save_every < 1 || nsave < 1) return cudaErrorInvalidValue;
+    const bool cot = ncot > 0, jumps = cot && nsave > 1 && (cot_r || cot_i), hist = hist_r || hist_i;
     if (P.solver != 1 || P.objFuncType == 1 || A0.hist_r || 2 * P.n > 512 || (cot && !plan_obj)) return cudaErrorNotSupported;
+    if (hist && !(hist_r && hist_i)) return cudaErrorInvalidValue;
     const size_t n2 = 2 * (size_t)P.n, nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)A0.ntraj, ns = (size_t)nseg;
     LaunchArgs A = A0;
     A.evaladjoint = cot ? 1 : 0;
@@ -667,7 +676,14 @@ cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *pla
         A.seg.gpart = take(ns * nt * (size_t)A.Npar);
         A.seg.gpart2 = take(ns * nt * (size_t)A.Npar);
         A.seg.Lam = A.seg.Lam2;
+        if (jumps) A.seg.cpart = take(ns * nt * nm2);
     }
+    // the history VJP's additions to the launches: the saves of mode 2 (cotangent 0 of every (candidate, sample)), the third mode of
+    // launch 2 and the cotangent jumps of modes 7 and 5
+    SegHist H{};
+    H.hist_nc = std::max(ncot, 1);
+    if (jumps) { H.cot_r = cot_r; H.cot_i = cot_i; }
+    const size_t nm = nm2 / 2;
     int launches = 0;
     cudaMemsetAsync(flags, 0, 4 * sizeof(int), st);
     if (ld != n2) {            // the padding of the propagators must read as zero
@@ -684,18 +700,35 @@ cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *pla
     if (e != cudaSuccess) return e;
     timer.mark();
     run_join(P, A, 0, st);
+    launches += 2;
     timer.mark();
-    const size_t nel = nt * nm2 / 2;
-    jq_seg_vjp_terminal_kernel<<<(unsigned)std::min<size_t>((nel + 255) / 256, 148 * 8), 256, 0, st>>>(P, A, std::max(ncot, 1), cot_r, cot_i,
-                                                                                                      state_r, state_i);
-    launches += 3;
-    timer.mark();
-    if (cot) {
-        A.seg.mode[0] = 6; A.seg.mode[1] = 0;
-        e = jq_traj_launch(plan, P, A, st, nullptr, nullptr, nullptr, nullptr);
+    if (cot || state_r || state_i) {
+        const size_t nel = nt * nm;
+        jq_seg_vjp_terminal_kernel<<<(unsigned)std::min<size_t>((nel + 255) / 256, 148 * 8), 256, 0, st>>>(
+            P, A, std::max(ncot, 1), cot_r ? cot_r + (size_t)(nsave - 1) * nm : nullptr, cot_i ? cot_i + (size_t)(nsave - 1) * nm : nullptr,
+            (size_t)nsave * nm, state_r, state_i);
+        ++launches;
+        timer.mark();
+    }
+    if (hist || cot) {         // launch 2: the modes of this call, in the order 2, 6, 7
+        int modes[3] = {0, 0, 0}, k = 0;
+        if (hist) modes[k++] = 2;
+        if (cot) modes[k++] = 6;
+        if (jumps) modes[k++] = 7;
+        A.seg.mode[0] = modes[0]; A.seg.mode[1] = modes[1]; H.mode2 = modes[2];
+        if (hist) { A.hist_r = hist_r; A.hist_i = hist_i; A.save_every = save_every; A.nsave = nsave; }
+        if (jumps) { A.save_every = save_every; A.nsave = nsave; }
+        e = jq_traj_launch(plan, P, A, st, nullptr, nullptr, nullptr, nullptr, hist || jumps ? &H : nullptr);
         if (e != cudaSuccess) return e;
+        A.hist_r = A.hist_i = nullptr;
+        H.mode2 = 0;
+        ++launches;
+        timer.mark();
+    }
+    if (cot) {
         run_join(P, A, 2, st);
-        launches += 2;
+        ++launches;
+        A.seg.mode[0] = 6; A.seg.mode[1] = 0;
         for (int r = 1; r <= 2; ++r) {         // refinement passes: no-ops unless the defects are large (coarse time steps)
             A.seg.pass = r;
             e = jq_traj_launch(plan, P, A, st, nullptr, nullptr, nullptr, nullptr);
@@ -705,10 +738,10 @@ cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *pla
         }
         A.seg.pass = 0;
         timer.mark();
-        run_join(P, A, 4, st);
+        run_join(P, A, jumps ? 1 : 4, st);
         timer.mark();
         A.seg.mode[0] = 5;
-        e = jq_traj_launch(plan_obj, P, A, st, nullptr, nullptr, nullptr, nullptr);
+        e = jq_traj_launch(plan_obj, P, A, st, nullptr, nullptr, nullptr, nullptr, jumps ? &H : nullptr);
         if (e != cudaSuccess) return e;
         timer.mark();
         const long long total = (long long)nt * A.pstride;

@@ -17,13 +17,13 @@ const InstPart kInstA = inst_part(kInst);
 // with glt == 0 serves any group size, a query with nw == 0 takes the entry's own warp count, pipe is compared as zero / non-zero.
 const Inst *find_inst(const InstKey &want, int J) {
     for (int jt : {J, 0})
-        for (const InstPart *part : {&kInstA, &kInstB, &kInstC, &kInstD, &kInstE, &kInstF})
+        for (const InstPart *part : {&kInstA, &kInstB, &kInstC, &kInstD, &kInstE, &kInstF, &kInstG})
             for (const Inst *i = part->inst; i < part->inst + part->count; ++i) {
                 const InstKey &k = i->key;
                 if (k.kind == want.kind && k.R == want.R && k.C == want.C && k.NC == want.NC && k.WQ == want.WQ && k.LMASK == want.LMASK &&
                     k.UPL == want.UPL && k.obj2 == want.obj2 && k.jacobi == want.jacobi && k.hx == want.hx &&
                     k.general_hanti == want.general_hanti && k.NF == want.NF && k.jt == jt && (k.glt == 0 || k.glt == want.glt) &&
-                    (want.nw == 0 || k.nw == want.nw) && (k.pipe != 0) == (want.pipe != 0) && k.seg == want.seg) return i;
+                    (want.nw == 0 || k.nw == want.nw) && (k.pipe != 0) == (want.pipe != 0) && k.seg == want.seg && k.hist == want.hist) return i;
             }
     return nullptr;
 }
@@ -390,11 +390,12 @@ void jq_traj_plan_destroy(TrajPlan *pl) {
 
 // Segment-sweep instantiations exist only for Neumann problems on non-pipelined 4-warp (tile: their own) plans without drift
 // couplings and with the ladder form of Hanti.
-bool jq_seg_supported(const TrajPlan *pl, const DevProblem &P, bool second_adjoint) {
+bool jq_seg_supported(const TrajPlan *pl, const DevProblem &P, bool second_adjoint, bool hist) {
     if (!pl || 2 * P.n > 512) return false;
     InstKey want = query(pl->key, P);
     want.seg = 1;
     want.obj2 = second_adjoint;
+    want.hist = hist;
     return find_inst(want, P.J) != nullptr;
 }
 
@@ -402,13 +403,14 @@ int jq_traj_plan_tpc(const TrajPlan *pl) { return pl ? pl->TPC : 0; }
 int jq_traj_plan_lanes(const TrajPlan *pl) { return pl ? pl->GPT * pl->key.glt : 0; }
 
 cudaError_t jq_traj_launch(TrajPlan *pl, const DevProblem &P, const LaunchArgs &A, cudaStream_t st, int *nctas, int *regs,
-                           size_t *smem, int *traj_per_cta) {
+                           size_t *smem, int *traj_per_cta, const SegHist *hist) {
     // never substitute: Neumann for Jacobi, one adjoint set for two, no drift couplings
     InstKey want = query(pl->key, P);
     const bool seg = A.seg.nseg > 0;
     if (seg) {                  // segment sweeps of the time-parallel evaluation
-        if (A.hist_r) return cudaErrorNotSupported;
+        if (A.hist_r && !hist) return cudaErrorNotSupported;
         want.seg = 1;
+        want.hist = hist != nullptr;        // the history VJP's paths live in their own instantiations
         // objFuncType 2/3: only the gradient sweep (mode 5) carries the second adjoint set; every other mode is the plain one
         want.obj2 = want.obj2 && A.seg.mode[0] == 5;
     }
@@ -417,6 +419,7 @@ cudaError_t jq_traj_launch(TrajPlan *pl, const DevProblem &P, const LaunchArgs &
     if (!inst || (inst->key.jt != 0 && inst->key.jt != P.J)) return cudaErrorNotSupported;
     TrajParams S{};
     S.P = P; S.A = A;
+    if (seg && hist) S.H = *hist;
     S.NL = pl->NL; S.NLR = pl->NLR; S.GL = pl->key.glt; S.GPT = pl->GPT; S.CPG = pl->CPG;
     S.plan_i = pl->d_i; S.plan_d = pl->d_d; S.plan_d0 = pl->d_d0; S.plan_w = pl->d_w;
     S.exch_per_unit = pl->exch_per_unit;
@@ -469,10 +472,11 @@ cudaError_t jq_traj_launch(TrajPlan *pl, const DevProblem &P, const LaunchArgs &
             const long long per = (mode == 1 || mode == 3) ? (long long)nblk * A.ntraj : (long long)A.ntraj;
             return (long long)(A.seg.seg_cnt > 0 ? A.seg.seg_cnt : A.seg.nseg) * ((per + TPC - 1) / TPC);
         };
-        const long long c0 = ctas(A.seg.mode[0]), c1 = ctas(A.seg.mode[1]);
-        if (c0 + c1 > 0x7fffffffLL || c0 + c1 < 1) return cudaErrorInvalidConfiguration;
+        const long long c0 = ctas(A.seg.mode[0]), c1 = ctas(A.seg.mode[1]), c2 = ctas(S.H.mode2);
+        if (c0 + c1 + c2 > 0x7fffffffLL || c0 + c1 + c2 < 1) return cudaErrorInvalidConfiguration;
         S.A.seg.ctas0 = (int)c0;
-        grid = (int)(c0 + c1);
+        S.H.ctas1 = (int)(c0 + c1);
+        grid = (int)(c0 + c1 + c2);
     }
     inst->fn<<<grid, (pipe == 1 ? 3 * nw + 1 : pipe == 2 ? 2 * nw : nw) * 32, bytes, st>>>(S);
     if (nctas) *nctas = grid;

@@ -59,6 +59,7 @@ struct TrajParams {
     int GPW;                                 // groups per warp (32 / GL, rounded down: GL need not be a power of two)
     // pipelined (PIPE) instantiations: state-role and adjoint-role warps of one CTA
     int o_ring, o_cnt, tab_role_stride;      // rings of (vr0, vi05, vr) and of lane-partial traces, the int step / chunk counters, size of one control-table buffer
+    SegHist H;                               // HIST instantiations: the history VJP's launch arguments (zero otherwise)
 };
 
 typedef void (*traj_kernel_t)(const TrajParams);
@@ -71,18 +72,19 @@ typedef void (*traj_kernel_t)(const TrajParams);
 //   ladder form (AS = 0);
 //   glt group size (entry: compile-time, 0 = any); jt Neumann terms compiled in (0 = run-time J; a query passes J instead);
 //   nw warps per CTA and role (query: 0 = the entry's own); pipe pipelined roles (matched as zero / non-zero); seg segment sweep
-//   of the time-parallel evaluation.
+//   of the time-parallel evaluation; hist segment sweep with the history VJP's paths (SegHist).
 struct InstKey {
     int kind, R, C, NC, WQ, LMASK, UPL;
     bool obj2 = false, jacobi = false, hx = false, general_hanti = false;
     int glt = 0, jt = 0, nw = TRAJ_WARPS, pipe = 0, seg = 0;
     int NF = 0;
+    bool hist = false;
 };
 struct Inst { InstKey key; traj_kernel_t fn; };
 // The instantiation table is split over jq_traj.cu and the jq_traj_inst_*.cu files so that they compile in parallel.
 struct InstPart { const Inst *inst; int count; };
 template <int N> constexpr InstPart inst_part(const Inst (&t)[N]) { return {t, N}; }
-extern const InstPart kInstB, kInstC, kInstD, kInstE, kInstF;
+extern const InstPart kInstB, kInstC, kInstD, kInstE, kInstF, kInstG;
 
 struct TrajPlan {
     InstKey key;                             // glt: the group size GL; nw: warps per CTA (per role), 0 for the instantiation's own
@@ -1047,11 +1049,17 @@ __device__ __forceinline__ void grad_scatter(Updater (&U)[UPL], double *gsm, con
 // SEG = true (time-parallel evaluation, jq_seg.cu): every CTA sweeps ONE segment of the time axis in one of the modes of SegArgs --
 // forward from a block of unit vectors or from the true boundary state, adjoint without forcing from unit vectors, or the backward
 // sweep between two known boundaries -- with the same steppers on the same lane layout.
-template <class LaneT, int UPL, int MINB = 1, int JT = 0, int OBJ = 0, int GLT = 0, int NW = TRAJ_WARPS, int PIPE_ = 0, bool SEG = false>
+//
+// HIST = true (segment sweeps of the history VJP, jq_seg_vjp_launch with a SegHist): mode 2 also saves the states, mode 7 sweeps the
+// particular solutions with the cotangent jumps, mode 5 applies the jumps to the second adjoint set.  Separate instantiations, so that
+// the ones kernel 7's evaluation and the final-state VJP run keep their code.
+template <class LaneT, int UPL, int MINB = 1, int JT = 0, int OBJ = 0, int GLT = 0, int NW = TRAJ_WARPS, int PIPE_ = 0, bool SEG = false,
+          bool HIST = false>
 __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW : NW) * 32, MINB) jq_traj_kernel(const __grid_constant__ TrajParams S) {
     constexpr int E = LaneT::E, NC = LaneT::NC;
     constexpr bool PIPE = PIPE_ != 0;
     static_assert(!SEG || PIPE_ == 0, "segment sweeps: plain layout");
+    static_assert(!HIST || SEG, "history paths: segment sweeps only");
     // PIPE_ = 1: roles state | adjoint | gradient + one table warp; PIPE_ = 2 (shapes whose register budget allows 8 warps only):
     // state and adjoint in one role, and the gradient role also produces the control tables in the slack of its own steps
     constexpr int NR = PIPE_ == 1 ? 3 : PIPE_ == 2 ? 2 : 1, R_ADJ = PIPE_ == 1 ? 1 : 0, R_GRAD = NR - 1;
@@ -1078,6 +1086,7 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
         const int part = b >= A.seg.ctas0 ? 1 : 0;
         if (part) b -= A.seg.ctas0;
         smode = A.seg.mode[part];
+        if constexpr (HIST) { if (S.H.mode2 != 0 && (int)blockIdx.x >= S.H.ctas1) { smode = S.H.mode2; b = (int)blockIdx.x - S.H.ctas1; } }
         sper = (smode == 1 || smode == 3) ? ((2 * P.n + P.m - 1) / P.m) * A.ntraj : A.ntraj;
         const int cps = (sper + S.TPC - 1) / S.TPC;
         seg = A.seg.seg_lo + b / cps; sq0 = (b % cps) * S.TPC;
@@ -1170,7 +1179,7 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
             const int j = sblk * m + L.col(e);                           // unit vector of this column: u_j (j < n) or v_{j-n}
             if (smode == 1) { vr[e] = ok[e] && L.row(e) == j ? 1.0 : 0.0; vi[e] = ok[e] && L.row(e) + n == j ? 1.0 : 0.0; }
             else if (smode == 2) { vr[e] = ok[e] ? A.seg.X[sbt * 2 * nm + bx] : 0.0; vi[e] = ok[e] ? A.seg.X[sbt * 2 * nm + bx + n] : 0.0; }
-            else if (smode >= 4) {                                       // backward sweeps: Xb = X + J' Eta at the segment end (6: X itself)
+            else if (smode >= 4 && (!HIST || smode != 7)) {              // backward sweeps: Xb = X + J' Eta at the segment end (6: X itself)
                 const size_t b1 = (sbt + A.ntraj) * 2 * nm + bx;
                 const bool plain = smode == 6 && A.seg.pass == 0;       // first defect sweep: from the forward boundary state
                 vr[e] = ok[e] ? A.seg.X[b1] - (plain ? 0.0 : A.seg.Eta[b1 + n]) : 0.0;
@@ -1200,9 +1209,18 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
     double dt = P.T / (double)P.nsteps, t = 0.0, pen = 0.0;
     if constexpr (SEG) t = A.seg.times[seg];
     // forward history (jq_eval_forward; src/evalobjgrad.jl:2847-2849): Re = vr, Im = -vi after every save_every-th step
-    const bool hist = A.hist_r != nullptr;
+    const bool hist = A.hist_r != nullptr && (!HIST || smode == 2);
     size_t hpos = hist ? (size_t)(live_t ? traj : 0) * A.nsave * ((size_t)n * m) : 0;      // start of the next saved block
     int hcount = hist ? A.save_every : 0;                                                // steps until the next save
+    if constexpr (HIST) {
+        // mode 2: the saves in (k0, k1] -- the first is j1 = k0 / save_every + 1 -- and block 0 in segment 0, written by one trajectory
+        // per history row; the others start at hcount = 0, which the countdown never reaches again
+        if (hist) {
+            const long long q0 = (long long)seg * P.nsteps / A.seg.nseg, j1 = q0 / A.save_every + 1;
+            hpos = ((size_t)(traj / S.H.hist_nc) * A.nsave + (seg == 0 ? 0 : j1)) * ((size_t)n * m);
+            hcount = live_t && traj % S.H.hist_nc == 0 ? (int)(j1 * A.save_every - q0) : 0;
+        }
+    }
     auto save_state = [&]() {
         UNROLL for (int e = 0; e < E; ++e)
             if (ok[e]) {
@@ -1211,7 +1229,7 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
             }
         hpos += (size_t)n * m;
     };
-    if (hist) save_state();
+    if (hist && (!HIST || (seg == 0 && hcount != 0))) save_state();
     // two copies of the loop (generic lambda, both inlined): the evaluation path carries no per-step history test
     // SHARE (weighted layouts, not pipelined): a step's last product pass also gives the next step's boundary products (bp, with
     // the next p05 from the table row past the step: the table carries one extra point for the last step of a chunk).  The penalty
@@ -1263,7 +1281,8 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
     double lr[E], li[E], vr0[E];
     if constexpr (SEG) {
         if (smode <= 2) {
-            forward_sweep(std::false_type{});
+            if constexpr (HIST && OBJ == 0) { if (hist) forward_sweep(std::true_type{}); else forward_sweep(std::false_type{}); }
+            else forward_sweep(std::false_type{});
             if (smode == 1) {                                // column j of the segment's propagator
                 UNROLL for (int e = 0; e < E; ++e) {
                     const int j = sblk * m + L.col(e);
@@ -1281,7 +1300,7 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
             if (live_t && g.gi == 0 && g.lg == 0) {
                 double pens = 0.0;
                 for (int j = 0; j < S.GPT; ++j) pens += red[(tl * S.GPT + j) * 4 + 2];
-                A.seg.penpart[sbt] = 0.5 * dt * pens;
+                if (!HIST || A.seg.penpart) A.seg.penpart[sbt] = 0.5 * dt * pens;      // the history VJP has no penalty shares
             }
             return;
         }
@@ -1397,6 +1416,20 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
             trace_hs(L, vr, li, tcar);
             if constexpr (OBJ != 0) trace_hs(L, vr, lin, tcar2);
         }
+        // history VJP (modes 5 and 7): the cotangent of save j = K / save_every >= 1 jumps into the unforced set after the iteration
+        // that recomputes state K; the block of the next save is prefetched into L1 then, so that its loads stay off the critical path
+        // of the steps in between.  Derived from the loop position (warp-uniform), so the sweeps carry no extra state.
+        auto jump = [&](double (&xr)[E], double (&xi)[E], int K) -> bool {
+            if (!(S.H.cot_r || S.H.cot_i) || K == 0 || K % A.save_every != 0) return false;      // save 0 is Uinit: no effect
+            const size_t j = (size_t)(K / A.save_every), base = ((size_t)traj * A.nsave + j) * nm;
+            UNROLL for (int e = 0; e < E; ++e)
+                if (ok[e]) {
+                    const size_t ix = base + L.row(e) + (size_t)n * L.col(e);
+                    if (S.H.cot_r) { xr[e] = fma(-0.5, S.H.cot_r[ix], xr[e]); if (j > 1) asm volatile("prefetch.global.L1 [%0];" ::"l"(S.H.cot_r + ix - nm)); }
+                    if (S.H.cot_i) { xi[e] = fma(0.5, S.H.cot_i[ix], xi[e]); if (j > 1) asm volatile("prefetch.global.L1 [%0];" ::"l"(S.H.cot_i + ix - nm)); }
+                }
+            return true;
+        };
         for (long long s0 = 0; s0 < (SEG ? nstl : P.nsteps); s0 += TRAJ_CH) {
             const int nst = (int)(((SEG ? nstl : P.nsteps) - s0) < TRAJ_CH ? ((SEG ? nstl : P.nsteps) - s0) : TRAJ_CH);
             fill_table<NC>(S, sm, t, dt, nst, dtknot);
@@ -1406,7 +1439,10 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
                 if constexpr (SEG) {
                     if (smode != 5) {        // no gradient: the traces are dead code (DEFER leaves them in registers nobody reads)
                         double tp[NC * 5];
-                        if (smode == 3) adjoint_step<JT, false, LaneT, true>(L, J, dt, lr, li, vr, vi05, vr, nullptr, GL, gbase_lane, false, tp);
+                        if (smode == 3 || (HIST && smode == 7)) {
+                            adjoint_step<JT, false, LaneT, true>(L, J, dt, lr, li, vr, vi05, vr, nullptr, GL, gbase_lane, false, tp);
+                            if constexpr (HIST && OBJ == 0) { if (smode == 7) jump(lr, li, (int)(k1 - 1 - s0) - ls); }      // particular solution
+                        }
                         else if (smode == 6) state_step<JT>(L, J, dt, vr, vi, vi05);
                         else {
                             UNROLL for (int e = 0; e < E; ++e) vr0[e] = vr[e];
@@ -1424,6 +1460,9 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
                 if constexpr (OBJ != 0) {
                     adjoint_step<JT, false>(L, J, dt, lrn, lin, vr0, vi05, vr, tred, GL, gbase_lane, lane_on && g.lg == 0, nullptr, CARRY ? tcar2 : nullptr);
                     grad_scatter<NC, UPL>(U2, gsm2, tred, tabb, tabph, tabk, ls, Nfreq);
+                    if constexpr (HIST) {                    // after this step's traces; the carried trace is tr(vr, Hs, lin) of the jumped lin
+                        if (jump(lrn, lin, (int)(k1 - 1 - s0) - ls)) { if constexpr (CARRY) trace_hs(L, vr, lin, tcar2); }
+                    }
                 }
                 t = t + dt;
             }
@@ -1500,7 +1539,7 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
                     if (ok[e] && j < 2 * n) { double *o = A.seg.Adj + (sbt * A.seg.ld + j) * A.seg.ld + L.row(e); o[0] = lr[e]; o[n] = li[e]; }
                 } else if (ok[e]) {
                     const size_t b0 = sbt * 2 * nm + L.row(e) + (size_t)2 * n * L.col(e);
-                    if (smode == 4) { A.seg.cpart[b0] = lr[e]; A.seg.cpart[b0 + n] = li[e]; }
+                    if (smode == 4 || (HIST && smode == 7)) { A.seg.cpart[b0] = lr[e]; A.seg.cpart[b0 + n] = li[e]; }
                     else {
                         // defect of the backward recomputation against the current boundary state X_p (+ J' Eta_p in a refinement pass)
                         const bool plain = A.seg.pass == 0;
@@ -1540,10 +1579,11 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
 }
 
 // Table entry of one instantiation: the key is derived from the template arguments, so it cannot disagree with the kernel.
-template <class LaneT, int UPL, int MINB = 1, int JT = 0, int OBJ = 0, int GLT = 0, int NW = TRAJ_WARPS, int PIPE = 0, bool SEG = false>
+template <class LaneT, int UPL, int MINB = 1, int JT = 0, int OBJ = 0, int GLT = 0, int NW = TRAJ_WARPS, int PIPE = 0, bool SEG = false,
+          bool HIST = false>
 constexpr Inst traj_inst() {
     return {{LaneT::KIND, LaneT::R, LaneT::C, LaneT::NC, LaneT::WQ, LaneT::LMASK, UPL, OBJ != 0, JT < 0, LaneT::HX != 0, !LaneT::AS,
-             GLT, JT > 0 ? JT : 0, NW, PIPE, SEG, LaneT::NF},
-            jq_traj_kernel<LaneT, UPL, MINB, JT, OBJ, GLT, NW, PIPE, SEG>};
+             GLT, JT > 0 ? JT : 0, NW, PIPE, SEG, LaneT::NF, HIST},
+            jq_traj_kernel<LaneT, UPL, MINB, JT, OBJ, GLT, NW, PIPE, SEG, HIST>};
 }
 }  // namespace
