@@ -22,6 +22,41 @@ def _f64(a):
     return np.ascontiguousarray(a, dtype=np.float64)
 
 
+def _ptr(a):
+    return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def _samples(shifts, weights, ntot):
+    """shifts [nsamples, Ntot] and weights [nsamples], either None, checked and made contiguous float64: (nsamples, shifts, weights)."""
+    nsamples = 1
+    if shifts is not None:
+        shifts = _f64(np.atleast_2d(shifts))
+        if shifts.ndim != 2 or shifts.shape[1] != ntot:
+            raise ValueError("shifts must be [nsamples, Ntot]")
+        nsamples = shifts.shape[0]
+    if weights is not None:
+        weights = _f64(np.atleast_1d(weights))
+        if weights.shape != (nsamples,):
+            raise ValueError("weights must have one entry per sample")
+    return nsamples, shifts, weights
+
+
+def _cotangents(cot, nbatch, nsamples, trailing, none_error):
+    """cot, complex [nbatch, nsamples, ncot, *trailing] with trailing (Ntot, N) or (nsave, Ntot, N), as the C layout's real and
+    imaginary parts: (ncot, cot_r, cot_i).  cot=None is ncot = 0, or ValueError(none_error) when that is not None."""
+    if cot is None:
+        if none_error is not None:
+            raise ValueError(none_error)
+        return 0, None, None
+    cot = np.asarray(cot)
+    if cot.ndim != 3 + len(trailing) or cot.shape[:2] != (nbatch, nsamples) or cot.shape[2] < 1 or cot.shape[3:] != tuple(trailing):
+        names, dims = ", ".join(("nsave", "Ntot", "N")[-len(trailing):]), ", ".join(str(d) for d in trailing)
+        raise ValueError(f"cot must be [nbatch, nsamples, ncot, {names}] = [{nbatch}, {nsamples}, ncot >= 1, {dims}], not {list(cot.shape)}")
+    cr = _f64(cot.real.swapaxes(-1, -2))                 # the C layout: column-major Ntot x N blocks
+    ci = _f64(cot.imag.swapaxes(-1, -2)) if np.iscomplexobj(cot) else None
+    return cot.shape[2], cr, ci
+
+
 def _csc(a):
     a = np.asarray(a, dtype=np.float64)
     n = a.shape[0]
@@ -207,19 +242,7 @@ class Working_Arrays:
         self._check_params()
         pcof = _f64(np.atleast_2d(pcof))
         nbatch, npar = pcof.shape
-        nsamples = 1
-        sp = wp = None
-        if shifts is not None:
-            shifts = _f64(np.atleast_2d(shifts))
-            if shifts.shape[1] != p.Ntot:
-                raise ValueError("shifts must be [nsamples, Ntot]")
-            nsamples = shifts.shape[0]
-            sp = shifts.ctypes.data_as(C.c_void_p)
-        if weights is not None:
-            weights = _f64(np.atleast_1d(weights))
-            if len(weights) != nsamples:
-                raise ValueError("weights must have one entry per sample")
-            wp = weights.ctypes.data_as(C.c_void_p)
+        nsamples, shifts, weights = _samples(shifts, weights, p.Ntot)
         shape = (nbatch,) if weights is not None else (nbatch, nsamples)
         two_sets = p.objFuncType != 1
 
@@ -232,19 +255,18 @@ class Working_Arrays:
         gptr = [None, None, None]
         if evaladjoint:
             res["grad"] = buf("grad", shape + (npar,))
-            gptr[0] = res["grad"].ctypes.data_as(C.c_void_p)
+            gptr[0] = _ptr(res["grad"])
             if two_sets:
                 res["infidgrad"] = buf("infidgrad", shape + (npar,))
                 res["leakgrad"] = buf("leakgrad", shape + (npar,))
-                gptr[1:] = [res[k].ctypes.data_as(C.c_void_p) for k in ("infidgrad", "leakgrad")]
+                gptr[1:] = [_ptr(res[k]) for k in ("infidgrad", "leakgrad")]
             else:
                 res["infidgrad"] = res["grad"]
                 res["leakgrad"] = np.broadcast_to(0.0, shape + (npar,))
         out = res
         _lib.check(self._lib.jq_traceobjgrad_batch(
-            self._handle, nbatch, pcof.ctypes.data_as(C.c_void_p), npar, nsamples, sp, wp, int(bool(evaladjoint)),
-            out["infid"].ctypes.data_as(C.c_void_p), out["leak"].ctypes.data_as(C.c_void_p),
-            out["trace_infid"].ctypes.data_as(C.c_void_p), *gptr))
+            self._handle, nbatch, _ptr(pcof), npar, nsamples, _ptr(shifts), _ptr(weights), int(bool(evaladjoint)), _ptr(out["infid"]),
+            _ptr(out["leak"]), _ptr(out["trace_infid"]), *gptr))
         out["objf"] = out["infid"] + out["leak"]
         return out
 
@@ -255,21 +277,15 @@ class Working_Arrays:
         self._check_params()
         pcof = _f64(np.atleast_2d(pcof))
         nbatch, npar = pcof.shape
-        nsamples, sp = 1, None
-        if shifts is not None:
-            shifts = _f64(np.atleast_2d(shifts))
-            if shifts.shape[1] != p.Ntot:
-                raise ValueError("shifts must be [nsamples, Ntot]")
-            nsamples, sp = shifts.shape[0], shifts.ctypes.data_as(C.c_void_p)
+        nsamples, shifts, _ = _samples(shifts, None, p.Ntot)
         if save_every < 1 or p.nsteps % save_every != 0:
             raise ValueError(f"nsteps must be divisible by saveEvery. nsteps={p.nsteps}, saveEvery={save_every}")
         nsave = p.nsteps // save_every + 1
         hr = np.zeros((nbatch, nsamples, nsave, p.N, p.Ntot))
         hi = np.zeros_like(hr)
         infid, leak = np.zeros((nbatch, nsamples)), np.zeros((nbatch, nsamples))
-        _lib.check(self._lib.jq_eval_forward(self._handle, nbatch, pcof.ctypes.data_as(C.c_void_p), npar, nsamples, sp, int(save_every),
-                                             hr.ctypes.data_as(C.c_void_p), hi.ctypes.data_as(C.c_void_p),
-                                             infid.ctypes.data_as(C.c_void_p), leak.ctypes.data_as(C.c_void_p)))
+        _lib.check(self._lib.jq_eval_forward(self._handle, nbatch, _ptr(pcof), npar, nsamples, _ptr(shifts), int(save_every), _ptr(hr),
+                                             _ptr(hi), _ptr(infid), _ptr(leak)))
         return hr + 1j * hi, infid, leak
 
     def forward_sensitivity(self, pcof, dirs, shifts=None, weights=None, final_state: bool = False):
@@ -291,29 +307,18 @@ class Working_Arrays:
             raise ValueError(f"dirs must be [nbatch, ndir, npar] = [{nbatch}, ndir >= 1, {npar}], not {list(dirs.shape)}")
         dirs = _f64(dirs)
         ndir = dirs.shape[1]
-        nsamples, sp, wp = 1, None, None
-        if shifts is not None:
-            shifts = _f64(np.atleast_2d(shifts))
-            if shifts.ndim != 2 or shifts.shape[1] != p.Ntot:
-                raise ValueError("shifts must be [nsamples, Ntot]")
-            nsamples, sp = shifts.shape[0], shifts.ctypes.data_as(C.c_void_p)
-        if weights is not None:
-            weights = _f64(np.atleast_1d(weights))
-            if weights.shape != (nsamples,):
-                raise ValueError("weights must have one entry per sample")
-            if final_state:
-                raise ValueError("final_state=True needs per-sample outputs (weights=None): a weighted sum of states is not defined")
-            wp = weights.ctypes.data_as(C.c_void_p)
+        nsamples, shifts, weights = _samples(shifts, weights, p.Ntot)
+        if weights is not None and final_state:
+            raise ValueError("final_state=True needs per-sample outputs (weights=None): a weighted sum of states is not defined")
         shape = (nbatch,) if weights is not None else (nbatch, nsamples)
         out = {"infid": np.zeros(shape), "leak": np.zeros(shape), "dinfid": np.zeros(shape + (ndir,)), "dleak": np.zeros(shape + (ndir,))}
         sr = si = None
         if final_state:
             sr = np.zeros((nbatch, nsamples, ndir, p.N, p.Ntot))      # the C layout: column-major Ntot x N blocks
             si = np.zeros_like(sr)
-        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
         _lib.check(self._lib.jq_forward_sensitivity(
-            self._handle, nbatch, ptr(pcof), npar, nsamples, sp, wp, ndir, ptr(dirs), ptr(out["infid"]), ptr(out["leak"]),
-            ptr(out["dinfid"]), ptr(out["dleak"]), ptr(sr), ptr(si)))
+            self._handle, nbatch, _ptr(pcof), npar, nsamples, _ptr(shifts), _ptr(weights), ndir, _ptr(dirs), _ptr(out["infid"]),
+            _ptr(out["leak"]), _ptr(out["dinfid"]), _ptr(out["dleak"]), _ptr(sr), _ptr(si)))
         out["objf"] = out["infid"] + out["leak"]
         out["dobjf"] = out["dinfid"] + out["dleak"]
         if final_state:
@@ -338,32 +343,16 @@ class Working_Arrays:
             raise ValueError("pcof must be [nbatch, npar]")
         pcof = _f64(pcof)
         nbatch, npar = pcof.shape
-        nsamples, sp = 1, None
-        if shifts is not None:
-            shifts = _f64(np.atleast_2d(shifts))
-            if shifts.ndim != 2 or shifts.shape[1] != p.Ntot:
-                raise ValueError("shifts must be [nsamples, Ntot]")
-            nsamples, sp = shifts.shape[0], shifts.ctypes.data_as(C.c_void_p)
-        if cot is None:
-            if not (time_parallel and final_state):
-                raise ValueError("cot=None (U(T) only) needs time_parallel=True and final_state=True")
-            ncot, cr, ci = 0, None, None
-        else:
-            cot = np.asarray(cot)
-            if cot.ndim != 5 or cot.shape[:2] != (nbatch, nsamples) or cot.shape[2] < 1 or cot.shape[3:] != (p.Ntot, p.N):
-                raise ValueError(f"cot must be [nbatch, nsamples, ncot, Ntot, N] = [{nbatch}, {nsamples}, ncot >= 1, {p.Ntot}, {p.N}], "
-                                 f"not {list(cot.shape)}")
-            ncot = cot.shape[2]
-            cr = _f64(cot.real.swapaxes(-1, -2))                 # the C layout: column-major Ntot x N blocks
-            ci = _f64(cot.imag.swapaxes(-1, -2)) if np.iscomplexobj(cot) else None
+        nsamples, shifts, _ = _samples(shifts, None, p.Ntot)
+        ncot, cr, ci = _cotangents(cot, nbatch, nsamples, (p.Ntot, p.N), None if time_parallel and final_state else
+                                   "cot=None (U(T) only) needs time_parallel=True and final_state=True")
         vjp = np.zeros((nbatch, nsamples, ncot, npar)) if ncot else None
         sr = si = None
         if final_state:
             sr = np.zeros((nbatch, nsamples, p.N, p.Ntot))
             si = np.zeros_like(sr)
-        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
         fn = self._lib.jq_final_state_vjp_time_parallel if time_parallel else self._lib.jq_final_state_vjp
-        _lib.check(fn(self._handle, nbatch, ptr(pcof), npar, nsamples, sp, ncot, ptr(cr), ptr(ci), ptr(vjp), ptr(sr), ptr(si)))
+        _lib.check(fn(self._handle, nbatch, _ptr(pcof), npar, nsamples, _ptr(shifts), ncot, _ptr(cr), _ptr(ci), _ptr(vjp), _ptr(sr), _ptr(si)))
         out = {} if vjp is None else {"vjp": vjp}
         if final_state:
             out["state"] = (sr + 1j * si).swapaxes(-1, -2)
@@ -378,15 +367,10 @@ class Working_Arrays:
             raise ValueError("pcof must be [nbatch, npar]")
         pcof = _f64(pcof)
         nbatch, npar = pcof.shape
-        nsamples, sp = 1, None
-        if shifts is not None:
-            shifts = _f64(np.atleast_2d(shifts))
-            if shifts.ndim != 2 or shifts.shape[1] != p.Ntot:
-                raise ValueError("shifts must be [nsamples, Ntot]")
-            nsamples, sp = shifts.shape[0], shifts
+        nsamples, shifts, _ = _samples(shifts, None, p.Ntot)
         if int(save_every) != save_every or save_every < 1 or p.nsteps % save_every != 0:
             raise ValueError(f"nsteps must be divisible by saveEvery. nsteps={p.nsteps}, saveEvery={save_every}")
-        return pcof, nbatch, npar, nsamples, sp, p.nsteps // int(save_every) + 1
+        return pcof, nbatch, npar, nsamples, shifts, p.nsteps // int(save_every) + 1
 
     def history_vjp(self, pcof, cot, shifts=None, save_every: int = 1, history: bool = False, time_parallel: bool = False):
         """Vector-Jacobian products of the state history (jq_history_vjp): one forward and one backward sweep per cotangent.
@@ -402,27 +386,16 @@ class Working_Arrays:
         saved states alone."""
         p = self.params
         pcof, nbatch, npar, nsamples, sh, nsave = self._history_inputs(pcof, shifts, save_every)
-        if cot is None:
-            if not (time_parallel and history):
-                raise ValueError("cot=None (the history only) needs time_parallel=True and history=True")
-            ncot, cr, ci = 0, None, None
-        else:
-            cot = np.asarray(cot)
-            if cot.ndim != 6 or cot.shape[:2] != (nbatch, nsamples) or cot.shape[2] < 1 or cot.shape[3:] != (nsave, p.Ntot, p.N):
-                raise ValueError(f"cot must be [nbatch, nsamples, ncot, nsave, Ntot, N] = [{nbatch}, {nsamples}, ncot >= 1, {nsave}, "
-                                 f"{p.Ntot}, {p.N}], not {list(cot.shape)}")
-            ncot = cot.shape[2]
-            cr = _f64(cot.real.swapaxes(-1, -2))                 # the C layout: column-major Ntot x N blocks
-            ci = _f64(cot.imag.swapaxes(-1, -2)) if np.iscomplexobj(cot) else None
+        ncot, cr, ci = _cotangents(cot, nbatch, nsamples, (nsave, p.Ntot, p.N), None if time_parallel and history else
+                                   "cot=None (the history only) needs time_parallel=True and history=True")
         vjp = np.zeros((nbatch, nsamples, ncot, npar)) if ncot else None
         hr = hi = None
         if history:
             hr = np.zeros((nbatch, nsamples, nsave, p.N, p.Ntot))
             hi = np.zeros_like(hr)
-        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
         fn = self._lib.jq_history_vjp_time_parallel if time_parallel else self._lib.jq_history_vjp
-        _lib.check(fn(self._handle, nbatch, ptr(pcof), npar, nsamples, ptr(sh), int(save_every), ncot, ptr(cr), ptr(ci), ptr(vjp),
-                      ptr(hr), ptr(hi)))
+        _lib.check(fn(self._handle, nbatch, _ptr(pcof), npar, nsamples, _ptr(sh), int(save_every), ncot, _ptr(cr), _ptr(ci), _ptr(vjp),
+                      _ptr(hr), _ptr(hi)))
         out = {} if vjp is None else {"vjp": vjp}
         if history:
             out["history"] = (hr + 1j * hi).swapaxes(-1, -2)
@@ -442,9 +415,8 @@ class Working_Arrays:
         ndir = dirs.shape[1]
         dr = np.zeros((nbatch, nsamples, ndir, nsave, p.N, p.Ntot))
         di = np.zeros_like(dr)
-        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
-        _lib.check(self._lib.jq_history_jvp(self._handle, nbatch, ptr(pcof), npar, nsamples, ptr(sh), int(save_every), ndir, ptr(dirs),
-                                            ptr(dr), ptr(di)))
+        _lib.check(self._lib.jq_history_jvp(self._handle, nbatch, _ptr(pcof), npar, nsamples, _ptr(sh), int(save_every), ndir, _ptr(dirs),
+                                            _ptr(dr), _ptr(di)))
         return (dr + 1j * di).swapaxes(-1, -2)
 
     def eval_f_grad(self, pcof, shifts=None, weights=None, tik0: float = 0.0, prior=None):
@@ -455,28 +427,17 @@ class Working_Arrays:
         self._check_params()
         pcof = _f64(np.ravel(pcof))
         npar = len(pcof)
-        nsamples, sp, wp, pp = 1, None, None, None
-        if shifts is not None:
-            shifts = _f64(np.atleast_2d(shifts))
-            if shifts.shape[1] != p.Ntot:
-                raise ValueError("shifts must be [nsamples, Ntot]")
-            nsamples, sp = shifts.shape[0], shifts.ctypes.data_as(C.c_void_p)
-        if weights is not None:
-            weights = _f64(np.atleast_1d(weights))
-            if len(weights) != nsamples:
-                raise ValueError("weights must have one entry per sample")
-            wp = weights.ctypes.data_as(C.c_void_p)
+        nsamples, shifts, weights = _samples(shifts, weights, p.Ntot)
         if prior is not None:
             prior = _f64(np.ravel(prior))
             if len(prior) != npar:
                 raise ValueError("prior must have the length of pcof")
-            pp = prior.ctypes.data_as(C.c_void_p)
         f, infid, leak = C.c_double(), C.c_double(), C.c_double()
         ev = C.c_int32()
         grad, lgrad = np.zeros(npar), np.zeros(npar if p.objFuncType != 1 else 0)
-        _lib.check(self._lib.jq_eval_f_grad(self._handle, pcof.ctypes.data_as(C.c_void_p), npar, nsamples, sp, wp, float(tik0), pp,
-                                            C.byref(f), grad.ctypes.data_as(C.c_void_p), C.byref(infid), C.byref(leak),
-                                            lgrad.ctypes.data_as(C.c_void_p) if len(lgrad) else None, C.byref(ev)))
+        _lib.check(self._lib.jq_eval_f_grad(self._handle, _ptr(pcof), npar, nsamples, _ptr(shifts), _ptr(weights), float(tik0), _ptr(prior),
+                                            C.byref(f), _ptr(grad), C.byref(infid), C.byref(leak), _ptr(lgrad) if len(lgrad) else None,
+                                            C.byref(ev)))
         return {"f": f.value, "grad_f": grad, "infid": infid.value, "leak": leak.value, "leakgrad": lgrad, "evaluated": bool(ev.value)}
 
     def controls(self, pcof, times):
@@ -568,7 +529,32 @@ def forward_sensitivity(pcof0, params: objparams, wa: Working_Arrays, dirs, node
     return {k: v[0] for k, v in r.items()}
 
 
-_FinalState = None
+_StateFn = None
+
+
+def _state_function():
+    """The torch.autograd.Function of final_state and state_history: apply(fwd, bwd, pcof) is fwd(pcof) (host arrays) as a tensor on
+    pcof's device; its backward pass is bwd(pcof, cot) with the incoming gradient as the one cotangent, summed over the samples,
+    which all share pcof.  First derivatives in reverse mode only."""
+    global _StateFn
+    if _StateFn is None:
+        import torch
+
+        class _Fn(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, fwd, bwd, pc):
+                ctx.bwd, ctx.pcof = bwd, pc.detach().cpu().numpy()
+                return torch.from_numpy(np.ascontiguousarray(fwd(ctx.pcof))).to(pc.device)
+
+            @staticmethod
+            @torch.autograd.function.once_differentiable
+            def backward(ctx, grad_out):
+                cot = grad_out.detach().resolve_conj().cpu().numpy()[:, :, None]
+                g = ctx.bwd(ctx.pcof, cot)[:, :, 0].sum(axis=1)
+                return None, None, torch.from_numpy(g).to(grad_out.device)
+
+        _StateFn = _Fn
+    return _StateFn
 
 
 def final_state(wa: Working_Arrays, pcof, shifts=None, time_parallel: bool = False):
@@ -579,35 +565,16 @@ def final_state(wa: Working_Arrays, pcof, shifts=None, time_parallel: bool = Fal
     cotangent (summed over the samples, which all share pcof).  time_parallel=True runs both on the time-parallel path (kernel 7,
     for a few trajectories): the forward pass is the U(T)-only call (cot=None), the backward pass one time-parallel VJP.  First
     derivatives in reverse mode only."""
-    global _FinalState
     import torch
     if pcof.dim() != 2 or pcof.dtype != torch.float64:
         raise ValueError("pcof must be a float64 tensor [nbatch, npar]")
-    if _FinalState is None:
-        class _Fn(torch.autograd.Function):
-            @staticmethod
-            def forward(ctx, wa_, pc, sh, tp):
-                ctx.wa, ctx.pcof, ctx.shifts, ctx.tp = wa_, pc.detach().cpu().numpy(), sh, tp
-                if tp:
-                    U = wa_.final_state_vjp(ctx.pcof, None, sh, final_state=True, time_parallel=True)["state"]
-                else:
-                    hist, _, _ = wa_.forward_history(ctx.pcof, sh, save_every=wa_.params.nsteps)
-                    U = hist[:, :, -1].swapaxes(-1, -2)
-                return torch.from_numpy(np.ascontiguousarray(U)).to(pc.device)
-
-            @staticmethod
-            @torch.autograd.function.once_differentiable
-            def backward(ctx, grad_out):
-                cot = grad_out.detach().resolve_conj().cpu().numpy()[:, :, None]
-                kw = {"time_parallel": True} if ctx.tp else {}
-                g = ctx.wa.final_state_vjp(ctx.pcof, cot, ctx.shifts, **kw)["vjp"][:, :, 0].sum(axis=1)
-                return None, torch.from_numpy(g).to(grad_out.device), None, None
-
-        _FinalState = _Fn
-    return _FinalState.apply(wa, pcof, shifts, bool(time_parallel))
-
-
-_StateHistory = None
+    if time_parallel:
+        fwd = lambda pc: wa.final_state_vjp(pc, None, shifts, final_state=True, time_parallel=True)["state"]
+        bwd = lambda pc, cot: wa.final_state_vjp(pc, cot, shifts, time_parallel=True)["vjp"]
+    else:
+        fwd = lambda pc: wa.forward_history(pc, shifts, save_every=wa.params.nsteps)[0][:, :, -1].swapaxes(-1, -2)
+        bwd = lambda pc, cot: wa.final_state_vjp(pc, cot, shifts)["vjp"]
+    return _state_function().apply(fwd, bwd, pcof)
 
 
 def state_history(wa: Working_Arrays, pcof, shifts=None, save_every: int = 1, time_parallel: bool = False):
@@ -619,31 +586,16 @@ def state_history(wa: Working_Arrays, pcof, shifts=None, save_every: int = 1, ti
     samples, which all share pcof).  time_parallel=True runs both on the time-parallel path (kernel 7, for a few trajectories): the
     forward pass is the history-only call (cot=None), the backward pass one time-parallel history VJP.  First derivatives in reverse
     mode only."""
-    global _StateHistory
     import torch
     if pcof.dim() != 2 or pcof.dtype != torch.float64:
         raise ValueError("pcof must be a float64 tensor [nbatch, npar]")
-    if _StateHistory is None:
-        class _Fn(torch.autograd.Function):
-            @staticmethod
-            def forward(ctx, wa_, pc, sh, se, tp):
-                ctx.wa, ctx.pcof, ctx.shifts, ctx.save_every, ctx.tp = wa_, pc.detach().cpu().numpy(), sh, se, tp
-                if tp:
-                    H = wa_.history_vjp(ctx.pcof, None, sh, se, history=True, time_parallel=True)["history"]
-                else:
-                    H = wa_.forward_history(ctx.pcof, sh, save_every=se)[0].swapaxes(-1, -2)
-                return torch.from_numpy(np.ascontiguousarray(H)).to(pc.device)
-
-            @staticmethod
-            @torch.autograd.function.once_differentiable
-            def backward(ctx, grad_out):
-                cot = grad_out.detach().resolve_conj().cpu().numpy()[:, :, None]
-                kw = {"time_parallel": True} if ctx.tp else {}
-                g = ctx.wa.history_vjp(ctx.pcof, cot, ctx.shifts, ctx.save_every, **kw)["vjp"][:, :, 0].sum(axis=1)
-                return None, torch.from_numpy(g).to(grad_out.device), None, None, None
-
-        _StateHistory = _Fn
-    return _StateHistory.apply(wa, pcof, shifts, save_every, bool(time_parallel))
+    if time_parallel:
+        fwd = lambda pc: wa.history_vjp(pc, None, shifts, save_every, history=True, time_parallel=True)["history"]
+        bwd = lambda pc, cot: wa.history_vjp(pc, cot, shifts, save_every, time_parallel=True)["vjp"]
+    else:
+        fwd = lambda pc: wa.forward_history(pc, shifts, save_every=save_every)[0].swapaxes(-1, -2)
+        bwd = lambda pc, cot: wa.history_vjp(pc, cot, shifts, save_every)["vjp"]
+    return _state_function().apply(fwd, bwd, pcof)
 
 
 def eval_forward(pcof0, params: objparams, wa: Working_Arrays, saveEndOnly: bool = True, saveEvery: int = 1):

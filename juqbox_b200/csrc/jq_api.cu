@@ -12,6 +12,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <memory>
 #include <vector>
 
@@ -132,6 +133,82 @@ static int grow(double **buf, size_t *cap, size_t need) {
     *cap = 0;
     CU(cudaMalloc((void **)buf, need * sizeof(double)));
     *cap = need;
+    return 0;
+}
+
+// grow() for the buffers of the history derivatives, which reach hundreds of MB (cnot3 at save_every = 1: ~128 MB per trajectory and
+// cotangent or direction): a request larger than the device, or one cudaMalloc cannot satisfy, is JQ_ERR_ALLOC with the size
+static int grow_history(double **buf, size_t *cap, double need, const char *who) {
+    size_t free_b = 0, total_b = 0;
+    CU(cudaMemGetInfo(&free_b, &total_b));
+    if (need * sizeof(double) > (double)total_b)
+        return fail(JQ_ERR_ALLOC, "%s: needs %.1f GB in one device buffer, the device has %.1f GB", who, need * sizeof(double) / 1e9,
+                    total_b / 1e9);
+    if ((size_t)need <= *cap) return 0;
+    if (*buf) cudaFree(*buf);
+    *buf = nullptr;
+    *cap = 0;
+    const cudaError_t e = cudaMalloc((void **)buf, (size_t)need * sizeof(double));
+    if (e != cudaSuccess) {
+        *buf = nullptr;
+        cudaGetLastError();
+        return fail(e == cudaErrorMemoryAllocation ? JQ_ERR_ALLOC : JQ_ERR_CUDA, "%s: cudaMalloc of %.1f GB: %s", who,
+                    need * sizeof(double) / 1e9, cudaGetErrorString(e));
+    }
+    *cap = (size_t)need;
+    return 0;
+}
+
+// The host arrays of an entry, staged through the handle's d_in / d_out: n doubles at *dev.  An input takes space and a device pointer
+// when the caller gave it (src) and is copied there before the launch; an output takes them when it has entries and is copied to dst,
+// when given, after the launch.  Counts are doubles because history sizes can overflow size_t; grow_history rejects them by size.
+struct In { double **dev; double n; const double *src; };
+struct Out { double **dev; double n; double *dst; };
+
+// Size d_in and d_out for an entry's arrays (grow(), or grow_history() for the history entries, `history` naming the entry), hand out
+// the device pointers in list order and copy the inputs to the device
+static int stage(jq_handle *h, const char *history, std::initializer_list<In> in, std::initializer_list<Out> out, cudaStream_t st) {
+    double n_in = 0.0, n_out = 0.0;
+    for (const In &a : in) n_in += a.src ? a.n : 0.0;
+    for (const Out &a : out) n_out += a.n;
+    int rc = history ? grow_history(&h->d_in, &h->cap_in, n_in, history) : grow(&h->d_in, &h->cap_in, (size_t)n_in);
+    if (rc || (rc = history ? grow_history(&h->d_out, &h->cap_out, n_out, history) : grow(&h->d_out, &h->cap_out, (size_t)n_out)) != 0)
+        return rc;
+    double *p = h->d_in;
+    for (const In &a : in) {
+        *a.dev = a.src ? p : nullptr;
+        if (a.src) p += (size_t)a.n;
+    }
+    p = h->d_out;
+    for (const Out &a : out) {
+        *a.dev = a.n > 0 ? p : nullptr;
+        p += (size_t)a.n;
+    }
+    for (const In &a : in)
+        if (a.src && a.n > 0) CU(cudaMemcpyAsync(*a.dev, a.src, (size_t)a.n * sizeof(double), cudaMemcpyHostToDevice, st));
+    return 0;
+}
+
+// Copy an entry's outputs back to the host and wait for them
+static int read_back(std::initializer_list<Out> out, cudaStream_t st) {
+    for (const Out &a : out)
+        if (a.dst && a.n > 0) CU(cudaMemcpyAsync(a.dst, *a.dev, (size_t)a.n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// Run `launch(ran)`, the trajectory work of an entry on kernel `kernel` (jq_query(0)), between the timing events, and record what ran:
+// jq_query reports it, and the entry's launch count starts from it
+template <class Launch>
+static int record_launch(jq_handle *h, int kernel, cudaStream_t st, Launch &&launch) {
+    CU(cudaEventRecord(h->ev0, st));
+    Ran ran;
+    ran.kernel = kernel;
+    if (int rc = launch(ran)) return rc;
+    CU(cudaEventRecord(h->ev1, st));
+    h->timed = true;
+    h->ran = ran;
+    h->last_launches = ran.launches;
     return 0;
 }
 
@@ -642,12 +719,20 @@ static int scratch_release(jq_handle *h, cudaStream_t st) {
     return 0;
 }
 
+// The spline coefficients of a caller's vector of npar entries (pFidType 3: the last entry is the global phase, src/evalobjgrad.jl:591-596)
+// and D1, their number per control function and carrier
+struct Splines { int nspl, D1; };
+static Splines splines(const jq_handle *h, int npar) {
+    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
+    return {nspl, nspl / (2 * h->Nc * h->Nfreq)};
+}
+
 // Arguments of a launch over nbatch x nsamples trajectories.  npar is the caller's vector length: the spline coefficients, plus the
 // global phase as last entry for pFidType 3; gradients have the same length.
 static LaunchArgs launch_args(const jq_handle *h, int nbatch, int npar, int nsamples, const double *pcof, const double *shift) {
-    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
+    const Splines s = splines(h, npar);
     LaunchArgs A{};
-    A.ntraj = nbatch * nsamples; A.nsamples = nsamples; A.Npar = nspl; A.D1 = nspl / (2 * h->Nc * h->Nfreq);
+    A.ntraj = nbatch * nsamples; A.nsamples = nsamples; A.Npar = s.nspl; A.D1 = s.D1;
     A.pstride = npar; A.gstride = npar;
     A.pcof = pcof; A.shift = shift; A.scal = h->d_scal;
     return A;
@@ -725,7 +810,7 @@ static int launch_time_parallel(jq_handle *h, const LaunchArgs &A, cudaStream_t 
         if (nseg > h->P.nsteps) nseg = (int)(h->P.nsteps / h->comm_size) * h->comm_size;       // >= comm_size by the test above
     }
     SegCoop coop{h->comm_rank, h->comm_size, seg_allgather, h};
-    int rc = grow(&h->d_seg, &h->cap_seg, jq_seg_workspace_doubles(h->P, A.ntraj, A.Npar, nseg, A.evaladjoint));
+    int rc = grow(&h->d_seg, &h->cap_seg, jq_seg_workspace(h->P, A.ntraj, A.Npar, nseg, false, A.evaladjoint, false));
     if (rc) return rc;
     if ((rc = seg_times_upload(h, nseg, st)) != 0) return rc;
     ran.nseg = nseg;
@@ -754,34 +839,33 @@ static int launch_trajectories(jq_handle *h, const LaunchArgs &A, cudaStream_t s
     const int pref = h->kernel_pref;
     const Route *routes[NROUTES];
     const int n = launch_routes(h, A, pref, routes);
-    CU(cudaEventRecord(h->ev0, st));
-    Ran ran;
-    int rc = HANDED_OVER;
-    for (int i = 0; i < n && rc == HANDED_OVER; ++i) {
-        ran = Ran();
-        ran.kernel = routes[i]->kernel;
-        rc = launch_route(h, *routes[i], A, st, ran, pref == 0 && i + 1 < n);
-    }
-    if (rc) return rc;
-    CU(cudaEventRecord(h->ev1, st));
-    h->timed = true;
-    h->ran = ran;
-    return 0;
+    return record_launch(h, 0, st, [&](Ran &ran) {
+        int rc = HANDED_OVER;
+        for (int i = 0; i < n && rc == HANDED_OVER; ++i) {
+            ran = Ran();
+            ran.kernel = routes[i]->kernel;
+            rc = launch_route(h, *routes[i], A, st, ran, pref == 0 && i + 1 < n);
+        }
+        return rc;
+    });
 }
 
+// The batch arguments every entry checks.  The derivative entries run `per_traj` trajectories (directions or cotangents) per candidate
+// and sample; `who` names the entry in the trajectory-count message.
 static int check_batch_args(jq_handle *h, int nbatch, const double *pcof, int npar, int nsamples, const double *shift,
-                            bool empty_shard_ok = false) {
+                            bool empty_shard_ok = false, int per_traj = 1, const char *who = nullptr) {
     if (!h) return fail(JQ_ERR_ARG, "null handle");
     if (nbatch < 1 || !pcof) return fail(JQ_ERR_ARG, "need nbatch >= 1 and a pcof array");
-    const int nsig = 2 * h->Nc;
-    npar -= h->pfid == 3 ? 1 : 0;              // pFidType 3: the last entry is the global phase (src/evalobjgrad.jl:591-596)
-    if (npar % nsig != 0 || npar < 3 * nsig)   // src/evalobjgrad.jl:604-606
-        return fail(JQ_ERR_PCOF_LENGTH, "pcof must have an even number of elements >= %d, not %d", 3 * nsig, npar);
-    if (npar % (nsig * h->Nfreq) != 0 || npar / (nsig * h->Nfreq) < 3)   // src/bsplines.jl:177-181 (and k >= 3 needs D1 >= 3)
-        return fail(JQ_ERR_PCOF_LENGTH, "Inconsistent number of coefficients and size of parameter vector (nCoeff = %d, Nfreq = %d, Ncoupled + Nunc = %d)", npar, h->Nfreq, h->Nc);
+    const int nsig = 2 * h->Nc, nspl = splines(h, npar).nspl;
+    if (nspl % nsig != 0 || nspl < 3 * nsig)   // src/evalobjgrad.jl:604-606
+        return fail(JQ_ERR_PCOF_LENGTH, "pcof must have an even number of elements >= %d, not %d", 3 * nsig, nspl);
+    if (nspl % (nsig * h->Nfreq) != 0 || nspl / (nsig * h->Nfreq) < 3)   // src/bsplines.jl:177-181 (and k >= 3 needs D1 >= 3)
+        return fail(JQ_ERR_PCOF_LENGTH, "Inconsistent number of coefficients and size of parameter vector (nCoeff = %d, Nfreq = %d, Ncoupled + Nunc = %d)", nspl, h->Nfreq, h->Nc);
     // an empty sample shard (more ranks than quadrature nodes) contributes zeros and still joins the all-reduce
     if (nsamples < (empty_shard_ok ? 0 : 1)) return fail(JQ_ERR_ARG, "nsamples must be >= 1 (0 only with weights: an empty sample shard)");
-    if ((long long)nbatch * nsamples > 0x7fffffffLL) return fail(JQ_ERR_ARG, "nbatch * nsamples exceeds 2^31 - 1 trajectories per call");
+    if ((long long)nbatch * nsamples * per_traj > 0x7fffffffLL)
+        return fail(JQ_ERR_ARG, "%s%snbatch * nsamples%s exceeds 2^31 - 1 trajectories per call", who ? who : "", who ? ": " : "",
+                    per_traj > 1 ? " * (directions or cotangents)" : "");
     if (!shift && nsamples > 1) return fail(JQ_ERR_ARG, "nsamples > 1 needs h0_diag_shift");
     return 0;
 }
@@ -873,30 +957,22 @@ extern "C" int jq_eval_f_grad(jq_handle *h, const double *pcof, int32_t npar, in
         CU(cudaSetDevice(h->device));
         h->cache_valid = false;
         const bool two = h->P.objFuncType != 1;
-        const size_t n_in = (size_t)npar + n_shift + (n_w ? n_w : 1) + (prior ? npar : 0);
-        const size_t n_out = 3 + (size_t)npar * (two ? 3 : 1) + 3 + 3 * (size_t)npar;
-        if ((rc = grow(&h->d_in, &h->cap_in, n_in)) != 0) return rc;
-        if ((rc = grow(&h->d_out, &h->cap_out, n_out)) != 0) return rc;
         cudaStream_t st = h->stream;
-        double *d_pcof = h->d_in, *d_shift = shift ? d_pcof + npar : nullptr, *d_w = d_pcof + npar + n_shift;
-        double *d_prior = prior ? d_w + (n_w ? n_w : 1) : nullptr;
-        CU(cudaMemcpyAsync(d_pcof, pcof, (size_t)npar * sizeof(double), cudaMemcpyHostToDevice, st));
-        if (n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
-        const double one = 1.0;
-        if (n_w) CU(cudaMemcpyAsync(d_w, weights, n_w * sizeof(double), cudaMemcpyHostToDevice, st));
-        else CU(cudaMemcpyAsync(d_w, &one, sizeof(double), cudaMemcpyHostToDevice, st));      // no weights: the single sample has weight 1
-        if (prior) CU(cudaMemcpyAsync(d_prior, prior, (size_t)npar * sizeof(double), cudaMemcpyHostToDevice, st));
-        double *o_infid = h->d_out, *o_leak = o_infid + 1, *o_tinf = o_leak + 1, *o_g = o_tinf + 1;
-        double *o_ig = two ? o_g + npar : nullptr, *o_lg = two ? o_ig + npar : nullptr;
-        double *o_pack = o_g + (size_t)npar * (two ? 3 : 1);
+        const double one = 1.0;                 // no weights: the single sample has weight 1
+        std::vector<double> pack(3 + 3 * (size_t)npar);
+        double *d_pcof, *d_shift, *d_w, *d_prior, *o_infid, *o_leak, *o_tinf, *o_g, *o_ig, *o_lg, *o_pack;
+        const std::initializer_list<Out> out = {{&o_infid, 1, nullptr}, {&o_leak, 1, nullptr}, {&o_tinf, 1, nullptr}, {&o_g, (double)npar, nullptr},
+                                                {&o_ig, two ? (double)npar : 0.0, nullptr}, {&o_lg, two ? (double)npar : 0.0, nullptr},
+                                                {&o_pack, (double)pack.size(), pack.data()}};
+        rc = stage(h, nullptr, {{&d_pcof, (double)npar, pcof}, {&d_shift, (double)n_shift, shift}, {&d_w, n_w ? (double)n_w : 1.0, n_w ? weights : &one},
+                                {&d_prior, (double)npar, prior}}, out, st);
+        if (rc) return rc;
         rc = jq_traceobjgrad_batch_device(h, 1, d_pcof, npar, nsamples, d_shift, d_w, 1, o_infid, o_leak, o_tinf, o_g, o_ig, o_lg, st);
         if (rc) return rc;
         jq_tikhonov_kernel<<<1, 256, 0, st>>>(npar, h->P.objFuncType, tik0, d_pcof, d_prior, o_infid, o_leak, two ? o_ig : o_g, o_lg, o_pack);
         CU(cudaGetLastError());
         h->last_launches += 1;
-        std::vector<double> pack(3 + 3 * (size_t)npar);
-        CU(cudaMemcpyAsync(pack.data(), o_pack, pack.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+        if ((rc = read_back(out, st)) != 0) return rc;
         // store what the reference stores (last_infidelity, last_leak, last_infidelity_grad, last_leak_grad): the Tikhonov terms are
         // re-applied on a cache hit because tik0 / prior are inputs of every call
         h->c_pcof.assign(pcof, pcof + npar);
@@ -939,23 +1015,18 @@ extern "C" int jq_eval_forward(jq_handle *h, int32_t nbatch, const double *pcof,
     if (!hist_r || !hist_i) return fail(JQ_ERR_ARG, "jq_eval_forward: null history buffer");
     if ((rc = check_save_every(h, save_every)) != 0) return rc;
     CU(cudaSetDevice(h->device));
-    const size_t ntraj = (size_t)nbatch * nsamples, len = (size_t)h->n * h->m;
-    const long long nsave = h->P.nsteps / save_every + 1;
-    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)nsamples * h->n : 0, n_hist = ntraj * (size_t)nsave * len;
-    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_shift)) != 0) return rc;
-    if ((rc = grow(&h->d_out, &h->cap_out, 2 * n_hist)) != 0) return rc;
-    if ((rc = grow(&h->d_scal, &h->cap_traj, ntraj * 4)) != 0) return rc;
     cudaStream_t st = h->stream;
-    double *d_pcof = h->d_in, *d_shift = shift ? h->d_in + n_pcof : nullptr;
-    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
+    const size_t ntraj = (size_t)nbatch * nsamples;
+    const long long nsave = h->P.nsteps / save_every + 1;
+    const double n_hist = (double)ntraj * nsave * h->n * h->m;
+    double *d_pcof, *d_shift, *o_hr, *o_hi;
+    const std::initializer_list<Out> out = {{&o_hr, n_hist, hist_r}, {&o_hi, n_hist, hist_i}};
+    if ((rc = stage(h, nullptr, {{&d_pcof, (double)nbatch * npar, pcof}, {&d_shift, (double)nsamples * h->n, shift}}, out, st)) != 0) return rc;
+    if ((rc = grow(&h->d_scal, &h->cap_traj, ntraj * 4)) != 0) return rc;
     LaunchArgs A = launch_args(h, nbatch, npar, nsamples, d_pcof, d_shift);
-    A.hist_r = h->d_out; A.hist_i = h->d_out + n_hist; A.save_every = save_every; A.nsave = nsave;
+    A.hist_r = o_hr; A.hist_i = o_hi; A.save_every = save_every; A.nsave = nsave;
     if ((rc = launch_trajectories(h, A, st)) != 0) return rc;      // same kernel choice as jq_traceobjgrad_batch
-    h->last_launches = 1;
-    CU(cudaMemcpyAsync(hist_r, A.hist_r, n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(hist_i, A.hist_i, n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    if ((rc = read_back(out, st)) != 0) return rc;
     if (infid || leak) {
         std::vector<double> sc(ntraj * 4);
         CU(cudaMemcpy(sc.data(), h->d_scal, sc.size() * sizeof(double), cudaMemcpyDeviceToHost));
@@ -970,17 +1041,13 @@ extern "C" int jq_eval_controls(jq_handle *h, const double *pcof, int32_t npar, 
     if (ntimes < 0 || (ntimes > 0 && (!times || !p || !q))) return fail(JQ_ERR_ARG, "jq_eval_controls: null time or output array");
     if (ntimes == 0) return 0;
     CU(cudaSetDevice(h->device));
-    const size_t nout = (size_t)h->Nc * ntimes;
-    if ((rc = grow(&h->d_in, &h->cap_in, (size_t)npar + ntimes)) != 0) return rc;
-    if ((rc = grow(&h->d_out, &h->cap_out, 2 * nout)) != 0) return rc;
     cudaStream_t st = h->stream;
-    CU(cudaMemcpyAsync(h->d_in, pcof, (size_t)npar * sizeof(double), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(h->d_in + npar, times, (size_t)ntimes * sizeof(double), cudaMemcpyHostToDevice, st));
-    CU(jq_controls_launch(h->P, (npar - (h->pfid == 3 ? 1 : 0)) / (2 * h->Nc * h->Nfreq), h->d_in, ntimes, h->d_in + npar, h->d_out, h->d_out + nout, st));
-    CU(cudaMemcpyAsync(p, h->d_out, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(q, h->d_out + nout, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    return 0;
+    const double nout = (double)h->Nc * ntimes;
+    double *d_pcof, *d_times, *o_p, *o_q;
+    const std::initializer_list<Out> out = {{&o_p, nout, p}, {&o_q, nout, q}};
+    if ((rc = stage(h, nullptr, {{&d_pcof, (double)npar, pcof}, {&d_times, (double)ntimes, times}}, out, st)) != 0) return rc;
+    CU(jq_controls_launch(h->P, splines(h, npar).D1, d_pcof, ntimes, d_times, o_p, o_q, st));
+    return read_back(out, st);
 }
 
 extern "C" int jq_traceobjgrad_batch(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
@@ -989,271 +1056,162 @@ extern "C" int jq_traceobjgrad_batch(jq_handle *h, int32_t nbatch, const double 
     int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift, weights != nullptr);
     if (rc) return rc;
     CU(cudaSetDevice(h->device));
-    const size_t ntraj = (size_t)nbatch * nsamples, nout = weights ? (size_t)nbatch : ntraj;
-    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)nsamples * h->n : 0, n_w = weights ? (size_t)nsamples : 0;
-    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_shift + n_w + 1)) != 0) return rc;      // + 1: a valid weights pointer for an empty shard
-    const bool want_g = evaladjoint && grad, want_ig = evaladjoint && infidgrad, want_lg = evaladjoint && leakgrad && h->P.objFuncType != 1;
-    const size_t n_outs = 3 * nout + (size_t)(want_g + want_ig + want_lg) * nout * npar;
-    if ((rc = grow(&h->d_out, &h->cap_out, n_outs)) != 0) return rc;
     cudaStream_t st = h->stream;
-    double *d_pcof = h->d_in, *d_shift = shift ? h->d_in + n_pcof : nullptr, *d_w = weights ? h->d_in + n_pcof + n_shift : nullptr;
-    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (shift && n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (weights && n_w) CU(cudaMemcpyAsync(d_w, weights, n_w * sizeof(double), cudaMemcpyHostToDevice, st));
-    double *o_infid = h->d_out, *o_leak = o_infid + nout, *o_tinf = o_leak + nout, *cur = o_tinf + nout;
-    double *o_g = nullptr, *o_ig = nullptr, *o_lg = nullptr;
-    if (want_g) { o_g = cur; cur += nout * npar; }
-    if (want_ig) { o_ig = cur; cur += nout * npar; }
-    if (want_lg) { o_lg = cur; cur += nout * npar; }
+    const double nout = weights ? nbatch : (double)nbatch * nsamples, ngrad = nout * npar;
+    const bool want_g = evaladjoint && grad, want_ig = evaladjoint && infidgrad, want_lg = evaladjoint && leakgrad && h->P.objFuncType != 1;
+    double *d_pcof, *d_shift, *d_w, *o_infid, *o_leak, *o_tinf, *o_g, *o_ig, *o_lg;
+    const std::initializer_list<Out> out = {{&o_infid, nout, infid}, {&o_leak, nout, leak}, {&o_tinf, nout, trace_infid},
+                                            {&o_g, want_g ? ngrad : 0.0, grad}, {&o_ig, want_ig ? ngrad : 0.0, infidgrad},
+                                            {&o_lg, want_lg ? ngrad : 0.0, leakgrad}};
+    // an empty sample shard's weights take no space but keep a valid pointer
+    rc = stage(h, nullptr, {{&d_pcof, (double)nbatch * npar, pcof}, {&d_shift, (double)nsamples * h->n, shift}, {&d_w, (double)nsamples, weights}},
+               out, st);
+    if (rc) return rc;
     rc = jq_traceobjgrad_batch_device(h, nbatch, d_pcof, npar, nsamples, d_shift, d_w, evaladjoint, o_infid, o_leak, o_tinf, o_g, o_ig,
                                       o_lg, st);
     if (rc) return rc;
-    if (infid) CU(cudaMemcpyAsync(infid, o_infid, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (leak) CU(cudaMemcpyAsync(leak, o_leak, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (trace_infid) CU(cudaMemcpyAsync(trace_infid, o_tinf, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (want_g) CU(cudaMemcpyAsync(grad, o_g, nout * npar * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (want_ig) CU(cudaMemcpyAsync(infidgrad, o_ig, nout * npar * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (want_lg) CU(cudaMemcpyAsync(leakgrad, o_lg, nout * npar * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    return read_back(out, st);
+}
+
+// The tangent kernel's (kernel 8) checks that both forward-mode entries make
+static int check_tangent_kernel(const jq_handle *h, const char *who, int npar) {
+    if (h->P.solver == 2) return fail(JQ_ERR_ARG, "%s: the Jacobi solver has no tangent sweep (use the Neumann solver)", who);
+    if (jq_fwdsens_smem_bytes(h->P, splines(h, npar).nspl) > 227 * 1024)
+        return fail(JQ_ERR_ARG, "%s: problem too large for the tangent kernel's shared memory (n*m = %d)", who, h->n * h->m);
+    return 0;
+}
+
+// The tangent kernel's arguments for ndir directions per (candidate, sample) of staged inputs.  Its scalars and directional derivatives
+// go to the handle's scratch (d_scal, d_grad, d_igrad), grown here.
+static int tangent_args(jq_handle *h, int nbatch, int npar, int nsamples, int ndir, const double *pcof, const double *dirs,
+                        const double *shift, SensArgs *S) {
+    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ndir;
+    int rc = grow(&h->d_scal, &h->cap_traj, nt * 4);
+    if (rc || (rc = grow(&h->d_grad, &h->cap_grad, ntraj)) != 0 || (rc = grow(&h->d_igrad, &h->cap_igrad, ntraj)) != 0) return rc;
+    const Splines s = splines(h, npar);
+    *S = SensArgs{};
+    S->ntraj = (int)ntraj; S->nsamples = nsamples; S->ndir = ndir; S->Npar = s.nspl; S->D1 = s.D1; S->pstride = npar;
+    S->pcof = pcof; S->dirs = dirs; S->shift = shift;
+    S->scal = h->d_scal; S->dinfid = h->d_grad; S->dleak = h->d_igrad;
     return 0;
 }
 
 extern "C" int jq_forward_sensitivity(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
                                       const double *shift, const double *weights, int32_t ndir, const double *dirs, double *infid,
                                       double *leak, double *dinfid, double *dleak, double *dstate_r, double *dstate_i) {
-    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
+    const char *who = "jq_forward_sensitivity";
+    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift, false, ndir, who);
     if (rc) return rc;
-    if (ndir < 1 || !dirs) return fail(JQ_ERR_ARG, "jq_forward_sensitivity: need ndir >= 1 and a dirs array");
-    if ((long long)nbatch * nsamples * ndir > 0x7fffffffLL)
-        return fail(JQ_ERR_ARG, "jq_forward_sensitivity: nbatch * nsamples * ndir exceeds 2^31 - 1 trajectories per call");
-    if (h->P.solver == 2) return fail(JQ_ERR_ARG, "jq_forward_sensitivity: the Jacobi solver has no tangent sweep (use the Neumann solver)");
+    if (ndir < 1 || !dirs) return fail(JQ_ERR_ARG, "%s: need ndir >= 1 and a dirs array", who);
+    if ((rc = check_tangent_kernel(h, who, npar)) != 0) return rc;
     if (weights && (dstate_r || dstate_i))
-        return fail(JQ_ERR_ARG, "jq_forward_sensitivity: a weighted sum of final-state tangents is not defined (pass weights or dstate, not both)");
+        return fail(JQ_ERR_ARG, "%s: a weighted sum of final-state tangents is not defined (pass weights or dstate, not both)", who);
     if (weights && h->comm && h->comm_size > 1)
-        return fail(JQ_ERR_ARG, "jq_forward_sensitivity: never communicates; with a communicator attached shard the directions, not the samples (no weights)");
-    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
-    if (jq_fwdsens_smem_bytes(h->P, nspl) > 227 * 1024)
-        return fail(JQ_ERR_ARG, "jq_forward_sensitivity: problem too large for the tangent kernel's shared memory (n*m = %d)", h->n * h->m);
+        return fail(JQ_ERR_ARG, "%s: never communicates; with a communicator attached shard the directions, not the samples (no weights)", who);
     CU(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
     if ((rc = scratch_acquire(h, st)) != 0) return rc;
-    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ndir, len = (size_t)h->n * h->m;
-    const size_t nout = weights ? (size_t)nbatch : nt, ndout = nout * ndir;
-    const size_t n_pcof = (size_t)nbatch * npar, n_dirs = (size_t)nbatch * ndir * npar;
-    const size_t n_shift = shift ? (size_t)nsamples * h->n : 0, n_w = weights ? (size_t)nsamples : 0;
-    const bool want_state = dstate_r || dstate_i;
-    const size_t n_state = want_state ? ntraj * len : 0;
-    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_dirs + n_shift + n_w)) != 0) return rc;
-    if ((rc = grow(&h->d_out, &h->cap_out, 2 * nout + 2 * ndout + 2 * n_state)) != 0) return rc;
-    if ((rc = grow(&h->d_scal, &h->cap_traj, nt * 4)) != 0) return rc;
-    if ((rc = grow(&h->d_grad, &h->cap_grad, ntraj)) != 0) return rc;
-    if ((rc = grow(&h->d_igrad, &h->cap_igrad, ntraj)) != 0) return rc;
-    double *d_pcof = h->d_in, *d_dirs = d_pcof + n_pcof, *d_shift = shift ? d_dirs + n_dirs : nullptr;
-    double *d_w = weights ? d_dirs + n_dirs + n_shift : nullptr;
-    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_dirs, dirs, n_dirs * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (n_w) CU(cudaMemcpyAsync(d_w, weights, n_w * sizeof(double), cudaMemcpyHostToDevice, st));
-    double *o_infid = h->d_out, *o_leak = o_infid + nout, *o_dinf = o_leak + nout, *o_dleak = o_dinf + ndout;
-    double *o_sr = want_state ? o_dleak + ndout : nullptr, *o_si = want_state ? o_sr + n_state : nullptr;
-
-    SensArgs S{};
-    S.ntraj = (int)ntraj; S.nsamples = nsamples; S.ndir = ndir; S.Npar = nspl; S.D1 = nspl / (2 * h->Nc * h->Nfreq); S.pstride = npar;
-    S.pcof = d_pcof; S.dirs = d_dirs; S.shift = d_shift;
-    S.scal = h->d_scal; S.dinfid = h->d_grad; S.dleak = h->d_igrad; S.dstate_r = o_sr; S.dstate_i = o_si;
-    Ran ran;
-    ran.kernel = 8;
-    CU(cudaEventRecord(h->ev0, st));
-    CU(jq_fwdsens_launch(h->P, S, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc));
-    CU(cudaEventRecord(h->ev1, st));
-    h->timed = true;
-    h->ran = ran;
+    const double nout = weights ? nbatch : (double)nbatch * nsamples, ndout = nout * ndir;
+    const double n_state = dstate_r || dstate_i ? (double)nbatch * nsamples * ndir * h->n * h->m : 0.0;
+    double *d_pcof, *d_dirs, *d_shift, *d_w, *o_infid, *o_leak, *o_dinf, *o_dleak, *o_sr, *o_si;
+    const std::initializer_list<Out> out = {{&o_infid, nout, infid}, {&o_leak, nout, leak}, {&o_dinf, ndout, dinfid}, {&o_dleak, ndout, dleak},
+                                            {&o_sr, n_state, dstate_r}, {&o_si, n_state, dstate_i}};
+    rc = stage(h, nullptr, {{&d_pcof, (double)nbatch * npar, pcof}, {&d_dirs, (double)nbatch * ndir * npar, dirs},
+                            {&d_shift, (double)nsamples * h->n, shift}, {&d_w, (double)nsamples, weights}}, out, st);
+    SensArgs S;
+    if (rc || (rc = tangent_args(h, nbatch, npar, nsamples, ndir, d_pcof, d_dirs, d_shift, &S)) != 0) return rc;
+    S.dstate_r = o_sr; S.dstate_i = o_si;
+    rc = record_launch(h, 8, st, [&](Ran &r) {
+        CU(jq_fwdsens_launch(h->P, S, st, &r.ctas, &r.regs, &r.smem, &r.tpc));
+        return 0;
+    });
+    if (rc) return rc;
     // per-trajectory outputs or the weighted sums over the samples, in the fixed order of the evaluation path's reductions: the
     // directions take the place of the gradient columns (dinfid as `grad`, dleak as `infidgrad`)
     launch_finalize(nbatch, nsamples, ndir, 2, 1, d_w, h->d_scal, h->d_grad, h->d_igrad, o_infid, o_leak, nullptr, o_dinf, o_dleak, nullptr, st);
     CU(cudaGetLastError());
-    h->last_launches = 2;
+    h->last_launches += 1;
     if ((rc = scratch_release(h, st)) != 0) return rc;
-    if (infid) CU(cudaMemcpyAsync(infid, o_infid, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (leak) CU(cudaMemcpyAsync(leak, o_leak, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (dinfid) CU(cudaMemcpyAsync(dinfid, o_dinf, ndout * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (dleak) CU(cudaMemcpyAsync(dleak, o_dleak, ndout * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (dstate_r) CU(cudaMemcpyAsync(dstate_r, o_sr, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (dstate_i) CU(cudaMemcpyAsync(dstate_i, o_si, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    return 0;
+    return read_back(out, st);
+}
+
+extern "C" int jq_history_jvp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples, const double *shift,
+                              int32_t save_every, int32_t ndir, const double *dirs, double *dhist_r, double *dhist_i) {
+    const char *who = "jq_history_jvp";
+    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift, false, ndir, who);
+    if (rc) return rc;
+    if ((rc = check_save_every(h, save_every)) != 0) return rc;
+    if (ndir < 1 || !dirs) return fail(JQ_ERR_ARG, "%s: need ndir >= 1 and a dirs array", who);
+    if (!dhist_r || !dhist_i) return fail(JQ_ERR_ARG, "%s: null tangent-history output", who);
+    if ((rc = check_tangent_kernel(h, who, npar)) != 0) return rc;
+    CU(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    if ((rc = scratch_acquire(h, st)) != 0) return rc;
+    const long long nsave = h->P.nsteps / save_every + 1;
+    const double n_hist = (double)nbatch * nsamples * ndir * nsave * h->n * h->m;
+    double *d_pcof, *d_dirs, *d_shift, *o_hr, *o_hi;
+    const std::initializer_list<Out> out = {{&o_hr, n_hist, dhist_r}, {&o_hi, n_hist, dhist_i}};
+    // tangent histories reach hundreds of MB: JQ_ERR_ALLOC with the size when they do not fit
+    rc = stage(h, who, {{&d_pcof, (double)nbatch * npar, pcof}, {&d_dirs, (double)nbatch * ndir * npar, dirs}, {&d_shift, (double)nsamples * h->n, shift}},
+               out, st);
+    SensArgs S;
+    if (rc || (rc = tangent_args(h, nbatch, npar, nsamples, ndir, d_pcof, d_dirs, d_shift, &S)) != 0) return rc;
+    S.dhist_r = o_hr; S.dhist_i = o_hi; S.save_every = save_every; S.nsave = nsave;     // dinfid, dleak: written, not returned
+    rc = record_launch(h, 8, st, [&](Ran &r) {
+        CU(jq_fwdsens_launch(h->P, S, st, &r.ctas, &r.regs, &r.smem, &r.tpc));
+        return 0;
+    });
+    if (rc || (rc = scratch_release(h, st)) != 0) return rc;
+    return read_back(out, st);
+}
+
+// The serial VJP entries (kernel 9): cotangents [traj][nsave][n*m] of the saved states.  The final-state entry has one save, U(T)
+// (save_every = nsteps), returned in state_r / state_i; `history`: the history entry, nsave saves returned in hist_r / hist_i, its
+// buffers grown with grow_history.
+static int vjp_serial(jq_handle *h, const char *who, bool history, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
+                      const double *shift, int32_t save_every, int32_t ncot, const double *cot_r, const double *cot_i, double *vjp,
+                      double *save_r, double *save_i) {
+    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift, false, ncot, who);
+    if (rc) return rc;
+    if (history && (rc = check_save_every(h, save_every)) != 0) return rc;
+    if (ncot < 1 || (!cot_r && !cot_i)) return fail(JQ_ERR_ARG, "%s: need ncot >= 1 and at least one of cot_r, cot_i", who);
+    if (!vjp) return fail(JQ_ERR_ARG, "%s: null vjp output", who);
+    const Splines s = splines(h, npar);
+    if (jq_vjp_smem_bytes(h->P, s.nspl) > 227 * 1024)
+        return fail(JQ_ERR_ARG, "%s: problem too large for the VJP kernel's shared memory (n*m = %d)", who, h->n * h->m);
+    CU(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    const long long nsave = history ? h->P.nsteps / save_every + 1 : 1;
+    const double nt = (double)nbatch * nsamples, len = (double)h->n * h->m, n_cot = nt * ncot * nsave * len;
+    const double n_save = save_r || save_i ? nt * nsave * len : 0.0;
+    double *d_pcof, *d_shift, *d_cr, *d_ci, *o_vjp, *o_sr, *o_si;
+    const std::initializer_list<Out> out = {{&o_vjp, nt * ncot * npar, vjp}, {&o_sr, n_save, save_r}, {&o_si, n_save, save_i}};
+    rc = stage(h, history ? who : nullptr, {{&d_pcof, (double)nbatch * npar, pcof}, {&d_shift, (double)nsamples * h->n, shift},
+                                            {&d_cr, n_cot, cot_r}, {&d_ci, n_cot, cot_i}}, out, st);
+    if (rc) return rc;
+    VjpArgs V{};
+    V.ntraj = nbatch * nsamples * ncot; V.nsamples = nsamples; V.ncot = ncot; V.Npar = s.nspl; V.D1 = s.D1; V.pstride = npar;
+    V.pcof = d_pcof; V.shift = d_shift; V.cot_r = d_cr; V.cot_i = d_ci; V.save_every = history ? save_every : h->P.nsteps; V.nsave = nsave;
+    V.vjp = o_vjp;
+    (history ? V.hist_r : V.state_r) = o_sr;
+    (history ? V.hist_i : V.state_i) = o_si;
+    rc = record_launch(h, 9, st, [&](Ran &r) {
+        CU(jq_vjp_launch(h->P, V, st, &r.ctas, &r.regs, &r.smem, &r.tpc));
+        return 0;
+    });
+    if (rc) return rc;
+    return read_back(out, st);
 }
 
 extern "C" int jq_final_state_vjp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples, const double *shift,
                                   int32_t ncot, const double *cot_r, const double *cot_i, double *vjp, double *state_r, double *state_i) {
-    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
-    if (rc) return rc;
-    if (ncot < 1 || (!cot_r && !cot_i)) return fail(JQ_ERR_ARG, "jq_final_state_vjp: need ncot >= 1 and at least one of cot_r, cot_i");
-    if (!vjp) return fail(JQ_ERR_ARG, "jq_final_state_vjp: null vjp output");
-    if ((long long)nbatch * nsamples * ncot > 0x7fffffffLL)
-        return fail(JQ_ERR_ARG, "jq_final_state_vjp: nbatch * nsamples * ncot exceeds 2^31 - 1 trajectories per call");
-    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
-    if (jq_vjp_smem_bytes(h->P, nspl) > 227 * 1024)
-        return fail(JQ_ERR_ARG, "jq_final_state_vjp: problem too large for the VJP kernel's shared memory (n*m = %d)", h->n * h->m);
-    CU(cudaSetDevice(h->device));
-    cudaStream_t st = h->stream;
-    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ncot, len = (size_t)h->n * h->m;
-    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)nsamples * h->n : 0, n_cot = ntraj * len;
-    const size_t n_vjp = ntraj * npar, n_state = (state_r || state_i) ? nt * len : 0;
-    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_shift + (cot_r ? n_cot : 0) + (cot_i ? n_cot : 0))) != 0) return rc;
-    if ((rc = grow(&h->d_out, &h->cap_out, n_vjp + 2 * n_state)) != 0) return rc;
-    double *d_pcof = h->d_in, *cur = d_pcof + n_pcof;
-    double *d_shift = shift ? cur : nullptr; cur += n_shift;
-    double *d_cr = cot_r ? cur : nullptr; cur += cot_r ? n_cot : 0;
-    double *d_ci = cot_i ? cur : nullptr;
-    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (cot_r) CU(cudaMemcpyAsync(d_cr, cot_r, n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (cot_i) CU(cudaMemcpyAsync(d_ci, cot_i, n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
-
-    VjpArgs V{};
-    V.ntraj = (int)ntraj; V.nsamples = nsamples; V.ncot = ncot; V.Npar = nspl; V.D1 = nspl / (2 * h->Nc * h->Nfreq); V.pstride = npar;
-    V.pcof = d_pcof; V.shift = d_shift; V.cot_r = d_cr; V.cot_i = d_ci; V.save_every = h->P.nsteps; V.nsave = 1;
-    V.vjp = h->d_out;
-    V.state_r = n_state ? h->d_out + n_vjp : nullptr; V.state_i = n_state ? h->d_out + n_vjp + n_state : nullptr;
-    Ran ran;
-    ran.kernel = 9;
-    CU(cudaEventRecord(h->ev0, st));
-    CU(jq_vjp_launch(h->P, V, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc));
-    CU(cudaEventRecord(h->ev1, st));
-    h->timed = true;
-    h->ran = ran;
-    h->last_launches = 1;
-    CU(cudaMemcpyAsync(vjp, V.vjp, n_vjp * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (state_r) CU(cudaMemcpyAsync(state_r, V.state_r, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (state_i) CU(cudaMemcpyAsync(state_i, V.state_i, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    return 0;
-}
-
-// grow() for the buffers of the history derivatives, which reach hundreds of MB (cnot3 at save_every = 1: ~128 MB per trajectory and
-// cotangent or direction): a request larger than the device, or one cudaMalloc cannot satisfy, is JQ_ERR_ALLOC with the size
-static int grow_history(double **buf, size_t *cap, double need, const char *who) {
-    size_t free_b = 0, total_b = 0;
-    CU(cudaMemGetInfo(&free_b, &total_b));
-    if (need * sizeof(double) > (double)total_b)
-        return fail(JQ_ERR_ALLOC, "%s: needs %.1f GB in one device buffer, the device has %.1f GB", who, need * sizeof(double) / 1e9,
-                    total_b / 1e9);
-    if ((size_t)need <= *cap) return 0;
-    if (*buf) cudaFree(*buf);
-    *buf = nullptr;
-    *cap = 0;
-    const cudaError_t e = cudaMalloc((void **)buf, (size_t)need * sizeof(double));
-    if (e != cudaSuccess) {
-        *buf = nullptr;
-        cudaGetLastError();
-        return fail(e == cudaErrorMemoryAllocation ? JQ_ERR_ALLOC : JQ_ERR_CUDA, "%s: cudaMalloc of %.1f GB: %s", who,
-                    need * sizeof(double) / 1e9, cudaGetErrorString(e));
-    }
-    *cap = (size_t)need;
-    return 0;
+    return vjp_serial(h, "jq_final_state_vjp", false, nbatch, pcof, npar, nsamples, shift, 0, ncot, cot_r, cot_i, vjp, state_r, state_i);
 }
 
 extern "C" int jq_history_vjp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples, const double *shift,
                               int32_t save_every, int32_t ncot, const double *cot_r, const double *cot_i, double *vjp, double *hist_r,
                               double *hist_i) {
-    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
-    if (rc) return rc;
-    if ((rc = check_save_every(h, save_every)) != 0) return rc;
-    if (ncot < 1 || (!cot_r && !cot_i)) return fail(JQ_ERR_ARG, "jq_history_vjp: need ncot >= 1 and at least one of cot_r, cot_i");
-    if (!vjp) return fail(JQ_ERR_ARG, "jq_history_vjp: null vjp output");
-    if ((long long)nbatch * nsamples * ncot > 0x7fffffffLL)
-        return fail(JQ_ERR_ARG, "jq_history_vjp: nbatch * nsamples * ncot exceeds 2^31 - 1 trajectories per call");
-    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
-    if (jq_vjp_smem_bytes(h->P, nspl) > 227 * 1024)
-        return fail(JQ_ERR_ARG, "jq_history_vjp: problem too large for the VJP kernel's shared memory (n*m = %d)", h->n * h->m);
-    CU(cudaSetDevice(h->device));
-    cudaStream_t st = h->stream;
-    const long long nsave = h->P.nsteps / save_every + 1;
-    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ncot, len = (size_t)h->n * h->m;
-    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)nsamples * h->n : 0;
-    const double n_cot = (double)ntraj * nsave * len, n_hist = (hist_r || hist_i) ? (double)nt * nsave * len : 0.0;
-    const size_t n_vjp = ntraj * npar;
-    if ((rc = grow_history(&h->d_in, &h->cap_in, n_pcof + n_shift + (cot_r ? n_cot : 0) + (cot_i ? n_cot : 0), "jq_history_vjp")) != 0)
-        return rc;
-    if ((rc = grow_history(&h->d_out, &h->cap_out, n_vjp + 2 * n_hist, "jq_history_vjp")) != 0) return rc;
-    double *d_pcof = h->d_in, *cur = d_pcof + n_pcof;
-    double *d_shift = shift ? cur : nullptr; cur += n_shift;
-    double *d_cr = cot_r ? cur : nullptr; cur += cot_r ? (size_t)n_cot : 0;
-    double *d_ci = cot_i ? cur : nullptr;
-    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (cot_r) CU(cudaMemcpyAsync(d_cr, cot_r, (size_t)n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (cot_i) CU(cudaMemcpyAsync(d_ci, cot_i, (size_t)n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
-
-    VjpArgs V{};
-    V.ntraj = (int)ntraj; V.nsamples = nsamples; V.ncot = ncot; V.Npar = nspl; V.D1 = nspl / (2 * h->Nc * h->Nfreq); V.pstride = npar;
-    V.pcof = d_pcof; V.shift = d_shift; V.cot_r = d_cr; V.cot_i = d_ci; V.save_every = save_every; V.nsave = nsave;
-    V.vjp = h->d_out;
-    V.hist_r = n_hist > 0 ? h->d_out + n_vjp : nullptr; V.hist_i = n_hist > 0 ? h->d_out + n_vjp + (size_t)n_hist : nullptr;
-    Ran ran;
-    ran.kernel = 9;
-    CU(cudaEventRecord(h->ev0, st));
-    CU(jq_vjp_launch(h->P, V, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc));
-    CU(cudaEventRecord(h->ev1, st));
-    h->timed = true;
-    h->ran = ran;
-    h->last_launches = 1;
-    CU(cudaMemcpyAsync(vjp, V.vjp, n_vjp * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (hist_r) CU(cudaMemcpyAsync(hist_r, V.hist_r, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (hist_i) CU(cudaMemcpyAsync(hist_i, V.hist_i, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    return 0;
-}
-
-extern "C" int jq_history_jvp(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples, const double *shift,
-                              int32_t save_every, int32_t ndir, const double *dirs, double *dhist_r, double *dhist_i) {
-    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
-    if (rc) return rc;
-    if ((rc = check_save_every(h, save_every)) != 0) return rc;
-    if (ndir < 1 || !dirs) return fail(JQ_ERR_ARG, "jq_history_jvp: need ndir >= 1 and a dirs array");
-    if (!dhist_r || !dhist_i) return fail(JQ_ERR_ARG, "jq_history_jvp: null tangent-history output");
-    if ((long long)nbatch * nsamples * ndir > 0x7fffffffLL)
-        return fail(JQ_ERR_ARG, "jq_history_jvp: nbatch * nsamples * ndir exceeds 2^31 - 1 trajectories per call");
-    if (h->P.solver == 2) return fail(JQ_ERR_ARG, "jq_history_jvp: the Jacobi solver has no tangent sweep (use the Neumann solver)");
-    const int nspl = npar - (h->pfid == 3 ? 1 : 0);
-    if (jq_fwdsens_smem_bytes(h->P, nspl) > 227 * 1024)
-        return fail(JQ_ERR_ARG, "jq_history_jvp: problem too large for the tangent kernel's shared memory (n*m = %d)", h->n * h->m);
-    CU(cudaSetDevice(h->device));
-    cudaStream_t st = h->stream;
-    if ((rc = scratch_acquire(h, st)) != 0) return rc;
-    const long long nsave = h->P.nsteps / save_every + 1;
-    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * ndir, len = (size_t)h->n * h->m;
-    const size_t n_pcof = (size_t)nbatch * npar, n_dirs = (size_t)nbatch * ndir * npar, n_shift = shift ? (size_t)nsamples * h->n : 0;
-    const double n_hist = (double)ntraj * nsave * len;
-    if ((rc = grow(&h->d_in, &h->cap_in, n_pcof + n_dirs + n_shift)) != 0) return rc;
-    if ((rc = grow_history(&h->d_out, &h->cap_out, 2 * n_hist, "jq_history_jvp")) != 0) return rc;
-    if ((rc = grow(&h->d_scal, &h->cap_traj, nt * 4)) != 0) return rc;
-    if ((rc = grow(&h->d_grad, &h->cap_grad, ntraj)) != 0) return rc;
-    if ((rc = grow(&h->d_igrad, &h->cap_igrad, ntraj)) != 0) return rc;
-    double *d_pcof = h->d_in, *d_dirs = d_pcof + n_pcof, *d_shift = shift ? d_dirs + n_dirs : nullptr;
-    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_dirs, dirs, n_dirs * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (n_shift) CU(cudaMemcpyAsync(d_shift, shift, n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
-
-    SensArgs S{};
-    S.ntraj = (int)ntraj; S.nsamples = nsamples; S.ndir = ndir; S.Npar = nspl; S.D1 = nspl / (2 * h->Nc * h->Nfreq); S.pstride = npar;
-    S.pcof = d_pcof; S.dirs = d_dirs; S.shift = d_shift;
-    S.scal = h->d_scal; S.dinfid = h->d_grad; S.dleak = h->d_igrad;         // written by the kernel, not returned
-    S.dhist_r = h->d_out; S.dhist_i = h->d_out + (size_t)n_hist; S.save_every = save_every; S.nsave = nsave;
-    Ran ran;
-    ran.kernel = 8;
-    CU(cudaEventRecord(h->ev0, st));
-    CU(jq_fwdsens_launch(h->P, S, st, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc));
-    CU(cudaEventRecord(h->ev1, st));
-    h->timed = true;
-    h->ran = ran;
-    h->last_launches = 1;
-    if ((rc = scratch_release(h, st)) != 0) return rc;
-    CU(cudaMemcpyAsync(dhist_r, S.dhist_r, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(dhist_i, S.dhist_i, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    return 0;
+    return vjp_serial(h, "jq_history_vjp", true, nbatch, pcof, npar, nsamples, shift, save_every, ncot, cot_r, cot_i, vjp, hist_r, hist_i);
 }
 
 // The VJP entries on the time-parallel path: cotangents [traj][nsave][n*m] of the saved states (nsave = 1, save_every = nsteps: of U(T),
@@ -1262,7 +1220,8 @@ extern "C" int jq_history_jvp(jq_handle *h, int32_t nbatch, const double *pcof, 
 static int vjp_time_parallel(jq_handle *h, const char *who, bool history, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,
                              const double *shift, int32_t save_every, int32_t ncot, const double *cot_r, const double *cot_i, double *vjp,
                              double *state_r, double *state_i, double *hist_r, double *hist_i) {
-    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift);
+    const int nc = std::max<int>(ncot, 1);
+    int rc = check_batch_args(h, nbatch, pcof, npar, nsamples, shift, false, nc, who);
     if (rc) return rc;
     if (history && (rc = check_save_every(h, save_every)) != 0) return rc;
     if (ncot < 0) return fail(JQ_ERR_ARG, "%s: need ncot >= 0 (0: %s only)", who, history ? "the history" : "U(T)");
@@ -1270,9 +1229,6 @@ static int vjp_time_parallel(jq_handle *h, const char *who, bool history, int32_
     if (ncot == 0 && history && !hist_r && !hist_i) return fail(JQ_ERR_ARG, "%s: ncot = 0 returns the history only and needs hist_r or hist_i", who);
     if (ncot > 0 && !cot_r && !cot_i) return fail(JQ_ERR_ARG, "%s: need at least one of cot_r, cot_i", who);
     if (ncot > 0 && !vjp) return fail(JQ_ERR_ARG, "%s: null vjp output", who);
-    const int nc = std::max<int>(ncot, 1);
-    if ((long long)nbatch * nsamples * nc > 0x7fffffffLL)
-        return fail(JQ_ERR_ARG, "%s: nbatch * nsamples * ncot exceeds 2^31 - 1 trajectories per call", who);
     if (!h->route[TIME_PARALLEL].ok) return fail(JQ_ERR_ARG, "%s: %s", who, h->route[TIME_PARALLEL].why);
     // the pulled-back adjoint is the unforced second set of objFuncType 2/3: every launch sees objFuncType 2, whatever the problem's
     DevProblem P = h->P;
@@ -1288,56 +1244,34 @@ static int vjp_time_parallel(jq_handle *h, const char *who, bool history, int32_
     // trajectory (b, s, k) is kernel-7 trajectory b * nsamples * nc + s * nc + k: sample s * nc + k of candidate b, whose shift row is s
     const int ns2 = nsamples * nc;
     const long long nsave = history ? h->P.nsteps / save_every + 1 : 1;
-    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * nc, len = (size_t)h->n * h->m;
-    const size_t n_pcof = (size_t)nbatch * npar, n_shift = shift ? (size_t)ns2 * h->n : 0;
-    const double n_cot = ncot > 0 ? (double)ntraj * nsave * len : 0.0;
-    const size_t n_vjp = ncot > 0 ? ntraj * npar : 0, n_state = (state_r || state_i) ? nt * len : 0;
-    const double n_hist = (hist_r || hist_i) ? (double)nt * nsave * len : 0.0;
-    const double *cr = ncot > 0 ? cot_r : nullptr, *ci = ncot > 0 ? cot_i : nullptr;
+    const size_t nt = (size_t)nbatch * nsamples, ntraj = nt * nc;
+    const double len = (double)h->n * h->m, n_cot = ncot > 0 ? (double)ntraj * nsave * len : 0.0;
+    const double n_vjp = ncot > 0 ? (double)ntraj * npar : 0.0, n_state = state_r || state_i ? nt * len : 0.0;
+    const double n_hist = hist_r || hist_i ? nt * nsave * len : 0.0;
     const int nseg = seg_count(h, (int)ntraj, 1);
-    const size_t need = jq_seg_vjp_workspace_doubles(P, (int)ntraj, npar - (h->pfid == 3 ? 1 : 0), nseg, ncot > 0, nsave > 1);
+    const size_t need = jq_seg_workspace(P, (int)ntraj, splines(h, npar).nspl, nseg, true, ncot > 0, nsave > 1);
     if (need > h->cap_seg && (rc = grow_history(&h->d_seg, &h->cap_seg, (double)need, who)) != 0) return rc;
     if ((rc = seg_times_upload(h, nseg, st)) != 0) return rc;
-    // histories reach hundreds of MB: JQ_ERR_ALLOC with the size when they do not fit
-    auto grow_io = [&](double **buf, size_t *cap, double cnt) { return history ? grow_history(buf, cap, cnt, who) : grow(buf, cap, (size_t)cnt); };
-    if ((rc = grow_io(&h->d_in, &h->cap_in, n_pcof + n_shift + (cr ? n_cot : 0) + (ci ? n_cot : 0))) != 0) return rc;
-    if ((rc = grow_io(&h->d_out, &h->cap_out, n_vjp + 2 * n_state + 2 * n_hist)) != 0) return rc;
-    double *d_pcof = h->d_in, *cur = d_pcof + n_pcof;
-    double *d_shift = shift ? cur : nullptr; cur += n_shift;
-    double *d_cr = cr ? cur : nullptr; cur += cr ? (size_t)n_cot : 0;
-    double *d_ci = ci ? cur : nullptr;
-    std::vector<double> shifts(n_shift);
+    std::vector<double> shifts(shift ? (size_t)ns2 * h->n : 0);
     for (size_t r = 0; r < (shift ? (size_t)ns2 : 0); ++r) memcpy(&shifts[r * h->n], shift + (r / nc) * h->n, h->n * sizeof(double));
-    CU(cudaMemcpyAsync(d_pcof, pcof, n_pcof * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (n_shift) CU(cudaMemcpyAsync(d_shift, shifts.data(), n_shift * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (cr) CU(cudaMemcpyAsync(d_cr, cr, (size_t)n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (ci) CU(cudaMemcpyAsync(d_ci, ci, (size_t)n_cot * sizeof(double), cudaMemcpyHostToDevice, st));
-    double *o_vjp = n_vjp ? h->d_out : nullptr, *o_sr = n_state ? h->d_out + n_vjp : nullptr, *o_si = n_state ? o_sr + n_state : nullptr;
-    double *o_hr = n_hist > 0 ? h->d_out + n_vjp + 2 * n_state : nullptr, *o_hi = n_hist > 0 ? o_hr + (size_t)n_hist : nullptr;
-
-    const LaunchArgs A = launch_args(h, nbatch, npar, ns2, d_pcof, d_shift);
-    Ran ran;
-    ran.kernel = 7;
-    ran.nseg = nseg;
-    CU(cudaEventRecord(h->ev0, st));
-    rc = launched(jq_seg_vjp_launch(h->seg_prop, h->route[TIME_PARALLEL].plan, fiber, P, A, nseg, h->d_segt,
-                                    reinterpret_cast<int *>(h->d_segt + 2 * (size_t)nseg), h->d_seg, st, ncot,
-                                    history ? save_every : (int)h->P.nsteps, nsave, d_cr, d_ci, o_vjp, state_r ? o_sr : nullptr,
-                                    state_i ? o_si : nullptr, o_hr, o_hi, &ran.ctas, &ran.regs, &ran.smem, &ran.tpc, &ran.launches),
-                  false, who);
+    double *d_pcof, *d_shift, *d_cr, *d_ci, *o_vjp, *o_sr, *o_si, *o_hr, *o_hi;
+    const std::initializer_list<Out> out = {{&o_vjp, n_vjp, vjp}, {&o_sr, n_state, state_r}, {&o_si, n_state, state_i},
+                                            {&o_hr, n_hist, hist_r}, {&o_hi, n_hist, hist_i}};
+    // histories reach hundreds of MB: JQ_ERR_ALLOC with the size when they do not fit
+    rc = stage(h, history ? who : nullptr, {{&d_pcof, (double)nbatch * npar, pcof}, {&d_shift, (double)shifts.size(), shift ? shifts.data() : nullptr},
+                                            {&d_cr, n_cot, ncot > 0 ? cot_r : nullptr}, {&d_ci, n_cot, ncot > 0 ? cot_i : nullptr}}, out, st);
     if (rc) return rc;
-    CU(cudaEventRecord(h->ev1, st));
-    h->timed = true;
-    h->ran = ran;
-    h->last_launches = ran.launches;
-    if ((rc = scratch_release(h, st)) != 0) return rc;
-    if (n_vjp) CU(cudaMemcpyAsync(vjp, o_vjp, n_vjp * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (state_r) CU(cudaMemcpyAsync(state_r, o_sr, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (state_i) CU(cudaMemcpyAsync(state_i, o_si, n_state * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (hist_r) CU(cudaMemcpyAsync(hist_r, o_hr, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (hist_i) CU(cudaMemcpyAsync(hist_i, o_hi, (size_t)n_hist * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    return 0;
+    const LaunchArgs A = launch_args(h, nbatch, npar, ns2, d_pcof, d_shift);
+    rc = record_launch(h, 7, st, [&](Ran &r) {
+        r.nseg = nseg;
+        return launched(jq_seg_vjp_launch(h->seg_prop, h->route[TIME_PARALLEL].plan, fiber, P, A, nseg, h->d_segt,
+                                          reinterpret_cast<int *>(h->d_segt + 2 * (size_t)nseg), h->d_seg, st, ncot,
+                                          history ? save_every : (int)h->P.nsteps, nsave, d_cr, d_ci, o_vjp, state_r ? o_sr : nullptr,
+                                          state_i ? o_si : nullptr, o_hr, o_hi, &r.ctas, &r.regs, &r.smem, &r.tpc, &r.launches),
+                        false, who);
+    });
+    if (rc || (rc = scratch_release(h, st)) != 0) return rc;
+    return read_back(out, st);
 }
 
 extern "C" int jq_final_state_vjp_time_parallel(jq_handle *h, int32_t nbatch, const double *pcof, int32_t npar, int32_t nsamples,

@@ -169,7 +169,10 @@ cudaError_t jq_traj_launch(TrajPlan *plan, const DevProblem &P, const LaunchArgs
 bool jq_seg_supported(const TrajPlan *plan, const DevProblem &P, bool second_adjoint = false, bool hist = false);
 int jq_seg_ld(const DevProblem &P);
 int jq_seg_auto_segments(const DevProblem &P, int ntraj, int evaladjoint, int tpc, int sms);
-size_t jq_seg_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, int evaladjoint);
+// Doubles of the segment workspace of the evaluation (vjp false; adjoint: evaladjoint) or of the VJP (adjoint: cotangents, jumps: a
+// history); with `work`, also its arrays in S
+size_t jq_seg_workspace(const DevProblem &P, int ntraj, int Npar, int nseg, bool vjp, bool adjoint, bool jumps, double *work = nullptr,
+                        SegArgs *S = nullptr);
 void jq_seg_times(const DevProblem &P, int nseg, double *times /* [2][nseg], host */);
 // plan_prop: plan of the propagator launch (many independent sweeps: a throughput layout pays), plan: the boundary-to-boundary sweeps
 // plan_obj: plan of the gradient sweep when objFuncType != 1 (second adjoint set; nullptr otherwise)
@@ -186,7 +189,6 @@ cudaError_t jq_seg_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_ob
 // Vector-Jacobian products of the saved states on the segment sweeps (the unforced adjoint set of jq_seg_launch from caller-supplied
 // cotangents [traj][nsave][n*m]; nsave = 1, save_every = nsteps: of U(T) alone; ncot = 0: U(T) and / or the history only).  P:
 // objFuncType 2 or 3 whatever the problem's own; plan_obj: the two-set gradient sweep.
-size_t jq_seg_vjp_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, bool cotangents, bool jumps);
 cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_obj, const DevProblem &P, const LaunchArgs &A, int nseg,
                               const double *times, int *flags /* 4 ints, device */, double *work, cudaStream_t st, int ncot,
                               int save_every, long long nsave, const double *cot_r, const double *cot_i, double *vjp, double *state_r,

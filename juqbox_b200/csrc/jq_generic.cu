@@ -816,29 +816,7 @@ cudaError_t jq_controls_launch(const DevProblem &P, int D1, const double *pcof, 
     return cudaGetLastError();
 }
 
-cudaError_t jq_generic_launch(const DevProblem &P, const LaunchArgs &A, cudaStream_t st, int *nctas, int *regs, size_t *smem) {
-    size_t bytes = 0;
-    const GenGeom G = generic_geometry(P, per_group_doubles(P, A.Npar), &bytes);
-    cudaError_t e = cudaFuncSetAttribute(jq_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e != cudaSuccess) return e;
-    cudaFuncAttributes fa;
-    e = cudaFuncGetAttributes(&fa, jq_generic_kernel);
-    if (e != cudaSuccess) return e;
-    int dev = 0, sms = 148, occ = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, jq_generic_kernel, G.tpt * G.gpc, bytes);
-    if (occ < 1) occ = 1;
-    const int want = (A.ntraj + G.gpc - 1) / G.gpc;
-    int grid = want < sms * occ ? want : sms * occ;   // persistent: groups loop over trajectories
-    jq_generic_kernel<<<grid, G.tpt * G.gpc, bytes, st>>>(P, A, G);
-    if (nctas) *nctas = grid;
-    if (regs) *regs = fa.numRegs;
-    if (smem) *smem = bytes;
-    return cudaGetLastError();
-}
-
-// One launch of a persistent generic-layout kernel (forward sensitivities, final-state VJPs): at most one resident wave of CTAs, whose
+// One launch of a persistent generic-layout kernel (evaluation, forward sensitivities, VJPs): at most one resident wave of CTAs, whose
 // groups loop over the ntraj trajectories.
 template <class Args>
 static cudaError_t persistent_launch(void (*kernel)(DevProblem, Args, GenGeom), const DevProblem &P, const Args &A, int ntraj,
@@ -863,6 +841,10 @@ static cudaError_t persistent_launch(void (*kernel)(DevProblem, Args, GenGeom), 
     if (smem) *smem = bytes;
     if (gpc) *gpc = G.gpc;
     return cudaGetLastError();
+}
+
+cudaError_t jq_generic_launch(const DevProblem &P, const LaunchArgs &A, cudaStream_t st, int *nctas, int *regs, size_t *smem) {
+    return persistent_launch(jq_generic_kernel, P, A, A.ntraj, per_group_doubles(P, A.Npar), st, nctas, regs, smem, /*gpc*/ nullptr);
 }
 
 cudaError_t jq_fwdsens_launch(const DevProblem &P, const SensArgs &S, cudaStream_t st, int *nctas, int *regs, size_t *smem, int *gpc) {

@@ -490,12 +490,31 @@ int jq_seg_auto_segments(const DevProblem &P, int ntraj, int evaladjoint, int tp
 // Leading dimension of the segment propagators: 8, 16 or 32 for the one-warp joins (zero padded), 2n for the block join.
 int jq_seg_ld(const DevProblem &P) { const int n2 = 2 * P.n; return n2 <= 8 ? 8 : n2 <= 16 ? 16 : n2 <= 32 ? 32 : n2; }
 
-size_t jq_seg_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, int evaladjoint) {
-    const size_t n2 = (size_t)jq_seg_ld(P), nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)ntraj, ns = (size_t)nseg;
-    size_t tot = ns * nt * n2 * n2 + (ns + 1) * nt * nm2 + ns * nt;                      // Phi, X, penpart
-    if (evaladjoint) tot += ns * nt * n2 * n2 + 2 * (ns + 1) * nt * nm2 + 2 * ns * nt * nm2 + ns * nt * (size_t)Npar;     // Adj, Lam, Eta, cpart, dpart, gpart
-    if (evaladjoint && P.objFuncType != 1) tot += (ns + 1) * nt * nm2 + ns * nt * (size_t)Npar;                      // Lam2, gpart2
-    tot += 20;                                                                                                          // even-count padding of every array
+// The segment workspace of a driver, counted and, given `work`, carved into S's arrays in that driver's order.
+// Every array is rounded to an even number of doubles, so that each starts 16-byte aligned.
+//   evaluation (vjp false): Phi, X, penpart; with `adjoint` also Adj, Lam, Eta, cpart, dpart, gpart and, for objFuncType 2/3, Lam2, gpart2
+//   VJP: Phi, X; with `adjoint` (cotangents) also Adj, Lam2, Eta, dpart, gpart, gpart2 and, with `jumps` (a history), cpart
+size_t jq_seg_workspace(const DevProblem &P, int ntraj, int Npar, int nseg, bool vjp, bool adjoint, bool jumps, double *work, SegArgs *S) {
+    const size_t ld = (size_t)jq_seg_ld(P), nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)ntraj, ns = (size_t)nseg;
+    const size_t prop = ns * nt * ld * ld, bound = (ns + 1) * nt * nm2, part = ns * nt * nm2, grad = ns * nt * (size_t)Npar;
+    SegArgs count{};
+    SegArgs &A = S ? *S : count;
+    size_t tot = 0;
+    auto take = [&](double *&dst, size_t cnt) { dst = work ? work + tot : nullptr; tot += (cnt + 1) & ~(size_t)1; };
+    take(A.Phi, prop);
+    take(A.X, bound);
+    if (!vjp) take(A.penpart, ns * nt);
+    if (adjoint) {
+        take(A.Adj, prop);
+        take(vjp ? A.Lam2 : A.Lam, bound);
+        take(A.Eta, bound);
+        if (!vjp) take(A.cpart, part);
+        take(A.dpart, part);
+        take(A.gpart, grad);
+        if (!vjp && P.objFuncType != 1) take(A.Lam2, bound);
+        if (vjp || P.objFuncType != 1) take(A.gpart2, grad);
+        if (vjp && jumps) take(A.cpart, part);
+    }
     return tot;
 }
 
@@ -519,43 +538,34 @@ void jq_seg_times(const DevProblem &P, int nseg, double *times) {
     }
 }
 
-cudaError_t jq_seg_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_obj, const DevProblem &P, const LaunchArgs &A0, int nseg, const double *times, int *flags, double *work, cudaStream_t st, const SegCoop *coop,
-                          int *nctas, int *regs, size_t *smem, int *traj_per_cta, int *nlaunch) {
-    if (nseg < 1 || nseg > P.nsteps) return cudaErrorInvalidValue;
-    if (P.solver != 1 || A0.hist_r || (P.objFuncType != 1 && (!plan_obj || (A0.evaladjoint && !A0.infidgrad)))) return cudaErrorNotSupported;
-    const size_t n2 = 2 * (size_t)P.n, nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)A0.ntraj, ns = (size_t)nseg;
-    if (n2 > 512) return cudaErrorNotSupported;
-    LaunchArgs A = A0;
+// The segment set-up of both drivers: A's segment count, times, propagator stride and refinement state, the workspace arrays of
+// jq_seg_workspace (with the adjoint sets when A.evaladjoint), the refinement flags cleared and the padding of the propagators zeroed
+static void seg_setup(const DevProblem &P, LaunchArgs &A, int nseg, const double *times, int *flags, double *work, bool vjp, bool jumps,
+                      cudaStream_t st) {
+    const size_t ld = (size_t)jq_seg_ld(P), nt = (size_t)A.ntraj, ns = (size_t)nseg;
     A.seg.nseg = nseg;
     A.seg.times = times;
-    const size_t ld = (size_t)jq_seg_ld(P);
     A.seg.ld = (int)ld;
     A.seg.pass = 0;
     A.seg.flags = flags;
     A.seg.refine_tol = 1.0e-9 / (double)nseg;              // |eps| <~ nseg |d|: below 1e-9 the first-order join is exact to 1e-12 and better
-    double *w = work;
-    auto take = [&](size_t cnt) { double *p = w; w += (cnt + 1) & ~(size_t)1; return p; };
-    A.seg.Phi = take(ns * nt * ld * ld);
-    A.seg.X = take((ns + 1) * nt * nm2);
-    A.seg.penpart = take(ns * nt);
-    if (A.evaladjoint) {
-        A.seg.Adj = take(ns * nt * ld * ld);
-        A.seg.Lam = take((ns + 1) * nt * nm2);
-        A.seg.Eta = take((ns + 1) * nt * nm2);
-        A.seg.cpart = take(ns * nt * nm2);
-        A.seg.dpart = take(ns * nt * nm2);
-        A.seg.gpart = take(ns * nt * (size_t)A.Npar);
-        if (P.objFuncType != 1) {
-            A.seg.Lam2 = take((ns + 1) * nt * nm2);
-            A.seg.gpart2 = take(ns * nt * (size_t)A.Npar);
-        }
-    }
-    int launches = 0;
+    jq_seg_workspace(P, A.ntraj, A.Npar, nseg, vjp, A.evaladjoint, jumps, work, &A.seg);
     cudaMemsetAsync(flags, 0, 4 * sizeof(int), st);
-    if (ld != n2) {            // the padding of the propagators must read as zero
+    if (ld != 2 * (size_t)P.n) {            // the padding of the propagators must read as zero
         cudaMemsetAsync(A.seg.Phi, 0, ns * nt * ld * ld * sizeof(double), st);
         if (A.evaladjoint) cudaMemsetAsync(A.seg.Adj, 0, ns * nt * ld * ld * sizeof(double), st);
     }
+}
+
+cudaError_t jq_seg_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_obj, const DevProblem &P, const LaunchArgs &A0, int nseg, const double *times, int *flags, double *work, cudaStream_t st, const SegCoop *coop,
+                          int *nctas, int *regs, size_t *smem, int *traj_per_cta, int *nlaunch) {
+    if (nseg < 1 || nseg > P.nsteps) return cudaErrorInvalidValue;
+    if (P.solver != 1 || A0.hist_r || (P.objFuncType != 1 && (!plan_obj || (A0.evaladjoint && !A0.infidgrad)))) return cudaErrorNotSupported;
+    const size_t nt = (size_t)A0.ntraj, ld = (size_t)jq_seg_ld(P);
+    if (2 * P.n > 512) return cudaErrorNotSupported;
+    LaunchArgs A = A0;
+    seg_setup(P, A, nseg, times, flags, work, false, false, st);
+    int launches = 0;
     StageTimer timer(st);
     timer.mark();
     // launch 1: propagators
@@ -618,14 +628,6 @@ cudaError_t jq_seg_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *plan_ob
     return cudaGetLastError();
 }
 
-size_t jq_seg_vjp_workspace_doubles(const DevProblem &P, int ntraj, int Npar, int nseg, bool cotangents, bool jumps) {
-    const size_t ld = (size_t)jq_seg_ld(P), nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)ntraj, ns = (size_t)nseg;
-    size_t tot = ns * nt * ld * ld + (ns + 1) * nt * nm2;                                               // Phi, X
-    if (cotangents) tot += ns * nt * ld * ld + 2 * (ns + 1) * nt * nm2 + ns * nt * nm2 + 2 * ns * nt * (size_t)Npar;    // Adj, Lam2, Eta, dpart, gpart, gpart2
-    if (cotangents && jumps) tot += ns * nt * nm2;                                                      // cpart
-    return tot + 18;                                                                                    // even-count padding of every array
-}
-
 // Vector-Jacobian products of the saved states on the segment sweeps (DESIGN.md §4.9, §4.10): the stages of jq_seg_launch that the
 // unforced adjoint set (kind 4, Lam2) needs, started from the callers' cotangents instead of the objective's terminal adjoint --
 //   launch 1  Phi_p (mode 1) and, with cotangents, Adj_p (mode 3)
@@ -654,30 +656,11 @@ cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *pla
     const bool cot = ncot > 0, jumps = cot && nsave > 1 && (cot_r || cot_i), hist = hist_r || hist_i;
     if (P.solver != 1 || P.objFuncType == 1 || A0.hist_r || 2 * P.n > 512 || (cot && !plan_obj)) return cudaErrorNotSupported;
     if (hist && !(hist_r && hist_i)) return cudaErrorInvalidValue;
-    const size_t n2 = 2 * (size_t)P.n, nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)A0.ntraj, ns = (size_t)nseg;
+    const size_t nm2 = 2 * (size_t)P.n * P.m, nt = (size_t)A0.ntraj;
     LaunchArgs A = A0;
     A.evaladjoint = cot ? 1 : 0;
-    A.seg.nseg = nseg;
-    A.seg.times = times;
-    const size_t ld = (size_t)jq_seg_ld(P);
-    A.seg.ld = (int)ld;
-    A.seg.pass = 0;
-    A.seg.flags = flags;
-    A.seg.refine_tol = 1.0e-9 / (double)nseg;              // as in jq_seg_launch
-    double *w = work;
-    auto take = [&](size_t cnt) { double *p = w; w += (cnt + 1) & ~(size_t)1; return p; };
-    A.seg.Phi = take(ns * nt * ld * ld);
-    A.seg.X = take((ns + 1) * nt * nm2);
-    if (cot) {
-        A.seg.Adj = take(ns * nt * ld * ld);
-        A.seg.Lam2 = take((ns + 1) * nt * nm2);
-        A.seg.Eta = take((ns + 1) * nt * nm2);
-        A.seg.dpart = take(ns * nt * nm2);
-        A.seg.gpart = take(ns * nt * (size_t)A.Npar);
-        A.seg.gpart2 = take(ns * nt * (size_t)A.Npar);
-        A.seg.Lam = A.seg.Lam2;
-        if (jumps) A.seg.cpart = take(ns * nt * nm2);
-    }
+    seg_setup(P, A, nseg, times, flags, work, true, jumps, st);
+    if (cot) A.seg.Lam = A.seg.Lam2;        // mode 5 sweeps the forced set from Lam2 (its gradient shares are discarded)
     // the history VJP's additions to the launches: the saves of mode 2 (cotangent 0 of every (candidate, sample)), the third mode of
     // launch 2 and the cotangent jumps of modes 7 and 5
     SegHist H{};
@@ -685,11 +668,6 @@ cudaError_t jq_seg_vjp_launch(TrajPlan *plan_prop, TrajPlan *plan, TrajPlan *pla
     if (jumps) { H.cot_r = cot_r; H.cot_i = cot_i; }
     const size_t nm = nm2 / 2;
     int launches = 0;
-    cudaMemsetAsync(flags, 0, 4 * sizeof(int), st);
-    if (ld != n2) {            // the padding of the propagators must read as zero
-        cudaMemsetAsync(A.seg.Phi, 0, ns * nt * ld * ld * sizeof(double), st);
-        if (cot) cudaMemsetAsync(A.seg.Adj, 0, ns * nt * ld * ld * sizeof(double), st);
-    }
     // Eta_0, which no join writes, enters the refinement passes' defect of segment 0 (dpart_0 feeds nothing, but the flag does): zero,
     // so that a stale workspace cannot start a pass
     if (cot) cudaMemsetAsync(A.seg.Eta, 0, nt * nm2 * sizeof(double), st);
