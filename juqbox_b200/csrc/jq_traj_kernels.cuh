@@ -645,6 +645,42 @@ __device__ __forceinline__ void group_sum_n(double (&v)[N], int GL, int base) {
     UNROLL for (int i = 0; i < N; ++i) v[i] = s[i];
 }
 
+// Reduce-scatter of N values over the GL lanes of a group (GL a compile-time power of two) by recursive halving: the values,
+// padded with zeros to M = a power of two, are halved over the low lane bits -- a lane sends the half it gives up to its partner
+// and adds the half it keeps -- and when fewer than GL lanes share them, the last K = max(M / GL, 1) are summed by xor butterfly over
+// the remaining bits.  Lane lg ends with the full sums of values first .. first + K - 1 in s (returned: first); the lanes whose
+// butterfly bits are zero own them.  The pair sums are the same on both partners (addition commutes), so the summation tree, and
+// every result bit, depends only on the group's lanes, not on where the group sits.  A lane sends M - K values over the halving
+// rounds and K per butterfly round, where the butterfly of group_sum_n sends N per round.
+constexpr int ilog2(int x) { return x > 1 ? 1 + ilog2(x / 2) : 0; }
+template <int N, int GL>
+struct ScatterShape {
+    static_assert(GL > 0 && (GL & (GL - 1)) == 0, "reduce-scatter: power-of-two group");
+    static constexpr int M = 1 << ilog2(2 * N - 1), K = M > GL ? M / GL : 1, H = ilog2(M / K);     // H: halving rounds
+};
+template <int N, int GL>
+__device__ __forceinline__ int group_scatter_sum(const double (&v)[N], int lg, double (&s)[ScatterShape<N, GL>::K]) {
+    constexpr int M = ScatterShape<N, GL>::M, K = ScatterShape<N, GL>::K, H = ScatterShape<N, GL>::H;
+    double c[M];
+    UNROLL for (int i = 0; i < M; ++i) c[i] = i < N ? v[i] : 0.0;
+    int first = 0;
+    UNROLL for (int r = 0; r < H; ++r) {                 // all sends of a round are independent: one shuffle latency per round
+        const int half = M >> (r + 1);
+        const bool hi = (lg >> r) & 1;
+        double g[M > 1 ? M / 2 : 1];
+        UNROLL for (int i = 0; i < half; ++i) g[i] = __shfl_xor_sync(0xffffffffu, hi ? c[i] : c[half + i], 1 << r);
+        UNROLL for (int i = 0; i < half; ++i) c[i] = (hi ? c[half + i] : c[i]) + g[i];
+        if (hi) first += half;
+    }
+    UNROLL for (int o = 1 << H; o < GL; o <<= 1) {
+        double g[K];
+        UNROLL for (int i = 0; i < K; ++i) g[i] = __shfl_xor_sync(0xffffffffu, c[i], o);
+        UNROLL for (int i = 0; i < K; ++i) c[i] += g[i];
+    }
+    UNROLL for (int i = 0; i < K; ++i) s[i] = c[i];
+    return first;
+}
+
 // (H0 x)_e for the lane's element e: diagonal entry times x_e, plus the off-diagonal drift product x0 in HX layouts.
 template <class LaneT>
 __device__ __forceinline__ double kdiag(const LaneT &L, int e, double xe, double x0) {
@@ -806,17 +842,39 @@ __device__ __forceinline__ void state_step(LaneT &L, int J, double h, double (&u
 // traces per control of adjoint_grad_calc! (src/evalobjgrad.jl:2578-2618):
 //   T[q][0] = tr(vr0,Ha,lr05)  T[q][1] = tr(vi05,Hs,lr05)  T[q][2] = tr(vr,Ha,lr05)
 //   T[q][3] = tr(vr,Hs,li)+tr(vr0,Hs,li0)                   T[q][4] = tr(vi05,Ha,li)+tr(vi05,Ha,li0)
-// The group-reduced traces are left in shared memory at tred[q*5 + a] (written by lane 0 of the group).
+// The group-reduced traces are left in shared memory at tred[q*5 + a] (written by lane 0 of the group, or with RS by their
+// owners).
 // DEFER: the lane's partial traces are returned in tpart[q*5 + a] instead of being reduced over the group (pipelined
 // instantiations hand them to the gradient role).
+// RS > 0: the traces are reduce-scattered over the group of RS lanes (group_scatter_sum), and `writer` only says that the lane
+// belongs to a group.
 // tcar: the lane-partial tr(vr0,Hs,li0) of this step on entry -- the tr(vr,Hs,li) of the step before (trace_hs before the first) --
 // and tr(vr,Hs,li) on return, so that every boundary trace is summed once.
-template <int JT, bool FORCING, class LaneT, bool DEFER = false>
+template <int JT, bool FORCING, class LaneT, bool DEFER = false, int RS = 0>
 __device__ __forceinline__ void adjoint_step(LaneT &L, int J, double h, double (&mu)[LaneT::E], double (&nu)[LaneT::E],
                                              const double (&vr0)[LaneT::E], const double (&vi05)[LaneT::E],
                                              const double (&vr)[LaneT::E], double *tred, int GL, int gbase_lane, bool writer,
                                              double *tpart = nullptr, double *tcar = nullptr) {
     constexpr int E = LaneT::E, NC = LaneT::NC;
+    // the group's reduced traces into tred: v holds A of the five traces per control, starting at trace a0
+    auto reduce = [&](auto &v, auto a0c) {
+        constexpr int A = std::extent_v<std::remove_reference_t<decltype(v)>> / NC, a0 = decltype(a0c)::value;
+        if constexpr (RS > 0) {
+            constexpr int K = ScatterShape<NC * A, RS>::K, H = ScatterShape<NC * A, RS>::H;
+            const int lg = (threadIdx.x & 31) & (RS - 1);
+            double sv[K];
+            const int first = group_scatter_sum<NC * A, RS>(v, lg, sv);
+            if (writer && (lg >> H) == 0) {
+                UNROLL for (int i = 0; i < K; ++i) {
+                    const int j = first + i;
+                    if (j < NC * A) tred[(j / A) * 5 + a0 + j % A] = sv[i];
+                }
+            }
+        } else {
+            group_sum_n(v, GL, gbase_lane);
+            if (writer) { UNROLL for (int qq = 0; qq < NC; ++qq) UNROLL for (int a = 0; a < A; ++a) tred[qq * 5 + a0 + a] = v[qq * A + a]; }
+        }
+    };
     double rhs[E], s05n[E], Tb[NC][2];
     typename LaneT::SC sc;
     L.sync_reset();
@@ -861,10 +919,7 @@ __device__ __forceinline__ void adjoint_step(LaneT &L, int J, double h, double (
         UNROLL for (int qq = 0; qq < NC; ++qq) UNROLL for (int a = 0; a < 3; ++a) tv3[qq * 3 + a] = Ta[qq][a];
         if constexpr (LaneSigned<LaneT>::value) { UNROLL for (int qq = 0; qq < NC; ++qq) { tv3[qq * 3] *= L.dsign(qq); tv3[qq * 3 + 2] *= L.dsign(qq); } }
         if constexpr (DEFER) { UNROLL for (int qq = 0; qq < NC; ++qq) UNROLL for (int a = 0; a < 3; ++a) tpart[qq * 5 + a] = tv3[qq * 3 + a]; }
-        else {
-            group_sum_n(tv3, GL, gbase_lane);
-            if (writer) { UNROLL for (int qq = 0; qq < NC; ++qq) UNROLL for (int a = 0; a < 3; ++a) tred[qq * 5 + a] = tv3[qq * 3 + a]; }
-        }
+        else reduce(tv3, std::integral_constant<int, 0>{});
     }
     L.s_prescale(1, sc);
     double l1[E];
@@ -894,10 +949,7 @@ __device__ __forceinline__ void adjoint_step(LaneT &L, int J, double h, double (
         if (tcar) { UNROLL for (int qq = 0; qq < NC; ++qq) { tv2[qq * 2] += tcar[qq]; tcar[qq] = Tb[qq][0]; } }
         if constexpr (LaneSigned<LaneT>::value) { UNROLL for (int qq = 0; qq < NC; ++qq) tv2[qq * 2 + 1] *= L.dsign(qq); }
         if constexpr (DEFER) { UNROLL for (int qq = 0; qq < NC; ++qq) UNROLL for (int a = 0; a < 2; ++a) tpart[qq * 5 + 3 + a] = tv2[qq * 2 + a]; }
-        else {
-            group_sum_n(tv2, GL, gbase_lane);
-            if (writer) { UNROLL for (int qq = 0; qq < NC; ++qq) UNROLL for (int a = 0; a < 2; ++a) tred[qq * 5 + 3 + a] = tv2[qq * 2 + a]; }
-        }
+        else reduce(tv2, std::integral_constant<int, 3>{});
     }
     if constexpr (!DEFER) __syncwarp();
 }
@@ -1411,6 +1463,8 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
         // weighted layouts carry the boundary trace from step to step; in the other layouts' backward loops, several of which
         // spill, the carried sums would be more live registers
         constexpr bool CARRY = LaneWeighted<LaneT>::value;
+        // the same layouts reduce-scatter the traces when the group size is known at compile time
+        constexpr int RSG = CARRY && GLT > 0 ? GLT : 0;
         double tcar[NC], tcar2[OBJ ? NC : 1];
         if constexpr (CARRY) {
             trace_hs(L, vr, li, tcar);
@@ -1455,10 +1509,10 @@ __global__ void __launch_bounds__((PIPE_ == 1 ? 3 * NW + 1 : PIPE_ == 2 ? 2 * NW
                 }
                 UNROLL for (int e = 0; e < E; ++e) vr0[e] = vr[e];
                 state_step<JT>(L, J, dt, vr, vi, vi05);
-                adjoint_step<JT, true>(L, J, dt, lr, li, vr0, vi05, vr, tred, GL, gbase_lane, lane_on && g.lg == 0, nullptr, CARRY ? tcar : nullptr);   // traces -> tred
+                adjoint_step<JT, true, LaneT, false, RSG>(L, J, dt, lr, li, vr0, vi05, vr, tred, GL, gbase_lane, RSG > 0 ? lane_on : lane_on && g.lg == 0, nullptr, CARRY ? tcar : nullptr);   // traces -> tred
                 grad_scatter<NC, UPL>(U, gsm, tred, tabb, tabph, tabk, ls, Nfreq);
                 if constexpr (OBJ != 0) {
-                    adjoint_step<JT, false>(L, J, dt, lrn, lin, vr0, vi05, vr, tred, GL, gbase_lane, lane_on && g.lg == 0, nullptr, CARRY ? tcar2 : nullptr);
+                    adjoint_step<JT, false, LaneT, false, RSG>(L, J, dt, lrn, lin, vr0, vi05, vr, tred, GL, gbase_lane, RSG > 0 ? lane_on : lane_on && g.lg == 0, nullptr, CARRY ? tcar2 : nullptr);
                     grad_scatter<NC, UPL>(U2, gsm2, tred, tabb, tabph, tabk, ls, Nfreq);
                     if constexpr (HIST) {                    // after this step's traces; the carried trace is tr(vr, Hs, lin) of the jumped lin
                         if (jump(lrn, lin, (int)(k1 - 1 - s0) - ls)) { if constexpr (CARRY) trace_hs(L, vr, lin, tcar2); }
